@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark of the B200 DEFLATE engine (BASELINE.json metric / configs[1]).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--configs all|none|c1,c3,...]
+                    [--dump-outputs DIR]
 
 A "step" is one chunk-parallel raw deflate (DYNAMIC blocks, 64 KiB chunks, reference-compatible bytes)
 of one 256 MiB `mixed(268435456, seed)` buffer per GPU (SURVEY.md section 8(d), config C2). The same JSON line also
@@ -25,6 +26,7 @@ import subprocess
 import sys
 import tempfile
 import time
+import zlib
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
@@ -51,7 +53,14 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--configs", default="all", help="BASELINE configs to add to the line: all | none | c1,c3,c4,c5")
     ap.add_argument("--no-extras", action="store_true", help="skip the fast / primed / pageable / adversarial legs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/*.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs; the reference arm keeps none")
+    return args
 
 
 def peaks():
@@ -233,6 +242,34 @@ def adversarial_inputs(n):
             "records8": r.reshape(-1)}
 
 
+DUMP_SAMPLE = 1 << 22   # stream positions --dump-outputs keeps: 16 MiB of float32 bytes + 32 MiB of float64 indices
+
+
+def dump_outputs(out_dir, stream, results, rank=0, world=1):
+    """--dump-outputs: what the timed deflate call hands its caller, as .npy files under `out_dir`, so that two builds
+    can be compared output for output (the inputs are seeded):
+      deflate_<field>.npy       every field of the per-item result record (status, crc32, ..., out_len), float64
+      deflate_stream.npy        bytes of the compressed stream (uint8 host array `stream`), float32, at the positions
+      deflate_stream_index.npy  listed here (float64): every position of a stream of at most DUMP_SAMPLE bytes, else
+                                one drawn with a fixed seed from each of DUMP_SAMPLE equal slices of the stream
+      deflate_stream_crc32.npy  CRC-32 of the whole stream (float64): covers what the sample skips
+    Under --gpus N every rank writes its own files (suffix _rank<r>), sampling DUMP_SAMPLE / N positions: 48 MiB at
+    most in all."""
+    os.makedirs(out_dir, exist_ok=True)
+    sfx = "" if world == 1 else "_rank%d" % rank
+    k = DUMP_SAMPLE // world
+    if stream.size <= k:
+        idx = np.arange(stream.size)
+    else:
+        edges = np.arange(k + 1, dtype=np.int64) * stream.size // k
+        idx = edges[:-1] + (np.random.default_rng(0).random(k) * np.diff(edges)).astype(np.int64)
+    arrays = {"stream": stream[idx].astype(np.float32), "stream_index": idx.astype(np.float64),
+              "stream_crc32": np.array([zlib.crc32(stream)], dtype=np.float64)}
+    arrays.update((f, results[f].astype(np.float64)) for f in results.dtype.names)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, "deflate_%s%s.npy" % (name, sfx)), a)
+
+
 def run_b200(args, rank, world, local_rank):
     import torch
     import zlibts_b200 as z
@@ -314,6 +351,8 @@ def run_b200(args, rank, world, local_rank):
     assert int(r["status"][0]) == 0, r
     clen = int(r["out_len"][0])
     value = world * n * args.steps / (ms * 1e-3) / 1e9
+    if args.dump_outputs:   # before the legs below reuse d_out
+        dump_outputs(args.dump_outputs, d_out[:clen].cpu().numpy(), r, rank, world)
 
     extras = not args.no_extras
     few = max(1, min(args.steps, 5))
