@@ -81,8 +81,8 @@ enum { ZLB_MODE_COMPAT = 0, ZLB_MODE_FAST = 1, ZLB_MODE_PRIMED = 2, ZLB_MODE_SMA
  * and chunk share the 64 KiB a CTA indexes, so chunks are at most ZLB_PRIMED_CHUNK bytes (chunk_bytes 0 = that; pass
  * the same value to zlb_deflate_bound). Blocks are still one per chunk with their own codes, joined by the
  * byte-aligning empty stored block, so the item remains one RFC-1951 stream for the reference's RawInflate; what is
- * given up is per-chunk byte identity with RawDeflate(chunk) and chunk-parallel decoding (ZLB_INFLATE_SPLIT detects
- * the back references and takes the one-warp route). Without FAST the search is the reference's exhaustive one, and
+ * given up is per-chunk byte identity with RawDeflate(chunk). ZLB_INFLATE_SPLIT still decodes the chunks side by side
+ * (its window mode resolves the back references across the markers). Without FAST the search is the reference's exhaustive one, and
  * every block equals the reference's block construction run with that history (oracle: zo_raw_deflate_dict). */
 /* SMALLEST (SURVEY 8(f)-4; a flag for block_type DYNAMIC, may be or-ed with the others): each chunk is written as the
  * shortest of the reference's three block constructions over the chunk's tokens -- dynamic, fixed, or stored
@@ -108,9 +108,11 @@ enum {
     ZLB_INFLATE_CHECK_NLEN = 1u << 2,   /* verify NLEN == ~LEN in stored blocks (the reference
                                            never does: src/RawInflate.ts:277 is always false) */
     ZLB_INFLATE_SPLIT = 1u << 3,        /* large items may be cut at sync-flush markers (empty stored blocks,
-                                           `00 00 FF FF`) and their pieces decoded side by side when the pieces
-                                           turn out to be independent (what zlb_deflate_batch emits); anything
-                                           else falls back to the one-warp decoder. Results are identical. */
+                                           `00 00 FF FF`) and their pieces decoded side by side: independent
+                                           pieces (what zlb_deflate_batch emits) directly, pieces that reach up to
+                                           32 KiB into the ones before (ZLB_MODE_PRIMED, zlib's Z_SYNC_FLUSH) in
+                                           window mode; anything else falls back to the one-warp decoder. Results
+                                           are identical. */
     ZLB_INFLATE_SEGMENT = 1u << 4       /* internal: an item may end at a block boundary without BFINAL */
 };
 

@@ -25,6 +25,10 @@ enum ZtsKernelSlot {
     ZK_GATHER,
     ZK_FRAME_BODY,
     ZK_FRAME_HEADER,
+    ZK_INFLATE_WINDOW,  // marker split, window mode (zts_inflate.cu)
+    ZK_WINDOW_RUN,
+    ZK_WINDOW_SCAN,
+    ZK_WINDOW_RESOLVE,
     ZK_COUNT
 };
 
@@ -33,7 +37,8 @@ static const char* const kZtsKernelNames[ZK_COUNT] = {
     "lz77_chunk_kernel",   "huffman_build_kernel",   "chunk_scan_kernel",
     "bitpack_kernel",      "stored_block_kernel",    "deflate_finalize_kernel",
     "marker_scan_kernel",  "segment_gather_kernel",
-    "frame_body_kernel",   "frame_header_kernel"};
+    "frame_body_kernel",   "frame_header_kernel",
+    "inflate_warp_kernel_window", "window_run_kernel", "window_scan_kernel", "window_resolve_kernel"};
 
 struct ZtsDevBuf {
     void* p = nullptr;
@@ -55,7 +60,7 @@ struct zlb_ctx {
 
     // device arenas (grow-only, freed in zlb_destroy)
     ZtsDevBuf d_items, d_results, d_chunks, d_chunk_info, d_tokens, d_spec, d_hist, d_codes, d_sortT,
-        d_sums, d_misc, d_stage_in, d_stage_out, d_split, d_body, d_frames;
+        d_sums, d_misc, d_stage_in, d_stage_out, d_split, d_window, d_body, d_frames;
     // pinned host staging for the small tables
     void* h_pin = nullptr;
     size_t h_pin_cap = 0;

@@ -223,7 +223,7 @@ void zlb_destroy(zlb_ctx* ctx)
         if (ctx->s_aux[i]) cudaStreamSynchronize(ctx->s_aux[i]);
     ZtsDevBuf* bufs[] = {&ctx->d_items, &ctx->d_results, &ctx->d_chunks, &ctx->d_chunk_info, &ctx->d_tokens,
                          &ctx->d_spec,  &ctx->d_hist,    &ctx->d_codes,  &ctx->d_sortT,      &ctx->d_sums,
-                         &ctx->d_misc,  &ctx->d_stage_in, &ctx->d_stage_out, &ctx->d_split,
+                         &ctx->d_misc,  &ctx->d_stage_in, &ctx->d_stage_out, &ctx->d_split, &ctx->d_window,
                          &ctx->d_body,  &ctx->d_frames};
     for (ZtsDevBuf* b : bufs)
         if (b->p) cudaFree(b->p);

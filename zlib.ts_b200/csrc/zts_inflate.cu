@@ -28,6 +28,7 @@
 #include <algorithm>
 #include <cstddef>
 #include <chrono>
+#include <type_traits>
 
 #include "zts_common.cuh"
 
@@ -331,10 +332,17 @@ __device__ uint32_t inf_classify_symbols(const InfWarpSmem* S, const uint8_t* sr
     return ZLB_ST_INPUT_BROKEN;
 }
 
+// WINDOW = false: the decoder. WINDOW = true: the window mode of the marker split (see there): the output is one 16-bit
+// word per byte, out_off / out_cap count bytes / words, and the 32768 words in front of out_off belong to the item as
+// well -- the kernel fills them with 0x8000 | w, "byte w of the window" (the 32 KiB of output in front of the piece),
+// so that the copy code below is the same for both: a match that reaches before the piece copies window words.
+#define WIN_WORDS 32768u
+template <bool WINDOW>
 __global__ void __launch_bounds__(INF_WARPS_PER_CTA * 32, INF_MIN_CTAS)
 inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, const zlb_item* __restrict__ items,
                     zlb_result* __restrict__ results, uint32_t n_items, uint32_t flags)
 {
+    using T = typename std::conditional<WINDOW, uint16_t, uint8_t>::type;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const unsigned lane = zts_lane();
     const unsigned warp = threadIdx.x >> 5;
@@ -344,7 +352,15 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
 
     const zlb_item it = items[item];
     const uint8_t* src = in + it.in_off;
-    uint8_t* dst = out + it.out_off;
+    T* dst = reinterpret_cast<T*>(out + it.out_off);
+    if constexpr (WINDOW) {
+        uint4* w = reinterpret_cast<uint4*>(dst - WIN_WORDS);  // (slots are 256-byte aligned)
+        for (uint32_t i = lane; i < WIN_WORDS / 8; i += 32) {
+            const uint32_t a = 0x80008000u | (8u * i) | ((8u * i + 1u) << 16);
+            w[i] = make_uint4(a, a + 0x00020002u, a + 0x00040004u, a + 0x00060006u);
+        }
+        __syncwarp();
+    }
     const unsigned long long in_bits = it.in_len * 8ull;
     const unsigned long long cap = it.out_cap;
 
@@ -621,12 +637,12 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
             // `rel` = where this token's bytes start; the output written so far and the room left are clamped to
             // values that decide the same (a distance is at most 32768, a batch at most 8256 bytes).
             const uint32_t rel = inc - len;
-            uint8_t* const bdst = dst + op;  // first byte of the batch
+            T* const bdst = dst + op;  // first byte of the batch
             const uint32_t behind = op > 0x00FFFFFFull ? 0x00FFFFFFu : (uint32_t)op;         // bytes in front of the batch
             const uint32_t room = cap - op > 0x00FFFFFFull ? 0x00FFFFFFu : (uint32_t)(cap - op);  // (op <= cap always)
             // a distance beyond the start of the output (the reference would copy `undefined` -> 0) or an
             // output slot that is too small ends the batch before the offending token
-            const bool bad_dist = is_match && dist > behind + rel;
+            const bool bad_dist = is_match && dist > behind + rel + (WINDOW ? WIN_WORDS : 0u);
             const bool over = mine && rel + len > room;
             const unsigned bad_mask = __ballot_sync(0xFFFFFFFFu, bad_dist || over);
             uint32_t nvalid = ntok;
@@ -637,7 +653,7 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
             }
             const bool live = lane < nvalid;
             // -- literals: one store
-            ZTS_ASSERT(!live || (op + rel + len <= cap && (!is_match || dist <= op + rel)));
+            ZTS_ASSERT(!live || (op + rel + len <= cap && (!is_match || dist <= op + rel + (WINDOW ? WIN_WORDS : 0u))));
             if (live && !is_match) bdst[rel] = (uint8_t)(mytok >> 16);
             __syncwarp();  // (a match may read the literals of its own batch)
             // -- matches, sub-batch by sub-batch: a sub-batch ends in front of the first match that reads what a match
@@ -658,11 +674,11 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
                 const bool small = in_sub && len <= 8u && dist >= len;
                 if (__any_sync(0xFFFFFFFFu, small)) {
                     // short non-overlapping matches: every lane copies its own, loads first, then stores
-                    uint8_t v[8];
-                    uint8_t* dp = bdst + rel;
-                    const uint8_t* sp = dp - dist;
+                    T v[8];
+                    T* dp = bdst + rel;
+                    const T* sp = dp - dist;
 #pragma unroll
-                    for (int k = 0; k < 8; ++k) v[k] = (small && (uint32_t)k < len) ? sp[k] : (uint8_t)0;
+                    for (int k = 0; k < 8; ++k) v[k] = (small && (uint32_t)k < len) ? sp[k] : (T)0;
 #pragma unroll
                     for (int k = 0; k < 8; ++k)
                         if (small && (uint32_t)k < len) dp[k] = v[k];
@@ -674,8 +690,8 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
                     const uint32_t jl = __shfl_sync(0xFFFFFFFFu, len, j);
                     const uint32_t jd = __shfl_sync(0xFFFFFFFFu, dist, j);
                     const uint32_t jr = __shfl_sync(0xFFFFFFFFu, rel, j);
-                    uint8_t* o = bdst + jr;
-                    const uint8_t* s0 = o - jd;
+                    T* o = bdst + jr;
+                    const T* s0 = o - jd;
                     if (jd >= jl) {
                         for (uint32_t k = lane; k < jl; k += 32) o[k] = s0[k];
                     } else {
@@ -710,25 +726,27 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
     }
 }
 
+template <bool WINDOW = false>
 static int inflate_launch(zlb_ctx* ctx, cudaStream_t st, const uint8_t* d_in, uint8_t* d_out, const zlb_item* d_items,
                           zlb_result* d_results, size_t n, uint32_t flags)
 {
     const size_t smem = sizeof(InfWarpSmem) * INF_WARPS_PER_CTA;
-    ZTS_CUDA(ctx, cudaFuncSetAttribute(inflate_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    ZTS_CUDA(ctx, cudaFuncSetAttribute(inflate_warp_kernel<WINDOW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     unsigned grid = (unsigned)((n + INF_WARPS_PER_CTA - 1) / INF_WARPS_PER_CTA);
-    ZTS_LAUNCH(ctx, ZK_INFLATE,
-               inflate_warp_kernel<<<grid, INF_WARPS_PER_CTA * 32, smem, st>>>(d_in, d_out, d_items, d_results,
-                                                                              (uint32_t)n, flags));
+    ZTS_LAUNCH(ctx, WINDOW ? ZK_INFLATE_WINDOW : ZK_INFLATE,
+               inflate_warp_kernel<WINDOW><<<grid, INF_WARPS_PER_CTA * 32, smem, st>>>(d_in, d_out, d_items, d_results,
+                                                                                      (uint32_t)n, flags));
     return ZLB_OK;
 }
 
 // ---- marker split (ZLB_INFLATE_SPLIT) ------------------------------------------------------------------------
-// A stream written by zlb_deflate_batch is a sequence of independent pieces: every chunk was compressed on its own
-// (no match reaches into an earlier chunk) and ends with an empty stored block, `00 00 FF FF` after byte alignment.
-// One warp per piece decodes a 1 GiB stream in the time of a 64 KiB one. Nothing is assumed about the input: the
-// pieces are decoded into scratch slots in segment mode, and only if every piece (a) ends exactly where the next
-// one starts, (b) never reaches before its own first byte and (c) fits its slot is the result gathered; a false
-// marker or a foreign stream with history across blocks fails one of these and the item is decoded serially.
+// A stream written by zlb_deflate_batch is a sequence of pieces joined by empty stored blocks, `00 00 FF FF` after
+// byte alignment. One warp per piece decodes a 1 GiB stream in the time of a 64 KiB one. Nothing is assumed about the
+// input: the pieces are decoded into scratch slots in segment mode, and only if every piece (a) ends exactly where the
+// next one starts, (b) never reaches before its own first byte and (c) fits its slot is the result gathered. Items
+// that fail (b) alone -- primed streams, zlib's Z_SYNC_FLUSH, whose matches reach across the markers -- are decoded
+// once more in window mode (below); a false marker, a reference before the start of the stream or anything else that
+// fails a check sends the item to the one-warp decoder.
 #define SPLIT_MIN_BYTES (256u << 10)   // items at least this large are worth splitting
 #define SPLIT_SLOT (128u << 10)        // scratch bytes per piece (pieces of this engine's streams are <= 64 KiB)
 #define SPLIT_MAX_MARKS (1u << 22)
@@ -777,12 +795,332 @@ segment_gather_kernel(const uint8_t* __restrict__ scratch, uint8_t* __restrict__
     for (unsigned long long i = head + body + threadIdx.x; i < e.len; i += 256) d[i] = s[i];
 }
 
-static int inflate_launch(zlb_ctx* ctx, cudaStream_t st, const uint8_t* d_in, uint8_t* d_out, const zlb_item* d_items,
-                          zlb_result* d_results, size_t n, uint32_t flags);
+// ---- window mode: pieces that reach up to 32 KiB in front of their first byte -----------------------------------
+// Every piece of such an item is decoded again by inflate_warp_kernel<true>, into 16-bit words: a byte (< 0x100), or
+// 0x8000 | w, "byte w of the piece's window" (the 32768 output bytes in front of its first byte). The last 32768
+// words of window ++ piece are the piece's tail map T_j: W_{j+1} in terms of W_j (a piece shorter than a window
+// shifts the older part of W_j along, so a window may span many short pieces). Composition
+// (A;B)[i] = B[i] < 0x100 ? B[i] : A[B[i] & 0x7FFF] is associative, so W_j in terms of W_0 -- the window in front of
+// the stream, of which no byte exists -- is an exclusive scan of the tail maps over the pieces of the item, starting
+// from the identity. A byte of a piece that still names W_0 after that reaches before the start of the stream: the
+// item fails and goes to the one-warp decoder. The scan has a fixed depth and no CTA ever waits for another: a CTA
+// composes a run of about sqrt(n) consecutive pieces (window_run_kernel), one per item composes the runs
+// (window_scan_kernel), and a CTA per run applies its prefix piece by piece while it turns the words into bytes in
+// the pieces' byte slots (window_resolve_kernel), which are gathered like those of independent pieces.
+struct ZtsWinPiece {
+    unsigned long long words;  // byte offset in the window arena of the piece's first output word
+    unsigned long long bytes;  // byte offset in the split scratch of its resolved bytes
+    uint32_t len, cap;         // output words, slot words
+};
+struct ZtsWinRun {
+    uint32_t first, count;  // pieces [first, first + count)
+    uint32_t item;          // index of its item among those resolved
+    uint32_t pad;
+};
+struct ZtsWinItem {
+    uint32_t first_run, runs;
+};
+#define WIN_THREADS 1024
+#define WIN_SMEM (2u * WIN_WORDS * 2u)  // the map being composed and the next one
+
+__device__ __forceinline__ void win_identity(uint16_t* E)
+{
+    uint32_t* e = reinterpret_cast<uint32_t*>(E);
+    for (uint32_t i = threadIdx.x; i < WIN_WORDS / 2; i += WIN_THREADS) e[i] = 0x80008000u | (2u * i) | ((2u * i + 1u) << 16);
+    __syncthreads();
+}
+// 64 KiB, both sides 16-byte aligned
+__device__ __forceinline__ void win_copy(uint16_t* dst, const uint16_t* src)
+{
+    uint4* d = reinterpret_cast<uint4*>(dst);
+    const uint4* s = reinterpret_cast<const uint4*>(src);
+    for (uint32_t i = threadIdx.x; i < WIN_WORDS / 8; i += WIN_THREADS) d[i] = s[i];
+    __syncthreads();
+}
+// En = E;tail
+__device__ __forceinline__ void win_compose(const uint16_t* E, uint16_t* En, const uint16_t* __restrict__ tail)
+{
+    for (uint32_t i = threadIdx.x; i < WIN_WORDS; i += WIN_THREADS) {
+        const uint32_t t = tail[i];
+        En[i] = (t & 0x8000u) ? E[t & 0x7FFFu] : (uint16_t)t;
+    }
+    __syncthreads();
+}
+// T_j: the last 32768 words of window ++ piece
+__device__ __forceinline__ const uint16_t* win_tail(const uint8_t* arena, const ZtsWinPiece& p)
+{
+    ZTS_ASSERT(p.len <= p.cap && p.words >= 2ull * WIN_WORDS && p.words % 16 == 0);  // (the window words in front)
+    return reinterpret_cast<const uint16_t*>(arena + p.words) + ((long long)p.len - (long long)WIN_WORDS);
+}
+
+// aggregate of run r: W_{last + 1} in terms of W_first
+__global__ void __launch_bounds__(WIN_THREADS)
+window_run_kernel(const uint8_t* __restrict__ arena, const ZtsWinPiece* __restrict__ pieces,
+                  const ZtsWinRun* __restrict__ runs, uint16_t* __restrict__ agg)
+{
+    extern __shared__ __align__(16) uint16_t wmap[];
+    uint16_t *E = wmap, *En = wmap + WIN_WORDS;
+    const ZtsWinRun r = runs[blockIdx.x];
+    win_identity(E);
+    for (uint32_t j = r.first; j < r.first + r.count; ++j) {
+        win_compose(E, En, win_tail(arena, pieces[j]));
+        uint16_t* t = E;
+        E = En;
+        En = t;
+    }
+    win_copy(agg + (size_t)blockIdx.x * WIN_WORDS, E);
+}
+
+// prefix of every run of item i: the window in front of the run's first piece in terms of W_0
+__global__ void __launch_bounds__(WIN_THREADS)
+window_scan_kernel(const ZtsWinItem* __restrict__ items, const uint16_t* __restrict__ agg, uint16_t* __restrict__ prefix)
+{
+    extern __shared__ __align__(16) uint16_t wmap[];
+    uint16_t *E = wmap, *En = wmap + WIN_WORDS;
+    const ZtsWinItem it = items[blockIdx.x];
+    win_identity(E);
+    for (uint32_t r = it.first_run; r < it.first_run + it.runs; ++r) {
+        win_copy(prefix + (size_t)r * WIN_WORDS, E);
+        if (r + 1 < it.first_run + it.runs) {
+            win_compose(E, En, agg + (size_t)r * WIN_WORDS);
+            uint16_t* t = E;
+            E = En;
+            En = t;
+        }
+    }
+}
+
+__device__ __forceinline__ uint32_t win_resolve(const uint16_t* E, uint32_t w)
+{
+    return (w & 0x8000u) ? E[w & 0x7FFFu] : w;
+}
+
+// the bytes of every piece of run r; fail[item] = 1 when one of them lies before the start of the stream
+__global__ void __launch_bounds__(WIN_THREADS)
+window_resolve_kernel(const uint8_t* __restrict__ arena, uint8_t* __restrict__ scratch, const ZtsWinPiece* __restrict__ pieces,
+                      const ZtsWinRun* __restrict__ runs, const uint16_t* __restrict__ prefix, uint32_t* __restrict__ fail)
+{
+    extern __shared__ __align__(16) uint16_t wmap[];
+    uint16_t *E = wmap, *En = wmap + WIN_WORDS;
+    const ZtsWinRun r = runs[blockIdx.x];
+    win_copy(E, prefix + (size_t)blockIdx.x * WIN_WORDS);
+    uint32_t seen = 0;  // or of the resolved words: bit 15 = a byte before the stream
+    for (uint32_t j = r.first; j < r.first + r.count; ++j) {
+        const ZtsWinPiece p = pieces[j];
+        ZTS_ASSERT(p.len <= p.cap);
+        const uint16_t* w = reinterpret_cast<const uint16_t*>(arena + p.words);
+        uint8_t* o = scratch + p.bytes;
+        // four words at a time (both slots are 256-byte aligned)
+        const uint32_t n4 = p.len / 4u;
+        for (uint32_t q = threadIdx.x; q < n4; q += WIN_THREADS) {
+            const uint2 v = reinterpret_cast<const uint2*>(w)[q];
+            const uint32_t b0 = win_resolve(E, v.x & 0xFFFFu), b1 = win_resolve(E, v.x >> 16);
+            const uint32_t b2 = win_resolve(E, v.y & 0xFFFFu), b3 = win_resolve(E, v.y >> 16);
+            seen |= b0 | b1 | b2 | b3;
+            reinterpret_cast<uint32_t*>(o)[q] = (b0 & 0xFFu) | ((b1 & 0xFFu) << 8) | ((b2 & 0xFFu) << 16) | (b3 << 24);
+        }
+        for (uint32_t k = 4u * n4 + threadIdx.x; k < p.len; k += WIN_THREADS) {
+            const uint32_t b = win_resolve(E, w[k]);
+            seen |= b;
+            o[k] = (uint8_t)b;
+        }
+        if (j + 1 < r.first + r.count) {
+            win_compose(E, En, win_tail(arena, p));
+            uint16_t* t = E;
+            E = En;
+            En = t;
+        }
+    }
+    if (__syncthreads_or((int)(seen & 0x8000u)) && threadIdx.x == 0) fail[r.item] = 1u;
+}
+
+struct SplitPiece {
+    uint32_t item;  // index into big
+    unsigned long long start;
+};
+
+// The chain checks of the pieces r[0 .. n) of an item: each one decoded cleanly, ended exactly where the next one
+// starts, and only the last one saw BFINAL. With `window`, a piece behind the first that stopped at an undefined code
+// or distance may have reached before its first byte: SPLIT_WINDOW says window mode may still decode the item.
+enum { SPLIT_BAD = 0, SPLIT_OK = 1, SPLIT_WINDOW = 2 };
+static int split_chain(const zlb_result* r, const zlb_item* seg, size_t n, bool window)
+{
+    bool reaches = false;
+    for (size_t j = 0; j < n; ++j) {
+        const bool last = j + 1 == n;
+        const bool fin = (r[j].blocks & 0x80000000u) != 0;
+        if (window && j > 0 && r[j].status == ZLB_ST_BAD_CODE) {
+            reaches = true;
+            continue;
+        }
+        if (r[j].status != ZLB_ST_OK) return SPLIT_BAD;
+        if (last ? !fin : (fin || r[j].in_used != seg[j].in_len)) return SPLIT_BAD;
+    }
+    return reaches ? SPLIT_WINDOW : SPLIT_OK;
+}
+
+// result of an item whose n pieces passed the checks; their bytes (r[j].out_len at scratch offset seg[j].out_off)
+// are queued for the gather when they fit
+static void split_finish(const zlb_item& it, const zlb_result* r, const zlb_item* seg, size_t n, unsigned long long last_start,
+                         zlb_result& o, std::vector<ZtsGather>& gath)
+{
+    unsigned long long total = 0, blocks = 0;
+    for (size_t j = 0; j < n; ++j) {
+        total += r[j].out_len;
+        blocks += r[j].blocks & 0x7FFFFFFFu;
+    }
+    o.status = total > it.out_cap ? ZLB_ST_OUT_OVERFLOW : ZLB_ST_OK;
+    o.out_len = total > it.out_cap ? 0 : total;
+    o.in_used = last_start + r[n - 1].in_used;
+    o.blocks = (uint32_t)blocks;
+    if (total <= it.out_cap && total) {
+        unsigned long long at = 0;
+        for (size_t j = 0; j < n; ++j) {
+            if (r[j].out_len) gath.push_back({seg[j].out_off, it.out_off + at, r[j].out_len});
+            at += r[j].out_len;
+        }
+    }
+}
+
+// Window mode for the items big[cand[*]] (pieces as laid out by inflate_split_batch, byte slots at seg[j].out_off of
+// d_scratch): all of them in one decode launch and one scan; done[k] / res[k] / gath as there.
+static int inflate_split_window(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_scratch, const zlb_item* h_items,
+                                const std::vector<size_t>& big, uint32_t flags, const std::vector<SplitPiece>& pieces,
+                                const std::vector<size_t>& first, const std::vector<zlb_item>& seg,
+                                const std::vector<size_t>& cand, std::vector<zlb_result>& res, std::vector<char>& done,
+                                std::vector<ZtsGather>& gath)
+{
+    cudaStream_t st = ctx->stream;
+    // runs of about sqrt(n) pieces: the scan's depth is then about 3 sqrt(n) compositions
+    auto run_len = [](size_t n) {
+        size_t g = 8;
+        while (g * g < n) ++g;
+        return g;
+    };
+    const size_t map_b = (size_t)WIN_WORDS * 2;
+    // arena: word slots (each behind its window) | aggregates | prefixes | items | results | pieces | runs | items | fail
+    auto layout = [&](size_t words, size_t np, size_t nr, size_t ni, size_t* off) {
+        off[0] = words;
+        off[1] = off[0] + nr * map_b;
+        off[2] = off[1] + nr * map_b;
+        off[3] = off[2] + np * sizeof(zlb_item);
+        off[4] = off[3] + np * sizeof(zlb_result);
+        off[5] = off[4] + np * sizeof(ZtsWinPiece);
+        off[6] = off[5] + nr * sizeof(ZtsWinRun);
+        off[7] = off[6] + ni * sizeof(ZtsWinItem);
+        return off[7] + ni * 4 + 256;
+    };
+    // The scratch is bounded like the byte slots' (a quarter of what the device has free, 16 GiB), and by what the
+    // input could legitimately need: three times the byte slots' bound (two bytes per word, the windows, the maps).
+    // Items that do not fit go to the one-warp decoder.
+    size_t free_b = 0, total_b = 0;
+    if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) free_b = 0;
+    size_t budget = (free_b + ctx->d_window.cap) / 4;
+    if (budget > ((size_t)16 << 30)) budget = (size_t)16 << 30;
+    std::vector<size_t> take;
+    size_t words = 0, np = 0, nr = 0, in_b = 0, need = 0, off[8];
+    for (size_t k : cand) {
+        const size_t a = first[k], b = first[k + 1], n = b - a;
+        size_t w = 0;
+        for (size_t j = a; j < b; ++j) w += map_b + 2 * (size_t)seg[j].out_cap;  // (out_cap: a multiple of 256)
+        const size_t g = run_len(n);
+        const size_t need_k = layout(words + w, np + n, nr + (n + g - 1) / g, take.size() + 1, off);
+        size_t by_input = (in_b + h_items[big[k]].in_len) * 2048u;
+        if (by_input < ((size_t)64 << 20)) by_input = (size_t)64 << 20;
+        if (need_k > budget || need_k > 3 * by_input) continue;
+        take.push_back(k);
+        words += w;
+        np += n;
+        nr += (n + g - 1) / g;
+        in_b += h_items[big[k]].in_len;
+        need = need_k;
+    }
+    if (take.empty()) return ZLB_OK;
+    int rc = zts_reserve(ctx, &ctx->d_window, need);
+    if (rc == ZLB_E_NOMEM) {
+        ctx->err[0] = 0;
+        return ZLB_OK;
+    }
+    if (rc) return rc;
+    layout(words, np, nr, take.size(), off);
+    uint8_t* arena = (uint8_t*)ctx->d_window.p;
+    uint16_t* d_agg = (uint16_t*)(arena + off[0]);
+    uint16_t* d_prefix = (uint16_t*)(arena + off[1]);
+    zlb_item* d_wseg = (zlb_item*)(arena + off[2]);
+    zlb_result* d_wres = (zlb_result*)(arena + off[3]);
+    ZtsWinPiece* d_pieces = (ZtsWinPiece*)(arena + off[4]);
+    ZtsWinRun* d_runs = (ZtsWinRun*)(arena + off[5]);
+    ZtsWinItem* d_witems = (ZtsWinItem*)(arena + off[6]);
+    uint32_t* d_fail = (uint32_t*)(arena + off[7]);
+    // 1. every piece of those items in window mode, one launch
+    std::vector<zlb_item> wseg;
+    wseg.reserve(np);
+    size_t at = 0;
+    for (size_t k : take)
+        for (size_t j = first[k]; j < first[k + 1]; ++j) {
+            zlb_item w = seg[j];
+            w.out_off = at + map_b;  // the window's words in front
+            at += map_b + 2 * (size_t)seg[j].out_cap;
+            wseg.push_back(w);
+        }
+    ZTS_CUDA(ctx, cudaMemcpyAsync(d_wseg, wseg.data(), np * sizeof(zlb_item), cudaMemcpyHostToDevice, st));
+    ZTS_CUDA(ctx, cudaMemsetAsync(d_wres, 0, np * sizeof(zlb_result), st));
+    rc = inflate_launch<true>(ctx, st, d_in, arena, d_wseg, d_wres, np, (flags & ZLB_INFLATE_CHECK_NLEN) | ZLB_INFLATE_SEGMENT);
+    if (rc) return rc;
+    std::vector<zlb_result> wres(np);
+    ZTS_CUDA(ctx, cudaMemcpyAsync(wres.data(), d_wres, np * sizeof(zlb_result), cudaMemcpyDeviceToHost, st));
+    ZTS_CUDA(ctx, cudaStreamSynchronize(st));
+    // 2. the chain checks; the items that pass are resolved
+    std::vector<ZtsWinPiece> wp;
+    std::vector<ZtsWinRun> runs;
+    std::vector<ZtsWinItem> witems;
+    std::vector<size_t> wk, wfirst;  // per resolved item: its k, its first piece in wseg / wres
+    for (size_t t = 0, wj = 0; t < take.size(); ++t) {
+        const size_t k = take[t], a = first[k], n = first[k + 1] - a;
+        const size_t w0 = wj;
+        wj += n;
+        if (split_chain(&wres[w0], &seg[a], n, false) != SPLIT_OK) continue;
+        const size_t g = run_len(n);
+        witems.push_back({(uint32_t)runs.size(), (uint32_t)((n + g - 1) / g)});
+        for (size_t s = 0; s < n; s += g)
+            runs.push_back({(uint32_t)(wp.size() + s), (uint32_t)std::min(g, n - s), (uint32_t)wk.size(), 0u});
+        for (size_t j = 0; j < n; ++j)
+            wp.push_back({wseg[w0 + j].out_off, seg[a + j].out_off, (uint32_t)wres[w0 + j].out_len, (uint32_t)seg[a + j].out_cap});
+        wk.push_back(k);
+        wfirst.push_back(w0);
+    }
+    if (wk.empty()) return ZLB_OK;
+    // 3. tail maps, scan, resolve
+    ZTS_CUDA(ctx, cudaMemcpyAsync(d_pieces, wp.data(), wp.size() * sizeof(ZtsWinPiece), cudaMemcpyHostToDevice, st));
+    ZTS_CUDA(ctx, cudaMemcpyAsync(d_runs, runs.data(), runs.size() * sizeof(ZtsWinRun), cudaMemcpyHostToDevice, st));
+    ZTS_CUDA(ctx, cudaMemcpyAsync(d_witems, witems.data(), witems.size() * sizeof(ZtsWinItem), cudaMemcpyHostToDevice, st));
+    ZTS_CUDA(ctx, cudaMemsetAsync(d_fail, 0, wk.size() * 4, st));
+    ZTS_CUDA(ctx, cudaFuncSetAttribute(window_run_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WIN_SMEM));
+    ZTS_CUDA(ctx, cudaFuncSetAttribute(window_scan_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WIN_SMEM));
+    ZTS_CUDA(ctx, cudaFuncSetAttribute(window_resolve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WIN_SMEM));
+    ZTS_LAUNCH(ctx, ZK_WINDOW_RUN,
+               window_run_kernel<<<(unsigned)runs.size(), WIN_THREADS, WIN_SMEM, st>>>(arena, d_pieces, d_runs, d_agg));
+    ZTS_LAUNCH(ctx, ZK_WINDOW_SCAN,
+               window_scan_kernel<<<(unsigned)witems.size(), WIN_THREADS, WIN_SMEM, st>>>(d_witems, d_agg, d_prefix));
+    ZTS_LAUNCH(ctx, ZK_WINDOW_RESOLVE,
+               window_resolve_kernel<<<(unsigned)runs.size(), WIN_THREADS, WIN_SMEM, st>>>(arena, d_scratch, d_pieces, d_runs,
+                                                                                            d_prefix, d_fail));
+    std::vector<uint32_t> fail(wk.size());
+    ZTS_CUDA(ctx, cudaMemcpyAsync(fail.data(), d_fail, wk.size() * 4, cudaMemcpyDeviceToHost, st));
+    ZTS_CUDA(ctx, cudaStreamSynchronize(st));
+    for (size_t i = 0; i < wk.size(); ++i) {
+        if (fail[i]) continue;  // a byte before the start of the stream
+        const size_t k = wk[i], a = first[k], n = first[k + 1] - a;
+        split_finish(h_items[big[k]], &wres[wfirst[i]], &seg[a], n, pieces[a + n - 1].start, res[k], gath);
+        done[k] = 1;
+    }
+    return ZLB_OK;
+}
 
 // Tries to decode the items h_items[big[*]] piecewise, all of them in one pass: one marker scan per item (queued back
-// to back, one read-back for all), one segment-mode launch over the pieces of every item, one gather. done[k] tells
-// whether big[k] worked (then res[k] is filled); the others have to go through the serial decoder. < 0 on API errors.
+// to back, one read-back for all), one segment-mode launch over the pieces of every item, one window-mode pass for
+// the items whose pieces reach into their predecessors, one gather. done[k] tells whether big[k] worked (then res[k]
+// is filled); the others have to go through the serial decoder. < 0 on API errors.
 #define SPLIT_TAG_SHIFT 40  // marks carry the item's index above the byte offset (offsets < 1 TiB, < 16 M large items)
 static int inflate_split_batch(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const zlb_item* h_items,
                                const std::vector<size_t>& big, uint32_t flags, std::vector<zlb_result>& res,
@@ -816,11 +1154,7 @@ static int inflate_split_batch(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out
     ZTS_CUDA(ctx, cudaStreamSynchronize(st));
     std::sort(marks.begin(), marks.end());  // by item, then by offset
     // pieces of every item: it starts at 0 and behind every marker that leaves at least one byte
-    struct Piece {
-        uint32_t item;  // index into big
-        unsigned long long start;
-    };
-    std::vector<Piece> pieces;
+    std::vector<SplitPiece> pieces;
     std::vector<size_t> first(nb + 1, 0);  // pieces of item k: [first[k], first[k + 1])
     {
         size_t mi = 0;
@@ -890,38 +1224,22 @@ static int inflate_split_batch(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out
     std::vector<zlb_result> sres(np);
     ZTS_CUDA(ctx, cudaMemcpyAsync(sres.data(), d_segres, np * sizeof(zlb_result), cudaMemcpyDeviceToHost, st));
     ZTS_CUDA(ctx, cudaStreamSynchronize(st));
-    // validate every item's chain of pieces; the valid ones are gathered in one launch
+    // validate every item's chain of pieces; the valid ones are gathered in one launch, together with those that
+    // window mode decodes
     std::vector<ZtsGather> gath;
+    std::vector<size_t> window;
     for (size_t k = 0; k < nb; ++k) {
-        const zlb_item& it = h_items[big[k]];
         const size_t a = first[k], b = first[k + 1];
         if (b - a < 2) continue;
-        unsigned long long total = 0, blocks = 0;
-        bool ok = true;
-        for (size_t j = a; j < b && ok; ++j) {
-            const zlb_result& r = sres[j];
-            const bool last = j + 1 == b;
-            const bool fin = (r.blocks & 0x80000000u) != 0;
-            if (r.status != ZLB_ST_OK) ok = false;                 // incl. a distance before the piece's first byte
-            else if (!last && (fin || r.in_used != seg[j].in_len)) ok = false;
-            else if (last && !fin) ok = false;
-            total += r.out_len;
-            blocks += r.blocks & 0x7FFFFFFFu;
-        }
-        if (!ok) continue;
-        zlb_result& o = res[k];
-        o.status = total > it.out_cap ? ZLB_ST_OUT_OVERFLOW : ZLB_ST_OK;
-        o.out_len = total > it.out_cap ? 0 : total;
-        o.in_used = pieces[b - 1].start + sres[b - 1].in_used;
-        o.blocks = (uint32_t)blocks;
+        const int chain = split_chain(&sres[a], &seg[a], b - a, true);
+        if (chain == SPLIT_WINDOW) window.push_back(k);
+        if (chain != SPLIT_OK) continue;
+        split_finish(h_items[big[k]], &sres[a], &seg[a], b - a, pieces[b - 1].start, res[k], gath);
         done[k] = 1;
-        if (total <= it.out_cap && total) {
-            unsigned long long at = 0;
-            for (size_t j = a; j < b; ++j) {
-                if (sres[j].out_len) gath.push_back({seg[j].out_off, it.out_off + at, sres[j].out_len});
-                at += sres[j].out_len;
-            }
-        }
+    }
+    if (!window.empty()) {
+        rc = inflate_split_window(ctx, d_in, d_scratch, h_items, big, flags, pieces, first, seg, window, res, done, gath);
+        if (rc) return rc;
     }
     if (!gath.empty()) {
         ZTS_CUDA(ctx, cudaMemcpyAsync(d_gather, gath.data(), gath.size() * sizeof(ZtsGather), cudaMemcpyHostToDevice, st));  // <= np entries
