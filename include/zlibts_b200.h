@@ -13,6 +13,8 @@
  *                                                         src/Zip.ts:93,144    src/Unzip.ts:294
  *   Adler-32     Adler32.create / update                  src/Deflate.ts:81    src/Inflate.ts:84
  *                                                                                  -> zlb_checksum_batch[_host]
+ *   preset dictionaries (zlib's deflateSetDictionary / inflateSetDictionary; the reference's Inflate refuses FDICT,
+ *   src/Inflate.ts:56-57)                                 -> zlb_deflate_batch_dict[_host], zlb_inflate_batch_dict[_host]
  *
  * Conventions
  *   - plain pointers and sizes only; no exceptions cross the ABI.
@@ -172,6 +174,33 @@ int zlb_deflate_batch_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes, void
 /* output bytes that always suffice for an item of in_len bytes */
 uint64_t zlb_deflate_bound(uint64_t in_len, uint32_t chunk_bytes, int block_type);
 
+/* ---- preset dictionaries (zlib's deflateSetDictionary / inflateSetDictionary, RFC 1950 FDICT) ----------------
+ * An engine extension: the reference's Inflate refuses FDICT streams (src/Inflate.ts:56-57). dicts[i] names item i's
+ * dictionary as a span of one dictionary blob (d_dict: device pointer; h_dict: host pointer); a shared dictionary is
+ * every entry naming the same span. dicts == NULL, or len == 0, means no dictionary; zlb_deflate_batch[_host] and
+ * zlb_inflate_batch[_host] are these calls with dicts == NULL. Only the last 32768 bytes of a dictionary can be
+ * reached (the DEFLATE window). Results keep their meaning: CRC-32 / Adler-32 cover the item's own bytes.
+ * ZLB_E_ARG: a span outside dict_bytes (host entry points), or len > 0 with a NULL blob.                        */
+typedef struct {
+    uint64_t off;   /* first byte of this item's dictionary in the dictionary blob                    */
+    uint64_t len;   /* 0 = no dictionary; only the last 32768 bytes are used (the DEFLATE window)      */
+} zlb_dict;
+
+/* Deflate with a dictionary: a chunk's match search also reaches into the last min(32768, ...) bytes of
+ * dictionary || the item's bytes in front of the chunk. Without ZLB_MODE_PRIMED only an item's first chunk has the
+ * dictionary as history (later chunks stay independent); with it every chunk searches its 32 KiB of dictionary || item.
+ * When any item of the call has a dictionary, chunks are at most ZLB_PRIMED_CHUNK bytes (history and chunk share
+ * the 64 KiB a CTA indexes; size slots with zlb_deflate_bound(in_len, ZLB_PRIMED_CHUNK, ...)). In the compat mode the
+ * first chunk's block is the reference's block construction run with that history; block_type ZLB_NONE ignores the
+ * dictionary.                                                                                                    */
+int zlb_deflate_batch_dict(zlb_ctx* ctx, const void* d_in, void* d_out, const void* d_dict, const zlb_dict* dicts,
+                           const zlb_item* items, zlb_result* results, size_t n_items, int mode, int block_type,
+                           uint32_t chunk_bytes, uint32_t flags);
+int zlb_deflate_batch_dict_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes, void* h_out, size_t out_bytes,
+                                const void* h_dict, size_t dict_bytes, const zlb_dict* dicts, const zlb_item* items,
+                                zlb_result* results, size_t n_items, int mode, int block_type, uint32_t chunk_bytes,
+                                uint32_t flags);
+
 /* ---- raw inflate (replaces RawInflate.decompress, src/RawInflate.ts:127-140) ----------------
  * One warp per item. in_off points at the first deflate byte (the caller has applied the
  * reference's `index` option); trailing container bytes may follow the stream.               */
@@ -179,6 +208,14 @@ int zlb_inflate_batch(zlb_ctx* ctx, const void* d_in, void* d_out, const zlb_ite
                       zlb_result* results, size_t n_items, uint32_t flags);
 int zlb_inflate_batch_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes, void* h_out, size_t out_bytes,
                            const zlb_item* items, zlb_result* results, size_t n_items, uint32_t flags);
+/* Inflate with a dictionary (zlb_dict above): a distance may reach up to the dictionary's first usable byte in
+ * front of the output; one beyond it is ZLB_ST_BAD_CODE as before. ZLB_INFLATE_SPLIT takes the same routes, the
+ * window in front of an item's first piece being the dictionary.                                                */
+int zlb_inflate_batch_dict(zlb_ctx* ctx, const void* d_in, void* d_out, const void* d_dict, const zlb_dict* dicts,
+                           const zlb_item* items, zlb_result* results, size_t n_items, uint32_t flags);
+int zlb_inflate_batch_dict_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes, void* h_out, size_t out_bytes,
+                                const void* h_dict, size_t dict_bytes, const zlb_dict* dicts, const zlb_item* items,
+                                zlb_result* results, size_t n_items, uint32_t flags);
 
 /* ---- checksums (replace CRC32.create src/CRC32.ts:13, Adler32.create src/Adler32.ts:13) ----- */
 int zlb_checksum_batch(zlb_ctx* ctx, const void* d_in, const zlb_item* items, zlb_result* results,

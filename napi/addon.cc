@@ -153,11 +153,30 @@ static std::vector<double> get_numbers(napi_env env, napi_value arr)
     return v;
 }
 
-// deflateBatch(inputs, compressionType, chunkBytes, flags, mode = 0)  <- new RawDeflate(input, opts).compress()
+// an optional preset dictionary argument (Uint8Array, shared by every item; undefined / empty = none): the zlb_dict
+// table of n items that all name it
+static bool get_dict(napi_env env, size_t argc, napi_value* argv, size_t k, size_t n, Bytes* dict,
+                     std::vector<zlb_dict>* dicts)
+{
+    dict->p = nullptr;
+    dict->n = 0;
+    if (argc <= k) return true;
+    napi_valuetype t;
+    napi_typeof(env, argv[k], &t);
+    if (t == napi_undefined || t == napi_null) return true;
+    if (!get_u8(env, argv[k], dict)) {
+        napi_throw_type_error(env, nullptr, "dictionary must be Uint8Array");
+        return false;
+    }
+    if (dict->n) dicts->assign(n, zlb_dict{0, (uint64_t)dict->n});
+    return true;
+}
+
+// deflateBatch(inputs, compressionType, chunkBytes, flags, mode = 0, dictionary?)  <- new RawDeflate(input, opts).compress()
 static napi_value DeflateBatch(napi_env env, napi_callback_info info)
 {
-    size_t argc = 5;
-    napi_value argv[5];
+    size_t argc = 6;
+    napi_value argv[6];
     napi_get_cb_info(env, info, &argc, argv, nullptr, nullptr);
     if (!ensure_ctx(env)) return nullptr;
     uint32_t n = 0, ctype = 2, chunk = 0, flags = 0, mode = ZLB_MODE_COMPAT;
@@ -166,7 +185,11 @@ static napi_value DeflateBatch(napi_env env, napi_callback_info info)
     napi_get_value_uint32(env, argv[2], &chunk);
     napi_get_value_uint32(env, argv[3], &flags);
     if (argc > 4) napi_get_value_uint32(env, argv[4], &mode);   // ZLB_MODE_FAST | ZLB_MODE_PRIMED | ZLB_MODE_SMALLEST
-    if ((mode & ZLB_MODE_PRIMED) && (chunk == 0 || chunk > ZLB_PRIMED_CHUNK)) chunk = ZLB_PRIMED_CHUNK;
+    Bytes dict;
+    std::vector<zlb_dict> dicts;
+    if (!get_dict(env, argc, argv, 5, n, &dict, &dicts)) return nullptr;
+    // primed mode and dictionaries: chunks of at most 32 KiB (the slots are sized with the chunk size used)
+    if ((mode & ZLB_MODE_PRIMED || !dicts.empty()) && (chunk == 0 || chunk > ZLB_PRIMED_CHUNK)) chunk = ZLB_PRIMED_CHUNK;
     std::vector<zlb_item> items(n);
     std::vector<zlb_result> res(n);
     std::vector<Bytes> in(n);
@@ -195,8 +218,9 @@ static napi_value DeflateBatch(napi_env env, napi_callback_info info)
     if (!direct)
         for (uint32_t i = 0; i < n; ++i)
             if (in[i].n) memcpy(blob.p + items[i].in_off, in[i].p, in[i].n);
-    int rc = zlb_deflate_batch_host(g_ctx, direct ? in[0].p : blob.p, in_total, out.p, out_total, items.data(), res.data(), n,
-                                    (int)mode, (int)ctype, chunk, flags);
+    int rc = zlb_deflate_batch_dict_host(g_ctx, direct ? in[0].p : blob.p, in_total, out.p, out_total, dict.p, dict.n,
+                                         dicts.empty() ? nullptr : dicts.data(), items.data(), res.data(), n, (int)mode,
+                                         (int)ctype, chunk, flags);
     if (rc != ZLB_OK) {
         napi_throw_error(env, nullptr, zlb_last_error(g_ctx));
         return nullptr;
@@ -218,11 +242,11 @@ static napi_value DeflateBatch(napi_env env, napi_callback_info info)
     return result;
 }
 
-// inflateBatch(input, offsets, lengths, caps, flags)  <- new RawInflate(input, {index}).decompress()
+// inflateBatch(input, offsets, lengths, caps, flags, dictionary?)  <- new RawInflate(input, {index}).decompress()
 static napi_value InflateBatch(napi_env env, napi_callback_info info)
 {
-    size_t argc = 5;
-    napi_value argv[5];
+    size_t argc = 6;
+    napi_value argv[6];
     napi_get_cb_info(env, info, &argc, argv, nullptr, nullptr);
     if (!ensure_ctx(env)) return nullptr;
     Bytes in;
@@ -234,6 +258,9 @@ static napi_value InflateBatch(napi_env env, napi_callback_info info)
     uint32_t flags = 0;
     napi_get_value_uint32(env, argv[4], &flags);
     const size_t n = offs.size();
+    Bytes dict;
+    std::vector<zlb_dict> dicts;
+    if (!get_dict(env, argc, argv, 5, n, &dict, &dicts)) return nullptr;
     std::vector<zlb_item> items(n);
     std::vector<zlb_result> res(n);
     uint64_t out_total = 0;
@@ -251,7 +278,8 @@ static napi_value InflateBatch(napi_env env, napi_callback_info info)
         napi_throw_error(env, nullptr, "zlib.ts-b200: out of host memory");
         return nullptr;
     }
-    int rc = zlb_inflate_batch_host(g_ctx, in.p, in.n, out.p, out_total, items.data(), res.data(), n, flags);
+    int rc = zlb_inflate_batch_dict_host(g_ctx, in.p, in.n, out.p, out_total, dict.p, dict.n,
+                                         dicts.empty() ? nullptr : dicts.data(), items.data(), res.data(), n, flags);
     if (rc != ZLB_OK) {
         napi_throw_error(env, nullptr, zlb_last_error(g_ctx));
         return nullptr;

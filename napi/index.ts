@@ -8,12 +8,14 @@ export enum CompressionType { NONE = 0, FIXED = 1, DYNAMIC = 2, RESERVED = 3 }  
 export enum BufferType { BLOCK = 0, ADAPTIVE = 1 }                                   // src/RawInflate.ts:5-8
 export interface RawDeflateOptions { lazy?: number; compressionType?: CompressionType;
     outputBuffer?: number[] | Uint8Array; outputIndex?: number;
-    b200?: { chunkBytes?: number; mode?: 'compat' | 'fast' | 'primed' | 'fast-primed'; depth?: number; smallest?: boolean; lazy?: boolean } }
+    b200?: { chunkBytes?: number; mode?: 'compat' | 'fast' | 'primed' | 'fast-primed'; depth?: number; smallest?: boolean; lazy?: boolean;
+             dictionary?: Uint8Array } }   // dictionary: a preset dictionary (zlib's deflateSetDictionary)
 // engine-only knob -> ZLB_MODE_* (include/zlibts_b200.h); the default is the reference-compatible mode
 const modeOf = (o: RawDeflateOptions = {}) => { const b = o.b200 ?? {}; const m = b.mode ?? 'compat';
     return (m.startsWith('fast') ? 1 | ((b.depth ?? 0) << 8) : 0) | (m.endsWith('primed') ? 2 : 0) | (b.smallest ? 4 : 0) |
         (b.lazy && m.startsWith('fast') ? 8 : 0); };   // lazy: ZLB_MODE_LAZY, a fast-mode option
-export interface RawInflateOptions { index?: number; bufferSize?: number; bufferType?: BufferType; resize?: boolean }
+export interface RawInflateOptions { index?: number; bufferSize?: number; bufferType?: BufferType; resize?: boolean;
+    b200?: { dictionary?: Uint8Array } }   // a preset dictionary (zlib's inflateSetDictionary)
 
 const STATUS_TEXT: { [k: number]: string } = {                                       // include/zlibts_b200.h
     1: 'input buffer is broken', 2: 'unknown BTYPE: 3', 3: 'invalid code length',
@@ -26,7 +28,7 @@ const u8 = (x: number[] | Uint8Array) => x instanceof Uint8Array ? x : new Uint8
 
 export class RawDeflate {                                                            // src/RawDeflate.ts:50-114
     input: Uint8Array; output: Uint8Array; op: number; compressionType: CompressionType; lazy: number; chunk: number;
-    mode: number;
+    mode: number; dictionary?: Uint8Array;
     constructor(input: number[] | Uint8Array, opts: RawDeflateOptions = {}) {
         this.input = u8(input);
         this.lazy = opts.lazy ?? 0;
@@ -36,9 +38,11 @@ export class RawDeflate {                                                       
         this.op = opts.outputIndex ?? 0;
         this.chunk = opts.b200?.chunkBytes ?? 0;
         this.mode = modeOf(opts);
+        this.dictionary = opts.b200?.dictionary;
     }
-    compress(): Uint8Array {
-        const r = native.deflateBatch([this.input], this.compressionType, this.chunk, 0, this.mode);
+    compress(flags = 0): Uint8Array {
+        const r = native.deflateBatch([this.input], this.compressionType, this.chunk, flags, this.mode, this.dictionary);
+        (this as any).adler32 = r.adler32[0];
         const body: Uint8Array = r.outputs[0];
         const out = new Uint8Array(this.op + body.length);
         out.set(this.output.subarray(0, Math.min(this.op, this.output.length)));     // caller's prefix survives
@@ -49,14 +53,15 @@ export class RawDeflate {                                                       
 }
 
 export class RawInflate {                                                            // src/RawInflate.ts:70-140
-    input: Uint8Array; ip: number; bufferSize?: number; buffer: Uint8Array | null = null; op = 0;
+    input: Uint8Array; ip: number; bufferSize?: number; buffer: Uint8Array | null = null; op = 0; dictionary?: Uint8Array;
     constructor(input: Uint8Array, opts: RawInflateOptions = {}) {
         this.input = u8(input); this.ip = opts.index ?? 0; this.bufferSize = opts.bufferSize;
+        this.dictionary = opts.b200?.dictionary;
     }
     decompress(flags = 0): Uint8Array {
         let cap = this.bufferSize ?? Math.max(0x8000, 4 * (this.input.length - this.ip));
         for (;;) {                                                                   // the reference grows its buffer
-            const r = native.inflateBatch(this.input, [this.ip], [this.input.length - this.ip], [cap], flags);
+            const r = native.inflateBatch(this.input, [this.ip], [this.input.length - this.ip], [cap], flags, this.dictionary);
             if (r.status[0] === 4) { cap *= 4; continue; }
             if (r.status[0] !== 0) throw new Error(statusText(r.status[0]));
             this.ip += r.inUsed[0]; this.buffer = r.outputs[0]; this.op = r.outputs[0].length;
@@ -89,6 +94,16 @@ export class Deflate {                                                          
     static compress(input: number[] | Uint8Array, opts: RawDeflateOptions) { return new Deflate(input, opts).compress(); }
     compress(): Uint8Array {
         const type = this.opts.compressionType ?? CompressionType.DYNAMIC;
+        const dict = this.opts.b200?.dictionary;
+        if (dict && dict.length) {
+            // preset dictionary: FDICT, DICTID (the dictionary's Adler-32), the dictionary deflate, Adler-32 of the input
+            const cmf = 120; let flg = type << 6 | 0x20; flg |= 31 - ((cmf << 8) + flg) % 31;
+            const raw = new RawDeflate(this.input, this.opts), body = raw.compress(2), id = Adler32.create(dict);
+            this.adler32 = (raw as any).adler32 as number;
+            const out = new Uint8Array(6 + body.length + 4), v = new DataView(out.buffer);
+            out[0] = cmf; out[1] = flg; v.setUint32(2, id); out.set(body, 6); v.setUint32(6 + body.length, this.adler32);
+            return this.output = out;
+        }
         const cmf = 120; let flg = type << 6; flg |= 31 - ((cmf << 8) + flg) % 31;     // :67-78
         // header, raw stream and big-endian Adler-32 (:95) are put together on the device (zlb_archive_host, kind 1)
         const r = native.archive(1, [u8(this.input)], [new Uint8Array([cmf, flg])], null, null, new Uint8Array(0),
@@ -105,8 +120,17 @@ export class Inflate {                                                          
         const cmf = input[this.ip++], flg = input[this.ip++];
         if ((cmf & 0x0f) !== 8) throw new Error('unsupported compression method');
         if (((cmf << 8) + flg) % 31 !== 0) throw new Error('invalid fcheck flag:' + ((cmf << 8) + flg) % 31);
-        if (flg & 0x20) throw new Error('fdict flag is not supported');
-        this.rawinflate = new RawInflate(input, { index: this.ip, bufferSize: opts.bufferSize });
+        // a preset dictionary is used for FDICT streams only; other streams ignore it, like zlib
+        const dict = flg & 0x20 ? opts.b200?.dictionary : undefined;
+        if (flg & 0x20) {
+            if (!dict) throw new Error('fdict flag is not supported');
+            const p = this.ip, id = (input[p] << 24 | input[p + 1] << 16 | input[p + 2] << 8 | input[p + 3]) >>> 0;
+            const have = Adler32.create(dict) >>> 0;
+            if (have !== id) throw new Error('invalid dictionary: adler-32 0x' + have.toString(16).padStart(8, '0') +
+                                             ', DICTID 0x' + id.toString(16).padStart(8, '0'));
+            this.ip += 4;
+        }
+        this.rawinflate = new RawInflate(input, { index: this.ip, bufferSize: opts.bufferSize, b200: { dictionary: dict } });
     }
     decompress(): Uint8Array {
         const buffer = this.rawinflate.decompress(this.verify ? 2 : 0);

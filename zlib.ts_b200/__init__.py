@@ -2,6 +2,7 @@
 from ._native import (  # noqa: F401
     Engine, EngineError, load_library, default_engine, make_items, make_entries, deflate_bound, archive_bound,
     crc32_combine, adler32_combine, host_alloc, host_free, host_is_pinned, ITEM_DTYPE, RESULT_DTYPE, ENTRY_DTYPE, EXPORTS, LIB_PATH,
+    DICT_DTYPE, make_dicts,
     FRAME_ZLIB, FRAME_GZIP, FRAME_ZIP,
     NONE, FIXED, DYNAMIC, MODE_COMPAT, MODE_FAST, MODE_PRIMED, MODE_SMALLEST, MODE_LAZY, PRIMED_CHUNK, mode_fast, mode_chunk,
     DEFLATE_WANT_CRC32, DEFLATE_WANT_ADLER32, DEFLATE_NOT_FINAL,

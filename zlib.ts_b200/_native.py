@@ -16,7 +16,8 @@ RESULT_DTYPE = np.dtype([("status", "<u4"), ("crc32", "<u4"), ("adler32", "<u4")
                          ("out_len", "<u8"), ("in_used", "<u8")])
 ENTRY_DTYPE = np.dtype([("in_off", "<u8"), ("in_len", "<u8"), ("head_off", "<u8"), ("head_len", "<u4"),
                         ("method", "<u4"), ("cdir_off", "<u8"), ("cdir_len", "<u4"), ("reserved", "<u4")])
-assert ITEM_DTYPE.itemsize == 32 and RESULT_DTYPE.itemsize == 32 and ENTRY_DTYPE.itemsize == 48
+DICT_DTYPE = np.dtype([("off", "<u8"), ("len", "<u8")])   # zlb_dict: an item's preset dictionary in the dictionary blob
+assert ITEM_DTYPE.itemsize == 32 and RESULT_DTYPE.itemsize == 32 and ENTRY_DTYPE.itemsize == 48 and DICT_DTYPE.itemsize == 16
 
 # CompressionType (src/RawDeflate.ts:12-17)
 NONE, FIXED, DYNAMIC = 0, 1, 2
@@ -44,6 +45,7 @@ EXPORTS = [
     "zlb_profile_enable", "zlb_profile_read", "zlb_profile_reset", "zlb_launch_count",
     "zlb_debug_lz77", "zlb_debug_code_lengths",
     "zlb_host_alloc", "zlb_host_free", "zlb_host_is_pinned",
+    "zlb_deflate_batch_dict", "zlb_deflate_batch_dict_host", "zlb_inflate_batch_dict", "zlb_inflate_batch_dict_host",
 ]
 
 _lib = None
@@ -79,6 +81,14 @@ def load_library():
     lib.zlb_inflate_batch.restype = i32
     lib.zlb_inflate_batch_host.argtypes = [vp, vp, sz, vp, sz, vp, vp, sz, u32]
     lib.zlb_inflate_batch_host.restype = i32
+    lib.zlb_deflate_batch_dict.argtypes = [vp, vp, vp, vp, vp, vp, vp, sz, i32, i32, u32, u32]
+    lib.zlb_deflate_batch_dict.restype = i32
+    lib.zlb_deflate_batch_dict_host.argtypes = [vp, vp, sz, vp, sz, vp, sz, vp, vp, vp, sz, i32, i32, u32, u32]
+    lib.zlb_deflate_batch_dict_host.restype = i32
+    lib.zlb_inflate_batch_dict.argtypes = [vp, vp, vp, vp, vp, vp, vp, sz, u32]
+    lib.zlb_inflate_batch_dict.restype = i32
+    lib.zlb_inflate_batch_dict_host.argtypes = [vp, vp, sz, vp, sz, vp, sz, vp, vp, vp, sz, u32]
+    lib.zlb_inflate_batch_dict_host.restype = i32
     lib.zlb_checksum_batch.argtypes = [vp, vp, vp, vp, sz, u32]
     lib.zlb_checksum_batch.restype = i32
     lib.zlb_checksum_batch_host.argtypes = [vp, vp, sz, vp, vp, sz, u32]
@@ -163,15 +173,21 @@ def adler32_combine(adler_a, adler_b, len_b):
     return load_library().zlb_adler32_combine(adler_a, adler_b, len_b)
 
 
-def deflate_bound(in_len, chunk_bytes=0, block_type=DYNAMIC, mode=MODE_COMPAT):
-    return int(load_library().zlb_deflate_bound(in_len, mode_chunk(mode, chunk_bytes), block_type))
+def deflate_bound(in_len, chunk_bytes=0, block_type=DYNAMIC, mode=MODE_COMPAT, dictionary=False):
+    """Output bytes that always suffice for an item; `dictionary`: some item of the call has a preset dictionary."""
+    return int(load_library().zlb_deflate_bound(in_len, mode_chunk(mode, chunk_bytes, dictionary), block_type))
 
 
-def mode_chunk(mode, chunk_bytes=0):
-    """The chunk size a deflate call with this mode really uses (primed modes: at most 32 KiB)."""
-    if mode & MODE_PRIMED and (chunk_bytes == 0 or chunk_bytes > PRIMED_CHUNK):
+def mode_chunk(mode, chunk_bytes=0, dictionary=False):
+    """The chunk size a deflate call with this mode really uses (primed modes, and calls in which some item has a
+    preset dictionary: at most 32 KiB)."""
+    if (mode & MODE_PRIMED or dictionary) and (chunk_bytes == 0 or chunk_bytes > PRIMED_CHUNK):
         return PRIMED_CHUNK
     return chunk_bytes
+
+
+def make_dicts(n):
+    return np.zeros(n, dtype=DICT_DTYPE)
 
 
 def make_items(n):
@@ -251,17 +267,39 @@ class Engine:
         results = np.zeros(len(items), dtype=RESULT_DTYPE)
         return items, results
 
-    def deflate_batch(self, d_in, d_out, items, block_type=DYNAMIC, chunk_bytes=0, flags=0, mode=MODE_COMPAT):
+    @staticmethod
+    def _dicts(dicts):
+        """The zlb_dict table as an array (None: no dictionaries, a NULL table)."""
+        return None if dicts is None else np.ascontiguousarray(dicts, dtype=DICT_DTYPE)
+
+    def deflate_batch(self, d_in, d_out, items, block_type=DYNAMIC, chunk_bytes=0, flags=0, mode=MODE_COMPAT,
+                      d_dict=None, dicts=None):
+        """zlb_deflate_batch; with `dicts` (a DICT_DTYPE table, one entry per item, spans of the device blob d_dict)
+        zlb_deflate_batch_dict."""
         items, results = self._tables(items)
-        rc = self.lib.zlb_deflate_batch(self.h, d_in.data_ptr(), d_out.data_ptr(), items.ctypes.data,
-                                        results.ctypes.data, len(items), mode, block_type, chunk_bytes, flags)
+        dicts = self._dicts(dicts)
+        if dicts is None:
+            rc = self.lib.zlb_deflate_batch(self.h, d_in.data_ptr(), d_out.data_ptr(), items.ctypes.data,
+                                            results.ctypes.data, len(items), mode, block_type, chunk_bytes, flags)
+        else:
+            rc = self.lib.zlb_deflate_batch_dict(self.h, d_in.data_ptr(), d_out.data_ptr(),
+                                                 d_dict.data_ptr() if d_dict is not None else None, dicts.ctypes.data,
+                                                 items.ctypes.data, results.ctypes.data, len(items), mode, block_type,
+                                                 chunk_bytes, flags)
         self._check(rc, "zlb_deflate_batch")
         return results
 
-    def inflate_batch(self, d_in, d_out, items, flags=0):
+    def inflate_batch(self, d_in, d_out, items, flags=0, d_dict=None, dicts=None):
+        """zlb_inflate_batch; with `dicts` zlb_inflate_batch_dict (see deflate_batch)."""
         items, results = self._tables(items)
-        rc = self.lib.zlb_inflate_batch(self.h, d_in.data_ptr(), d_out.data_ptr(), items.ctypes.data,
-                                        results.ctypes.data, len(items), flags)
+        dicts = self._dicts(dicts)
+        if dicts is None:
+            rc = self.lib.zlb_inflate_batch(self.h, d_in.data_ptr(), d_out.data_ptr(), items.ctypes.data,
+                                            results.ctypes.data, len(items), flags)
+        else:
+            rc = self.lib.zlb_inflate_batch_dict(self.h, d_in.data_ptr(), d_out.data_ptr(),
+                                                 d_dict.data_ptr() if d_dict is not None else None, dicts.ctypes.data,
+                                                 items.ctypes.data, results.ctypes.data, len(items), flags)
         self._check(rc, "zlb_inflate_batch")
         return results
 
@@ -282,21 +320,37 @@ class Engine:
         arr = np.ascontiguousarray(arr)
         return arr.ctypes.data, arr.nbytes, arr
 
-    def deflate_batch_host(self, h_in, h_out, items, block_type=DYNAMIC, chunk_bytes=0, flags=0, mode=MODE_COMPAT):
+    def deflate_batch_host(self, h_in, h_out, items, block_type=DYNAMIC, chunk_bytes=0, flags=0, mode=MODE_COMPAT,
+                           h_dict=None, dicts=None):
+        """zlb_deflate_batch_host; with `dicts` (spans of the host blob h_dict) zlb_deflate_batch_dict_host."""
         items, results = self._tables(items)
         pi, ni, ki = self._host_ptr(h_in)
         po, no, ko = self._host_ptr(h_out)
-        rc = self.lib.zlb_deflate_batch_host(self.h, pi, ni, po, no, items.ctypes.data, results.ctypes.data,
-                                             len(items), mode, block_type, chunk_bytes, flags)
+        dicts = self._dicts(dicts)
+        if dicts is None:
+            rc = self.lib.zlb_deflate_batch_host(self.h, pi, ni, po, no, items.ctypes.data, results.ctypes.data,
+                                                 len(items), mode, block_type, chunk_bytes, flags)
+        else:
+            pd, nd, kd = self._host_ptr(h_dict) if h_dict is not None else (None, 0, None)
+            rc = self.lib.zlb_deflate_batch_dict_host(self.h, pi, ni, po, no, pd, nd, dicts.ctypes.data,
+                                                      items.ctypes.data, results.ctypes.data, len(items), mode,
+                                                      block_type, chunk_bytes, flags)
         self._check(rc, "zlb_deflate_batch_host")
         return results
 
-    def inflate_batch_host(self, h_in, h_out, items, flags=0):
+    def inflate_batch_host(self, h_in, h_out, items, flags=0, h_dict=None, dicts=None):
+        """zlb_inflate_batch_host; with `dicts` zlb_inflate_batch_dict_host (see deflate_batch_host)."""
         items, results = self._tables(items)
         pi, ni, ki = self._host_ptr(h_in)
         po, no, ko = self._host_ptr(h_out)
-        rc = self.lib.zlb_inflate_batch_host(self.h, pi, ni, po, no, items.ctypes.data, results.ctypes.data,
-                                             len(items), flags)
+        dicts = self._dicts(dicts)
+        if dicts is None:
+            rc = self.lib.zlb_inflate_batch_host(self.h, pi, ni, po, no, items.ctypes.data, results.ctypes.data,
+                                                 len(items), flags)
+        else:
+            pd, nd, kd = self._host_ptr(h_dict) if h_dict is not None else (None, 0, None)
+            rc = self.lib.zlb_inflate_batch_dict_host(self.h, pi, ni, po, no, pd, nd, dicts.ctypes.data,
+                                                      items.ctypes.data, results.ctypes.data, len(items), flags)
         self._check(rc, "zlb_inflate_batch_host")
         return results
 

@@ -19,6 +19,11 @@ Deviations from the reference, all deliberate (SURVEY.md Appendix B):
     which no inflater accepts) because LZ77's output array has length 0 there (src/LZ77.ts:122,278).
   * corrupt streams that make the reference loop or emit zeros (B-8) raise ZlibError instead.
   * ZipCrypto (password) is out of scope (SURVEY section 2: serial byte cipher, broken upstream).
+  * preset dictionaries (zlib's deflateSetDictionary / inflateSetDictionary): `b200: {dictionary}` on RawDeflate,
+    RawInflate, Deflate and Inflate, `dictionary=` on the batch functions. Deflate then writes FLG.FDICT and DICTID
+    (RFC 1950); Inflate reads FDICT streams when given the dictionary whose Adler-32 is DICTID, where the reference
+    always throws "fdict flag is not supported" (it still does here without a dictionary). A dictionary given for a
+    stream without FDICT is ignored, as zlib does. Only a dictionary's last 32 KiB can be reached.
 """
 import datetime
 import struct
@@ -118,26 +123,55 @@ def _mode_of(opts):
     return mode | (N.MODE_PRIMED if name.endswith("primed") else 0) | (N.MODE_SMALLEST if b.get("smallest") else 0)
 
 
+def _dict_table(dictionary, n):
+    """(dictionary blob, zlb_dict table) for `dictionary` = None | bytes-like (every item) | list (one entry per
+    item, None = no dictionary); (None, None) when no item has one. Equal dictionaries are stored once."""
+    if dictionary is None:
+        return None, None
+    per_item = [dictionary] * n if not isinstance(dictionary, (list, tuple)) else list(dictionary)
+    if len(per_item) != n:
+        raise ZlibError("dictionary list must have one entry per input")
+    table = N.make_dicts(n)
+    parts, at, where = [], 0, {}
+    for i, d in enumerate(per_item):
+        if d is None:
+            continue
+        key = _u8(d).tobytes()
+        if not key:
+            continue
+        if key not in where:
+            where[key] = at
+            parts.append(key)
+            at += len(key)
+        table[i] = (where[key], len(key))
+    if not parts:
+        return None, None
+    return np.frombuffer(b"".join(parts), dtype=np.uint8), table
+
+
 def deflate_many(inputs, compression_type=CompressionType.DYNAMIC, chunk_bytes=0, want_crc32=False,
-                 want_adler32=False, prefixes=None, mode=N.MODE_COMPAT):
+                 want_adler32=False, prefixes=None, mode=N.MODE_COMPAT, dictionary=None):
     """Raw-deflates every input in one GPU batch. Returns (list of uint8 arrays, results table). With `prefixes`
-    each output starts with its prefix bytes (RawDeflate's outputBuffer / outputIndex contract)."""
+    each output starts with its prefix bytes (RawDeflate's outputBuffer / outputIndex contract). `dictionary`: a
+    preset dictionary for every input (bytes-like) or one per input (a list; None entries have none)."""
     arrs = [_u8(x) for x in inputs]
     n = len(arrs)
     if n == 0:
         return [], np.zeros(0, dtype=N.RESULT_DTYPE)
     if compression_type not in (0, 1, 2):
         raise ZlibError("invalid compression type")  # src/RawDeflate.ts:110 (a thrown string there)
+    dblob, dicts = _dict_table(dictionary, n)
     lens = np.array([a.size for a in arrs], dtype=np.uint64)
     in_off = np.concatenate([[0], np.cumsum(lens)[:-1]]).astype(np.uint64)
     blob = np.concatenate(arrs) if int(lens.sum()) else np.zeros(1, dtype=np.uint8)
-    caps = np.array([N.deflate_bound(int(l), chunk_bytes, compression_type, mode) for l in lens], dtype=np.uint64)
+    caps = np.array([N.deflate_bound(int(l), chunk_bytes, compression_type, mode, dicts is not None) for l in lens],
+                    dtype=np.uint64)
     out_off = np.concatenate([[0], np.cumsum(caps)[:-1]]).astype(np.uint64)
     out = np.zeros(int(caps.sum()), dtype=np.uint8)
     items = N.make_items(n)
     items["in_off"], items["in_len"], items["out_off"], items["out_cap"] = in_off, lens, out_off, caps
     flags = (N.DEFLATE_WANT_CRC32 if want_crc32 else 0) | (N.DEFLATE_WANT_ADLER32 if want_adler32 else 0)
-    res = engine().deflate_batch_host(blob, out, items, compression_type, chunk_bytes, flags, mode)
+    res = engine().deflate_batch_host(blob, out, items, compression_type, chunk_bytes, flags, mode, dblob, dicts)
     outs = []
     for i in range(n):
         if int(res["status"][i]) != N.ST_OK:
@@ -149,16 +183,18 @@ def deflate_many(inputs, compression_type=CompressionType.DYNAMIC, chunk_bytes=0
     return outs, res
 
 
-def inflate_blob(blob, offs, lens, size_hints=None, want_crc32=False, want_adler32=False, split=True, tolerant=False):
+def inflate_blob(blob, offs, lens, size_hints=None, want_crc32=False, want_adler32=False, split=True, tolerant=False,
+                 dictionary=None):
     """Raw-inflates the streams blob[offs[i] : offs[i] + lens[i]] in one GPU batch; output slots that turn out
     too small are retried larger (the reference grows its buffer instead, src/RawInflate.ts:550-581).
     Returns (list of uint8 arrays, results table); raises ZlibError with the reference's text on corrupt input.
     `tolerant`: nothing is raised or retried -- a stream that fails or overflows its slot comes back as None with its
-    status in the table (speculative decoding of gzip member candidates)."""
+    status in the table (speculative decoding of gzip member candidates). `dictionary`: as for deflate_many."""
     blob = _u8(blob)
     n = len(offs)
     if n == 0:
         return [], np.zeros(0, dtype=N.RESULT_DTYPE)
+    dblob, dicts = _dict_table(dictionary, n)
     offs = np.asarray(offs, dtype=np.uint64)
     lens = np.asarray(lens, dtype=np.uint64)
     caps = np.zeros(n, dtype=np.uint64)
@@ -180,7 +216,7 @@ def inflate_blob(blob, offs, lens, size_hints=None, want_crc32=False, want_adler
         items = N.make_items(m)
         items["in_off"], items["in_len"] = offs[todo], lens[todo]
         items["out_off"], items["out_cap"] = out_off, caps[todo]
-        res = engine().inflate_batch_host(blob, out, items, flags)
+        res = engine().inflate_batch_host(blob, out, items, flags, dblob, None if dicts is None else dicts[todo])
         again = []
         for k, i in enumerate(todo):
             st = int(res["status"][k])
@@ -201,8 +237,9 @@ def inflate_blob(blob, offs, lens, size_hints=None, want_crc32=False, want_adler
     raise ZlibError("inflate output does not fit")
 
 
-def inflate_many(buffers, indices=None, size_hints=None, want_crc32=False, want_adler32=False):
-    """One stream per buffer, starting at indices[i] (RawInflate's `index` option)."""
+def inflate_many(buffers, indices=None, size_hints=None, want_crc32=False, want_adler32=False, dictionary=None):
+    """One stream per buffer, starting at indices[i] (RawInflate's `index` option); `dictionary` as for
+    deflate_many."""
     arrs = [_u8(x) for x in buffers]
     n = len(arrs)
     if n == 0:
@@ -212,7 +249,7 @@ def inflate_many(buffers, indices=None, size_hints=None, want_crc32=False, want_
     base = np.concatenate([[0], np.cumsum(lens)[:-1]]).astype(np.uint64)
     blob = np.concatenate(arrs) if int(lens.sum()) else np.zeros(1, dtype=np.uint8)
     idx = np.minimum(idx, lens)
-    return inflate_blob(blob, base + idx, lens - idx, size_hints, want_crc32, want_adler32)
+    return inflate_blob(blob, base + idx, lens - idx, size_hints, want_crc32, want_adler32, dictionary=dictionary)
 
 
 def checksum_many(buffers, crc32=True, adler32=True):
@@ -318,6 +355,7 @@ class RawDeflate:
         self.op = _opt(opts, "outputIndex", 0)
         self.chunkBytes = _b200(opts).get("chunkBytes", 0)
         self.mode = _mode_of(opts)
+        self.dictionary = _b200(opts).get("dictionary")  # preset dictionary (engine extension)
         if self.lazy:
             raise ZlibError("lazy matching is not supported: the reference corrupts data with lazy > 0")
 
@@ -325,7 +363,8 @@ class RawDeflate:
         prefix = self.output[:self.op]
         if prefix.size < self.op:  # outputIndex beyond the given buffer: the reference doubles it, zero filled
             prefix = np.concatenate([prefix, np.zeros(self.op - prefix.size, dtype=np.uint8)])
-        outs, _ = deflate_many([self.input], self.compressionType, self.chunkBytes, prefixes=[prefix], mode=self.mode)
+        outs, _ = deflate_many([self.input], self.compressionType, self.chunkBytes, prefixes=[prefix], mode=self.mode,
+                               dictionary=self.dictionary)
         self.output = outs[0]
         self.op = int(self.output.size)
         return self.output
@@ -338,11 +377,12 @@ class RawInflate:
         self.bufferSize = (opts or {}).get("bufferSize")
         self.bufferType = _opt(opts, "bufferType", BufferType.ADAPTIVE)
         self.resize = _opt(opts, "resize", False)
+        self.dictionary = _b200(opts).get("dictionary")  # preset dictionary (engine extension)
         self.buffer = None
         self.op = 0
 
     def decompress(self):
-        outs, res = inflate_many([self.input], [self.ip], [self.bufferSize])
+        outs, res = inflate_many([self.input], [self.ip], [self.bufferSize], dictionary=self.dictionary)
         self.ip += int(res["in_used"][0])  # first byte after the deflate data (src/RawInflate.ts:511-514)
         self.buffer = outs[0]
         self.op = int(outs[0].size)
@@ -352,11 +392,16 @@ class RawInflate:
 # ------------------------------------------------------------------------------------------------------------
 # zlib container (src/Deflate.ts, src/Inflate.ts)
 # ------------------------------------------------------------------------------------------------------------
-def _zlib_header(compression_type):  # src/Deflate.ts:67-78
+def _zlib_header(compression_type, fdict=False):  # src/Deflate.ts:67-78 (FDICT: RFC 1950)
     cmf = 120
-    flg = (compression_type << 6) | (0 << 5)
+    flg = (compression_type << 6) | ((1 if fdict else 0) << 5)
     flg |= 31 - ((cmf << 8) + flg) % 31
     return bytes([cmf, flg & 0xFF])
+
+
+def _dictid(dictionary):
+    """DICTID of a preset dictionary: its Adler-32 (RFC 1950), computed on the GPU."""
+    return int(checksum_many([_u8(dictionary)], False, True)["adler32"][0])
 
 
 class Deflate:
@@ -374,6 +419,16 @@ class Deflate:
         return Deflate(input, opts).compress()
 
     def compress(self):
+        dictionary = _b200(self.opts).get("dictionary")
+        if dictionary is not None and _u8(dictionary).size:
+            # preset dictionary: header with FDICT, DICTID, the dictionary deflate, Adler-32 of the input (zlb_archive
+            # has no dictionary, so this stream is framed here)
+            outs, res = deflate_many([self.input], self.compressionType, _b200(self.opts).get("chunkBytes", 0),
+                                     want_adler32=True, mode=_mode_of(self.opts), dictionary=dictionary)
+            self.adler32 = int(res["adler32"][0])
+            head = _zlib_header(self.compressionType, fdict=True) + struct.pack(">I", _dictid(dictionary))
+            self.output = np.concatenate([_u8(head), outs[0], _u8(struct.pack(">I", self.adler32))])
+            return self.output
         # header (:67-78), raw stream (:84-85) and Adler-32 big endian (:95) are put together on the device
         self.output, res = archive_many(N.FRAME_ZLIB, [self.input], [_zlib_header(self.compressionType)],
                                         self.compressionType, _b200(self.opts).get("chunkBytes", 0), _mode_of(self.opts))
@@ -393,15 +448,24 @@ class Inflate:
             raise ZlibError("unsupported compression method")  # src/Inflate.ts:47
         if ((cmf << 8) + flg) % 31 != 0:
             raise ZlibError("invalid fcheck flag:%d" % (((cmf << 8) + flg) % 31))  # :52
+        # a preset dictionary (engine extension) is used for FDICT streams only; other streams ignore it, like zlib
+        dictionary = _b200(opts).get("dictionary") if flg & 0x20 else None
         if flg & 0x20:
-            raise ZlibError("fdict flag is not supported")  # :57
+            if dictionary is None:
+                raise ZlibError("fdict flag is not supported")  # :57
+            dictid = struct.unpack(">I", self.input[self.ip:self.ip + 4].tobytes().ljust(4, b"\0"))[0]
+            have = _dictid(dictionary)
+            if have != dictid:
+                raise ZlibError("invalid dictionary: adler-32 0x%08x, DICTID 0x%08x" % (have, dictid))
+            self.ip += 4
         self.rawinflate = RawInflate(self.input, {"index": self.ip, "bufferSize": (opts or {}).get("bufferSize"),
                                                   "bufferType": (opts or {}).get("bufferType"),
-                                                  "resize": (opts or {}).get("resize")})
+                                                  "resize": (opts or {}).get("resize"),
+                                                  "b200": {"dictionary": dictionary}})
 
     def decompress(self):
         r = self.rawinflate
-        outs, res = inflate_many([r.input], [r.ip], [r.bufferSize], want_adler32=self.verify)
+        outs, res = inflate_many([r.input], [r.ip], [r.bufferSize], want_adler32=self.verify, dictionary=r.dictionary)
         r.ip += int(res["in_used"][0])
         self.ip = r.ip
         buf = outs[0]

@@ -29,6 +29,8 @@ enum ZtsKernelSlot {
     ZK_WINDOW_RUN,
     ZK_WINDOW_SCAN,
     ZK_WINDOW_RESOLVE,
+    ZK_DICT_STAGE,      // preset dictionaries (zts_deflate.cu, zts_inflate.cu)
+    ZK_INFLATE_DICT,
     ZK_COUNT
 };
 
@@ -38,7 +40,8 @@ static const char* const kZtsKernelNames[ZK_COUNT] = {
     "bitpack_kernel",      "stored_block_kernel",    "deflate_finalize_kernel",
     "marker_scan_kernel",  "segment_gather_kernel",
     "frame_body_kernel",   "frame_header_kernel",
-    "inflate_warp_kernel_window", "window_run_kernel", "window_scan_kernel", "window_resolve_kernel"};
+    "inflate_warp_kernel_window", "window_run_kernel", "window_scan_kernel", "window_resolve_kernel",
+    "dict_stage_kernel", "inflate_warp_kernel_dict"};
 
 struct ZtsDevBuf {
     void* p = nullptr;
@@ -60,7 +63,7 @@ struct zlb_ctx {
 
     // device arenas (grow-only, freed in zlb_destroy)
     ZtsDevBuf d_items, d_results, d_chunks, d_chunk_info, d_tokens, d_spec, d_hist, d_codes, d_sortT,
-        d_sums, d_misc, d_stage_in, d_stage_out, d_split, d_window, d_body, d_frames;
+        d_sums, d_misc, d_stage_in, d_stage_out, d_split, d_window, d_body, d_frames, d_dict, d_dict_stage;
     // pinned host staging for the small tables
     void* h_pin = nullptr;
     size_t h_pin_cap = 0;
@@ -107,6 +110,9 @@ void zts_stage_destroy_ctx(zlb_ctx* ctx);
 int zts_copy_back(zlb_ctx* ctx, ZtsHostStage* st, cudaStream_t s, const uint8_t* d_out, uint8_t* h_out,
                   const zlb_item* h_items, const zlb_result* h_res, const zlb_item* d_items, const zlb_result* d_res,
                   size_t a, size_t b);
+// preset dictionaries: checks a table (NULL = none; blob_bytes = SIZE_MAX when the blob's size is not known, i.e. a
+// device blob) and tells whether any item has one
+int zts_check_dicts(zlb_ctx* ctx, const void* blob, size_t blob_bytes, const zlb_dict* dicts, size_t n, bool* any);
 void zts_prof_begin(zlb_ctx* ctx, int slot);
 void zts_prof_end(zlb_ctx* ctx, int slot);
 

@@ -34,6 +34,21 @@ int zts_reserve(zlb_ctx* ctx, ZtsDevBuf* b, size_t bytes)
     return ZLB_OK;
 }
 
+int zts_check_dicts(zlb_ctx* ctx, const void* blob, size_t blob_bytes, const zlb_dict* dicts, size_t n, bool* any)
+{
+    *any = false;
+    if (!dicts) return ZLB_OK;
+    for (size_t i = 0; i < n; ++i) {
+        const zlb_dict d = dicts[i];
+        if (d.len == 0) continue;
+        if (!blob) return zts_fail(ctx, ZLB_E_ARG, "item %zu has a dictionary but the dictionary blob is NULL", i);
+        if (d.off > blob_bytes || d.len > blob_bytes - d.off)
+            return zts_fail(ctx, ZLB_E_ARG, "dictionary of item %zu out of range", i);
+        *any = true;
+    }
+    return ZLB_OK;
+}
+
 int zts_reserve_pinned(zlb_ctx* ctx, size_t bytes)
 {
     if (bytes <= ctx->h_pin_cap) return ZLB_OK;
@@ -224,7 +239,7 @@ void zlb_destroy(zlb_ctx* ctx)
     ZtsDevBuf* bufs[] = {&ctx->d_items, &ctx->d_results, &ctx->d_chunks, &ctx->d_chunk_info, &ctx->d_tokens,
                          &ctx->d_spec,  &ctx->d_hist,    &ctx->d_codes,  &ctx->d_sortT,      &ctx->d_sums,
                          &ctx->d_misc,  &ctx->d_stage_in, &ctx->d_stage_out, &ctx->d_split, &ctx->d_window,
-                         &ctx->d_body,  &ctx->d_frames};
+                         &ctx->d_body,  &ctx->d_frames, &ctx->d_dict, &ctx->d_dict_stage};
     for (ZtsDevBuf* b : bufs)
         if (b->p) cudaFree(b->p);
     zts_stage_destroy_ctx(ctx);

@@ -10,8 +10,7 @@
 //                        block, image copied out with aligned word stores (byte stores at the edges)
 // Chunks of one item are joined by an empty stored block that byte-aligns (SURVEY App. A.7); the
 // reference's RawInflate accepts this (src/RawInflate.ts:128-130,261-262,311).
-#include <stdlib.h>
-
+#include <stdint.h>
 #include <stdlib.h>
 #include "zts_deflate.cuh"
 
@@ -293,6 +292,27 @@ bitpack_kernel(const ZtsChunk* __restrict__ chunks, const ZtsChunkInfo* __restri
     }
 }
 
+// ---- preset dictionaries: the window of every chunk whose history reaches into its item's dictionary ---------------
+// The window of a chunk at byte `pos` of its item is the last dict_len bytes of dictionary || item[0, pos), then the
+// chunk: its first dict_len - pos bytes are the dictionary's last ones. It is written to the chunk's place in the
+// staging arena (16-byte aligned, like the input the LZ77 kernel otherwise stages from), which that kernel reads
+// instead of the input (CHUNK_STAGED): its own chunk table names the window by an in_off taken relative to the input
+// (deflate_device). Only chunks that start in the first 32 KiB of their item have such a window.
+__global__ void __launch_bounds__(256)
+dict_stage_kernel(const uint8_t* __restrict__ in, const uint8_t* __restrict__ dict, const zlb_dict* __restrict__ dicts,
+                  const zlb_item* __restrict__ items, const ZtsChunk* __restrict__ chunks, uint8_t* __restrict__ stage)
+{
+    const ZtsChunk ch = chunks[blockIdx.x];
+    if (!(ch.flags & CHUNK_STAGED)) return;
+    const zlb_dict d = dicts[ch.item];
+    const zlb_item it = items[ch.item];
+    const uint32_t pos = (uint32_t)(ch.in_off - it.in_off);  // < 32768
+    const uint32_t from_dict = ch.dict_len - pos;             // > 0, <= d.len
+    uint8_t* dst = stage + 16ull * ch.stage_off;
+    zts_block_copy(dst, dict + d.off + d.len - from_dict, from_dict, threadIdx.x, 256);
+    zts_block_copy(dst + from_dict, in + it.in_off, pos + ch.len, threadIdx.x, 256);
+}
+
 // ---- stored blocks (CompressionType.NONE, src/RawDeflate.ts:93-100,122-153): 65535-byte pieces ----------
 __global__ void __launch_bounds__(256)
 stored_block_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, const zlb_item* __restrict__ items,
@@ -378,9 +398,10 @@ struct HostIO {
 #define HOST_DELTA_MAX_ITEMS 256u  // per-wave output read-back is done item by item up to this many items
 
 // Runs the pipeline on device buffers. Results land in h_results after the final synchronise.
-static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const zlb_item* h_items,
-                          zlb_result* h_results, size_t n, int mode, int block_type, uint32_t chunk_bytes,
-                          uint32_t flags, HostIO* hio)
+// d_dict / h_dicts: the preset dictionaries (h_dicts == NULL: none; checked by the caller)
+static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const uint8_t* d_dict,
+                          const zlb_dict* h_dicts, const zlb_item* h_items, zlb_result* h_results, size_t n, int mode,
+                          int block_type, uint32_t chunk_bytes, uint32_t flags, HostIO* hio)
 {
     if ((mode & 0xFF) & ~(ZLB_MODE_FAST | ZLB_MODE_PRIMED | ZLB_MODE_SMALLEST | ZLB_MODE_LAZY))
         return zts_fail(ctx, ZLB_E_UNSUPPORTED, "unknown deflate mode %d", mode);
@@ -394,8 +415,10 @@ static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
     const bool lazy = fast && (mode & ZLB_MODE_LAZY) != 0;  // a fast-mode option: the exact mode is the reference's greedy parse
     if (block_type != ZLB_NONE && block_type != ZLB_FIXED && block_type != ZLB_DYNAMIC)
         return zts_fail(ctx, ZLB_E_ARG, "invalid compression type");  // src/RawDeflate.ts:110
-    // primed: history + chunk share the 64 KiB a CTA stages and indexes, so a chunk is at most 32 KiB
-    const uint32_t cb_max = primed ? ZLB_PRIMED_CHUNK : LZ_MAX_CHUNK;
+    bool any_dict = false;  // some item has a dictionary
+    for (size_t i = 0; h_dicts && i < n && !any_dict; ++i) any_dict = h_dicts[i].len != 0;
+    // primed or a dictionary: history + chunk share the 64 KiB a CTA stages and indexes, so a chunk is at most 32 KiB
+    const uint32_t cb_max = (primed || any_dict) ? ZLB_PRIMED_CHUNK : LZ_MAX_CHUNK;
     const uint32_t cb = (chunk_bytes == 0 || chunk_bytes > cb_max) ? cb_max : chunk_bytes;
     if (n > 0x7FFFFFFFull) return zts_fail(ctx, ZLB_E_ARG, "too many items");
     ctx->work = ctx->stream;
@@ -475,15 +498,25 @@ static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
     size_t wave = 0;  // the largest wave sizes the scratch sets
     for (size_t k = 0; k < n_waves; ++k)
         if (wstart[k + 1] - wstart[k] > wave) wave = wstart[k + 1] - wstart[k];
-    rc = zts_reserve_pinned(ctx, n_chunks * sizeof(ZtsChunk) + n * sizeof(uint32_t));
+    // table upload: chunks | with dictionaries: the LZ77 kernel's view of the chunks and the dictionary table |
+    // blocks per item
+    const size_t view_b = any_dict ? n_chunks * sizeof(ZtsChunk) : 0;
+    const size_t dicts_b = any_dict ? n * sizeof(zlb_dict) : 0;
+    const size_t tables_b = n_chunks * sizeof(ZtsChunk) + view_b + dicts_b + n * sizeof(uint32_t);
+    rc = zts_reserve_pinned(ctx, tables_b);
     if (rc) return rc;
     ZtsChunk* h_chunks = (ZtsChunk*)ctx->h_pin;
-    uint32_t* h_blocks = (uint32_t*)(h_chunks + n_chunks);
+    ZtsChunk* h_view = h_chunks + n_chunks;
+    if (any_dict) memcpy((uint8_t*)h_view + view_b, h_dicts, dicts_b);
+    uint32_t* h_blocks = (uint32_t*)((uint8_t*)h_view + view_b + dicts_b);
+    size_t stage_b = 0;  // staging arena of the largest wave (dictionaries)
     {
-        size_t k = 0, wk = 0;
+        size_t k = 0, wk = 0, stage_at = 0;  // stage_at: 16-byte units used by the chunk's wave so far
         for (size_t i = 0; i < n; ++i) {
             const uint64_t len = h_items[i].in_len;
             const uint64_t nc = len ? (len + cb - 1) / cb : 1;
+            // dictionary bytes a chunk can reach (an empty item has nothing to search for)
+            const uint32_t dl = (any_dict && len) ? (uint32_t)(h_dicts[i].len < LZ_WINDOW ? h_dicts[i].len : LZ_WINDOW) : 0u;
             h_blocks[i] = (uint32_t)nc;
             for (uint64_t j = 0; j < nc; ++j, ++k) {
                 ZtsChunk& c = h_chunks[k];
@@ -492,7 +525,17 @@ static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
                 c.item = (uint32_t)i;
                 c.flags = (j + 1 == nc && !(flags & ZLB_DEFLATE_NOT_FINAL)) ? CHUNK_LAST : 0u;
                 c.dict_len = primed ? (uint32_t)(j * cb < LZ_WINDOW ? j * cb : LZ_WINDOW) : 0u;
-                c.pad1 = 0;
+                c.stage_off = 0;
+                if (k >= wstart[wk + 1]) stage_at = 0;  // a new wave (the loop below moves wk on)
+                // history from the dictionary: an item's first chunk, and in primed mode every chunk in its first 32 KiB
+                if (dl && (primed || j == 0) && j * cb < LZ_WINDOW) {
+                    const uint32_t pos = (uint32_t)(j * cb);
+                    c.dict_len = dl + pos < LZ_WINDOW ? dl + pos : LZ_WINDOW;
+                    c.flags |= CHUNK_STAGED;
+                    c.stage_off = (uint32_t)stage_at;
+                    stage_at += (c.dict_len + c.len + 15u) / 16u;
+                    if (16 * stage_at > stage_b) stage_b = 16 * stage_at;
+                }
                 // first chunk of this item inside the chunk's wave
                 while (k >= wstart[wk + 1]) ++wk;
                 const size_t wave_base = wstart[wk];
@@ -506,8 +549,23 @@ static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
     // wave's LZ77 CTAs take over the SMs as the previous wave's drain (no idle tail per wave) and its small kernels
     // overlap too; only the offset scan is chained from wave to wave.
     const int n_sets = (hio && n_waves > 1) ? 2 : 1;
-    rc = zts_reserve(ctx, &ctx->d_chunks, n_chunks * sizeof(ZtsChunk) + n * sizeof(uint32_t) + 64);
+    rc = zts_reserve(ctx, &ctx->d_chunks, tables_b + 64);
     if (rc) return rc;
+    stage_b = (stage_b + 255) & ~(size_t)255;
+    if (stage_b && (rc = zts_reserve(ctx, &ctx->d_dict_stage, n_sets * stage_b + 64))) return rc;
+    if (any_dict) {
+        // The LZ77 kernel stages `in + in_off - dict_len` (the history in front of the chunk, then the chunk). Its view
+        // of a staged chunk names the chunk's place in the staging arena of the chunk's wave that way, so that the
+        // kernel itself reads windows from the arena unchanged; the other kernels keep the chunk's place in the input.
+        for (size_t k = 0, wk = 0; k < n_chunks; ++k) {
+            while (k >= wstart[wk + 1]) ++wk;
+            h_view[k] = h_chunks[k];
+            if (h_chunks[k].flags & CHUNK_STAGED) {
+                const uint64_t arena = (uint64_t)(uintptr_t)ctx->d_dict_stage.p + (n_sets == 2 ? (wk & 1) : 0) * stage_b;
+                h_view[k].in_off = arena + 16ull * h_chunks[k].stage_off + h_chunks[k].dict_len - (uint64_t)(uintptr_t)d_in;
+            }
+        }
+    }
     const size_t info_b = (wave * sizeof(ZtsChunkInfo) + 255) & ~(size_t)255;
     const size_t list_b = (wave * (size_t)LZ_LIST_PER_CHUNK * 4 + 255) & ~(size_t)255;   // token list of every chunk
     const size_t tile_b = (zts_lz77_scratch_bytes(ctx->sm_count) + 255) & ~(size_t)255;  // per-CTA tile token scratch
@@ -529,13 +587,16 @@ static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
     rc = zts_reserve(ctx, &ctx->d_misc, n * 8 + n_sets * gpos_b + 256);
     if (rc) return rc;
     ZtsChunk* d_chunks = (ZtsChunk*)ctx->d_chunks.p;
-    uint32_t* d_blocks = (uint32_t*)(d_chunks + n_chunks);
+    const ZtsChunk* d_lz_chunks = any_dict ? d_chunks + n_chunks : d_chunks;  // what the LZ77 kernel reads
+    const zlb_dict* d_dicts = (const zlb_dict*)((uint8_t*)(d_chunks + n_chunks) + view_b);
+    uint32_t* d_blocks = (uint32_t*)((uint8_t*)d_dicts + dicts_b);
     unsigned long long* d_running = (unsigned long long*)ctx->d_misc.p;
     struct Set {
         ZtsChunkInfo* info;
         uint32_t *list, *tile_tok, *hist, *sortT, *counter;
         ZtsChunkCodes* codes;
         unsigned long long* gpos;
+        uint8_t* stage;
     } sets[2];
     for (int b = 0; b < n_sets; ++b) {
         sets[b].info = (ZtsChunkInfo*)((uint8_t*)ctx->d_chunk_info.p + b * info_b);
@@ -546,9 +607,9 @@ static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
         sets[b].sortT = (uint32_t*)((uint8_t*)ctx->d_sortT.p + b * sort_b);
         sets[b].gpos = (unsigned long long*)((uint8_t*)(d_running + n) + b * gpos_b);
         sets[b].counter = (uint32_t*)(sets[b].gpos + wave);
+        sets[b].stage = stage_b ? (uint8_t*)ctx->d_dict_stage.p + b * stage_b : nullptr;
     }
-    ZTS_CUDA(ctx, cudaMemcpyAsync(d_chunks, h_chunks, n_chunks * sizeof(ZtsChunk) + n * sizeof(uint32_t),
-                                  cudaMemcpyHostToDevice, ctx->stream));
+    ZTS_CUDA(ctx, cudaMemcpyAsync(d_chunks, h_chunks, tables_b, cudaMemcpyHostToDevice, ctx->stream));
     ZTS_CUDA(ctx, cudaMemsetAsync(d_running, 0, n * 8, ctx->stream));
     ZTS_CUDA(ctx, cudaFuncSetAttribute(bitpack_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)(PACK_STAGE_WORDS * 4)));
@@ -619,7 +680,11 @@ static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
         if (n_sets == 2 && k == 1)  // the tables uploaded on ctx->stream must be there before the second stream starts
             ZTS_CUDA(ctx, cudaStreamWaitEvent(st, zts_sync_event(ctx, 4 * n_waves), 0));
         if (pipe_in) ZTS_CUDA(ctx, cudaStreamWaitEvent(st, zts_sync_event(ctx, 2 * k), 0));
-        rc = zts_lz77_launch(ctx, d_in, d_chunks + w0, wn, S.info, S.tile_tok, S.list, S.hist, S.sortT, S.counter, g, depth, lazy ? 1u : 0u);
+        if (stage_b)
+            ZTS_LAUNCH(ctx, ZK_DICT_STAGE,
+                       dict_stage_kernel<<<wn, 256, 0, st>>>(d_in, d_dict, d_dicts, d_items, d_chunks + w0, S.stage));
+        rc = zts_lz77_launch(ctx, d_in, d_lz_chunks + w0, wn, S.info, S.tile_tok, S.list, S.hist, S.sortT, S.counter, g, depth,
+                             lazy ? 1u : 0u);
         if (rc) return rc;
         rc = zts_huffman_launch(ctx, d_chunks + w0, wn, S.hist, S.info, S.codes, block_type, smallest ? 1 : 0);
         if (rc) return rc;
@@ -673,29 +738,49 @@ static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
     return ZLB_OK;
 }
 
+extern "C" int zlb_deflate_batch_dict(zlb_ctx* ctx, const void* d_in, void* d_out, const void* d_dict,
+                                      const zlb_dict* dicts, const zlb_item* items, zlb_result* results, size_t n,
+                                      int mode, int block_type, uint32_t chunk_bytes, uint32_t flags)
+{
+    if (!ctx || (!items && n) || (!results && n) || (!d_out && n)) return ZLB_E_ARG;
+    if (n == 0) return ZLB_OK;
+    bool any = false;
+    int rc = zts_check_dicts(ctx, d_dict, SIZE_MAX, dicts, n, &any);
+    if (rc) return rc;
+    ZTS_CUDA(ctx, cudaSetDevice(ctx->device));
+    return deflate_device(ctx, (const uint8_t*)d_in, (uint8_t*)d_out, (const uint8_t*)d_dict, any ? dicts : nullptr,
+                          items, results, n, mode, block_type, chunk_bytes, flags, nullptr);
+}
+
 extern "C" int zlb_deflate_batch(zlb_ctx* ctx, const void* d_in, void* d_out, const zlb_item* items,
                                  zlb_result* results, size_t n, int mode, int block_type, uint32_t chunk_bytes,
                                  uint32_t flags)
 {
-    if (!ctx || (!items && n) || (!results && n) || (!d_out && n)) return ZLB_E_ARG;
-    if (n == 0) return ZLB_OK;
-    ZTS_CUDA(ctx, cudaSetDevice(ctx->device));
-    return deflate_device(ctx, (const uint8_t*)d_in, (uint8_t*)d_out, items, results, n, mode, block_type,
-                          chunk_bytes, flags, nullptr);
+    return zlb_deflate_batch_dict(ctx, d_in, d_out, nullptr, nullptr, items, results, n, mode, block_type, chunk_bytes,
+                                  flags);
 }
 
-extern "C" int zlb_deflate_batch_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes, void* h_out, size_t out_bytes,
-                                      const zlb_item* items, zlb_result* results, size_t n, int mode, int block_type,
-                                      uint32_t chunk_bytes, uint32_t flags)
+extern "C" int zlb_deflate_batch_dict_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes, void* h_out,
+                                           size_t out_bytes, const void* h_dict, size_t dict_bytes,
+                                           const zlb_dict* dicts, const zlb_item* items, zlb_result* results, size_t n,
+                                           int mode, int block_type, uint32_t chunk_bytes, uint32_t flags)
 {
     if (!ctx || (!items && n) || (!results && n) || (!h_in && in_bytes) || (!h_out && out_bytes)) return ZLB_E_ARG;
     if (n == 0) return ZLB_OK;
+    bool any = false;
+    int rc = zts_check_dicts(ctx, h_dict, dict_bytes, dicts, n, &any);
+    if (rc) return rc;
     ZTS_CUDA(ctx, cudaSetDevice(ctx->device));
     for (size_t i = 0; i < n; ++i) {
         if (items[i].in_off + items[i].in_len > in_bytes || items[i].out_off + items[i].out_cap > out_bytes)
             return zts_fail(ctx, ZLB_E_ARG, "item %zu out of range", i);
     }
-    int rc = zts_reserve(ctx, &ctx->d_stage_in, in_bytes + 256);
+    // the dictionaries go over first, on the context's stream (everything of the call is ordered behind it)
+    if (any) {
+        if ((rc = zts_reserve(ctx, &ctx->d_dict, dict_bytes + 256))) return rc;
+        ZTS_CUDA(ctx, cudaMemcpyAsync(ctx->d_dict.p, h_dict, dict_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    }
+    rc = zts_reserve(ctx, &ctx->d_stage_in, in_bytes + 256);
     if (rc) return rc;
     rc = zts_reserve(ctx, &ctx->d_stage_out, out_bytes + 256);
     if (rc) return rc;
@@ -703,8 +788,9 @@ extern "C" int zlb_deflate_batch_host(zlb_ctx* ctx, const void* h_in, size_t in_
     rc = zts_stage_begin(ctx, h_in, in_bytes, h_out, out_bytes, &stage);
     if (!rc) {
         HostIO hio = {zts_stage_in_ptr(stage), zts_stage_out_ptr(stage), in_bytes, out_bytes, false, stage};
-        rc = deflate_device(ctx, (const uint8_t*)ctx->d_stage_in.p, (uint8_t*)ctx->d_stage_out.p, items, results, n, mode,
-                            block_type, chunk_bytes, flags, &hio);
+        rc = deflate_device(ctx, (const uint8_t*)ctx->d_stage_in.p, (uint8_t*)ctx->d_stage_out.p,
+                            (const uint8_t*)ctx->d_dict.p, any ? dicts : nullptr, items, results, n, mode, block_type,
+                            chunk_bytes, flags, &hio);
         if (!rc && !hio.out_done) {
             // many items: what each of them wrote, adjacent ranges merged
             rc = zts_copy_back(ctx, stage, ctx->stream, (const uint8_t*)ctx->d_stage_out.p, hio.h_out, items, results,
@@ -714,6 +800,14 @@ extern "C" int zlb_deflate_batch_host(zlb_ctx* ctx, const void* h_in, size_t in_
     }
     zts_stage_end(ctx, stage);  // also on errors: the copy threads hold pointers into the caller's buffers
     return rc;
+}
+
+extern "C" int zlb_deflate_batch_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes, void* h_out, size_t out_bytes,
+                                      const zlb_item* items, zlb_result* results, size_t n, int mode, int block_type,
+                                      uint32_t chunk_bytes, uint32_t flags)
+{
+    return zlb_deflate_batch_dict_host(ctx, h_in, in_bytes, h_out, out_bytes, nullptr, 0, nullptr, items, results, n, mode,
+                                       block_type, chunk_bytes, flags);
 }
 
 // ---- test hooks ---------------------------------------------------------------------------------------

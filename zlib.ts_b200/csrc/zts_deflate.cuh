@@ -24,6 +24,7 @@
 #define ZTS_HDR_STORED 0xFFFFFFFFu       // ZtsChunkInfo.hdr_bits of a chunk written as stored block(s)
 
 #define CHUNK_LAST 1u                   // last chunk of its item: BFINAL = 1, no join marker
+#define CHUNK_STAGED 2u                 // history || chunk is put together in the staging arena (dict_stage_kernel)
 
 struct ZtsChunk {      // host-built, one per chunk
     uint64_t in_off;   // absolute offset of the chunk in d_in
@@ -31,8 +32,9 @@ struct ZtsChunk {      // host-built, one per chunk
     uint32_t item;
     uint32_t seg_first;  // index (within the wave) of the first chunk of the same item
     uint32_t flags;
-    uint32_t dict_len;   // primed mode: bytes in front of the chunk (same item, <= 32768) the match search may reach into
-    uint32_t pad1;
+    uint32_t dict_len;   // bytes of history in front of the chunk (<= 32768) the match search may reach into: the same
+                         // item's (primed mode) and / or a preset dictionary's
+    uint32_t stage_off;  // CHUNK_STAGED: the window's offset in the staging arena, in 16-byte units
 };
 
 // first position of tile t (t == LZ_NTILES gives the chunk size)

@@ -332,17 +332,22 @@ __device__ uint32_t inf_classify_symbols(const InfWarpSmem* S, const uint8_t* sr
     return ZLB_ST_INPUT_BROKEN;
 }
 
-// WINDOW = false: the decoder. WINDOW = true: the window mode of the marker split (see there): the output is one 16-bit
-// word per byte, out_off / out_cap count bytes / words, and the 32768 words in front of out_off belong to the item as
-// well -- the kernel fills them with 0x8000 | w, "byte w of the window" (the 32 KiB of output in front of the piece),
-// so that the copy code below is the same for both: a match that reaches before the piece copies window words.
+// INF_BYTES: the decoder. INF_WINDOW: the window mode of the marker split (see there): the output is one 16-bit word per
+// byte, out_off / out_cap count bytes / words, and the 32768 words in front of out_off belong to the item as well -- the
+// kernel fills them with 0x8000 | w, "byte w of the window" (the 32 KiB of output in front of the piece), so that the
+// copy code below is the same for both: a match that reaches before the piece copies window words. INF_DICT: the
+// decoder with a preset dictionary (dicts[item] in the blob `dict`, zlb_inflate_batch_dict): a match may reach up to
+// the dictionary's last 32768 bytes in front of the output; one whose source starts there takes a path of its own.
+// The dictionary arguments are read by INF_DICT only.
 #define WIN_WORDS 32768u
-template <bool WINDOW>
+enum { INF_BYTES = 0, INF_WINDOW = 1, INF_DICT = 2 };
+template <int MODE>
 __global__ void __launch_bounds__(INF_WARPS_PER_CTA * 32, INF_MIN_CTAS)
 inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, const zlb_item* __restrict__ items,
-                    zlb_result* __restrict__ results, uint32_t n_items, uint32_t flags)
+                    zlb_result* __restrict__ results, uint32_t n_items, uint32_t flags,
+                    const zlb_dict* __restrict__ dicts, const uint8_t* __restrict__ dict)
 {
-    using T = typename std::conditional<WINDOW, uint16_t, uint8_t>::type;
+    using T = typename std::conditional<MODE == INF_WINDOW, uint16_t, uint8_t>::type;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const unsigned lane = zts_lane();
     const unsigned warp = threadIdx.x >> 5;
@@ -353,7 +358,14 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
     const zlb_item it = items[item];
     const uint8_t* src = in + it.in_off;
     T* dst = reinterpret_cast<T*>(out + it.out_off);
-    if constexpr (WINDOW) {
+    uint32_t reach = MODE == INF_WINDOW ? WIN_WORDS : 0u;  // how far a distance may reach in front of the output
+    const uint8_t* dtail = nullptr;                       // INF_DICT: the `reach` bytes in front of the output
+    if constexpr (MODE == INF_DICT) {
+        const zlb_dict d = dicts[item];
+        reach = d.len < WIN_WORDS ? (uint32_t)d.len : WIN_WORDS;
+        dtail = dict + d.off + d.len - reach;
+    }
+    if constexpr (MODE == INF_WINDOW) {
         uint4* w = reinterpret_cast<uint4*>(dst - WIN_WORDS);  // (slots are 256-byte aligned)
         for (uint32_t i = lane; i < WIN_WORDS / 8; i += 32) {
             const uint32_t a = 0x80008000u | (8u * i) | ((8u * i + 1u) << 16);
@@ -642,7 +654,7 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
             const uint32_t room = cap - op > 0x00FFFFFFull ? 0x00FFFFFFu : (uint32_t)(cap - op);  // (op <= cap always)
             // a distance beyond the start of the output (the reference would copy `undefined` -> 0) or an
             // output slot that is too small ends the batch before the offending token
-            const bool bad_dist = is_match && dist > behind + rel + (WINDOW ? WIN_WORDS : 0u);
+            const bool bad_dist = is_match && dist > behind + rel + reach;
             const bool over = mine && rel + len > room;
             const unsigned bad_mask = __ballot_sync(0xFFFFFFFFu, bad_dist || over);
             uint32_t nvalid = ntok;
@@ -653,7 +665,7 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
             }
             const bool live = lane < nvalid;
             // -- literals: one store
-            ZTS_ASSERT(!live || (op + rel + len <= cap && (!is_match || dist <= op + rel + (WINDOW ? WIN_WORDS : 0u))));
+            ZTS_ASSERT(!live || (op + rel + len <= cap && (!is_match || dist <= op + rel + reach)));
             if (live && !is_match) bdst[rel] = (uint8_t)(mytok >> 16);
             __syncwarp();  // (a match may read the literals of its own batch)
             // -- matches, sub-batch by sub-batch: a sub-batch ends in front of the first match that reads what a match
@@ -671,7 +683,7 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
                 const unsigned dep_mask = __ballot_sync(0xFFFFFFFFu, dep);
                 const uint32_t cut = dep_mask ? (uint32_t)__ffs((int)dep_mask) - 1u : 32u;  // behind the first match always
                 const bool in_sub = live && is_match && lane >= start && lane < cut;
-                const bool small = in_sub && len <= 8u && dist >= len;
+                const bool small = in_sub && len <= 8u && dist >= len && (MODE != INF_DICT || dist <= behind + rel);
                 if (__any_sync(0xFFFFFFFFu, small)) {
                     // short non-overlapping matches: every lane copies its own, loads first, then stores
                     T v[8];
@@ -692,7 +704,19 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
                     const uint32_t jr = __shfl_sync(0xFFFFFFFFu, rel, j);
                     T* o = bdst + jr;
                     const T* s0 = o - jd;
-                    if (jd >= jl) {
+                    if (MODE == INF_DICT && jd > behind + jr) {
+                        // the source starts in the dictionary (then behind == op): byte k is byte
+                        // op + jr - jd + (k mod jd) of dictionary || output, which lies in front of the match
+                        const int x0 = (int)(behind + jr) - (int)jd;
+                        uint32_t r = lane % jd;
+                        const uint32_t step = 32u % jd;
+                        for (uint32_t k = lane; k < jl; k += 32) {
+                            const int x = x0 + (int)r;
+                            o[k] = x < 0 ? dtail[(int)reach + x] : dst[x];
+                            r += step;
+                            if (r >= jd) r -= jd;
+                        }
+                    } else if (jd >= jl) {
                         for (uint32_t k = lane; k < jl; k += 32) o[k] = s0[k];
                     } else {
                         // periodic source: byte k comes from s0[k mod dist]
@@ -726,17 +750,26 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
     }
 }
 
-template <bool WINDOW = false>
-static int inflate_launch(zlb_ctx* ctx, cudaStream_t st, const uint8_t* d_in, uint8_t* d_out, const zlb_item* d_items,
-                          zlb_result* d_results, size_t n, uint32_t flags)
+template <int MODE>
+static int inflate_launch_mode(zlb_ctx* ctx, cudaStream_t st, const uint8_t* d_in, uint8_t* d_out, const zlb_item* d_items,
+                               zlb_result* d_results, size_t n, uint32_t flags, const zlb_dict* d_dicts,
+                               const uint8_t* d_dict)
 {
     const size_t smem = sizeof(InfWarpSmem) * INF_WARPS_PER_CTA;
-    ZTS_CUDA(ctx, cudaFuncSetAttribute(inflate_warp_kernel<WINDOW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    ZTS_CUDA(ctx, cudaFuncSetAttribute(inflate_warp_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     unsigned grid = (unsigned)((n + INF_WARPS_PER_CTA - 1) / INF_WARPS_PER_CTA);
-    ZTS_LAUNCH(ctx, WINDOW ? ZK_INFLATE_WINDOW : ZK_INFLATE,
-               inflate_warp_kernel<WINDOW><<<grid, INF_WARPS_PER_CTA * 32, smem, st>>>(d_in, d_out, d_items, d_results,
-                                                                                      (uint32_t)n, flags));
+    ZTS_LAUNCH(ctx, MODE == INF_WINDOW ? ZK_INFLATE_WINDOW : MODE == INF_DICT ? ZK_INFLATE_DICT : ZK_INFLATE,
+               inflate_warp_kernel<MODE><<<grid, INF_WARPS_PER_CTA * 32, smem, st>>>(d_in, d_out, d_items, d_results,
+                                                                                    (uint32_t)n, flags, d_dicts, d_dict));
     return ZLB_OK;
+}
+// the decoder: with a dictionary table (d_dicts[i] belongs to d_items[i]) the dictionary instantiation
+static int inflate_launch(zlb_ctx* ctx, cudaStream_t st, const uint8_t* d_in, uint8_t* d_out, const zlb_item* d_items,
+                          zlb_result* d_results, size_t n, uint32_t flags, const zlb_dict* d_dicts = nullptr,
+                          const uint8_t* d_dict = nullptr)
+{
+    if (d_dicts) return inflate_launch_mode<INF_DICT>(ctx, st, d_in, d_out, d_items, d_results, n, flags, d_dicts, d_dict);
+    return inflate_launch_mode<INF_BYTES>(ctx, st, d_in, d_out, d_items, d_results, n, flags, nullptr, nullptr);
 }
 
 // ---- marker split (ZLB_INFLATE_SPLIT) ------------------------------------------------------------------------
@@ -819,6 +852,8 @@ struct ZtsWinRun {
 };
 struct ZtsWinItem {
     uint32_t first_run, runs;
+    const uint8_t* dict;  // W_0: the last dict_len (<= 32768) bytes of the item's preset dictionary (none: 0)
+    uint32_t dict_len, pad;
 };
 #define WIN_THREADS 1024
 #define WIN_SMEM (2u * WIN_WORDS * 2u)  // the map being composed and the next one
@@ -871,7 +906,8 @@ window_run_kernel(const uint8_t* __restrict__ arena, const ZtsWinPiece* __restri
     win_copy(agg + (size_t)blockIdx.x * WIN_WORDS, E);
 }
 
-// prefix of every run of item i: the window in front of the run's first piece in terms of W_0
+// prefix of every run of item i: the window in front of the run's first piece in terms of W_0. With a preset
+// dictionary W_0 is known in part: its last dict_len words are the dictionary's bytes, the scan starts from that map.
 __global__ void __launch_bounds__(WIN_THREADS)
 window_scan_kernel(const ZtsWinItem* __restrict__ items, const uint16_t* __restrict__ agg, uint16_t* __restrict__ prefix)
 {
@@ -879,6 +915,10 @@ window_scan_kernel(const ZtsWinItem* __restrict__ items, const uint16_t* __restr
     uint16_t *E = wmap, *En = wmap + WIN_WORDS;
     const ZtsWinItem it = items[blockIdx.x];
     win_identity(E);
+    if (it.dict_len) {
+        for (uint32_t i = threadIdx.x; i < it.dict_len; i += WIN_THREADS) E[WIN_WORDS - it.dict_len + i] = it.dict[i];
+        __syncthreads();
+    }
     for (uint32_t r = it.first_run; r < it.first_run + it.runs; ++r) {
         win_copy(prefix + (size_t)r * WIN_WORDS, E);
         if (r + 1 < it.first_run + it.runs) {
@@ -940,16 +980,17 @@ struct SplitPiece {
 };
 
 // The chain checks of the pieces r[0 .. n) of an item: each one decoded cleanly, ended exactly where the next one
-// starts, and only the last one saw BFINAL. With `window`, a piece behind the first that stopped at an undefined code
-// or distance may have reached before its first byte: SPLIT_WINDOW says window mode may still decode the item.
+// starts, and only the last one saw BFINAL. With `window`, a piece behind the first (or the first too, when the item
+// has a preset dictionary: `dict`) that stopped at an undefined code or distance may have reached before its first
+// byte: SPLIT_WINDOW says window mode may still decode the item.
 enum { SPLIT_BAD = 0, SPLIT_OK = 1, SPLIT_WINDOW = 2 };
-static int split_chain(const zlb_result* r, const zlb_item* seg, size_t n, bool window)
+static int split_chain(const zlb_result* r, const zlb_item* seg, size_t n, bool window, bool dict)
 {
     bool reaches = false;
     for (size_t j = 0; j < n; ++j) {
         const bool last = j + 1 == n;
         const bool fin = (r[j].blocks & 0x80000000u) != 0;
-        if (window && j > 0 && r[j].status == ZLB_ST_BAD_CODE) {
+        if (window && (j > 0 || dict) && r[j].status == ZLB_ST_BAD_CODE) {
             reaches = true;
             continue;
         }
@@ -983,8 +1024,10 @@ static void split_finish(const zlb_item& it, const zlb_result* r, const zlb_item
 }
 
 // Window mode for the items big[cand[*]] (pieces as laid out by inflate_split_batch, byte slots at seg[j].out_off of
-// d_scratch): all of them in one decode launch and one scan; done[k] / res[k] / gath as there.
+// d_scratch): all of them in one decode launch and one scan; done[k] / res[k] / gath as there. h_dicts / d_dict: the
+// preset dictionaries of h_items (NULL: none).
 static int inflate_split_window(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_scratch, const zlb_item* h_items,
+                                const zlb_dict* h_dicts, const uint8_t* d_dict,
                                 const std::vector<size_t>& big, uint32_t flags, const std::vector<SplitPiece>& pieces,
                                 const std::vector<size_t>& first, const std::vector<zlb_item>& seg,
                                 const std::vector<size_t>& cand, std::vector<zlb_result>& res, std::vector<char>& done,
@@ -1065,7 +1108,8 @@ static int inflate_split_window(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_sc
         }
     ZTS_CUDA(ctx, cudaMemcpyAsync(d_wseg, wseg.data(), np * sizeof(zlb_item), cudaMemcpyHostToDevice, st));
     ZTS_CUDA(ctx, cudaMemsetAsync(d_wres, 0, np * sizeof(zlb_result), st));
-    rc = inflate_launch<true>(ctx, st, d_in, arena, d_wseg, d_wres, np, (flags & ZLB_INFLATE_CHECK_NLEN) | ZLB_INFLATE_SEGMENT);
+    rc = inflate_launch_mode<INF_WINDOW>(ctx, st, d_in, arena, d_wseg, d_wres, np,
+                                         (flags & ZLB_INFLATE_CHECK_NLEN) | ZLB_INFLATE_SEGMENT, nullptr, nullptr);
     if (rc) return rc;
     std::vector<zlb_result> wres(np);
     ZTS_CUDA(ctx, cudaMemcpyAsync(wres.data(), d_wres, np * sizeof(zlb_result), cudaMemcpyDeviceToHost, st));
@@ -1079,9 +1123,11 @@ static int inflate_split_window(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_sc
         const size_t k = take[t], a = first[k], n = first[k + 1] - a;
         const size_t w0 = wj;
         wj += n;
-        if (split_chain(&wres[w0], &seg[a], n, false) != SPLIT_OK) continue;
+        if (split_chain(&wres[w0], &seg[a], n, false, false) != SPLIT_OK) continue;
         const size_t g = run_len(n);
-        witems.push_back({(uint32_t)runs.size(), (uint32_t)((n + g - 1) / g)});
+        const zlb_dict d = h_dicts ? h_dicts[big[k]] : zlb_dict{0, 0};
+        const uint32_t dl = d.len < WIN_WORDS ? (uint32_t)d.len : WIN_WORDS;
+        witems.push_back({(uint32_t)runs.size(), (uint32_t)((n + g - 1) / g), dl ? d_dict + d.off + d.len - dl : nullptr, dl, 0u});
         for (size_t s = 0; s < n; s += g)
             runs.push_back({(uint32_t)(wp.size() + s), (uint32_t)std::min(g, n - s), (uint32_t)wk.size(), 0u});
         for (size_t j = 0; j < n; ++j)
@@ -1123,8 +1169,8 @@ static int inflate_split_window(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_sc
 // is filled); the others have to go through the serial decoder. < 0 on API errors.
 #define SPLIT_TAG_SHIFT 40  // marks carry the item's index above the byte offset (offsets < 1 TiB, < 16 M large items)
 static int inflate_split_batch(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const zlb_item* h_items,
-                               const std::vector<size_t>& big, uint32_t flags, std::vector<zlb_result>& res,
-                               std::vector<char>& done)
+                               const zlb_dict* h_dicts, const uint8_t* d_dict, const std::vector<size_t>& big,
+                               uint32_t flags, std::vector<zlb_result>& res, std::vector<char>& done)
 {
     const size_t nb = big.size();
     res.assign(nb, zlb_result());
@@ -1231,14 +1277,15 @@ static int inflate_split_batch(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out
     for (size_t k = 0; k < nb; ++k) {
         const size_t a = first[k], b = first[k + 1];
         if (b - a < 2) continue;
-        const int chain = split_chain(&sres[a], &seg[a], b - a, true);
+        const int chain = split_chain(&sres[a], &seg[a], b - a, true, h_dicts && h_dicts[big[k]].len);
         if (chain == SPLIT_WINDOW) window.push_back(k);
         if (chain != SPLIT_OK) continue;
         split_finish(h_items[big[k]], &sres[a], &seg[a], b - a, pieces[b - 1].start, res[k], gath);
         done[k] = 1;
     }
     if (!window.empty()) {
-        rc = inflate_split_window(ctx, d_in, d_scratch, h_items, big, flags, pieces, first, seg, window, res, done, gath);
+        rc = inflate_split_window(ctx, d_in, d_scratch, h_items, h_dicts, d_dict, big, flags, pieces, first, seg, window, res,
+                                  done, gath);
         if (rc) return rc;
     }
     if (!gath.empty()) {
@@ -1259,11 +1306,19 @@ struct InfHostIO {
     ZtsHostStage* stage;   // copy threads behind the shadows (pageable caller buffers), see zts_hoststage.cu
 };
 
-static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const zlb_item* h_items,
-                          zlb_result* h_results, size_t n, uint32_t flags, const InfHostIO* hio)
+// d_dict / h_dicts: the preset dictionaries (h_dicts == NULL: none; checked by the caller)
+static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const uint8_t* d_dict,
+                          const zlb_dict* h_dicts, const zlb_item* h_items, zlb_result* h_results, size_t n, uint32_t flags,
+                          const InfHostIO* hio)
 {
     int rc = zts_reserve(ctx, &ctx->d_items, n * sizeof(zlb_item) + 64);
     if (rc) return rc;
+    const zlb_dict* d_dicts = nullptr;  // the dictionary table on the device, beside the item table
+    if (h_dicts) {
+        if ((rc = zts_reserve(ctx, &ctx->d_dict_stage, n * sizeof(zlb_dict) + 64))) return rc;
+        d_dicts = (const zlb_dict*)ctx->d_dict_stage.p;
+        ZTS_CUDA(ctx, cudaMemcpyAsync((void*)d_dicts, h_dicts, n * sizeof(zlb_dict), cudaMemcpyHostToDevice, ctx->stream));
+    }
     rc = zts_reserve(ctx, &ctx->d_results, n * sizeof(zlb_result) + 64);
     if (rc) return rc;
     zlb_item* d_items = (zlb_item*)ctx->d_items.p;
@@ -1286,12 +1341,13 @@ static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
                 ZTS_CUDA(ctx, cudaMemcpyAsync((void*)d_in, hio->h_in, hio->in_bytes, cudaMemcpyHostToDevice, ctx->stream));
             }
             std::vector<zlb_item> rest_items;
+            std::vector<zlb_dict> rest_dicts;
             std::vector<size_t> rest_idx;
             std::vector<char> is_done(n, 0);
             {
                 std::vector<zlb_result> bres;
                 std::vector<char> bdone;
-                rc = inflate_split_batch(ctx, d_in, d_out, h_items, big, flags, bres, bdone);
+                rc = inflate_split_batch(ctx, d_in, d_out, h_items, h_dicts, d_dict, big, flags, bres, bdone);
                 if (rc) return rc;
                 bool any = false;
                 for (size_t k = 0; k < big.size(); ++k)
@@ -1306,18 +1362,22 @@ static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
             for (size_t i = 0; i < n; ++i)
                 if (!is_done[i]) {
                     rest_items.push_back(h_items[i]);
+                    if (h_dicts) rest_dicts.push_back(h_dicts[i]);
                     rest_idx.push_back(i);
                 }
             if (!rest_items.empty()) {
                 // the remaining items in one batch; their results are scattered back to their slots
                 const size_t m = rest_items.size();
-                rc = zts_reserve(ctx, &ctx->d_sums, m * (sizeof(zlb_item) + sizeof(zlb_result)) + 256);
+                rc = zts_reserve(ctx, &ctx->d_sums, m * (sizeof(zlb_item) + sizeof(zlb_result) + sizeof(zlb_dict)) + 256);
                 if (rc) return rc;
                 zlb_item* d_ri = (zlb_item*)ctx->d_sums.p;
                 zlb_result* d_rr = (zlb_result*)(d_ri + m);
+                zlb_dict* d_rd = h_dicts ? (zlb_dict*)(d_rr + m) : nullptr;
                 ZTS_CUDA(ctx, cudaMemcpyAsync(d_ri, rest_items.data(), m * sizeof(zlb_item), cudaMemcpyHostToDevice, ctx->stream));
                 ZTS_CUDA(ctx, cudaMemsetAsync(d_rr, 0, m * sizeof(zlb_result), ctx->stream));
-                rc = inflate_launch(ctx, ctx->stream, d_in, d_out, d_ri, d_rr, m, flags & ~(uint32_t)ZLB_INFLATE_SPLIT);
+                if (d_rd)
+                    ZTS_CUDA(ctx, cudaMemcpyAsync(d_rd, rest_dicts.data(), m * sizeof(zlb_dict), cudaMemcpyHostToDevice, ctx->stream));
+                rc = inflate_launch(ctx, ctx->stream, d_in, d_out, d_ri, d_rr, m, flags & ~(uint32_t)ZLB_INFLATE_SPLIT, d_rd, d_dict);
                 if (rc) return rc;
                 std::vector<zlb_result> rr(m);
                 ZTS_CUDA(ctx, cudaMemcpyAsync(rr.data(), d_rr, m * sizeof(zlb_result), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1349,7 +1409,7 @@ static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
                 n_waves = 1;
     }
     if (!hio) {
-        rc = inflate_launch(ctx, ctx->stream, d_in, d_out, d_items, d_results, n, flags);
+        rc = inflate_launch(ctx, ctx->stream, d_in, d_out, d_items, d_results, n, flags, d_dicts, d_dict);
         if (rc) return rc;
         if (kinds) {
             rc = zts_checksum_device(ctx, d_out, d_items, d_results, h_items, n, kinds, 1);
@@ -1427,7 +1487,8 @@ static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
         ZTS_CUDA(ctx, cudaStreamWaitEvent(st, zts_sync_event(ctx, 1 + 2 * k), 0));
         if (a < b) {
             ctx->work = st;
-            rc = inflate_launch(ctx, st, d_in, d_out, d_items + a, d_results + a, b - a, flags);
+            rc = inflate_launch(ctx, st, d_in, d_out, d_items + a, d_results + a, b - a, flags, d_dicts ? d_dicts + a : nullptr,
+                                d_dict);
             ctx->work = ctx->stream;
             if (rc) return rc;
             if (kinds) {
@@ -1452,31 +1513,52 @@ static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
     return ZLB_OK;
 }
 
-extern "C" int zlb_inflate_batch(zlb_ctx* ctx, const void* d_in, void* d_out, const zlb_item* items,
-                                 zlb_result* results, size_t n, uint32_t flags)
+extern "C" int zlb_inflate_batch_dict(zlb_ctx* ctx, const void* d_in, void* d_out, const void* d_dict,
+                                      const zlb_dict* dicts, const zlb_item* items, zlb_result* results, size_t n,
+                                      uint32_t flags)
 {
     if (!ctx || (!items && n) || (!results && n) || (!d_in && n) || (!d_out && n)) return ZLB_E_ARG;
     if (n == 0) return ZLB_OK;
     if (n > 0x7FFFFFFFull) return zts_fail(ctx, ZLB_E_ARG, "too many items");
+    bool any = false;
+    int rc = zts_check_dicts(ctx, d_dict, SIZE_MAX, dicts, n, &any);
+    if (rc) return rc;
     ZTS_CUDA(ctx, cudaSetDevice(ctx->device));
-    int rc = inflate_device(ctx, (const uint8_t*)d_in, (uint8_t*)d_out, items, results, n, flags, nullptr);
+    rc = inflate_device(ctx, (const uint8_t*)d_in, (uint8_t*)d_out, (const uint8_t*)d_dict, any ? dicts : nullptr, items,
+                        results, n, flags, nullptr);
     if (rc) return rc;
     ZTS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return ZLB_OK;
 }
 
-extern "C" int zlb_inflate_batch_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes, void* h_out, size_t out_bytes,
-                                      const zlb_item* items, zlb_result* results, size_t n, uint32_t flags)
+extern "C" int zlb_inflate_batch(zlb_ctx* ctx, const void* d_in, void* d_out, const zlb_item* items,
+                                 zlb_result* results, size_t n, uint32_t flags)
+{
+    return zlb_inflate_batch_dict(ctx, d_in, d_out, nullptr, nullptr, items, results, n, flags);
+}
+
+extern "C" int zlb_inflate_batch_dict_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes, void* h_out,
+                                           size_t out_bytes, const void* h_dict, size_t dict_bytes,
+                                           const zlb_dict* dicts, const zlb_item* items, zlb_result* results, size_t n,
+                                           uint32_t flags)
 {
     if (!ctx || (!items && n) || (!results && n) || (!h_in && in_bytes) || (!h_out && out_bytes)) return ZLB_E_ARG;
     if (n == 0) return ZLB_OK;
     if (n > 0x7FFFFFFFull) return zts_fail(ctx, ZLB_E_ARG, "too many items");
+    bool any = false;
+    int rc = zts_check_dicts(ctx, h_dict, dict_bytes, dicts, n, &any);
+    if (rc) return rc;
     ZTS_CUDA(ctx, cudaSetDevice(ctx->device));
     for (size_t i = 0; i < n; ++i) {
         if (items[i].in_off + items[i].in_len > in_bytes || items[i].out_off + items[i].out_cap > out_bytes)
             return zts_fail(ctx, ZLB_E_ARG, "item %zu out of range", i);
     }
-    int rc = zts_reserve(ctx, &ctx->d_stage_in, in_bytes + 256);
+    // the dictionaries go over first, on the context's stream (every stream of the call starts behind it)
+    if (any) {
+        if ((rc = zts_reserve(ctx, &ctx->d_dict, dict_bytes + 256))) return rc;
+        ZTS_CUDA(ctx, cudaMemcpyAsync(ctx->d_dict.p, h_dict, dict_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    }
+    rc = zts_reserve(ctx, &ctx->d_stage_in, in_bytes + 256);
     if (rc) return rc;
     rc = zts_reserve(ctx, &ctx->d_stage_out, out_bytes + 256);
     if (rc) return rc;
@@ -1484,10 +1566,17 @@ extern "C" int zlb_inflate_batch_host(zlb_ctx* ctx, const void* h_in, size_t in_
     rc = zts_stage_begin(ctx, h_in, in_bytes, h_out, out_bytes, &stage);
     if (!rc) {
         InfHostIO hio = {zts_stage_in_ptr(stage), zts_stage_out_ptr(stage), in_bytes, out_bytes, stage};
-        rc = inflate_device(ctx, (const uint8_t*)ctx->d_stage_in.p, (uint8_t*)ctx->d_stage_out.p, items, results, n, flags,
-                            &hio);
+        rc = inflate_device(ctx, (const uint8_t*)ctx->d_stage_in.p, (uint8_t*)ctx->d_stage_out.p,
+                            (const uint8_t*)ctx->d_dict.p, any ? dicts : nullptr, items, results, n, flags, &hio);
         if (!rc && cudaStreamSynchronize(ctx->stream) != cudaSuccess) rc = zts_fail(ctx, ZLB_E_CUDA, "synchronize failed");
     }
     zts_stage_end(ctx, stage);  // also on errors: the copy threads hold pointers into the caller's buffers
     return rc;
+}
+
+extern "C" int zlb_inflate_batch_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes, void* h_out, size_t out_bytes,
+                                      const zlb_item* items, zlb_result* results, size_t n, uint32_t flags)
+{
+    return zlb_inflate_batch_dict_host(ctx, h_in, in_bytes, h_out, out_bytes, nullptr, 0, nullptr, items, results, n,
+                                       flags);
 }
