@@ -304,37 +304,68 @@ def test_compat_streams_keep_todays_route(engine):
 
 
 def test_host_entry_point_pinned_and_pageable(engine):
+    """The host entry point on a mixed batch -- large primed, compat, Z_SYNC_FLUSH and invalid items beside a few
+    thousand small streams -- without and with dictionaries, through page-locked and pageable buffers: the same results
+    and the same bytes, the slack included, as the call without INFLATE_SPLIT."""
     import zlibts_b200 as z
     from zlibts_b200 import synth
-    datas = [synth.text(3 << 20, 41).tobytes(), synth.mixed(5 << 20, 42).tobytes()]
-    streams = [_gpu_deflate(engine, datas[0], z.MODE_PRIMED), _sync_flushed(datas[1], 50000)]
-    blob, offs, lens = pack(streams)
-    caps = [len(d) for d in datas]
-    items = z.make_items(2)
-    items["in_off"], items["in_len"] = offs, lens
-    items["out_off"], items["out_cap"] = [0, caps[0]], caps
-    flags = z.INFLATE_SPLIT | z.INFLATE_WANT_CRC32 | z.INFLATE_WANT_ADLER32
-    for pinned in (True, False):
-        if pinned:
-            h_in, h_out = z.host_alloc(blob.size), z.host_alloc(sum(caps))
-            h_in[:] = blob
-        else:
-            h_in, h_out = blob.copy(), np.zeros(sum(caps), dtype=np.uint8)
-        engine.profile_enable(True)
-        engine.profile_reset()
-        try:
-            res = engine.inflate_batch_host(h_in, h_out, items, flags)
-            prof = engine.profile_read()
-        finally:
-            engine.profile_enable(False)
-        assert all(prof[k]["launches"] > 0 for k in WINDOW_KERNELS), prof
-        assert h_out[:caps[0]].tobytes() == datas[0] and h_out[caps[0]:].tobytes() == datas[1]
-        for d, s, r in zip(datas, streams, res):
-            assert int(r["status"]) == 0 and int(r["out_len"]) == len(d) and int(r["in_used"]) == len(s)
-            assert int(r["crc32"]) == zlib.crc32(d) and int(r["adler32"]) == zlib.adler32(d)
-        if pinned:
-            z.host_free(h_in)
-            z.host_free(h_out)
+    rng = np.random.default_rng(43)
+    zd = synth.text(32768, 40).tobytes()
+    big = [synth.text(3 << 20, 41).tobytes(), synth.mixed(4 << 20, 44).tobytes(), synth.mixed(5 << 20, 42).tobytes()]
+    small = [synth.text(int(n), 1000 + k).tobytes() for k, n in enumerate(rng.integers(1, 3000, 3000))]
+    fixed = [_gpu_deflate(engine, big[0], z.MODE_PRIMED), _gpu_deflate(engine, big[1], z.MODE_COMPAT)]
+    base = z.INFLATE_WANT_CRC32 | z.INFLATE_WANT_ADLER32
+    for with_dicts in (False, True):
+        # with dictionaries: the zlib streams (the Z_SYNC_FLUSH one, the invalid one and every other small one) have one
+        has = [False, False, with_dicts, with_dicts] + [with_dicts and k % 2 == 0 for k in range(len(small))]
+        co = zlib.compressobj(6, zlib.DEFLATED, -15, 9, zlib.Z_DEFAULT_STRATEGY, *([zd] if with_dicts else []))
+        sync = b"".join(co.compress(big[2][k:k + 50000]) + co.flush(zlib.Z_SYNC_FLUSH)
+                        for k in range(0, len(big[2]), 50000)) + co.flush()
+        streams = fixed + [sync, sync[:len(sync) // 2]]
+        for d, h in zip(small, has[4:]):
+            co = zlib.compressobj(6, zlib.DEFLATED, -15, 9, zlib.Z_DEFAULT_STRATEGY, *([zd] if h else []))
+            streams.append(co.compress(d) + co.flush())
+        datas = big + [None] + small
+        assert all(len(s) >= 256 << 10 for s in streams[:4])
+        blob, offs, lens = pack(streams)
+        caps = [len(big[0]) + 100, len(big[1]) + 100, len(big[2]) + 100, len(big[2])]
+        caps += [len(d) + (5 if k % 500 == 0 else 0) for k, d in enumerate(small)]
+        ooffs = np.concatenate([[0], np.cumsum(caps)]).astype(np.uint64)
+        items = z.make_items(len(streams))
+        items["in_off"], items["in_len"], items["out_off"], items["out_cap"] = offs, lens, ooffs[:-1], caps
+        h_dict, table = np.frombuffer(zd, dtype=np.uint8).copy(), z.make_dicts(len(streams))
+        table["len"] = [len(zd) if h else 0 for h in has]
+        for pinned in (True, False):
+            runs = []
+            for flags in (base | z.INFLATE_SPLIT, base):
+                if pinned:
+                    h_in, h_out = z.host_alloc(blob.size), z.host_alloc(int(ooffs[-1]))
+                    h_in[:] = blob
+                else:
+                    h_in, h_out = blob.copy(), np.empty(int(ooffs[-1]), dtype=np.uint8)
+                h_out[:] = 0xA5
+                engine.profile_enable(True)
+                engine.profile_reset()
+                try:
+                    res = engine.inflate_batch_host(h_in, h_out, items, flags, *((h_dict, table) if with_dicts else ()))
+                    prof = engine.profile_read()
+                finally:
+                    engine.profile_enable(False)
+                runs.append((res, h_out.tobytes(), prof))
+                if pinned:
+                    z.host_free(h_in)
+                    z.host_free(h_out)
+            (res, out, prof), (res0, out0, prof0) = runs
+            assert all(prof[k]["launches"] > 0 for k in WINDOW_KERNELS), prof
+            assert not any(prof0[k]["launches"] for k in WINDOW_KERNELS), prof0
+            assert res.tobytes() == res0.tobytes() and out == out0
+            assert int(res["status"][3]) != 0
+            for i, (d, s, r) in enumerate(zip(datas, streams, res)):
+                if d is None:
+                    continue
+                assert int(r["status"]) == 0 and int(r["out_len"]) == len(d) and int(r["in_used"]) == len(s), i
+                assert out[int(ooffs[i]):int(ooffs[i]) + len(d)] == d, i
+                assert int(r["crc32"]) == zlib.crc32(d) and int(r["adler32"]) == zlib.adler32(d), i
 
 
 def test_host_api_primed_round_trips(engine):

@@ -6,6 +6,7 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <functional>
 #include <vector>
 
 #include "../../include/zlibts_b200.h"
@@ -106,6 +107,26 @@ void zts_stage_wait_in(ZtsHostStage* st, size_t lo, size_t hi);  // blocks until
 int zts_stage_out_ready(zlb_ctx* ctx, ZtsHostStage* st, cudaStream_t s, size_t off, size_t len);
 int zts_stage_end(zlb_ctx* ctx, ZtsHostStage* st);
 void zts_stage_destroy_ctx(zlb_ctx* ctx);
+// The checks every batch entry point makes first, in this order: the pointers (bufs_ok: the caller's data buffers are
+// given where they are needed), n == 0 (returns 1: nothing to do), at most max_items items, the dictionary table
+// (zts_check_dicts); then the context's device is selected.
+int zts_entry_begin(zlb_ctx* ctx, bool bufs_ok, const zlb_item* items, const zlb_result* results, size_t n,
+                    size_t max_items, const void* dict_blob, size_t dict_bytes, const zlb_dict* dicts, bool* any);
+// Host buffers of a "_host" entry point, as its device path sees them. Their bytes travel through the staging arenas
+// ctx->d_stage_in / d_stage_out, the dictionary blob through ctx->d_dict.
+struct ZtsHostIO {
+    const uint8_t* h_in;   // where H2D copies read from: the caller's page-locked buffer, or the library's shadow
+    uint8_t* h_out;        // where D2H copies write to
+    size_t in_bytes;
+    bool out_done;         // set by a device path that has already copied the output back, wave by wave
+    ZtsHostStage* stage;   // copy threads behind the shadows (pageable caller buffers), see zts_hoststage.cu
+};
+// A "_host" entry point: zts_entry_begin, every item inside the blobs, the dictionary blob to the device, the staging
+// arenas and the copy threads; then body(io, dictionary table or NULL when no item has one) and a synchronise.
+// The copy threads are drained on every path, errors included.
+int zts_host_call(zlb_ctx* ctx, const void* h_in, size_t in_bytes, void* h_out, size_t out_bytes, const void* h_dict,
+                  size_t dict_bytes, const zlb_dict* dicts, const zlb_item* items, const zlb_result* results, size_t n,
+                  size_t max_items, const std::function<int(ZtsHostIO& io, const zlb_dict* dicts)>& body);
 // D2H of what items [a, b) wrote (adjacent ranges merged; see zts_ctx.cu); h_out = zts_stage_out_ptr() when staged
 int zts_copy_back(zlb_ctx* ctx, ZtsHostStage* st, cudaStream_t s, const uint8_t* d_out, uint8_t* h_out,
                   const zlb_item* h_items, const zlb_result* h_res, const zlb_item* d_items, const zlb_result* d_res,

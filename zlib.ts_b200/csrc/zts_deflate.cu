@@ -386,22 +386,15 @@ static int deflate_stored(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
     return ZLB_OK;
 }
 
-// Host buffers of the "_host" entry point. The device path below then also moves the data: the input of
-// wave k+1 travels while wave k is compressed, and what wave k produced travels while wave k+1 runs.
-struct HostIO {
-    const uint8_t* h_in;   // where H2D copies read from: the caller's page-locked buffer, or the library's shadow
-    uint8_t* h_out;        // where D2H copies write to
-    size_t in_bytes, out_bytes;
-    bool out_done;  // set when the output has already been copied wave by wave
-    ZtsHostStage* stage;   // copy threads behind the shadows (pageable caller buffers), see zts_hoststage.cu
-};
 #define HOST_DELTA_MAX_ITEMS 256u  // per-wave output read-back is done item by item up to this many items
 
 // Runs the pipeline on device buffers. Results land in h_results after the final synchronise.
 // d_dict / h_dicts: the preset dictionaries (h_dicts == NULL: none; checked by the caller)
+// hio: the host buffers of a "_host" call. The device path then also moves the data: the input of wave k+1 travels
+// while wave k is compressed, and with few items what wave k produced travels while wave k+1 runs (hio->out_done).
 static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const uint8_t* d_dict,
                           const zlb_dict* h_dicts, const zlb_item* h_items, zlb_result* h_results, size_t n, int mode,
-                          int block_type, uint32_t chunk_bytes, uint32_t flags, HostIO* hio)
+                          int block_type, uint32_t chunk_bytes, uint32_t flags, ZtsHostIO* hio)
 {
     if ((mode & 0xFF) & ~(ZLB_MODE_FAST | ZLB_MODE_PRIMED | ZLB_MODE_SMALLEST | ZLB_MODE_LAZY))
         return zts_fail(ctx, ZLB_E_UNSUPPORTED, "unknown deflate mode %d", mode);
@@ -742,12 +735,9 @@ extern "C" int zlb_deflate_batch_dict(zlb_ctx* ctx, const void* d_in, void* d_ou
                                       const zlb_dict* dicts, const zlb_item* items, zlb_result* results, size_t n,
                                       int mode, int block_type, uint32_t chunk_bytes, uint32_t flags)
 {
-    if (!ctx || (!items && n) || (!results && n) || (!d_out && n)) return ZLB_E_ARG;
-    if (n == 0) return ZLB_OK;
     bool any = false;
-    int rc = zts_check_dicts(ctx, d_dict, SIZE_MAX, dicts, n, &any);
-    if (rc) return rc;
-    ZTS_CUDA(ctx, cudaSetDevice(ctx->device));
+    int rc = zts_entry_begin(ctx, d_out || !n, items, results, n, SIZE_MAX, d_dict, SIZE_MAX, dicts, &any);
+    if (rc) return rc > 0 ? ZLB_OK : rc;
     return deflate_device(ctx, (const uint8_t*)d_in, (uint8_t*)d_out, (const uint8_t*)d_dict, any ? dicts : nullptr,
                           items, results, n, mode, block_type, chunk_bytes, flags, nullptr);
 }
@@ -765,41 +755,16 @@ extern "C" int zlb_deflate_batch_dict_host(zlb_ctx* ctx, const void* h_in, size_
                                            const zlb_dict* dicts, const zlb_item* items, zlb_result* results, size_t n,
                                            int mode, int block_type, uint32_t chunk_bytes, uint32_t flags)
 {
-    if (!ctx || (!items && n) || (!results && n) || (!h_in && in_bytes) || (!h_out && out_bytes)) return ZLB_E_ARG;
-    if (n == 0) return ZLB_OK;
-    bool any = false;
-    int rc = zts_check_dicts(ctx, h_dict, dict_bytes, dicts, n, &any);
-    if (rc) return rc;
-    ZTS_CUDA(ctx, cudaSetDevice(ctx->device));
-    for (size_t i = 0; i < n; ++i) {
-        if (items[i].in_off + items[i].in_len > in_bytes || items[i].out_off + items[i].out_cap > out_bytes)
-            return zts_fail(ctx, ZLB_E_ARG, "item %zu out of range", i);
-    }
-    // the dictionaries go over first, on the context's stream (everything of the call is ordered behind it)
-    if (any) {
-        if ((rc = zts_reserve(ctx, &ctx->d_dict, dict_bytes + 256))) return rc;
-        ZTS_CUDA(ctx, cudaMemcpyAsync(ctx->d_dict.p, h_dict, dict_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    }
-    rc = zts_reserve(ctx, &ctx->d_stage_in, in_bytes + 256);
-    if (rc) return rc;
-    rc = zts_reserve(ctx, &ctx->d_stage_out, out_bytes + 256);
-    if (rc) return rc;
-    ZtsHostStage* stage = nullptr;
-    rc = zts_stage_begin(ctx, h_in, in_bytes, h_out, out_bytes, &stage);
-    if (!rc) {
-        HostIO hio = {zts_stage_in_ptr(stage), zts_stage_out_ptr(stage), in_bytes, out_bytes, false, stage};
-        rc = deflate_device(ctx, (const uint8_t*)ctx->d_stage_in.p, (uint8_t*)ctx->d_stage_out.p,
-                            (const uint8_t*)ctx->d_dict.p, any ? dicts : nullptr, items, results, n, mode, block_type,
-                            chunk_bytes, flags, &hio);
-        if (!rc && !hio.out_done) {
-            // many items: what each of them wrote, adjacent ranges merged
-            rc = zts_copy_back(ctx, stage, ctx->stream, (const uint8_t*)ctx->d_stage_out.p, hio.h_out, items, results,
-                               (const zlb_item*)ctx->d_items.p, (const zlb_result*)ctx->d_results.p, 0, n);
-            if (!rc && cudaStreamSynchronize(ctx->stream) != cudaSuccess) rc = zts_fail(ctx, ZLB_E_CUDA, "synchronize failed");
-        }
-    }
-    zts_stage_end(ctx, stage);  // also on errors: the copy threads hold pointers into the caller's buffers
-    return rc;
+    return zts_host_call(ctx, h_in, in_bytes, h_out, out_bytes, h_dict, dict_bytes, dicts, items, results, n, SIZE_MAX,
+                         [&](ZtsHostIO& io, const zlb_dict* d) {
+        const uint8_t* d_out = (const uint8_t*)ctx->d_stage_out.p;
+        int rc = deflate_device(ctx, (const uint8_t*)ctx->d_stage_in.p, (uint8_t*)d_out, (const uint8_t*)ctx->d_dict.p, d,
+                                items, results, n, mode, block_type, chunk_bytes, flags, &io);
+        if (rc || io.out_done) return rc;
+        // many items: what each of them wrote, adjacent ranges merged
+        return zts_copy_back(ctx, io.stage, ctx->stream, d_out, io.h_out, items, results, (const zlb_item*)ctx->d_items.p,
+                             (const zlb_result*)ctx->d_results.p, 0, n);
+    });
 }
 
 extern "C" int zlb_deflate_batch_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes, void* h_out, size_t out_bytes,

@@ -1,5 +1,6 @@
 // zts_hoststage.cu -- host-side plumbing of the "_host" entry points for callers whose buffers are NOT page-locked
-// (a plain malloc'ed / JS-heap buffer), plus zlb_host_alloc / zlb_host_free for callers that can do better.
+// (a plain malloc'ed / JS-heap buffer), the prologue and epilogue the batch entry points share, plus zlb_host_alloc /
+// zlb_host_free for callers that can do better.
 //
 // cudaMemcpyAsync from pageable memory is staged by the driver through a small bounce buffer and serialises with
 // the caller's thread; the wave pipelines of the host paths (input of wave k+1 and output of wave k-1 travelling while
@@ -227,6 +228,51 @@ void zts_stage_destroy_ctx(zlb_ctx* ctx)
     if (ctx->h_shadow_out) cudaFreeHost(ctx->h_shadow_out);
     for (cudaEvent_t e : ctx->stage_ev_pool) cudaEventDestroy(e);
     ctx->stage_ev_pool.clear();
+}
+
+// ---- what the batch entry points share ------------------------------------------------------------------------------
+int zts_entry_begin(zlb_ctx* ctx, bool bufs_ok, const zlb_item* items, const zlb_result* results, size_t n,
+                    size_t max_items, const void* dict_blob, size_t dict_bytes, const zlb_dict* dicts, bool* any)
+{
+    if (!ctx || !bufs_ok || (!items && n) || (!results && n)) return ZLB_E_ARG;
+    if (n == 0) return 1;
+    if (n > max_items) return zts_fail(ctx, ZLB_E_ARG, "too many items");
+    int rc = zts_check_dicts(ctx, dict_blob, dict_bytes, dicts, n, any);
+    if (rc) return rc;
+    ZTS_CUDA(ctx, cudaSetDevice(ctx->device));
+    return ZLB_OK;
+}
+
+int zts_host_call(zlb_ctx* ctx, const void* h_in, size_t in_bytes, void* h_out, size_t out_bytes, const void* h_dict,
+                  size_t dict_bytes, const zlb_dict* dicts, const zlb_item* items, const zlb_result* results, size_t n,
+                  size_t max_items, const std::function<int(ZtsHostIO& io, const zlb_dict* dicts)>& body)
+{
+    bool any = false;
+    int rc = zts_entry_begin(ctx, (h_in || !in_bytes) && (h_out || !out_bytes), items, results, n, max_items, h_dict,
+                             dict_bytes, dicts, &any);
+    if (rc) return rc > 0 ? ZLB_OK : rc;
+    for (size_t i = 0; i < n; ++i) {
+        if (items[i].in_off + items[i].in_len > in_bytes || items[i].out_off + items[i].out_cap > out_bytes)
+            return zts_fail(ctx, ZLB_E_ARG, "item %zu out of range", i);
+    }
+    // the dictionaries go over first, on the context's stream (everything of the call is ordered behind it)
+    if (any) {
+        if ((rc = zts_reserve(ctx, &ctx->d_dict, dict_bytes + 256))) return rc;
+        ZTS_CUDA(ctx, cudaMemcpyAsync(ctx->d_dict.p, h_dict, dict_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    }
+    rc = zts_reserve(ctx, &ctx->d_stage_in, in_bytes + 256);
+    if (rc) return rc;
+    rc = zts_reserve(ctx, &ctx->d_stage_out, out_bytes + 256);
+    if (rc) return rc;
+    ZtsHostStage* stage = nullptr;
+    rc = zts_stage_begin(ctx, h_in, in_bytes, h_out, out_bytes, &stage);
+    if (!rc) {
+        ZtsHostIO io = {zts_stage_in_ptr(stage), zts_stage_out_ptr(stage), in_bytes, false, stage};
+        rc = body(io, any ? dicts : nullptr);
+        if (!rc && cudaStreamSynchronize(ctx->stream) != cudaSuccess) rc = zts_fail(ctx, ZLB_E_CUDA, "synchronize failed");
+    }
+    zts_stage_end(ctx, stage);  // also on errors: the copy threads hold pointers into the caller's buffers
+    return rc;
 }
 
 // ---- page-locked memory for callers (an N-API addon hands it out as external ArrayBuffers) -------------------------

@@ -1023,6 +1023,34 @@ static void split_finish(const zlb_item& it, const zlb_result* r, const zlb_item
     }
 }
 
+// Scratch budget of an arena of the split stage: a quarter of what the device has free plus what the arena already
+// holds, at most 16 GiB, and at most k times what `in_bytes` of input could legitimately inflate to (2048 x, at least
+// 64 MiB). Items whose scratch does not fit are not split: the one-warp decoder gives the same result.
+struct SplitBudget {
+    size_t device;
+    explicit SplitBudget(const ZtsDevBuf& arena)
+    {
+        size_t free_b = 0, total_b = 0;
+        if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) free_b = 0;
+        device = std::min((free_b + arena.cap) / 4, (size_t)16 << 30);
+    }
+    size_t operator()(size_t in_bytes, size_t k) const
+    {
+        return std::min(device, k * std::max(in_bytes * 2048u, (size_t)64 << 20));
+    }
+};
+
+// Reserves scratch of the split stage; *got = false, and no error left behind, when the device cannot give it (the
+// items then go to the one-warp decoder).
+static int split_reserve(zlb_ctx* ctx, ZtsDevBuf* arena, size_t bytes, bool* got)
+{
+    const int rc = zts_reserve(ctx, arena, bytes);
+    *got = rc == ZLB_OK;
+    if (rc != ZLB_E_NOMEM) return rc;
+    ctx->err[0] = 0;
+    return ZLB_OK;
+}
+
 // Window mode for the items big[cand[*]] (pieces as laid out by inflate_split_batch, byte slots at seg[j].out_off of
 // d_scratch): all of them in one decode launch and one scan; done[k] / res[k] / gath as there. h_dicts / d_dict: the
 // preset dictionaries of h_items (NULL: none).
@@ -1053,13 +1081,9 @@ static int inflate_split_window(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_sc
         off[7] = off[6] + ni * sizeof(ZtsWinItem);
         return off[7] + ni * 4 + 256;
     };
-    // The scratch is bounded like the byte slots' (a quarter of what the device has free, 16 GiB), and by what the
-    // input could legitimately need: three times the byte slots' bound (two bytes per word, the windows, the maps).
-    // Items that do not fit go to the one-warp decoder.
-    size_t free_b = 0, total_b = 0;
-    if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) free_b = 0;
-    size_t budget = (free_b + ctx->d_window.cap) / 4;
-    if (budget > ((size_t)16 << 30)) budget = (size_t)16 << 30;
+    // The scratch is bounded like the byte slots', with three times their bound by input (two bytes per word, the
+    // windows, the maps).
+    const SplitBudget budget(ctx->d_window);
     std::vector<size_t> take;
     size_t words = 0, np = 0, nr = 0, in_b = 0, need = 0, off[8];
     for (size_t k : cand) {
@@ -1068,9 +1092,7 @@ static int inflate_split_window(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_sc
         for (size_t j = a; j < b; ++j) w += map_b + 2 * (size_t)seg[j].out_cap;  // (out_cap: a multiple of 256)
         const size_t g = run_len(n);
         const size_t need_k = layout(words + w, np + n, nr + (n + g - 1) / g, take.size() + 1, off);
-        size_t by_input = (in_b + h_items[big[k]].in_len) * 2048u;
-        if (by_input < ((size_t)64 << 20)) by_input = (size_t)64 << 20;
-        if (need_k > budget || need_k > 3 * by_input) continue;
+        if (need_k > budget(in_b + h_items[big[k]].in_len, 3)) continue;
         take.push_back(k);
         words += w;
         np += n;
@@ -1079,12 +1101,9 @@ static int inflate_split_window(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_sc
         need = need_k;
     }
     if (take.empty()) return ZLB_OK;
-    int rc = zts_reserve(ctx, &ctx->d_window, need);
-    if (rc == ZLB_E_NOMEM) {
-        ctx->err[0] = 0;
-        return ZLB_OK;
-    }
-    if (rc) return rc;
+    bool got = false;
+    int rc = split_reserve(ctx, &ctx->d_window, need, &got);
+    if (rc || !got) return rc;
     layout(words, np, nr, take.size(), off);
     uint8_t* arena = (uint8_t*)ctx->d_window.p;
     uint16_t* d_agg = (uint16_t*)(arena + off[0]);
@@ -1238,26 +1257,10 @@ static int inflate_split_batch(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out
             scratch += slot;
         }
     }
-    {
-        // the scratch is bounded: what the input could legitimately inflate to (2048 x, floor 64 MiB), a quarter of
-        // what the device has free right now, 16 GiB at most. Whatever does not fit (or cannot be allocated) is simply
-        // not split -- the one-warp decoder gives the same result.
-        const size_t need = ((scratch + 255) & ~(size_t)255) + np * (sizeof(zlb_item) + sizeof(zlb_result) + sizeof(ZtsGather)) + 1024;
-        size_t free_b = 0, total_b = 0;
-        if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) free_b = 0;
-        size_t budget = (free_b + ctx->d_split.cap) / 4;
-        if (budget > ((size_t)16 << 30)) budget = (size_t)16 << 30;
-        size_t by_input = big_in * 2048u;
-        if (by_input < ((size_t)64 << 20)) by_input = (size_t)64 << 20;
-        if (budget > by_input) budget = by_input;
-        if (need > budget) return ZLB_OK;
-        rc = zts_reserve(ctx, &ctx->d_split, need);
-        if (rc == ZLB_E_NOMEM) {
-            ctx->err[0] = 0;
-            return ZLB_OK;
-        }
-        if (rc) return rc;
-    }
+    const size_t need = ((scratch + 255) & ~(size_t)255) + np * (sizeof(zlb_item) + sizeof(zlb_result) + sizeof(ZtsGather)) + 1024;
+    if (need > SplitBudget(ctx->d_split)(big_in, 1)) return ZLB_OK;
+    bool got = false;
+    if ((rc = split_reserve(ctx, &ctx->d_split, need, &got)) || !got) return rc;
     uint8_t* d_scratch = (uint8_t*)ctx->d_split.p;
     zlb_item* d_seg = (zlb_item*)(d_scratch + ((scratch + 255) & ~(size_t)255));
     zlb_result* d_segres = (zlb_result*)(d_seg + np);
@@ -1296,136 +1299,27 @@ static int inflate_split_batch(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out
     return ZLB_OK;
 }
 
-// Host buffers of the "_host" entry point: items are cut into a few waves; the input of a wave travels while the
-// previous waves are decoded (one compute stream per wave: a wave is latency-bound, so the waves run side by side) and its output
-// travels back as soon as it is done.
-struct InfHostIO {
-    const uint8_t* h_in;   // where H2D copies read from: the caller's page-locked buffer, or the library's shadow
-    uint8_t* h_out;        // where D2H copies write to
-    size_t in_bytes, out_bytes;
-    ZtsHostStage* stage;   // copy threads behind the shadows (pageable caller buffers), see zts_hoststage.cu
-};
-
-// d_dict / h_dicts: the preset dictionaries (h_dicts == NULL: none; checked by the caller)
-static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const uint8_t* d_dict,
-                          const zlb_dict* h_dicts, const zlb_item* h_items, zlb_result* h_results, size_t n, uint32_t flags,
-                          const InfHostIO* hio)
+// A "_host" call without a split, in waves; the tables are queued on ctx->stream already. The input of wave k+1 travels
+// on a copy stream while wave k is decoded, and as soon as the sizes of wave k are known (its results are read back
+// behind it, wave k+1 is already queued) what it wrote travels back on the other copy stream. The waves are launched
+// on up to four compute streams in turn: a stream is decoded by one warp from start to end (milliseconds, whatever the
+// batch size), so waves that do not fill the device by themselves run side by side, staggered by their input copies,
+// and their outputs leave as each one finishes; waves that do fill it simply take over the SMs as their predecessor
+// drains.
+static int inflate_waves(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const uint8_t* d_dict, const zlb_item* d_items,
+                         const zlb_dict* d_dicts, zlb_result* d_results, const zlb_item* h_items, zlb_result* h_results,
+                         size_t n, uint32_t flags, uint32_t kinds, const ZtsHostIO& hio)
 {
-    int rc = zts_reserve(ctx, &ctx->d_items, n * sizeof(zlb_item) + 64);
-    if (rc) return rc;
-    const zlb_dict* d_dicts = nullptr;  // the dictionary table on the device, beside the item table
-    if (h_dicts) {
-        if ((rc = zts_reserve(ctx, &ctx->d_dict_stage, n * sizeof(zlb_dict) + 64))) return rc;
-        d_dicts = (const zlb_dict*)ctx->d_dict_stage.p;
-        ZTS_CUDA(ctx, cudaMemcpyAsync((void*)d_dicts, h_dicts, n * sizeof(zlb_dict), cudaMemcpyHostToDevice, ctx->stream));
-    }
-    rc = zts_reserve(ctx, &ctx->d_results, n * sizeof(zlb_result) + 64);
-    if (rc) return rc;
-    zlb_item* d_items = (zlb_item*)ctx->d_items.p;
-    zlb_result* d_results = (zlb_result*)ctx->d_results.p;
-    ZTS_CUDA(ctx, cudaMemcpyAsync(d_items, h_items, n * sizeof(zlb_item), cudaMemcpyHostToDevice, ctx->stream));
-    ZTS_CUDA(ctx, cudaMemsetAsync(d_results, 0, n * sizeof(zlb_result), ctx->stream));
-    uint32_t kinds = 0;
-    if (flags & ZLB_INFLATE_WANT_CRC32) kinds |= ZLB_SUM_CRC32;
-    if (flags & ZLB_INFLATE_WANT_ADLER32) kinds |= ZLB_SUM_ADLER32;
-
-    // large items that may be cut at sync-flush markers are decoded piecewise, one after the other (each is
-    // massively parallel by itself); whatever is left goes through the batch path below
-    if ((flags & ZLB_INFLATE_SPLIT) && !(flags & ZLB_INFLATE_SEGMENT)) {
-        std::vector<size_t> big;
-        for (size_t i = 0; i < n; ++i)
-            if (h_items[i].in_len >= SPLIT_MIN_BYTES) big.push_back(i);
-        if (!big.empty()) {
-            if (hio) {
-                zts_stage_wait_in(hio->stage, 0, hio->in_bytes);
-                ZTS_CUDA(ctx, cudaMemcpyAsync((void*)d_in, hio->h_in, hio->in_bytes, cudaMemcpyHostToDevice, ctx->stream));
-            }
-            std::vector<zlb_item> rest_items;
-            std::vector<zlb_dict> rest_dicts;
-            std::vector<size_t> rest_idx;
-            std::vector<char> is_done(n, 0);
-            {
-                std::vector<zlb_result> bres;
-                std::vector<char> bdone;
-                rc = inflate_split_batch(ctx, d_in, d_out, h_items, h_dicts, d_dict, big, flags, bres, bdone);
-                if (rc) return rc;
-                bool any = false;
-                for (size_t k = 0; k < big.size(); ++k)
-                    if (bdone[k]) {
-                        is_done[big[k]] = 1;
-                        any = true;
-                        ZTS_CUDA(ctx, cudaMemcpyAsync(d_results + big[k], &bres[k], sizeof(zlb_result), cudaMemcpyHostToDevice,
-                                                      ctx->stream));
-                    }
-                if (any) ZTS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // bres goes out of scope
-            }
-            for (size_t i = 0; i < n; ++i)
-                if (!is_done[i]) {
-                    rest_items.push_back(h_items[i]);
-                    if (h_dicts) rest_dicts.push_back(h_dicts[i]);
-                    rest_idx.push_back(i);
-                }
-            if (!rest_items.empty()) {
-                // the remaining items in one batch; their results are scattered back to their slots
-                const size_t m = rest_items.size();
-                rc = zts_reserve(ctx, &ctx->d_sums, m * (sizeof(zlb_item) + sizeof(zlb_result) + sizeof(zlb_dict)) + 256);
-                if (rc) return rc;
-                zlb_item* d_ri = (zlb_item*)ctx->d_sums.p;
-                zlb_result* d_rr = (zlb_result*)(d_ri + m);
-                zlb_dict* d_rd = h_dicts ? (zlb_dict*)(d_rr + m) : nullptr;
-                ZTS_CUDA(ctx, cudaMemcpyAsync(d_ri, rest_items.data(), m * sizeof(zlb_item), cudaMemcpyHostToDevice, ctx->stream));
-                ZTS_CUDA(ctx, cudaMemsetAsync(d_rr, 0, m * sizeof(zlb_result), ctx->stream));
-                if (d_rd)
-                    ZTS_CUDA(ctx, cudaMemcpyAsync(d_rd, rest_dicts.data(), m * sizeof(zlb_dict), cudaMemcpyHostToDevice, ctx->stream));
-                rc = inflate_launch(ctx, ctx->stream, d_in, d_out, d_ri, d_rr, m, flags & ~(uint32_t)ZLB_INFLATE_SPLIT, d_rd, d_dict);
-                if (rc) return rc;
-                std::vector<zlb_result> rr(m);
-                ZTS_CUDA(ctx, cudaMemcpyAsync(rr.data(), d_rr, m * sizeof(zlb_result), cudaMemcpyDeviceToHost, ctx->stream));
-                ZTS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-                for (size_t k = 0; k < m; ++k)
-                    ZTS_CUDA(ctx, cudaMemcpyAsync(d_results + rest_idx[k], &rr[k], sizeof(zlb_result), cudaMemcpyHostToDevice, ctx->stream));
-                ZTS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-            }
-            if (kinds) {
-                rc = zts_checksum_device(ctx, d_out, d_items, d_results, h_items, n, kinds, 1);
-                if (rc) return rc;
-            }
-            ZTS_CUDA(ctx, cudaMemcpyAsync(h_results, d_results, n * sizeof(zlb_result), cudaMemcpyDeviceToHost, ctx->stream));
-            if (hio) {
-                ZTS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // the sizes decide what travels
-                rc = zts_copy_back(ctx, hio->stage, ctx->stream, d_out, hio->h_out, h_items, h_results, d_items, d_results, 0, n);
-                if (rc) return rc;
-            }
-            return ZLB_OK;
-        }
-    }
     // waves only pay when the items are laid out in order on both sides (then a wave is one contiguous copy each way)
     size_t n_waves = 1;
-    if (hio && n >= 1024) {
+    if (n >= 1024) {
         n_waves = n >= 32768 ? 16 : n >= 16384 ? 8 : 4;  // (the last wave's output travels alone: keep it small)
         for (size_t i = 1; i < n && n_waves > 1; ++i)
             if (h_items[i].in_off < h_items[i - 1].in_off + h_items[i - 1].in_len ||
                 h_items[i].out_off < h_items[i - 1].out_off + h_items[i - 1].out_cap)
                 n_waves = 1;
     }
-    if (!hio) {
-        rc = inflate_launch(ctx, ctx->stream, d_in, d_out, d_items, d_results, n, flags, d_dicts, d_dict);
-        if (rc) return rc;
-        if (kinds) {
-            rc = zts_checksum_device(ctx, d_out, d_items, d_results, h_items, n, kinds, 1);
-            if (rc) return rc;
-        }
-        ZTS_CUDA(ctx, cudaMemcpyAsync(h_results, d_results, n * sizeof(zlb_result), cudaMemcpyDeviceToHost, ctx->stream));
-        return ZLB_OK;
-    }
-
-    // Host buffers: the input of wave k+1 travels on a copy stream while wave k is decoded, and as soon as the sizes of
-    // wave k are known (its results are read back behind it, wave k+1 is already queued) what it wrote travels back on
-    // the other copy stream. The waves are launched on up to four compute streams in turn: a stream is decoded by one
-    // warp from start to end (milliseconds, whatever the batch size), so waves that do not fill the device by
-    // themselves run side by side, staggered by their input copies, and their outputs leave as each one finishes;
-    // waves that do fill it simply take over the SMs as their predecessor drains.
-    rc = zts_host_streams(ctx);
+    int rc = zts_host_streams(ctx);
     if (rc) return rc;
     rc = zts_reserve_pinned2(ctx, n * sizeof(zlb_result));
     if (rc) return rc;
@@ -1446,14 +1340,14 @@ static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
             uint64_t ilo, ihi;
             if (n_waves == 1) {  // items in any order: the whole blob
                 ilo = 0;
-                ihi = hio->in_bytes;
+                ihi = hio.in_bytes;
             } else {
                 ilo = h_items[a].in_off;
                 ihi = h_items[b - 1].in_off + h_items[b - 1].in_len;
             }
             if (ihi > ilo) {
-                zts_stage_wait_in(hio->stage, ilo, ihi);
-                ZTS_CUDA(ctx, cudaMemcpyAsync((void*)(d_in + ilo), hio->h_in + ilo, ihi - ilo, cudaMemcpyHostToDevice, ctx->s_in));
+                zts_stage_wait_in(hio.stage, ilo, ihi);
+                ZTS_CUDA(ctx, cudaMemcpyAsync((void*)(d_in + ilo), hio.h_in + ilo, ihi - ilo, cudaMemcpyHostToDevice, ctx->s_in));
             }
         }
         ZTS_CUDA(ctx, cudaEventRecord(zts_sync_event(ctx, 1 + 2 * k), ctx->s_in));
@@ -1475,7 +1369,7 @@ static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
         ZTS_CUDA(ctx, cudaMemcpyAsync(pin_res + a, d_results + a, (b - a) * sizeof(zlb_result), cudaMemcpyDeviceToHost, ctx->s_res));
         ZTS_CUDA(ctx, cudaStreamSynchronize(ctx->s_res));
         memcpy(h_results + a, pin_res + a, (b - a) * sizeof(zlb_result));
-        return zts_copy_back(ctx, hio->stage, ctx->s_out, d_out, hio->h_out, h_items, h_results, d_items, d_results, a, b);
+        return zts_copy_back(ctx, hio.stage, ctx->s_out, d_out, hio.h_out, h_items, h_results, d_items, d_results, a, b);
     };
     if ((rc = wave_in(0))) return rc;
     for (size_t k = 0; k < n_waves; ++k) {
@@ -1513,17 +1407,114 @@ static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
     return ZLB_OK;
 }
 
+// Decodes n items on device buffers; results land in h_results after the final synchronise. The item table goes to the
+// device with the dictionary table beside it. With ZLB_INFLATE_SPLIT the large items are tried piecewise first
+// (inflate_split_batch); the items left go through one decoder launch, over a compacted table when the split did some.
+// Then one tail: checksums, the result read-back and, on a "_host" call, the copy-back of the outputs. A "_host" call
+// without a split runs in waves instead (inflate_waves).
+// d_dict / h_dicts: the preset dictionaries (h_dicts == NULL: none; checked by the caller)
+static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const uint8_t* d_dict,
+                          const zlb_dict* h_dicts, const zlb_item* h_items, zlb_result* h_results, size_t n, uint32_t flags,
+                          const ZtsHostIO* hio)
+{
+    // large items that may be cut at sync-flush markers (each is massively parallel by itself)
+    std::vector<size_t> big;
+    if ((flags & ZLB_INFLATE_SPLIT) && !(flags & ZLB_INFLATE_SEGMENT))
+        for (size_t i = 0; i < n; ++i)
+            if (h_items[i].in_len >= SPLIT_MIN_BYTES) big.push_back(i);
+    // d_items holds the call's per-item tables: items | dictionaries, and with a split the same for the items left
+    const size_t row = sizeof(zlb_item) + (h_dicts ? sizeof(zlb_dict) : 0);
+    int rc = zts_reserve(ctx, &ctx->d_items, (big.empty() ? 1 : 2) * n * row + 64);
+    if (rc) return rc;
+    rc = zts_reserve(ctx, &ctx->d_results, n * sizeof(zlb_result) + 64);
+    if (rc) return rc;
+    auto upload = [&](size_t at, const zlb_item* items, const zlb_dict* dicts, size_t m, zlb_item*& d_it,
+                      zlb_dict*& d_di) -> int {
+        d_it = (zlb_item*)((uint8_t*)ctx->d_items.p + at);
+        d_di = dicts ? (zlb_dict*)(d_it + m) : nullptr;
+        ZTS_CUDA(ctx, cudaMemcpyAsync(d_it, items, m * sizeof(zlb_item), cudaMemcpyHostToDevice, ctx->stream));
+        if (dicts) ZTS_CUDA(ctx, cudaMemcpyAsync(d_di, dicts, m * sizeof(zlb_dict), cudaMemcpyHostToDevice, ctx->stream));
+        return ZLB_OK;
+    };
+    zlb_item* d_items;
+    zlb_dict* d_dicts;
+    if ((rc = upload(0, h_items, h_dicts, n, d_items, d_dicts))) return rc;
+    zlb_result* d_results = (zlb_result*)ctx->d_results.p;
+    ZTS_CUDA(ctx, cudaMemsetAsync(d_results, 0, n * sizeof(zlb_result), ctx->stream));
+    uint32_t kinds = 0;
+    if (flags & ZLB_INFLATE_WANT_CRC32) kinds |= ZLB_SUM_CRC32;
+    if (flags & ZLB_INFLATE_WANT_ADLER32) kinds |= ZLB_SUM_ADLER32;
+    if (hio && big.empty())
+        return inflate_waves(ctx, d_in, d_out, d_dict, d_items, d_dicts, d_results, h_items, h_results, n, flags, kinds, *hio);
+
+    // the split: the items it decodes get their results in h_results; when it decoded any, rest lists the others
+    zlb_item* d_rest = d_items;
+    zlb_dict* d_rest_dicts = d_dicts;
+    size_t m = n;
+    bool split_any = false;
+    std::vector<size_t> rest;
+    std::vector<zlb_item> rest_items;
+    std::vector<zlb_dict> rest_dicts;
+    if (!big.empty()) {
+        if (hio) {
+            zts_stage_wait_in(hio->stage, 0, hio->in_bytes);
+            ZTS_CUDA(ctx, cudaMemcpyAsync((void*)d_in, hio->h_in, hio->in_bytes, cudaMemcpyHostToDevice, ctx->stream));
+        }
+        std::vector<zlb_result> bres;
+        std::vector<char> bdone, done(n, 0);
+        rc = inflate_split_batch(ctx, d_in, d_out, h_items, h_dicts, d_dict, big, flags, bres, bdone);
+        if (rc) return rc;
+        for (size_t k = 0; k < big.size(); ++k)
+            if (bdone[k]) {
+                done[big[k]] = 1;
+                h_results[big[k]] = bres[k];
+                split_any = true;
+            }
+        if (split_any) {
+            for (size_t i = 0; i < n; ++i)
+                if (!done[i]) {
+                    rest.push_back(i);
+                    rest_items.push_back(h_items[i]);
+                    if (h_dicts) rest_dicts.push_back(h_dicts[i]);
+                }
+            m = rest.size();
+            if ((rc = upload(n * row, rest_items.data(), h_dicts ? rest_dicts.data() : nullptr, m, d_rest, d_rest_dicts)))
+                return rc;
+        }
+    }
+    // the items left, in one launch; after a split their results come back to the host, join the split's there, and
+    // the whole table goes to d_results in one copy (the checksums read out_len from it)
+    if (m) {
+        rc = inflate_launch(ctx, ctx->stream, d_in, d_out, d_rest, d_results, m, flags, d_rest_dicts, d_dict);
+        if (rc) return rc;
+    }
+    if (split_any) {
+        std::vector<zlb_result> rr(m);
+        ZTS_CUDA(ctx, cudaMemcpyAsync(rr.data(), d_results, m * sizeof(zlb_result), cudaMemcpyDeviceToHost, ctx->stream));
+        ZTS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        for (size_t j = 0; j < m; ++j) h_results[rest[j]] = rr[j];
+        ZTS_CUDA(ctx, cudaMemcpyAsync(d_results, h_results, n * sizeof(zlb_result), cudaMemcpyHostToDevice, ctx->stream));
+    }
+    if (kinds) {
+        rc = zts_checksum_device(ctx, d_out, d_items, d_results, h_items, n, kinds, 1);
+        if (rc) return rc;
+    }
+    ZTS_CUDA(ctx, cudaMemcpyAsync(h_results, d_results, n * sizeof(zlb_result), cudaMemcpyDeviceToHost, ctx->stream));
+    if (hio) {
+        ZTS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // the sizes decide what travels
+        rc = zts_copy_back(ctx, hio->stage, ctx->stream, d_out, hio->h_out, h_items, h_results, d_items, d_results, 0, n);
+        if (rc) return rc;
+    }
+    return ZLB_OK;
+}
+
 extern "C" int zlb_inflate_batch_dict(zlb_ctx* ctx, const void* d_in, void* d_out, const void* d_dict,
                                       const zlb_dict* dicts, const zlb_item* items, zlb_result* results, size_t n,
                                       uint32_t flags)
 {
-    if (!ctx || (!items && n) || (!results && n) || (!d_in && n) || (!d_out && n)) return ZLB_E_ARG;
-    if (n == 0) return ZLB_OK;
-    if (n > 0x7FFFFFFFull) return zts_fail(ctx, ZLB_E_ARG, "too many items");
     bool any = false;
-    int rc = zts_check_dicts(ctx, d_dict, SIZE_MAX, dicts, n, &any);
-    if (rc) return rc;
-    ZTS_CUDA(ctx, cudaSetDevice(ctx->device));
+    int rc = zts_entry_begin(ctx, (d_in && d_out) || !n, items, results, n, 0x7FFFFFFFull, d_dict, SIZE_MAX, dicts, &any);
+    if (rc) return rc > 0 ? ZLB_OK : rc;
     rc = inflate_device(ctx, (const uint8_t*)d_in, (uint8_t*)d_out, (const uint8_t*)d_dict, any ? dicts : nullptr, items,
                         results, n, flags, nullptr);
     if (rc) return rc;
@@ -1542,36 +1533,11 @@ extern "C" int zlb_inflate_batch_dict_host(zlb_ctx* ctx, const void* h_in, size_
                                            const zlb_dict* dicts, const zlb_item* items, zlb_result* results, size_t n,
                                            uint32_t flags)
 {
-    if (!ctx || (!items && n) || (!results && n) || (!h_in && in_bytes) || (!h_out && out_bytes)) return ZLB_E_ARG;
-    if (n == 0) return ZLB_OK;
-    if (n > 0x7FFFFFFFull) return zts_fail(ctx, ZLB_E_ARG, "too many items");
-    bool any = false;
-    int rc = zts_check_dicts(ctx, h_dict, dict_bytes, dicts, n, &any);
-    if (rc) return rc;
-    ZTS_CUDA(ctx, cudaSetDevice(ctx->device));
-    for (size_t i = 0; i < n; ++i) {
-        if (items[i].in_off + items[i].in_len > in_bytes || items[i].out_off + items[i].out_cap > out_bytes)
-            return zts_fail(ctx, ZLB_E_ARG, "item %zu out of range", i);
-    }
-    // the dictionaries go over first, on the context's stream (every stream of the call starts behind it)
-    if (any) {
-        if ((rc = zts_reserve(ctx, &ctx->d_dict, dict_bytes + 256))) return rc;
-        ZTS_CUDA(ctx, cudaMemcpyAsync(ctx->d_dict.p, h_dict, dict_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    }
-    rc = zts_reserve(ctx, &ctx->d_stage_in, in_bytes + 256);
-    if (rc) return rc;
-    rc = zts_reserve(ctx, &ctx->d_stage_out, out_bytes + 256);
-    if (rc) return rc;
-    ZtsHostStage* stage = nullptr;
-    rc = zts_stage_begin(ctx, h_in, in_bytes, h_out, out_bytes, &stage);
-    if (!rc) {
-        InfHostIO hio = {zts_stage_in_ptr(stage), zts_stage_out_ptr(stage), in_bytes, out_bytes, stage};
-        rc = inflate_device(ctx, (const uint8_t*)ctx->d_stage_in.p, (uint8_t*)ctx->d_stage_out.p,
-                            (const uint8_t*)ctx->d_dict.p, any ? dicts : nullptr, items, results, n, flags, &hio);
-        if (!rc && cudaStreamSynchronize(ctx->stream) != cudaSuccess) rc = zts_fail(ctx, ZLB_E_CUDA, "synchronize failed");
-    }
-    zts_stage_end(ctx, stage);  // also on errors: the copy threads hold pointers into the caller's buffers
-    return rc;
+    return zts_host_call(ctx, h_in, in_bytes, h_out, out_bytes, h_dict, dict_bytes, dicts, items, results, n,
+                         0x7FFFFFFFull, [&](ZtsHostIO& io, const zlb_dict* d) {
+        return inflate_device(ctx, (const uint8_t*)ctx->d_stage_in.p, (uint8_t*)ctx->d_stage_out.p,
+                              (const uint8_t*)ctx->d_dict.p, d, items, results, n, flags, &io);
+    });
 }
 
 extern "C" int zlb_inflate_batch_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes, void* h_out, size_t out_bytes,
