@@ -216,6 +216,20 @@ int zlb_inflate_batch_dict(zlb_ctx* ctx, const void* d_in, void* d_out, const vo
 int zlb_inflate_batch_dict_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes, void* h_out, size_t out_bytes,
                                 const void* h_dict, size_t dict_bytes, const zlb_dict* dicts, const zlb_item* items,
                                 zlb_result* results, size_t n_items, uint32_t flags);
+/* Decompressed size of every item without writing it (an engine extension: no format carries a usable size -- zlib
+ * none, gzip's ISIZE only mod 2^32, raw deflate none -- so callers can allocate exact output slots). items[i].in_off /
+ * in_len as for zlb_inflate_batch; out_off / out_cap are ignored. dicts (may be NULL): as for zlb_inflate_batch_dict,
+ * but only .len is read -- a dictionary decides how far a distance may reach, never a size -- so no dictionary blob is
+ * passed. flags: ZLB_INFLATE_SPLIT, ZLB_INFLATE_CHECK_NLEN; ZLB_INFLATE_WANT_CRC32 / _ADLER32 are ZLB_E_ARG (there are
+ * no bytes to sum), as is a NULL input with items. results[i].status / out_len / in_used / blocks equal those
+ * zlb_inflate_batch_dict returns for the same item, flags and dictionary with out_cap >= the item's size (never
+ * ZLB_ST_OUT_OVERFLOW); crc32 = adler32 = 0. A size-only decode stores nothing and skips stored data; with
+ * ZLB_INFLATE_SPLIT every stream the marker split can cut, primed and Z_SYNC_FLUSH ones included, is sized piecewise
+ * without scratch for its bytes.                                                                                 */
+int zlb_inflate_size_batch(zlb_ctx* ctx, const void* d_in, const zlb_dict* dicts, const zlb_item* items,
+                           zlb_result* results, size_t n_items, uint32_t flags);
+int zlb_inflate_size_batch_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes, const zlb_dict* dicts,
+                                const zlb_item* items, zlb_result* results, size_t n_items, uint32_t flags);
 
 /* ---- checksums (replace CRC32.create src/CRC32.ts:13, Adler32.create src/Adler32.ts:13) ----- */
 int zlb_checksum_batch(zlb_ctx* ctx, const void* d_in, const zlb_item* items, zlb_result* results,

@@ -14,6 +14,9 @@
 //   deflateBatch(inputs: Uint8Array[], compressionType, chunkBytes, flags, mode?) -> {outputs: Uint8Array[], crc32: number[], adler32: number[]}
 //   inflateBatch(input: Uint8Array, offsets: number[], lengths: number[], caps: number[], flags)
 //                                                          -> {outputs, status: number[], inUsed: number[], crc32, adler32}
+//   inflateSizes(input: Uint8Array, offsets: number[], lengths: number[], flags, dictionary?)
+//                                                          -> {status: number[], outLen: number[], inUsed: number[], blocks: number[]}
+//     decompressed sizes without writing them (exact `caps` for inflateBatch)
 //   checksumBatch(inputs: Uint8Array[], kinds)             -> {crc32: number[], adler32: number[]}
 //   crc32Combine(a, b, lenB), adler32Combine(a, b, lenB)
 //   hostAlloc(bytes) -> Uint8Array over page-locked memory (build inputs in it: they then travel without a copy)
@@ -305,6 +308,54 @@ static napi_value InflateBatch(napi_env env, napi_callback_info info)
     return result;
 }
 
+// inflateSizes(input, offsets, lengths, flags, dictionary?): what inflateBatch would return for each stream, without
+// the bytes (a dictionary matters by its length only)
+static napi_value InflateSizes(napi_env env, napi_callback_info info)
+{
+    size_t argc = 5;
+    napi_value argv[5];
+    napi_get_cb_info(env, info, &argc, argv, nullptr, nullptr);
+    if (!ensure_ctx(env)) return nullptr;
+    Bytes in;
+    if (!get_u8(env, argv[0], &in)) {
+        napi_throw_type_error(env, nullptr, "input must be Uint8Array");
+        return nullptr;
+    }
+    std::vector<double> offs = get_numbers(env, argv[1]), lens = get_numbers(env, argv[2]);
+    uint32_t flags = 0;
+    napi_get_value_uint32(env, argv[3], &flags);
+    const size_t n = offs.size();
+    Bytes dict;
+    std::vector<zlb_dict> dicts;
+    if (!get_dict(env, argc, argv, 4, n, &dict, &dicts)) return nullptr;
+    std::vector<zlb_item> items(n);
+    std::vector<zlb_result> res(n);
+    for (size_t i = 0; i < n; ++i) {
+        items[i].in_off = (uint64_t)offs[i];
+        items[i].in_len = (uint64_t)lens[i];
+    }
+    int rc = zlb_inflate_size_batch_host(g_ctx, in.p, in.n, dicts.empty() ? nullptr : dicts.data(), items.data(),
+                                         res.data(), n, flags);
+    if (rc != ZLB_OK) {
+        napi_throw_error(env, nullptr, zlb_last_error(g_ctx));
+        return nullptr;
+    }
+    std::vector<double> st(n), out_len(n), used(n), blocks(n);
+    for (size_t i = 0; i < n; ++i) {
+        st[i] = res[i].status;
+        out_len[i] = (double)res[i].out_len;
+        used[i] = (double)res[i].in_used;
+        blocks[i] = res[i].blocks;
+    }
+    napi_value result;
+    napi_create_object(env, &result);
+    napi_set_named_property(env, result, "status", num_array(env, st));
+    napi_set_named_property(env, result, "outLen", num_array(env, out_len));
+    napi_set_named_property(env, result, "inUsed", num_array(env, used));
+    napi_set_named_property(env, result, "blocks", num_array(env, blocks));
+    return result;
+}
+
 // checksumBatch(inputs, kinds)  <- CRC32.create / Adler32.create
 static napi_value ChecksumBatch(napi_env env, napi_callback_info info)
 {
@@ -493,6 +544,7 @@ static napi_value Init(napi_env env, napi_value exports)
     napi_property_descriptor d[] = {
         {"deflateBatch", nullptr, DeflateBatch, nullptr, nullptr, nullptr, napi_default, nullptr},
         {"inflateBatch", nullptr, InflateBatch, nullptr, nullptr, nullptr, napi_default, nullptr},
+        {"inflateSizes", nullptr, InflateSizes, nullptr, nullptr, nullptr, napi_default, nullptr},
         {"checksumBatch", nullptr, ChecksumBatch, nullptr, nullptr, nullptr, napi_default, nullptr},
         {"archive", nullptr, Archive, nullptr, nullptr, nullptr, napi_default, nullptr},
         {"crc32Combine", nullptr, Crc32Combine, nullptr, nullptr, nullptr, napi_default, nullptr},

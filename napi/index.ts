@@ -143,6 +143,12 @@ export class Inflate {                                                          
         return buffer;
     }
 }
+// Decompressed sizes of raw deflate streams input[offsets[i] .. + lengths[i]] without decoding their bytes (a
+// dictionary matters by its length only): exact RawInflate bufferSize / inflateBatch caps. flags: 8 = ZLB_INFLATE_SPLIT.
+export const inflateSizes = (input: Uint8Array, offsets: number[], lengths: number[], flags = 8, dictionary?: Uint8Array) =>
+    native.inflateSizes(input, offsets, lengths, flags, dictionary) as
+    { status: number[]; outLen: number[]; inUsed: number[]; blocks: number[] };
+
 // Whole containers in one call (what GZip.compress / Zip.compress do entry by entry, src/GZip.ts:96-194,
 // src/Zip.ts:117-372): every entry checksummed + deflated in one batch, headers / trailers / central directory / end
 // record written and packed on the device. heads / cdirs / tail are the byte templates described in the header.

@@ -13,6 +13,6 @@ from . import synth  # noqa: F401
 from . import api  # noqa: F401,E402
 from .api import (  # noqa: F401,E402
     Zlib, Deflate, Inflate, GZip, GUnzip, Zip, Unzip, RawDeflate, RawInflate, CRC32, Adler32, ZlibError,
-    CompressionType, BufferType, ZipCompressionMethod, deflate_many, inflate_many, inflate_blob, checksum_many,
+    CompressionType, BufferType, ZipCompressionMethod, deflate_many, inflate_many, inflate_blob, inflate_sizes, checksum_many,
     archive_many, zlib_many, gzip_many,
 )

@@ -46,6 +46,7 @@ EXPORTS = [
     "zlb_debug_lz77", "zlb_debug_code_lengths",
     "zlb_host_alloc", "zlb_host_free", "zlb_host_is_pinned",
     "zlb_deflate_batch_dict", "zlb_deflate_batch_dict_host", "zlb_inflate_batch_dict", "zlb_inflate_batch_dict_host",
+    "zlb_inflate_size_batch", "zlb_inflate_size_batch_host",
 ]
 
 _lib = None
@@ -89,6 +90,10 @@ def load_library():
     lib.zlb_inflate_batch_dict.restype = i32
     lib.zlb_inflate_batch_dict_host.argtypes = [vp, vp, sz, vp, sz, vp, sz, vp, vp, vp, sz, u32]
     lib.zlb_inflate_batch_dict_host.restype = i32
+    lib.zlb_inflate_size_batch.argtypes = [vp, vp, vp, vp, vp, sz, u32]
+    lib.zlb_inflate_size_batch.restype = i32
+    lib.zlb_inflate_size_batch_host.argtypes = [vp, vp, sz, vp, vp, vp, sz, u32]
+    lib.zlb_inflate_size_batch_host.restype = i32
     lib.zlb_checksum_batch.argtypes = [vp, vp, vp, vp, sz, u32]
     lib.zlb_checksum_batch.restype = i32
     lib.zlb_checksum_batch_host.argtypes = [vp, vp, sz, vp, vp, sz, u32]
@@ -303,6 +308,17 @@ class Engine:
         self._check(rc, "zlb_inflate_batch")
         return results
 
+    def inflate_size_batch(self, d_in, items, flags=0, dicts=None):
+        """zlb_inflate_size_batch: the decompressed size of every item (results' out_len), nothing written; `dicts`
+        (DICT_DTYPE) is read for its lengths only."""
+        items, results = self._tables(items)
+        dicts = self._dicts(dicts)
+        rc = self.lib.zlb_inflate_size_batch(self.h, d_in.data_ptr() if d_in is not None else None,
+                                             None if dicts is None else dicts.ctypes.data, items.ctypes.data,
+                                             results.ctypes.data, len(items), flags)
+        self._check(rc, "zlb_inflate_size_batch")
+        return results
+
     def checksum_batch(self, d_in, items, kinds=SUM_CRC32 | SUM_ADLER32):
         items, results = self._tables(items)
         rc = self.lib.zlb_checksum_batch(self.h, d_in.data_ptr(), items.ctypes.data, results.ctypes.data,
@@ -352,6 +368,16 @@ class Engine:
             rc = self.lib.zlb_inflate_batch_dict_host(self.h, pi, ni, po, no, pd, nd, dicts.ctypes.data,
                                                       items.ctypes.data, results.ctypes.data, len(items), flags)
         self._check(rc, "zlb_inflate_batch_host")
+        return results
+
+    def inflate_size_batch_host(self, h_in, items, flags=0, dicts=None):
+        """zlb_inflate_size_batch_host (see inflate_size_batch)."""
+        items, results = self._tables(items)
+        pi, ni, ki = self._host_ptr(h_in) if h_in is not None else (None, 0, None)
+        dicts = self._dicts(dicts)
+        rc = self.lib.zlb_inflate_size_batch_host(self.h, pi, ni, None if dicts is None else dicts.ctypes.data,
+                                                  items.ctypes.data, results.ctypes.data, len(items), flags)
+        self._check(rc, "zlb_inflate_size_batch_host")
         return results
 
     def checksum_batch_host(self, h_in, items, kinds=SUM_CRC32 | SUM_ADLER32):

@@ -24,6 +24,9 @@ Deviations from the reference, all deliberate (SURVEY.md Appendix B):
     (RFC 1950); Inflate reads FDICT streams when given the dictionary whose Adler-32 is DICTID, where the reference
     always throws "fdict flag is not supported" (it still does here without a dictionary). A dictionary given for a
     stream without FDICT is ignored, as zlib does. Only a dictionary's last 32 KiB can be reached.
+  * decompressed sizes without decoding the bytes: `inflate_sizes` (zlb_inflate_size_batch) returns what each stream
+    inflates to, so that the output slots of `inflate_many(..., size_hints=sizes)` or RawInflate's `bufferSize` are
+    exact and that call needs no retry. The reference has no such query (its buffer grows while it decodes).
 """
 import datetime
 import struct
@@ -250,6 +253,29 @@ def inflate_many(buffers, indices=None, size_hints=None, want_crc32=False, want_
     blob = np.concatenate(arrs) if int(lens.sum()) else np.zeros(1, dtype=np.uint8)
     idx = np.minimum(idx, lens)
     return inflate_blob(blob, base + idx, lens - idx, size_hints, want_crc32, want_adler32, dictionary=dictionary)
+
+
+def inflate_sizes(buffers, indices=None, dictionary=None):
+    """Decompressed size of the stream in every buffer (starting at indices[i]) as a uint64 array, from one size-only
+    GPU call that writes no output (ZLB_INFLATE_SPLIT, as inflate_many); `dictionary` as for deflate_many (only its
+    length matters). Raises ZlibError with the text inflate_many would raise for a corrupt stream."""
+    arrs = [_u8(x) for x in buffers]
+    n = len(arrs)
+    if n == 0:
+        return np.zeros(0, dtype=np.uint64)
+    idx = np.zeros(n, dtype=np.uint64) if indices is None else np.asarray(indices, dtype=np.uint64)
+    lens = np.array([a.size for a in arrs], dtype=np.uint64)
+    base = np.concatenate([[0], np.cumsum(lens)[:-1]]).astype(np.uint64)
+    blob = np.concatenate(arrs) if int(lens.sum()) else np.zeros(1, dtype=np.uint8)
+    idx = np.minimum(idx, lens)
+    _, dicts = _dict_table(dictionary, n)
+    items = N.make_items(n)
+    items["in_off"], items["in_len"] = base + idx, lens - idx
+    res = engine().inflate_size_batch_host(blob, items, N.INFLATE_SPLIT, dicts)
+    for st in res["status"]:
+        if int(st) != N.ST_OK:
+            raise ZlibError(status_text(st))
+    return res["out_len"].astype(np.uint64)
 
 
 def checksum_many(buffers, crc32=True, adler32=True):

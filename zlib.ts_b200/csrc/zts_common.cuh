@@ -32,6 +32,7 @@ enum ZtsKernelSlot {
     ZK_WINDOW_RESOLVE,
     ZK_DICT_STAGE,      // preset dictionaries (zts_deflate.cu, zts_inflate.cu)
     ZK_INFLATE_DICT,
+    ZK_INFLATE_SIZE,    // zlb_inflate_size_batch (zts_inflate.cu)
     ZK_COUNT
 };
 
@@ -42,7 +43,7 @@ static const char* const kZtsKernelNames[ZK_COUNT] = {
     "marker_scan_kernel",  "segment_gather_kernel",
     "frame_body_kernel",   "frame_header_kernel",
     "inflate_warp_kernel_window", "window_run_kernel", "window_scan_kernel", "window_resolve_kernel",
-    "dict_stage_kernel", "inflate_warp_kernel_dict"};
+    "dict_stage_kernel", "inflate_warp_kernel_dict", "inflate_warp_kernel_size"};
 
 struct ZtsDevBuf {
     void* p = nullptr;
@@ -109,9 +110,11 @@ int zts_stage_end(zlb_ctx* ctx, ZtsHostStage* st);
 void zts_stage_destroy_ctx(zlb_ctx* ctx);
 // The checks every batch entry point makes first, in this order: the pointers (bufs_ok: the caller's data buffers are
 // given where they are needed), n == 0 (returns 1: nothing to do), at most max_items items, the dictionary table
-// (zts_check_dicts); then the context's device is selected.
+// (zts_check_dicts); then the context's device is selected. dict_lens_only: a call that reads the dictionaries'
+// lengths only (a size call) and has no blob.
 int zts_entry_begin(zlb_ctx* ctx, bool bufs_ok, const zlb_item* items, const zlb_result* results, size_t n,
-                    size_t max_items, const void* dict_blob, size_t dict_bytes, const zlb_dict* dicts, bool* any);
+                    size_t max_items, const void* dict_blob, size_t dict_bytes, const zlb_dict* dicts, bool* any,
+                    bool dict_lens_only = false);
 // Host buffers of a "_host" entry point, as its device path sees them. Their bytes travel through the staging arenas
 // ctx->d_stage_in / d_stage_out, the dictionary blob through ctx->d_dict.
 struct ZtsHostIO {
@@ -123,17 +126,22 @@ struct ZtsHostIO {
 };
 // A "_host" entry point: zts_entry_begin, every item inside the blobs, the dictionary blob to the device, the staging
 // arenas and the copy threads; then body(io, dictionary table or NULL when no item has one) and a synchronise.
-// The copy threads are drained on every path, errors included.
+// The copy threads are drained on every path, errors included. ZTS_HOST_SIZES: a call without an output blob (h_out /
+// out_bytes unused; the items' out_off / out_cap are not looked at) that reads its dictionaries' lengths only (no
+// dictionary blob).
+enum ZtsHostKind { ZTS_HOST_DATA = 0, ZTS_HOST_SIZES = 1 };
 int zts_host_call(zlb_ctx* ctx, const void* h_in, size_t in_bytes, void* h_out, size_t out_bytes, const void* h_dict,
                   size_t dict_bytes, const zlb_dict* dicts, const zlb_item* items, const zlb_result* results, size_t n,
-                  size_t max_items, const std::function<int(ZtsHostIO& io, const zlb_dict* dicts)>& body);
+                  size_t max_items, const std::function<int(ZtsHostIO& io, const zlb_dict* dicts)>& body,
+                  ZtsHostKind kind = ZTS_HOST_DATA);
 // D2H of what items [a, b) wrote (adjacent ranges merged; see zts_ctx.cu); h_out = zts_stage_out_ptr() when staged
 int zts_copy_back(zlb_ctx* ctx, ZtsHostStage* st, cudaStream_t s, const uint8_t* d_out, uint8_t* h_out,
                   const zlb_item* h_items, const zlb_result* h_res, const zlb_item* d_items, const zlb_result* d_res,
                   size_t a, size_t b);
 // preset dictionaries: checks a table (NULL = none; blob_bytes = SIZE_MAX when the blob's size is not known, i.e. a
-// device blob) and tells whether any item has one
-int zts_check_dicts(zlb_ctx* ctx, const void* blob, size_t blob_bytes, const zlb_dict* dicts, size_t n, bool* any);
+// device blob; lens_only: there is no blob, only the lengths are used) and tells whether any item has one
+int zts_check_dicts(zlb_ctx* ctx, const void* blob, size_t blob_bytes, const zlb_dict* dicts, size_t n, bool* any,
+                    bool lens_only = false);
 void zts_prof_begin(zlb_ctx* ctx, int slot);
 void zts_prof_end(zlb_ctx* ctx, int slot);
 

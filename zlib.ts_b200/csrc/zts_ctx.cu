@@ -34,17 +34,19 @@ int zts_reserve(zlb_ctx* ctx, ZtsDevBuf* b, size_t bytes)
     return ZLB_OK;
 }
 
-int zts_check_dicts(zlb_ctx* ctx, const void* blob, size_t blob_bytes, const zlb_dict* dicts, size_t n, bool* any)
+int zts_check_dicts(zlb_ctx* ctx, const void* blob, size_t blob_bytes, const zlb_dict* dicts, size_t n, bool* any,
+                    bool lens_only)
 {
     *any = false;
     if (!dicts) return ZLB_OK;
     for (size_t i = 0; i < n; ++i) {
         const zlb_dict d = dicts[i];
         if (d.len == 0) continue;
+        *any = true;
+        if (lens_only) continue;
         if (!blob) return zts_fail(ctx, ZLB_E_ARG, "item %zu has a dictionary but the dictionary blob is NULL", i);
         if (d.off > blob_bytes || d.len > blob_bytes - d.off)
             return zts_fail(ctx, ZLB_E_ARG, "dictionary of item %zu out of range", i);
-        *any = true;
     }
     return ZLB_OK;
 }

@@ -232,12 +232,13 @@ void zts_stage_destroy_ctx(zlb_ctx* ctx)
 
 // ---- what the batch entry points share ------------------------------------------------------------------------------
 int zts_entry_begin(zlb_ctx* ctx, bool bufs_ok, const zlb_item* items, const zlb_result* results, size_t n,
-                    size_t max_items, const void* dict_blob, size_t dict_bytes, const zlb_dict* dicts, bool* any)
+                    size_t max_items, const void* dict_blob, size_t dict_bytes, const zlb_dict* dicts, bool* any,
+                    bool dict_lens_only)
 {
     if (!ctx || !bufs_ok || (!items && n) || (!results && n)) return ZLB_E_ARG;
     if (n == 0) return 1;
     if (n > max_items) return zts_fail(ctx, ZLB_E_ARG, "too many items");
-    int rc = zts_check_dicts(ctx, dict_blob, dict_bytes, dicts, n, any);
+    int rc = zts_check_dicts(ctx, dict_blob, dict_bytes, dicts, n, any, dict_lens_only);
     if (rc) return rc;
     ZTS_CUDA(ctx, cudaSetDevice(ctx->device));
     return ZLB_OK;
@@ -245,25 +246,30 @@ int zts_entry_begin(zlb_ctx* ctx, bool bufs_ok, const zlb_item* items, const zlb
 
 int zts_host_call(zlb_ctx* ctx, const void* h_in, size_t in_bytes, void* h_out, size_t out_bytes, const void* h_dict,
                   size_t dict_bytes, const zlb_dict* dicts, const zlb_item* items, const zlb_result* results, size_t n,
-                  size_t max_items, const std::function<int(ZtsHostIO& io, const zlb_dict* dicts)>& body)
+                  size_t max_items, const std::function<int(ZtsHostIO& io, const zlb_dict* dicts)>& body,
+                  ZtsHostKind kind)
 {
+    const bool sizes = kind == ZTS_HOST_SIZES;
+    if (sizes) {
+        h_out = nullptr;
+        out_bytes = 0;
+    }
     bool any = false;
     int rc = zts_entry_begin(ctx, (h_in || !in_bytes) && (h_out || !out_bytes), items, results, n, max_items, h_dict,
-                             dict_bytes, dicts, &any);
+                             dict_bytes, dicts, &any, sizes);
     if (rc) return rc > 0 ? ZLB_OK : rc;
     for (size_t i = 0; i < n; ++i) {
-        if (items[i].in_off + items[i].in_len > in_bytes || items[i].out_off + items[i].out_cap > out_bytes)
+        if (items[i].in_off + items[i].in_len > in_bytes || (!sizes && items[i].out_off + items[i].out_cap > out_bytes))
             return zts_fail(ctx, ZLB_E_ARG, "item %zu out of range", i);
     }
     // the dictionaries go over first, on the context's stream (everything of the call is ordered behind it)
-    if (any) {
+    if (any && !sizes) {
         if ((rc = zts_reserve(ctx, &ctx->d_dict, dict_bytes + 256))) return rc;
         ZTS_CUDA(ctx, cudaMemcpyAsync(ctx->d_dict.p, h_dict, dict_bytes, cudaMemcpyHostToDevice, ctx->stream));
     }
     rc = zts_reserve(ctx, &ctx->d_stage_in, in_bytes + 256);
     if (rc) return rc;
-    rc = zts_reserve(ctx, &ctx->d_stage_out, out_bytes + 256);
-    if (rc) return rc;
+    if (!sizes && (rc = zts_reserve(ctx, &ctx->d_stage_out, out_bytes + 256))) return rc;
     ZtsHostStage* stage = nullptr;
     rc = zts_stage_begin(ctx, h_in, in_bytes, h_out, out_bytes, &stage);
     if (!rc) {

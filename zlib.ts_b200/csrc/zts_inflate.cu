@@ -338,9 +338,13 @@ __device__ uint32_t inf_classify_symbols(const InfWarpSmem* S, const uint8_t* sr
 // copy code below is the same for both: a match that reaches before the piece copies window words. INF_DICT: the
 // decoder with a preset dictionary (dicts[item] in the blob `dict`, zlb_inflate_batch_dict): a match may reach up to
 // the dictionary's last 32768 bytes in front of the output; one whose source starts there takes a path of its own.
-// The dictionary arguments are read by INF_DICT only.
+// The dictionary arguments are read by INF_DICT only. INF_SIZE: the decoder without an output (zlb_inflate_size_batch):
+// it decodes and checks exactly like INF_BYTES but stores no byte, copies no match, skips stored data after its LEN
+// check and has no capacity; only the dictionary's length is read (dicts may be NULL). In segment mode a distance that
+// reaches before the piece's first byte does not fail it: results[item].crc32 tells how far in front the piece
+// reached, at most 32768 (the marker split compares that with the output of the pieces in front).
 #define WIN_WORDS 32768u
-enum { INF_BYTES = 0, INF_WINDOW = 1, INF_DICT = 2 };
+enum { INF_BYTES = 0, INF_WINDOW = 1, INF_DICT = 2, INF_SIZE = 3 };
 template <int MODE>
 __global__ void __launch_bounds__(INF_WARPS_PER_CTA * 32, INF_MIN_CTAS)
 inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, const zlb_item* __restrict__ items,
@@ -365,6 +369,15 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
         reach = d.len < WIN_WORDS ? (uint32_t)d.len : WIN_WORDS;
         dtail = dict + d.off + d.len - reach;
     }
+    if constexpr (MODE == INF_SIZE) {
+        if (flags & ZLB_INFLATE_SEGMENT) {
+            reach = WIN_WORDS;  // (every distance: how far it went is recorded instead)
+        } else if (dicts) {
+            const unsigned long long l = dicts[item].len;
+            reach = l < WIN_WORDS ? (uint32_t)l : WIN_WORDS;
+        }
+    }
+    uint32_t reached = 0;  // INF_SIZE: the farthest a match reached in front of the output
     if constexpr (MODE == INF_WINDOW) {
         uint4* w = reinterpret_cast<uint4*>(dst - WIN_WORDS);  // (slots are 256-byte aligned)
         for (uint32_t i = lane; i < WIN_WORDS / 8; i += 32) {
@@ -420,11 +433,12 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
                 status = ZLB_ST_INPUT_BROKEN;
                 break;
             }
-            if (op + len > cap) {
+            if (MODE != INF_SIZE && op + len > cap) {
                 status = ZLB_ST_OUT_OVERFLOW;
                 break;
             }
-            for (uint32_t k = lane; k < len; k += 32) dst[op + k] = src[byte_pos + k];
+            if constexpr (MODE != INF_SIZE)
+                for (uint32_t k = lane; k < len; k += 32) dst[op + k] = src[byte_pos + k];
             op += len;
             br_init(br, src + byte_pos + len, src + it.in_len, (byte_pos + len) * 8ull);
             __syncwarp();
@@ -655,7 +669,7 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
             // a distance beyond the start of the output (the reference would copy `undefined` -> 0) or an
             // output slot that is too small ends the batch before the offending token
             const bool bad_dist = is_match && dist > behind + rel + reach;
-            const bool over = mine && rel + len > room;
+            const bool over = MODE != INF_SIZE && mine && rel + len > room;
             const unsigned bad_mask = __ballot_sync(0xFFFFFFFFu, bad_dist || over);
             uint32_t nvalid = ntok;
             if (bad_mask) {
@@ -664,6 +678,13 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
                 status = first_is_dist ? ZLB_ST_BAD_CODE : ZLB_ST_OUT_OVERFLOW;
             }
             const bool live = lane < nvalid;
+            if constexpr (MODE == INF_SIZE) {
+                // nothing is written: the batch moves the cursor and tells how far its matches reached
+                if (live && is_match && dist > behind + rel) reached = max(reached, dist - (behind + rel));
+                op += nvalid ? __shfl_sync(0xFFFFFFFFu, inc, (int)nvalid - 1) : 0u;
+                __syncwarp();
+                continue;
+            }
             // -- literals: one store
             ZTS_ASSERT(!live || (op + rel + len <= cap && (!is_match || dist <= op + rel + reach)));
             if (live && !is_match) bdst[rel] = (uint8_t)(mytok >> 16);
@@ -740,8 +761,10 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
         if (status == ZLB_ST_OK && br_bits_used(br) > in_bits) status = ZLB_ST_INPUT_BROKEN;
     }
 
+    if constexpr (MODE == INF_SIZE) reached = __reduce_max_sync(0xFFFFFFFFu, reached);
     if (lane == 0) {
         zlb_result r = results[item];
+        if (MODE == INF_SIZE && (flags & ZLB_INFLATE_SEGMENT)) r.crc32 = reached;
         r.status = status;
         r.blocks = blocks | ((flags & ZLB_INFLATE_SEGMENT) && bfinal ? 0x80000000u : 0u);  // segment mode: saw BFINAL
         r.out_len = op;
@@ -758,16 +781,19 @@ static int inflate_launch_mode(zlb_ctx* ctx, cudaStream_t st, const uint8_t* d_i
     const size_t smem = sizeof(InfWarpSmem) * INF_WARPS_PER_CTA;
     ZTS_CUDA(ctx, cudaFuncSetAttribute(inflate_warp_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     unsigned grid = (unsigned)((n + INF_WARPS_PER_CTA - 1) / INF_WARPS_PER_CTA);
-    ZTS_LAUNCH(ctx, MODE == INF_WINDOW ? ZK_INFLATE_WINDOW : MODE == INF_DICT ? ZK_INFLATE_DICT : ZK_INFLATE,
+    ZTS_LAUNCH(ctx,
+               MODE == INF_WINDOW ? ZK_INFLATE_WINDOW : MODE == INF_DICT ? ZK_INFLATE_DICT : MODE == INF_SIZE ? ZK_INFLATE_SIZE : ZK_INFLATE,
                inflate_warp_kernel<MODE><<<grid, INF_WARPS_PER_CTA * 32, smem, st>>>(d_in, d_out, d_items, d_results,
                                                                                     (uint32_t)n, flags, d_dicts, d_dict));
     return ZLB_OK;
 }
-// the decoder: with a dictionary table (d_dicts[i] belongs to d_items[i]) the dictionary instantiation
+// the decoder: with a dictionary table (d_dicts[i] belongs to d_items[i]) the dictionary instantiation; without an
+// output (d_out == NULL, a size call) the size instantiation, which reads the table's lengths only
 static int inflate_launch(zlb_ctx* ctx, cudaStream_t st, const uint8_t* d_in, uint8_t* d_out, const zlb_item* d_items,
                           zlb_result* d_results, size_t n, uint32_t flags, const zlb_dict* d_dicts = nullptr,
                           const uint8_t* d_dict = nullptr)
 {
+    if (!d_out) return inflate_launch_mode<INF_SIZE>(ctx, st, d_in, nullptr, d_items, d_results, n, flags, d_dicts, nullptr);
     if (d_dicts) return inflate_launch_mode<INF_DICT>(ctx, st, d_in, d_out, d_items, d_results, n, flags, d_dicts, d_dict);
     return inflate_launch_mode<INF_BYTES>(ctx, st, d_in, d_out, d_items, d_results, n, flags, nullptr, nullptr);
 }
@@ -1000,20 +1026,33 @@ static int split_chain(const zlb_result* r, const zlb_item* seg, size_t n, bool 
     return reaches ? SPLIT_WINDOW : SPLIT_OK;
 }
 
-// result of an item whose n pieces passed the checks; their bytes (r[j].out_len at scratch offset seg[j].out_off)
+// result of an item whose n pieces passed the checks, the last one starting at input byte last_start of the item
+static zlb_result split_result(const zlb_result* r, size_t n, unsigned long long last_start)
+{
+    zlb_result o;
+    memset(&o, 0, sizeof o);
+    unsigned long long blocks = 0;
+    for (size_t j = 0; j < n; ++j) {
+        o.out_len += r[j].out_len;
+        blocks += r[j].blocks & 0x7FFFFFFFu;
+    }
+    o.status = ZLB_ST_OK;
+    o.in_used = last_start + r[n - 1].in_used;
+    o.blocks = (uint32_t)blocks;
+    return o;
+}
+
+// split_result, checked against the item's slot; the pieces' bytes (r[j].out_len at scratch offset seg[j].out_off)
 // are queued for the gather when they fit
 static void split_finish(const zlb_item& it, const zlb_result* r, const zlb_item* seg, size_t n, unsigned long long last_start,
                          zlb_result& o, std::vector<ZtsGather>& gath)
 {
-    unsigned long long total = 0, blocks = 0;
-    for (size_t j = 0; j < n; ++j) {
-        total += r[j].out_len;
-        blocks += r[j].blocks & 0x7FFFFFFFu;
+    o = split_result(r, n, last_start);
+    const unsigned long long total = o.out_len;
+    if (total > it.out_cap) {
+        o.status = ZLB_ST_OUT_OVERFLOW;
+        o.out_len = 0;
     }
-    o.status = total > it.out_cap ? ZLB_ST_OUT_OVERFLOW : ZLB_ST_OK;
-    o.out_len = total > it.out_cap ? 0 : total;
-    o.in_used = last_start + r[n - 1].in_used;
-    o.blocks = (uint32_t)blocks;
     if (total <= it.out_cap && total) {
         unsigned long long at = 0;
         for (size_t j = 0; j < n; ++j) {
@@ -1182,19 +1221,20 @@ static int inflate_split_window(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_sc
     return ZLB_OK;
 }
 
-// Tries to decode the items h_items[big[*]] piecewise, all of them in one pass: one marker scan per item (queued back
-// to back, one read-back for all), one segment-mode launch over the pieces of every item, one window-mode pass for
-// the items whose pieces reach into their predecessors, one gather. done[k] tells whether big[k] worked (then res[k]
-// is filled); the others have to go through the serial decoder. < 0 on API errors.
+// The pieces of the items h_items[big[*]]: one marker scan per item (queued back to back, one read-back for all), a
+// piece starting at 0 and behind every marker that leaves at least one byte. Pieces of item k: [first[k], first[k + 1]),
+// none when it has no marker inside; seg[j] = piece j's input span (out_off / out_cap 0). res / done are reset for
+// nb items, none done. No pieces at all: nothing to split. < 0 on API errors.
 #define SPLIT_TAG_SHIFT 40  // marks carry the item's index above the byte offset (offsets < 1 TiB, < 16 M large items)
-static int inflate_split_batch(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const zlb_item* h_items,
-                               const zlb_dict* h_dicts, const uint8_t* d_dict, const std::vector<size_t>& big,
-                               uint32_t flags, std::vector<zlb_result>& res, std::vector<char>& done)
+static int split_layout(zlb_ctx* ctx, const uint8_t* d_in, const zlb_item* h_items, const std::vector<size_t>& big,
+                        std::vector<zlb_result>& res, std::vector<char>& done, std::vector<SplitPiece>& pieces,
+                        std::vector<size_t>& first, std::vector<zlb_item>& seg)
 {
     const size_t nb = big.size();
     res.assign(nb, zlb_result());
     done.assign(nb, 0);
     for (size_t k = 0; k < nb; ++k) memset(&res[k], 0, sizeof(zlb_result));
+    pieces.clear();
     if (nb >= (1ull << 24)) return ZLB_OK;
     cudaStream_t st = ctx->stream;
     int rc = zts_reserve(ctx, &ctx->d_misc, (size_t)SPLIT_MAX_MARKS * 8 + 256);
@@ -1218,37 +1258,53 @@ static int inflate_split_batch(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out
     ZTS_CUDA(ctx, cudaMemcpyAsync(marks.data(), d_marks, (size_t)count * 8, cudaMemcpyDeviceToHost, st));
     ZTS_CUDA(ctx, cudaStreamSynchronize(st));
     std::sort(marks.begin(), marks.end());  // by item, then by offset
-    // pieces of every item: it starts at 0 and behind every marker that leaves at least one byte
-    std::vector<SplitPiece> pieces;
-    std::vector<size_t> first(nb + 1, 0);  // pieces of item k: [first[k], first[k + 1])
-    {
-        size_t mi = 0;
-        for (size_t k = 0; k < nb; ++k) {
-            first[k] = pieces.size();
-            const unsigned long long n = h_items[big[k]].in_len;
-            pieces.push_back({(uint32_t)k, 0ull});
-            for (; mi < marks.size() && (marks[mi] >> SPLIT_TAG_SHIFT) == k; ++mi) {
-                const unsigned long long m = marks[mi] & ((1ull << SPLIT_TAG_SHIFT) - 1);
-                // a piece of this engine's streams holds a whole block: never closer than SPLIT_MIN_PIECE bytes to the
-                // previous cut (a hostile stream of empty stored blocks would otherwise ask for a slot per 5 bytes)
-                if (m < n && m >= pieces.back().start + SPLIT_MIN_PIECE) pieces.push_back({(uint32_t)k, m});
-            }
-            if (pieces.size() - first[k] < 2) pieces.resize(first[k]);  // no marker inside: nothing to gain
+    first.assign(nb + 1, 0);
+    size_t mi = 0;
+    for (size_t k = 0; k < nb; ++k) {
+        first[k] = pieces.size();
+        const unsigned long long n = h_items[big[k]].in_len;
+        pieces.push_back({(uint32_t)k, 0ull});
+        for (; mi < marks.size() && (marks[mi] >> SPLIT_TAG_SHIFT) == k; ++mi) {
+            const unsigned long long m = marks[mi] & ((1ull << SPLIT_TAG_SHIFT) - 1);
+            // a piece of this engine's streams holds a whole block: never closer than SPLIT_MIN_PIECE bytes to the
+            // previous cut (a hostile stream of empty stored blocks would otherwise ask for a slot per 5 bytes)
+            if (m < n && m >= pieces.back().start + SPLIT_MIN_PIECE) pieces.push_back({(uint32_t)k, m});
         }
-        first[nb] = pieces.size();
+        if (pieces.size() - first[k] < 2) pieces.resize(first[k]);  // no marker inside: nothing to gain
     }
-    const size_t np = pieces.size();
-    if (np == 0) return ZLB_OK;
-    // slots: a piece of L compressed bytes cannot inflate to more than ~1032 L (258 bytes per 2 bits at best), and a
-    // piece of this engine's streams holds at most one 64 KiB chunk
-    std::vector<zlb_item> seg(np);
-    size_t scratch = 0, big_in = 0;
+    first[nb] = pieces.size();
+    seg.assign(pieces.size(), zlb_item{0, 0, 0, 0});
     for (size_t k = 0; k < nb; ++k) {
         const zlb_item& it = h_items[big[k]];
-        if (first[k + 1] > first[k]) big_in += it.in_len;
         for (size_t j = first[k]; j < first[k + 1]; ++j) {
             seg[j].in_off = it.in_off + pieces[j].start;
             seg[j].in_len = (j + 1 < first[k + 1] ? pieces[j + 1].start : it.in_len) - pieces[j].start;
+        }
+    }
+    return ZLB_OK;
+}
+
+// Tries to decode the items h_items[big[*]] piecewise, all of them in one pass: the marker scan (split_layout), one
+// segment-mode launch over the pieces of every item, one window-mode pass for the items whose pieces reach into their
+// predecessors, one gather. done[k] tells whether big[k] worked (then res[k] is filled); the others have to go through
+// the serial decoder. < 0 on API errors.
+static int inflate_split_batch(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const zlb_item* h_items,
+                               const zlb_dict* h_dicts, const uint8_t* d_dict, const std::vector<size_t>& big,
+                               uint32_t flags, std::vector<zlb_result>& res, std::vector<char>& done)
+{
+    std::vector<SplitPiece> pieces;
+    std::vector<size_t> first;
+    std::vector<zlb_item> seg;
+    int rc = split_layout(ctx, d_in, h_items, big, res, done, pieces, first, seg);
+    if (rc || pieces.empty()) return rc;
+    const size_t nb = big.size(), np = pieces.size();
+    cudaStream_t st = ctx->stream;
+    // slots: a piece of L compressed bytes cannot inflate to more than ~1032 L (258 bytes per 2 bits at best), and a
+    // piece of this engine's streams holds at most one 64 KiB chunk
+    size_t scratch = 0, big_in = 0;
+    for (size_t k = 0; k < nb; ++k) {
+        if (first[k + 1] > first[k]) big_in += h_items[big[k]].in_len;
+        for (size_t j = first[k]; j < first[k + 1]; ++j) {
             size_t slot = (size_t)seg[j].in_len * 1032u + 512u;
             if (slot > SPLIT_SLOT) slot = SPLIT_SLOT;
             slot = (slot + 255) & ~(size_t)255;
@@ -1295,6 +1351,51 @@ static int inflate_split_batch(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out
         ZTS_CUDA(ctx, cudaMemcpyAsync(d_gather, gath.data(), gath.size() * sizeof(ZtsGather), cudaMemcpyHostToDevice, st));  // <= np entries
         ZTS_LAUNCH(ctx, ZK_GATHER, segment_gather_kernel<<<(unsigned)gath.size(), 256, 0, st>>>(d_scratch, d_out, d_gather));
         ZTS_CUDA(ctx, cudaStreamSynchronize(st));  // gath goes out of scope
+    }
+    return ZLB_OK;
+}
+
+// The marker split of a size call: the items h_items[big[*]] are cut as inflate_split_batch cuts them and every piece of
+// every item is sized by one segment-mode launch of the size decoder. A piece's size does not depend on the bytes in
+// front of it, only whether a distance reaches before the stream (or before its dictionary) does, and a piece tells
+// how far in front of its first byte it reached (crc32). So an item is settled when its chain passes and no piece
+// reaches further than the output of the pieces in front of it plus the dictionary's reachable bytes; it then gets
+// the one-warp decoder's result by construction. No byte slots and no window scratch: the piece tables take the place
+// of the marks. done / res as for inflate_split_batch.
+static int inflate_split_sizes(zlb_ctx* ctx, const uint8_t* d_in, const zlb_item* h_items, const zlb_dict* h_dicts,
+                               const std::vector<size_t>& big, uint32_t flags, std::vector<zlb_result>& res,
+                               std::vector<char>& done)
+{
+    std::vector<SplitPiece> pieces;
+    std::vector<size_t> first;
+    std::vector<zlb_item> seg;
+    int rc = split_layout(ctx, d_in, h_items, big, res, done, pieces, first, seg);
+    if (rc || pieces.empty()) return rc;
+    const size_t nb = big.size(), np = pieces.size();
+    cudaStream_t st = ctx->stream;
+    if ((rc = zts_reserve(ctx, &ctx->d_misc, np * (sizeof(zlb_item) + sizeof(zlb_result)) + 256))) return rc;
+    zlb_item* d_seg = (zlb_item*)ctx->d_misc.p;
+    zlb_result* d_segres = (zlb_result*)(d_seg + np);
+    ZTS_CUDA(ctx, cudaMemcpyAsync(d_seg, seg.data(), np * sizeof(zlb_item), cudaMemcpyHostToDevice, st));
+    ZTS_CUDA(ctx, cudaMemsetAsync(d_segres, 0, np * sizeof(zlb_result), st));
+    rc = inflate_launch(ctx, st, d_in, nullptr, d_seg, d_segres, np, (flags & ZLB_INFLATE_CHECK_NLEN) | ZLB_INFLATE_SEGMENT);
+    if (rc) return rc;
+    std::vector<zlb_result> sres(np);
+    ZTS_CUDA(ctx, cudaMemcpyAsync(sres.data(), d_segres, np * sizeof(zlb_result), cudaMemcpyDeviceToHost, st));
+    ZTS_CUDA(ctx, cudaStreamSynchronize(st));
+    for (size_t k = 0; k < nb; ++k) {
+        const size_t a = first[k], b = first[k + 1];
+        if (b - a < 2 || split_chain(&sres[a], &seg[a], b - a, false, false) != SPLIT_OK) continue;
+        const unsigned long long dl = h_dicts ? std::min(h_dicts[big[k]].len, (uint64_t)WIN_WORDS) : 0;
+        unsigned long long before = 0;  // output of the pieces in front
+        bool fits = true;
+        for (size_t j = a; j < b && fits; ++j) {
+            fits = sres[j].crc32 <= before + dl;
+            before += sres[j].out_len;
+        }
+        if (!fits) continue;
+        res[k] = split_result(&sres[a], b - a, pieces[b - 1].start);
+        done[k] = 1;
     }
     return ZLB_OK;
 }
@@ -1413,6 +1514,9 @@ static int inflate_waves(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, cons
 // Then one tail: checksums, the result read-back and, on a "_host" call, the copy-back of the outputs. A "_host" call
 // without a split runs in waves instead (inflate_waves).
 // d_dict / h_dicts: the preset dictionaries (h_dicts == NULL: none; checked by the caller)
+// d_out == NULL: a size call (zlb_inflate_size_batch). The same route with the size decoder, the split's sizing stage
+// (inflate_split_sizes) and no checksums (refused by the caller); nothing is written, d_dict is not read, a "_host"
+// call copies its input over in one piece and nothing back.
 static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const uint8_t* d_dict,
                           const zlb_dict* h_dicts, const zlb_item* h_items, zlb_result* h_results, size_t n, uint32_t flags,
                           const ZtsHostIO* hio)
@@ -1444,7 +1548,8 @@ static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
     uint32_t kinds = 0;
     if (flags & ZLB_INFLATE_WANT_CRC32) kinds |= ZLB_SUM_CRC32;
     if (flags & ZLB_INFLATE_WANT_ADLER32) kinds |= ZLB_SUM_ADLER32;
-    if (hio && big.empty())
+    const bool sizes = d_out == nullptr;
+    if (hio && big.empty() && !sizes)
         return inflate_waves(ctx, d_in, d_out, d_dict, d_items, d_dicts, d_results, h_items, h_results, n, flags, kinds, *hio);
 
     // the split: the items it decodes get their results in h_results; when it decoded any, rest lists the others
@@ -1455,14 +1560,15 @@ static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
     std::vector<size_t> rest;
     std::vector<zlb_item> rest_items;
     std::vector<zlb_dict> rest_dicts;
+    if (hio) {  // (a "_host" call that does not run in waves: its whole input first)
+        zts_stage_wait_in(hio->stage, 0, hio->in_bytes);
+        ZTS_CUDA(ctx, cudaMemcpyAsync((void*)d_in, hio->h_in, hio->in_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    }
     if (!big.empty()) {
-        if (hio) {
-            zts_stage_wait_in(hio->stage, 0, hio->in_bytes);
-            ZTS_CUDA(ctx, cudaMemcpyAsync((void*)d_in, hio->h_in, hio->in_bytes, cudaMemcpyHostToDevice, ctx->stream));
-        }
         std::vector<zlb_result> bres;
         std::vector<char> bdone, done(n, 0);
-        rc = inflate_split_batch(ctx, d_in, d_out, h_items, h_dicts, d_dict, big, flags, bres, bdone);
+        rc = sizes ? inflate_split_sizes(ctx, d_in, h_items, h_dicts, big, flags, bres, bdone)
+                   : inflate_split_batch(ctx, d_in, d_out, h_items, h_dicts, d_dict, big, flags, bres, bdone);
         if (rc) return rc;
         for (size_t k = 0; k < big.size(); ++k)
             if (bdone[k]) {
@@ -1500,7 +1606,7 @@ static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
         if (rc) return rc;
     }
     ZTS_CUDA(ctx, cudaMemcpyAsync(h_results, d_results, n * sizeof(zlb_result), cudaMemcpyDeviceToHost, ctx->stream));
-    if (hio) {
+    if (hio && !sizes) {
         ZTS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // the sizes decide what travels
         rc = zts_copy_back(ctx, hio->stage, ctx->stream, d_out, hio->h_out, h_items, h_results, d_items, d_results, 0, n);
         if (rc) return rc;
@@ -1545,4 +1651,41 @@ extern "C" int zlb_inflate_batch_host(zlb_ctx* ctx, const void* h_in, size_t in_
 {
     return zlb_inflate_batch_dict_host(ctx, h_in, in_bytes, h_out, out_bytes, nullptr, 0, nullptr, items, results, n,
                                        flags);
+}
+
+// the refusals of a size call, with a text: an input buffer is needed whenever there are items, checksums cannot be
+// computed without the bytes
+static int size_flags_check(zlb_ctx* ctx, bool in_ok, uint32_t flags)
+{
+    if (!ctx) return ZLB_E_ARG;
+    if (!in_ok) return zts_fail(ctx, ZLB_E_ARG, "the input buffer is NULL");
+    if (flags & (ZLB_INFLATE_WANT_CRC32 | ZLB_INFLATE_WANT_ADLER32))
+        return zts_fail(ctx, ZLB_E_ARG, "a size call computes no checksums (ZLB_INFLATE_WANT_CRC32 / _ADLER32)");
+    return ZLB_OK;
+}
+
+extern "C" int zlb_inflate_size_batch(zlb_ctx* ctx, const void* d_in, const zlb_dict* dicts, const zlb_item* items,
+                                      zlb_result* results, size_t n, uint32_t flags)
+{
+    int rc = size_flags_check(ctx, d_in || !n, flags);
+    if (rc) return rc;
+    bool any = false;
+    rc = zts_entry_begin(ctx, true, items, results, n, 0x7FFFFFFFull, nullptr, SIZE_MAX, dicts, &any, true);
+    if (rc) return rc > 0 ? ZLB_OK : rc;
+    rc = inflate_device(ctx, (const uint8_t*)d_in, nullptr, nullptr, any ? dicts : nullptr, items, results, n, flags,
+                        nullptr);
+    if (rc) return rc;
+    ZTS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return ZLB_OK;
+}
+
+extern "C" int zlb_inflate_size_batch_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes, const zlb_dict* dicts,
+                                           const zlb_item* items, zlb_result* results, size_t n, uint32_t flags)
+{
+    const int rc = size_flags_check(ctx, h_in || !n, flags);
+    if (rc) return rc;
+    return zts_host_call(ctx, h_in, in_bytes, nullptr, 0, nullptr, 0, dicts, items, results, n, 0x7FFFFFFFull,
+                         [&](ZtsHostIO& io, const zlb_dict* d) {
+        return inflate_device(ctx, (const uint8_t*)ctx->d_stage_in.p, nullptr, nullptr, d, items, results, n, flags, &io);
+    }, ZTS_HOST_SIZES);
 }
