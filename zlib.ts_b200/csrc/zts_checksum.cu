@@ -267,9 +267,9 @@ int zts_checksum_device(zlb_ctx* ctx, const uint8_t* d_in, const zlb_item* d_ite
     }
     if (n_slices > 0x7FFFFFFFull) return zts_fail(ctx, ZLB_E_ARG, "too many checksum slices");
     size_t tab_bytes = n_slices * sizeof(ZtsSlice) + (n + 1) * sizeof(uint32_t);
-    int rc = zts_reserve_pinned(ctx, tab_bytes);
+    int rc = zts_reserve_pinned(ctx, &ctx->h_pin, tab_bytes);
     if (rc) return rc;
-    ZtsSlice* h_sl = (ZtsSlice*)ctx->h_pin;
+    ZtsSlice* h_sl = (ZtsSlice*)ctx->h_pin.p;
     uint32_t* h_begin = (uint32_t*)(h_sl + n_slices);
     size_t k = 0;
     for (size_t i = 0; i < n; ++i) {

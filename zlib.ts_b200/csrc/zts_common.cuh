@@ -50,6 +50,11 @@ struct ZtsDevBuf {
     size_t cap = 0;
 };
 
+struct ZtsHostBuf {  // page-locked (cudaMallocHost)
+    void* p = nullptr;
+    size_t cap = 0;
+};
+
 struct ZtsProfRec {
     int slot;
     cudaEvent_t a, b;
@@ -66,11 +71,8 @@ struct zlb_ctx {
     // device arenas (grow-only, freed in zlb_destroy)
     ZtsDevBuf d_items, d_results, d_chunks, d_chunk_info, d_tokens, d_spec, d_hist, d_codes, d_sortT,
         d_sums, d_misc, d_stage_in, d_stage_out, d_split, d_window, d_body, d_frames, d_dict, d_dict_stage;
-    // pinned host staging for the small tables
-    void* h_pin = nullptr;
-    size_t h_pin_cap = 0;
-    void* h_pin2 = nullptr;  // read-back area of the pipelined host paths
-    size_t h_pin2_cap = 0;
+    // pinned host staging for the small tables, and the read-back area of the pipelined host paths (grow-only)
+    ZtsHostBuf h_pin, h_pin2;
     // copy / second compute streams of the pipelined host paths (created on first use)
     cudaStream_t s_in = nullptr, s_out = nullptr, s_aux[3] = {nullptr, nullptr, nullptr};
     cudaStream_t s_res = nullptr;  // small read-backs that must not queue behind (or in front of) anything else
@@ -95,8 +97,7 @@ struct zlb_ctx {
 
 int zts_fail(zlb_ctx* ctx, int code, const char* fmt, ...);
 int zts_reserve(zlb_ctx* ctx, ZtsDevBuf* b, size_t bytes);
-int zts_reserve_pinned(zlb_ctx* ctx, size_t bytes);
-int zts_reserve_pinned2(zlb_ctx* ctx, size_t bytes);
+int zts_reserve_pinned(zlb_ctx* ctx, ZtsHostBuf* b, size_t bytes);
 int zts_host_streams(zlb_ctx* ctx);                 // creates s_in / s_out / s_aux
 cudaEvent_t zts_sync_event(zlb_ctx* ctx, size_t k);  // k-th reusable ordering event (nullptr on failure)
 // host staging for pageable caller buffers (zts_hoststage.cu); every function accepts st == nullptr / unstaged sides
@@ -121,7 +122,6 @@ struct ZtsHostIO {
     const uint8_t* h_in;   // where H2D copies read from: the caller's page-locked buffer, or the library's shadow
     uint8_t* h_out;        // where D2H copies write to
     size_t in_bytes;
-    bool out_done;         // set by a device path that has already copied the output back, wave by wave
     ZtsHostStage* stage;   // copy threads behind the shadows (pageable caller buffers), see zts_hoststage.cu
 };
 // A "_host" entry point: zts_entry_begin, every item inside the blobs, the dictionary blob to the device, the staging
@@ -134,7 +134,8 @@ int zts_host_call(zlb_ctx* ctx, const void* h_in, size_t in_bytes, void* h_out, 
                   size_t dict_bytes, const zlb_dict* dicts, const zlb_item* items, const zlb_result* results, size_t n,
                   size_t max_items, const std::function<int(ZtsHostIO& io, const zlb_dict* dicts)>& body,
                   ZtsHostKind kind = ZTS_HOST_DATA);
-// D2H of what items [a, b) wrote (adjacent ranges merged; see zts_ctx.cu); h_out = zts_stage_out_ptr() when staged
+// D2H of what items [a, b) wrote (adjacent ranges merged; see zts_ctx.cu); h_out = zts_stage_out_ptr() when staged;
+// h_res and d_res hold the same results
 int zts_copy_back(zlb_ctx* ctx, ZtsHostStage* st, cudaStream_t s, const uint8_t* d_out, uint8_t* h_out,
                   const zlb_item* h_items, const zlb_result* h_res, const zlb_item* d_items, const zlb_result* d_res,
                   size_t a, size_t b);

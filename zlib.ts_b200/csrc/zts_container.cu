@@ -232,11 +232,11 @@ static int archive_assemble(zlb_ctx* ctx, int kind, const uint8_t* d_in, const u
     const size_t bytes = n * sizeof(ZtsFrame);
     int rc = zts_reserve(ctx, &ctx->d_frames, bytes + 64);
     if (rc) return rc;
-    rc = zts_reserve_pinned(ctx, bytes + 64);
+    rc = zts_reserve_pinned(ctx, &ctx->h_pin, bytes + 64);
     if (rc) return rc;
-    if (n) memcpy(ctx->h_pin, plan.frames.data(), bytes);
+    if (n) memcpy(ctx->h_pin.p, plan.frames.data(), bytes);
     ZtsFrame* d_frames = (ZtsFrame*)ctx->d_frames.p;
-    if (n) ZTS_CUDA(ctx, cudaMemcpyAsync(d_frames, ctx->h_pin, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    if (n) ZTS_CUDA(ctx, cudaMemcpyAsync(d_frames, ctx->h_pin.p, bytes, cudaMemcpyHostToDevice, ctx->stream));
     ctx->work = ctx->stream;
     if (plan.n_pieces)
         ZTS_LAUNCH(ctx, ZK_FRAME_BODY,

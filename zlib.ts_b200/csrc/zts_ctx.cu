@@ -51,31 +51,18 @@ int zts_check_dicts(zlb_ctx* ctx, const void* blob, size_t blob_bytes, const zlb
     return ZLB_OK;
 }
 
-int zts_reserve_pinned(zlb_ctx* ctx, size_t bytes)
+int zts_reserve_pinned(zlb_ctx* ctx, ZtsHostBuf* b, size_t bytes)
 {
-    if (bytes <= ctx->h_pin_cap) return ZLB_OK;
+    if (bytes <= b->cap) return ZLB_OK;
     size_t want = bytes + bytes / 4 + 4096;
+    // the buffer may still be read by copies queued on the stream
     ZTS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    if (ctx->h_pin) cudaFreeHost(ctx->h_pin);
-    ctx->h_pin = nullptr;
-    ctx->h_pin_cap = 0;
-    cudaError_t e = cudaMallocHost(&ctx->h_pin, want);
+    if (b->p) cudaFreeHost(b->p);
+    b->p = nullptr;
+    b->cap = 0;
+    cudaError_t e = cudaMallocHost(&b->p, want);
     if (e != cudaSuccess) return zts_fail(ctx, ZLB_E_NOMEM, "cudaMallocHost(%zu) failed: %s", want, cudaGetErrorString(e));
-    ctx->h_pin_cap = want;
-    return ZLB_OK;
-}
-
-int zts_reserve_pinned2(zlb_ctx* ctx, size_t bytes)
-{
-    if (bytes <= ctx->h_pin2_cap) return ZLB_OK;
-    size_t want = bytes + bytes / 4 + 4096;
-    ZTS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    if (ctx->h_pin2) cudaFreeHost(ctx->h_pin2);
-    ctx->h_pin2 = nullptr;
-    ctx->h_pin2_cap = 0;
-    cudaError_t e = cudaMallocHost(&ctx->h_pin2, want);
-    if (e != cudaSuccess) return zts_fail(ctx, ZLB_E_NOMEM, "cudaMallocHost(%zu) failed: %s", want, cudaGetErrorString(e));
-    ctx->h_pin2_cap = want;
+    b->cap = want;
     return ZLB_OK;
 }
 
@@ -149,7 +136,8 @@ static void prof_resolve(zlb_ctx* ctx)
 // slots (or one span over all of them) back would put stale bytes of earlier calls between the items' outputs, so
 // only [out_off, out_off + out_len) of every item travels; adjacent ranges are merged into one copy (a batch of
 // streams that fill their slots is one copy). Should that still take more than ZTS_COPYBACK_MAX copies, the slack
-// behind every item is zeroed on the device and one span is copied instead.
+// behind every item is zeroed on the device and one span is copied instead. The runs are taken from h_res and the
+// slack from d_res, so both must hold the call's final results: the caller reads d_res back into h_res first.
 #define ZTS_COPYBACK_MAX 2048u
 
 __global__ void __launch_bounds__(256)
@@ -245,8 +233,8 @@ void zlb_destroy(zlb_ctx* ctx)
     for (ZtsDevBuf* b : bufs)
         if (b->p) cudaFree(b->p);
     zts_stage_destroy_ctx(ctx);
-    if (ctx->h_pin) cudaFreeHost(ctx->h_pin);
-    if (ctx->h_pin2) cudaFreeHost(ctx->h_pin2);
+    if (ctx->h_pin.p) cudaFreeHost(ctx->h_pin.p);
+    if (ctx->h_pin2.p) cudaFreeHost(ctx->h_pin2.p);
     for (cudaEvent_t e : ctx->sync_events) cudaEventDestroy(e);
     if (ctx->s_in) cudaStreamDestroy(ctx->s_in);
     if (ctx->s_out) cudaStreamDestroy(ctx->s_out);

@@ -347,11 +347,13 @@ extern "C" uint64_t zlb_deflate_bound(uint64_t in_len, uint32_t chunk_bytes, int
     return (in_len * 15 + 7) / 8 + n_chunks * (ZTS_HDR_BYTES + 8) + 16;
 }
 
+// Stored blocks: the results are known on the host. They go to d_results behind the launch, where the tail of
+// deflate_device reads them like those of the chunked route.
 static int deflate_stored(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const zlb_item* h_items,
-                          zlb_result* h_results, size_t n, zlb_item* d_items)
+                          zlb_result* h_results, size_t n, const zlb_item* d_items, zlb_result* d_results,
+                          const ZtsHostIO* hio)
 {
     size_t n_blocks = 0;
-    for (size_t i = 0; i < n; ++i) n_blocks += (h_items[i].in_len + 0xFFFE) / 0xFFFF;
     for (size_t i = 0; i < n; ++i) {
         uint64_t nb = (h_items[i].in_len + 0xFFFE) / 0xFFFF;
         uint64_t total = h_items[i].in_len + 5 * nb;
@@ -359,110 +361,62 @@ static int deflate_stored(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
         h_results[i].out_len = total;
         h_results[i].in_used = h_items[i].in_len;
         h_results[i].blocks = (uint32_t)nb;
+        n_blocks += nb;
     }
-    if (n_blocks == 0) return ZLB_OK;
     if (n_blocks > 0x7FFFFFFFull) return zts_fail(ctx, ZLB_E_ARG, "too many stored blocks");
-    int rc = zts_reserve_pinned(ctx, n_blocks * 8);
-    if (rc) return rc;
-    uint32_t* h_bi = (uint32_t*)ctx->h_pin;
-    uint32_t* h_bk = h_bi + n_blocks;
-    size_t k = 0;
-    for (size_t i = 0; i < n; ++i) {
-        uint64_t nb = (h_items[i].in_len + 0xFFFE) / 0xFFFF;
-        for (uint64_t j = 0; j < nb; ++j) {
-            h_bi[k] = (uint32_t)i;
-            h_bk[k] = (uint32_t)j;
-            ++k;
+    if (n_blocks) {
+        int rc = zts_reserve_pinned(ctx, &ctx->h_pin, n_blocks * 8);
+        if (rc) return rc;
+        uint32_t* h_bi = (uint32_t*)ctx->h_pin.p;
+        uint32_t* h_bk = h_bi + n_blocks;
+        size_t k = 0;
+        for (size_t i = 0; i < n; ++i) {
+            uint64_t nb = (h_items[i].in_len + 0xFFFE) / 0xFFFF;
+            for (uint64_t j = 0; j < nb; ++j) {
+                h_bi[k] = (uint32_t)i;
+                h_bk[k] = (uint32_t)j;
+                ++k;
+            }
         }
+        rc = zts_reserve(ctx, &ctx->d_misc, n_blocks * 8 + 64);
+        if (rc) return rc;
+        ZTS_CUDA(ctx, cudaMemcpyAsync(ctx->d_misc.p, h_bi, n_blocks * 8, cudaMemcpyHostToDevice, ctx->stream));
+        uint32_t* d_bi = (uint32_t*)ctx->d_misc.p;
+        if (hio) {
+            zts_stage_wait_in(hio->stage, 0, hio->in_bytes);
+            ZTS_CUDA(ctx, cudaMemcpyAsync((void*)d_in, hio->h_in, hio->in_bytes, cudaMemcpyHostToDevice, ctx->stream));
+        }
+        ZTS_LAUNCH(ctx, ZK_STORED,
+                   stored_block_kernel<<<(unsigned)n_blocks, 256, 0, ctx->stream>>>(d_in, d_out, d_items, d_bi,
+                                                                                    d_bi + n_blocks));
     }
-    rc = zts_reserve(ctx, &ctx->d_misc, n_blocks * 8 + 64);
-    if (rc) return rc;
-    ZTS_CUDA(ctx, cudaMemcpyAsync(ctx->d_misc.p, h_bi, n_blocks * 8, cudaMemcpyHostToDevice, ctx->stream));
-    uint32_t* d_bi = (uint32_t*)ctx->d_misc.p;
-    ZTS_LAUNCH(ctx, ZK_STORED,
-               stored_block_kernel<<<(unsigned)n_blocks, 256, 0, ctx->stream>>>(d_in, d_out, d_items, d_bi,
-                                                                                d_bi + n_blocks));
-    ZTS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    ZTS_CUDA(ctx, cudaMemcpyAsync(d_results, h_results, n * sizeof(zlb_result), cudaMemcpyHostToDevice, ctx->stream));
     return ZLB_OK;
 }
 
-#define HOST_DELTA_MAX_ITEMS 256u  // per-wave output read-back is done item by item up to this many items
+// The chunks of a call and its waves. The tables are built in ctx->h_pin and go to ctx->d_chunks in one piece:
+// chunks | with dictionaries, the LZ77 kernel's view of the chunks and the dictionary table | blocks per item.
+struct DeflatePlan {
+    std::vector<size_t> wstart;  // wstart[k] = first chunk of wave k, wstart[n_waves] = n_chunks
+    size_t wave;                 // the largest wave: it sizes the scratch sets
+    size_t view_b, dicts_b, tables_b;
+    size_t stage_b;              // staging arena of the largest wave (dictionaries), 0 without
+    int n_sets;                  // scratch sets: 2 when consecutive waves run on two streams
+    ZtsChunk* h_chunks;
+};
 
-// Runs the pipeline on device buffers. Results land in h_results after the final synchronise.
-// d_dict / h_dicts: the preset dictionaries (h_dicts == NULL: none; checked by the caller)
-// hio: the host buffers of a "_host" call. The device path then also moves the data: the input of wave k+1 travels
-// while wave k is compressed, and with few items what wave k produced travels while wave k+1 runs (hio->out_done).
-static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const uint8_t* d_dict,
-                          const zlb_dict* h_dicts, const zlb_item* h_items, zlb_result* h_results, size_t n, int mode,
-                          int block_type, uint32_t chunk_bytes, uint32_t flags, ZtsHostIO* hio)
+static int deflate_plan(zlb_ctx* ctx, const uint8_t* d_in, const zlb_dict* h_dicts, const zlb_item* h_items, size_t n,
+                        uint32_t cb, bool primed, bool any_dict, uint32_t flags, bool host, DeflatePlan& p)
 {
-    if ((mode & 0xFF) & ~(ZLB_MODE_FAST | ZLB_MODE_PRIMED | ZLB_MODE_SMALLEST | ZLB_MODE_LAZY))
-        return zts_fail(ctx, ZLB_E_UNSUPPORTED, "unknown deflate mode %d", mode);
-    uint32_t depth = 0xFFFFFFFFu;  // compat: every candidate, like the reference
-    // fast mode: the same kernel, but a search looks at the `depth` nearest entries of the position's bucket only
-    const bool fast = (mode & ZLB_MODE_FAST) != 0;
-    const bool primed = (mode & ZLB_MODE_PRIMED) != 0 && block_type != ZLB_NONE;
-    const bool smallest = (mode & ZLB_MODE_SMALLEST) != 0 && block_type == ZLB_DYNAMIC;
-    if (fast) depth = ((uint32_t)mode >> 8) ? ((uint32_t)mode >> 8) : ZLB_FAST_DEFAULT_DEPTH;
-    if (fast && depth > 64u) depth = 64u;  // (the lane-private search; longer lists belong to the exact mode)
-    const bool lazy = fast && (mode & ZLB_MODE_LAZY) != 0;  // a fast-mode option: the exact mode is the reference's greedy parse
-    if (block_type != ZLB_NONE && block_type != ZLB_FIXED && block_type != ZLB_DYNAMIC)
-        return zts_fail(ctx, ZLB_E_ARG, "invalid compression type");  // src/RawDeflate.ts:110
-    bool any_dict = false;  // some item has a dictionary
-    for (size_t i = 0; h_dicts && i < n && !any_dict; ++i) any_dict = h_dicts[i].len != 0;
-    // primed or a dictionary: history + chunk share the 64 KiB a CTA stages and indexes, so a chunk is at most 32 KiB
-    const uint32_t cb_max = (primed || any_dict) ? ZLB_PRIMED_CHUNK : LZ_MAX_CHUNK;
-    const uint32_t cb = (chunk_bytes == 0 || chunk_bytes > cb_max) ? cb_max : chunk_bytes;
-    if (n > 0x7FFFFFFFull) return zts_fail(ctx, ZLB_E_ARG, "too many items");
-    ctx->work = ctx->stream;
-
-    int rc = zts_reserve(ctx, &ctx->d_items, n * sizeof(zlb_item) + 64);
-    if (rc) return rc;
-    rc = zts_reserve(ctx, &ctx->d_results, n * sizeof(zlb_result) + 64);
-    if (rc) return rc;
-    zlb_item* d_items = (zlb_item*)ctx->d_items.p;
-    zlb_result* d_results = (zlb_result*)ctx->d_results.p;
-    ZTS_CUDA(ctx, cudaMemcpyAsync(d_items, h_items, n * sizeof(zlb_item), cudaMemcpyHostToDevice, ctx->stream));
-    ZTS_CUDA(ctx, cudaMemsetAsync(d_results, 0, n * sizeof(zlb_result), ctx->stream));
-    memset(h_results, 0, n * sizeof(zlb_result));
-
-    uint32_t kinds = 0;
-    if (flags & ZLB_DEFLATE_WANT_CRC32) kinds |= ZLB_SUM_CRC32;
-    if (flags & ZLB_DEFLATE_WANT_ADLER32) kinds |= ZLB_SUM_ADLER32;
-
-    if (hio && block_type == ZLB_NONE) {
-        zts_stage_wait_in(hio->stage, 0, hio->in_bytes);
-        ZTS_CUDA(ctx, cudaMemcpyAsync((void*)d_in, hio->h_in, hio->in_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    }
-    if (block_type == ZLB_NONE) {
-        rc = deflate_stored(ctx, d_in, d_out, h_items, h_results, n, d_items);
-        if (rc) return rc;
-        if (kinds) {
-            rc = zts_checksum_device(ctx, d_in, d_items, d_results, h_items, n, kinds, 0);
-            if (rc) return rc;
-            zlb_result* tmp = nullptr;
-            rc = zts_reserve_pinned(ctx, n * sizeof(zlb_result));
-            if (rc) return rc;
-            tmp = (zlb_result*)ctx->h_pin;
-            ZTS_CUDA(ctx, cudaMemcpyAsync(tmp, d_results, n * sizeof(zlb_result), cudaMemcpyDeviceToHost, ctx->stream));
-            ZTS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-            for (size_t i = 0; i < n; ++i) {
-                h_results[i].crc32 = tmp[i].crc32;
-                h_results[i].adler32 = tmp[i].adler32;
-            }
-        }
-        return ZLB_OK;
-    }
-
     // ---- chunk table
     size_t n_chunks = 0;
     for (size_t i = 0; i < n; ++i) n_chunks += h_items[i].in_len ? (h_items[i].in_len + cb - 1) / cb : 1;
     if (n_chunks > 0x7FFFFFFFull) return zts_fail(ctx, ZLB_E_ARG, "too many chunks");
-    // ---- wave plan: wstart[k] = first chunk of wave k, wstart[n_waves] = n_chunks
-    std::vector<size_t> wstart;
+    // ---- wave plan
+    std::vector<size_t>& wstart = p.wstart;
     {
         const size_t sm = (size_t)ctx->sm_count;
-        if (hio && n_chunks >= 16u * sm) {
+        if (host && n_chunks >= 16u * sm) {
             // host path, large job: the first wave's input and the last wave's small kernels + output are the
             // transfers nothing hides, so the waves ramp up (one, then two chunks per SM), cruise in about four
             // large waves (every wave costs ~0.15 ms of launches and tails) and end with a small one; consecutive
@@ -478,7 +432,7 @@ static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
             wstart.push_back(n_chunks);
         } else {
             size_t wave = n_chunks < WAVE_CHUNKS ? n_chunks : WAVE_CHUNKS;
-            if (hio && n_chunks > 4u * sm) {  // host path, medium job: about eight equal waves of at least two chunks per SM
+            if (host && n_chunks > 4u * sm) {  // host path, medium job: about eight equal waves of at least two chunks per SM
                 size_t w8 = (n_chunks + 7) / 8;
                 if (w8 < 2u * sm) w8 = 2u * sm;
                 if (w8 < wave) wave = w8;
@@ -488,21 +442,19 @@ static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
         }
     }
     const size_t n_waves = wstart.size() - 1;
-    size_t wave = 0;  // the largest wave sizes the scratch sets
+    p.wave = 0;
     for (size_t k = 0; k < n_waves; ++k)
-        if (wstart[k + 1] - wstart[k] > wave) wave = wstart[k + 1] - wstart[k];
-    // table upload: chunks | with dictionaries: the LZ77 kernel's view of the chunks and the dictionary table |
-    // blocks per item
-    const size_t view_b = any_dict ? n_chunks * sizeof(ZtsChunk) : 0;
-    const size_t dicts_b = any_dict ? n * sizeof(zlb_dict) : 0;
-    const size_t tables_b = n_chunks * sizeof(ZtsChunk) + view_b + dicts_b + n * sizeof(uint32_t);
-    rc = zts_reserve_pinned(ctx, tables_b);
+        if (wstart[k + 1] - wstart[k] > p.wave) p.wave = wstart[k + 1] - wstart[k];
+    const size_t view_b = p.view_b = any_dict ? n_chunks * sizeof(ZtsChunk) : 0;
+    const size_t dicts_b = p.dicts_b = any_dict ? n * sizeof(zlb_dict) : 0;
+    p.tables_b = n_chunks * sizeof(ZtsChunk) + view_b + dicts_b + n * sizeof(uint32_t);
+    int rc = zts_reserve_pinned(ctx, &ctx->h_pin, p.tables_b);
     if (rc) return rc;
-    ZtsChunk* h_chunks = (ZtsChunk*)ctx->h_pin;
+    ZtsChunk* h_chunks = p.h_chunks = (ZtsChunk*)ctx->h_pin.p;
     ZtsChunk* h_view = h_chunks + n_chunks;
     if (any_dict) memcpy((uint8_t*)h_view + view_b, h_dicts, dicts_b);
     uint32_t* h_blocks = (uint32_t*)((uint8_t*)h_view + view_b + dicts_b);
-    size_t stage_b = 0;  // staging arena of the largest wave (dictionaries)
+    size_t stage_b = 0;
     {
         size_t k = 0, wk = 0, stage_at = 0;  // stage_at: 16-byte units used by the chunk's wave so far
         for (size_t i = 0; i < n; ++i) {
@@ -537,14 +489,13 @@ static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
             }
         }
     }
-    const uint32_t grid = (uint32_t)(wave < (size_t)ctx->sm_count ? wave : (size_t)ctx->sm_count);
     // Host path with several waves: consecutive waves run on two streams with a scratch set each, so that the next
     // wave's LZ77 CTAs take over the SMs as the previous wave's drain (no idle tail per wave) and its small kernels
     // overlap too; only the offset scan is chained from wave to wave.
-    const int n_sets = (hio && n_waves > 1) ? 2 : 1;
-    rc = zts_reserve(ctx, &ctx->d_chunks, tables_b + 64);
+    const int n_sets = p.n_sets = (host && n_waves > 1) ? 2 : 1;
+    rc = zts_reserve(ctx, &ctx->d_chunks, p.tables_b + 64);
     if (rc) return rc;
-    stage_b = (stage_b + 255) & ~(size_t)255;
+    stage_b = p.stage_b = (stage_b + 255) & ~(size_t)255;
     if (stage_b && (rc = zts_reserve(ctx, &ctx->d_dict_stage, n_sets * stage_b + 64))) return rc;
     if (any_dict) {
         // The LZ77 kernel stages `in + in_off - dict_len` (the history in front of the chunk, then the chunk). Its view
@@ -559,6 +510,23 @@ static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
             }
         }
     }
+    return ZLB_OK;
+}
+
+// The scratch of one wave in flight
+struct DeflateSet {
+    ZtsChunkInfo* info;
+    uint32_t *list, *tile_tok, *hist, *sortT, *counter;
+    ZtsChunkCodes* codes;
+    unsigned long long* gpos;
+    uint8_t* stage;
+};
+
+// Reserves the plan's scratch sets and lays them out; ctx->d_misc starts with the running output size of every item.
+static int deflate_scratch(zlb_ctx* ctx, const DeflatePlan& p, size_t n, DeflateSet* sets)
+{
+    const size_t wave = p.wave;
+    const int n_sets = p.n_sets;
     const size_t info_b = (wave * sizeof(ZtsChunkInfo) + 255) & ~(size_t)255;
     const size_t list_b = (wave * (size_t)LZ_LIST_PER_CHUNK * 4 + 255) & ~(size_t)255;   // token list of every chunk
     const size_t tile_b = (zts_lz77_scratch_bytes(ctx->sm_count) + 255) & ~(size_t)255;  // per-CTA tile token scratch
@@ -566,7 +534,7 @@ static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
     const size_t codes_b = (wave * sizeof(ZtsChunkCodes) + 255) & ~(size_t)255;
     const size_t sort_b = ((size_t)ctx->sm_count * LZ_MAX_CHUNK * 4 + 255) & ~(size_t)255;
     const size_t gpos_b = (wave * 8 + 256 + 255) & ~(size_t)255;  // chunk offsets of the wave + the work counter
-    rc = zts_reserve(ctx, &ctx->d_chunk_info, n_sets * info_b + 64);
+    int rc = zts_reserve(ctx, &ctx->d_chunk_info, n_sets * info_b + 64);
     if (rc) return rc;
     rc = zts_reserve(ctx, &ctx->d_tokens, n_sets * list_b + 64);
     if (rc) return rc;
@@ -579,18 +547,7 @@ static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
     if (rc) return rc;
     rc = zts_reserve(ctx, &ctx->d_misc, n * 8 + n_sets * gpos_b + 256);
     if (rc) return rc;
-    ZtsChunk* d_chunks = (ZtsChunk*)ctx->d_chunks.p;
-    const ZtsChunk* d_lz_chunks = any_dict ? d_chunks + n_chunks : d_chunks;  // what the LZ77 kernel reads
-    const zlb_dict* d_dicts = (const zlb_dict*)((uint8_t*)(d_chunks + n_chunks) + view_b);
-    uint32_t* d_blocks = (uint32_t*)((uint8_t*)d_dicts + dicts_b);
     unsigned long long* d_running = (unsigned long long*)ctx->d_misc.p;
-    struct Set {
-        ZtsChunkInfo* info;
-        uint32_t *list, *tile_tok, *hist, *sortT, *counter;
-        ZtsChunkCodes* codes;
-        unsigned long long* gpos;
-        uint8_t* stage;
-    } sets[2];
     for (int b = 0; b < n_sets; ++b) {
         sets[b].info = (ZtsChunkInfo*)((uint8_t*)ctx->d_chunk_info.p + b * info_b);
         sets[b].list = (uint32_t*)((uint8_t*)ctx->d_tokens.p + b * list_b);
@@ -600,9 +557,32 @@ static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
         sets[b].sortT = (uint32_t*)((uint8_t*)ctx->d_sortT.p + b * sort_b);
         sets[b].gpos = (unsigned long long*)((uint8_t*)(d_running + n) + b * gpos_b);
         sets[b].counter = (uint32_t*)(sets[b].gpos + wave);
-        sets[b].stage = stage_b ? (uint8_t*)ctx->d_dict_stage.p + b * stage_b : nullptr;
+        sets[b].stage = p.stage_b ? (uint8_t*)ctx->d_dict_stage.p + b * p.stage_b : nullptr;
     }
-    ZTS_CUDA(ctx, cudaMemcpyAsync(d_chunks, h_chunks, tables_b, cudaMemcpyHostToDevice, ctx->stream));
+    return ZLB_OK;
+}
+
+#define HOST_DELTA_MAX_ITEMS 256u  // per-wave output read-back is done item by item up to this many items
+
+// The tables to the device, the waves, then deflate_finalize_kernel writes the results. hio: on a "_host" call the
+// input of wave k+1 travels while wave k is compressed (items laid out in order), and with at most
+// HOST_DELTA_MAX_ITEMS items what wave k produced travels back while wave k+1 runs (*out_copied).
+static int deflate_waves(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const uint8_t* d_dict, const zlb_item* d_items,
+                         zlb_result* d_results, const zlb_item* h_items, size_t n, const DeflatePlan& p,
+                         const DeflateSet* sets, int block_type, uint32_t depth, bool lazy, bool smallest,
+                         const ZtsHostIO* hio, bool* out_copied)
+{
+    const std::vector<size_t>& wstart = p.wstart;
+    const size_t n_chunks = wstart.back(), n_waves = wstart.size() - 1;
+    const int n_sets = p.n_sets;
+    const ZtsChunk* h_chunks = p.h_chunks;
+    const uint32_t grid = (uint32_t)(p.wave < (size_t)ctx->sm_count ? p.wave : (size_t)ctx->sm_count);
+    ZtsChunk* d_chunks = (ZtsChunk*)ctx->d_chunks.p;
+    const ZtsChunk* d_lz_chunks = p.view_b ? d_chunks + n_chunks : d_chunks;  // what the LZ77 kernel reads
+    const zlb_dict* d_dicts = (const zlb_dict*)((uint8_t*)(d_chunks + n_chunks) + p.view_b);
+    uint32_t* d_blocks = (uint32_t*)((uint8_t*)d_dicts + p.dicts_b);
+    unsigned long long* d_running = (unsigned long long*)ctx->d_misc.p;
+    ZTS_CUDA(ctx, cudaMemcpyAsync(d_chunks, h_chunks, p.tables_b, cudaMemcpyHostToDevice, ctx->stream));
     ZTS_CUDA(ctx, cudaMemsetAsync(d_running, 0, n * 8, ctx->stream));
     ZTS_CUDA(ctx, cudaFuncSetAttribute(bitpack_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)(PACK_STAGE_WORDS * 4)));
@@ -611,6 +591,7 @@ static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
     bool pipe_in = false, delta_out = false;
     unsigned long long* h_run = nullptr;      // [n_waves][n] running totals read back after each wave
     std::vector<unsigned long long> copied;   // bytes of every item already copied to the host
+    int rc;
     if (hio) {
         rc = zts_host_streams(ctx);
         if (rc) return rc;
@@ -619,9 +600,9 @@ static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
             if (h_chunks[k].in_off < h_chunks[k - 1].in_off + h_chunks[k - 1].len) pipe_in = false;  // not laid out in order
         delta_out = n <= HOST_DELTA_MAX_ITEMS;
         if (delta_out) {
-            rc = zts_reserve_pinned2(ctx, n_waves * n * sizeof(unsigned long long));
+            rc = zts_reserve_pinned(ctx, &ctx->h_pin2, n_waves * n * sizeof(unsigned long long));
             if (rc) return rc;
-            h_run = (unsigned long long*)ctx->h_pin2;
+            h_run = (unsigned long long*)ctx->h_pin2.p;
             copied.assign(n, 0ull);
         }
         if (!pipe_in) {
@@ -667,13 +648,13 @@ static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
         const size_t w0 = wstart[k];
         const uint32_t wn = (uint32_t)(wstart[k + 1] - w0);
         const uint32_t g = wn < grid ? wn : grid;
-        const Set& S = sets[n_sets == 2 ? (k & 1) : 0];
+        const DeflateSet& S = sets[n_sets == 2 ? (k & 1) : 0];
         cudaStream_t st = (n_sets == 2 && (k & 1)) ? ctx->s_aux[0] : ctx->stream;
         ctx->work = st;
         if (n_sets == 2 && k == 1)  // the tables uploaded on ctx->stream must be there before the second stream starts
             ZTS_CUDA(ctx, cudaStreamWaitEvent(st, zts_sync_event(ctx, 4 * n_waves), 0));
         if (pipe_in) ZTS_CUDA(ctx, cudaStreamWaitEvent(st, zts_sync_event(ctx, 2 * k), 0));
-        if (stage_b)
+        if (p.stage_b)
             ZTS_LAUNCH(ctx, ZK_DICT_STAGE,
                        dict_stage_kernel<<<wn, 256, 0, st>>>(d_in, d_dict, d_dicts, d_items, d_chunks + w0, S.stage));
         rc = zts_lz77_launch(ctx, d_in, d_lz_chunks + w0, wn, S.info, S.tile_tok, S.list, S.hist, S.sortT, S.counter, g, depth,
@@ -715,19 +696,81 @@ static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
     }
     if (delta_out) {
         if ((rc = wave_out_copy(n_waves - 1))) return rc;
-        hio->out_done = true;
+        *out_copied = true;
     }
     ZTS_LAUNCH(ctx, ZK_FINALIZE,
                deflate_finalize_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(d_items, d_results,
                                                                                              d_running, d_blocks,
                                                                                              (uint32_t)n));
+    return ZLB_OK;
+}
+
+// Deflates n items on device buffers; results land in h_results after the final synchronise. It validates the
+// arguments, uploads the item table and runs one route: stored blocks (deflate_stored) or chunks (deflate_plan,
+// deflate_scratch, deflate_waves). Either leaves every result in d_results. Then one tail: checksums, the result
+// read-back and, on a "_host" call whose waves did not copy the outputs back already, the copy-back.
+// d_dict / h_dicts: the preset dictionaries (h_dicts == NULL: none; checked by the caller)
+// hio: the host buffers of a "_host" call; the route then also copies the input over.
+static int deflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const uint8_t* d_dict,
+                          const zlb_dict* h_dicts, const zlb_item* h_items, zlb_result* h_results, size_t n, int mode,
+                          int block_type, uint32_t chunk_bytes, uint32_t flags, const ZtsHostIO* hio)
+{
+    if ((mode & 0xFF) & ~(ZLB_MODE_FAST | ZLB_MODE_PRIMED | ZLB_MODE_SMALLEST | ZLB_MODE_LAZY))
+        return zts_fail(ctx, ZLB_E_UNSUPPORTED, "unknown deflate mode %d", mode);
+    uint32_t depth = 0xFFFFFFFFu;  // compat: every candidate, like the reference
+    // fast mode: the same kernel, but a search looks at the `depth` nearest entries of the position's bucket only
+    const bool fast = (mode & ZLB_MODE_FAST) != 0;
+    const bool primed = (mode & ZLB_MODE_PRIMED) != 0 && block_type != ZLB_NONE;
+    const bool smallest = (mode & ZLB_MODE_SMALLEST) != 0 && block_type == ZLB_DYNAMIC;
+    if (fast) depth = ((uint32_t)mode >> 8) ? ((uint32_t)mode >> 8) : ZLB_FAST_DEFAULT_DEPTH;
+    if (fast && depth > 64u) depth = 64u;  // (the lane-private search; longer lists belong to the exact mode)
+    const bool lazy = fast && (mode & ZLB_MODE_LAZY) != 0;  // a fast-mode option: the exact mode is the reference's greedy parse
+    if (block_type != ZLB_NONE && block_type != ZLB_FIXED && block_type != ZLB_DYNAMIC)
+        return zts_fail(ctx, ZLB_E_ARG, "invalid compression type");  // src/RawDeflate.ts:110
+    bool any_dict = false;  // some item has a dictionary
+    for (size_t i = 0; h_dicts && i < n && !any_dict; ++i) any_dict = h_dicts[i].len != 0;
+    // primed or a dictionary: history + chunk share the 64 KiB a CTA stages and indexes, so a chunk is at most 32 KiB
+    const uint32_t cb_max = (primed || any_dict) ? ZLB_PRIMED_CHUNK : LZ_MAX_CHUNK;
+    const uint32_t cb = (chunk_bytes == 0 || chunk_bytes > cb_max) ? cb_max : chunk_bytes;
+    if (n > 0x7FFFFFFFull) return zts_fail(ctx, ZLB_E_ARG, "too many items");
+    ctx->work = ctx->stream;
+
+    int rc = zts_reserve(ctx, &ctx->d_items, n * sizeof(zlb_item) + 64);
+    if (rc) return rc;
+    rc = zts_reserve(ctx, &ctx->d_results, n * sizeof(zlb_result) + 64);
+    if (rc) return rc;
+    zlb_item* d_items = (zlb_item*)ctx->d_items.p;
+    zlb_result* d_results = (zlb_result*)ctx->d_results.p;
+    ZTS_CUDA(ctx, cudaMemcpyAsync(d_items, h_items, n * sizeof(zlb_item), cudaMemcpyHostToDevice, ctx->stream));
+    ZTS_CUDA(ctx, cudaMemsetAsync(d_results, 0, n * sizeof(zlb_result), ctx->stream));
+    memset(h_results, 0, n * sizeof(zlb_result));
+
+    bool out_copied = false;  // the waves copied the output back already
+    if (block_type == ZLB_NONE) {
+        rc = deflate_stored(ctx, d_in, d_out, h_items, h_results, n, d_items, d_results, hio);
+    } else {
+        DeflatePlan p;
+        DeflateSet sets[2];
+        rc = deflate_plan(ctx, d_in, h_dicts, h_items, n, cb, primed, any_dict, flags, hio != nullptr, p);
+        if (!rc) rc = deflate_scratch(ctx, p, n, sets);
+        if (!rc)
+            rc = deflate_waves(ctx, d_in, d_out, d_dict, d_items, d_results, h_items, n, p, sets, block_type, depth, lazy,
+                               smallest, hio, &out_copied);
+    }
+    if (rc) return rc;
+
+    uint32_t kinds = 0;
+    if (flags & ZLB_DEFLATE_WANT_CRC32) kinds |= ZLB_SUM_CRC32;
+    if (flags & ZLB_DEFLATE_WANT_ADLER32) kinds |= ZLB_SUM_ADLER32;
     if (kinds) {
         rc = zts_checksum_device(ctx, d_in, d_items, d_results, h_items, n, kinds, 0);
         if (rc) return rc;
     }
     ZTS_CUDA(ctx, cudaMemcpyAsync(h_results, d_results, n * sizeof(zlb_result), cudaMemcpyDeviceToHost, ctx->stream));
     ZTS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    if (delta_out) ZTS_CUDA(ctx, cudaStreamSynchronize(ctx->s_out));
+    if (out_copied) ZTS_CUDA(ctx, cudaStreamSynchronize(ctx->s_out));
+    else if (hio)  // what each item wrote, adjacent ranges merged; the sizes decide what travels
+        return zts_copy_back(ctx, hio->stage, ctx->stream, d_out, hio->h_out, h_items, h_results, d_items, d_results, 0, n);
     return ZLB_OK;
 }
 
@@ -757,13 +800,9 @@ extern "C" int zlb_deflate_batch_dict_host(zlb_ctx* ctx, const void* h_in, size_
 {
     return zts_host_call(ctx, h_in, in_bytes, h_out, out_bytes, h_dict, dict_bytes, dicts, items, results, n, SIZE_MAX,
                          [&](ZtsHostIO& io, const zlb_dict* d) {
-        const uint8_t* d_out = (const uint8_t*)ctx->d_stage_out.p;
-        int rc = deflate_device(ctx, (const uint8_t*)ctx->d_stage_in.p, (uint8_t*)d_out, (const uint8_t*)ctx->d_dict.p, d,
-                                items, results, n, mode, block_type, chunk_bytes, flags, &io);
-        if (rc || io.out_done) return rc;
-        // many items: what each of them wrote, adjacent ranges merged
-        return zts_copy_back(ctx, io.stage, ctx->stream, d_out, io.h_out, items, results, (const zlb_item*)ctx->d_items.p,
-                             (const zlb_result*)ctx->d_results.p, 0, n);
+        return deflate_device(ctx, (const uint8_t*)ctx->d_stage_in.p, (uint8_t*)ctx->d_stage_out.p,
+                              (const uint8_t*)ctx->d_dict.p, d, items, results, n, mode, block_type, chunk_bytes, flags,
+                              &io);
     });
 }
 

@@ -273,7 +273,7 @@ int zts_host_call(zlb_ctx* ctx, const void* h_in, size_t in_bytes, void* h_out, 
     ZtsHostStage* stage = nullptr;
     rc = zts_stage_begin(ctx, h_in, in_bytes, h_out, out_bytes, &stage);
     if (!rc) {
-        ZtsHostIO io = {zts_stage_in_ptr(stage), zts_stage_out_ptr(stage), in_bytes, false, stage};
+        ZtsHostIO io = {zts_stage_in_ptr(stage), zts_stage_out_ptr(stage), in_bytes, stage};
         rc = body(io, any ? dicts : nullptr);
         if (!rc && cudaStreamSynchronize(ctx->stream) != cudaSuccess) rc = zts_fail(ctx, ZLB_E_CUDA, "synchronize failed");
     }

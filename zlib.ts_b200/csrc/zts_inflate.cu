@@ -1422,9 +1422,9 @@ static int inflate_waves(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, cons
     }
     int rc = zts_host_streams(ctx);
     if (rc) return rc;
-    rc = zts_reserve_pinned2(ctx, n * sizeof(zlb_result));
+    rc = zts_reserve_pinned(ctx, &ctx->h_pin2, n * sizeof(zlb_result));
     if (rc) return rc;
-    zlb_result* pin_res = (zlb_result*)ctx->h_pin2;
+    zlb_result* pin_res = (zlb_result*)ctx->h_pin2.p;
     const size_t per = (n + n_waves - 1) / n_waves;
     // events: 0 = item table on the device; 1 + 2k = input of wave k arrived; 2 + 2k = wave k decoded, results read back
     cudaEvent_t ev_tab = zts_sync_event(ctx, 0);
