@@ -1000,9 +1000,18 @@ window_resolve_kernel(const uint8_t* __restrict__ arena, uint8_t* __restrict__ s
     if (__syncthreads_or((int)(seen & 0x8000u)) && threadIdx.x == 0) fail[r.item] = 1u;
 }
 
-struct SplitPiece {
-    uint32_t item;  // index into big
-    unsigned long long start;
+// One call's marker split: the caller's items and preset dictionaries (dicts == NULL: none), the indices of its large
+// items, and the pieces of item big[k], seg[first[k] .. first[k + 1]) (split_layout). seg[j] is piece j's input span;
+// the decode split gives it a byte slot of its scratch (out_off / out_cap).
+struct SplitJob {
+    const zlb_item* items;
+    const zlb_dict* dicts;
+    std::vector<size_t> big;
+    std::vector<size_t> first;
+    std::vector<zlb_item> seg;
+    size_t pieces(size_t k) const { return first[k + 1] - first[k]; }
+    // where the last piece of big[k] starts, from the item's first input byte
+    unsigned long long last_start(size_t k) const { return seg[first[k + 1] - 1].in_off - items[big[k]].in_off; }
 };
 
 // The chain checks of the pieces r[0 .. n) of an item: each one decoded cleanly, ended exactly where the next one
@@ -1026,9 +1035,10 @@ static int split_chain(const zlb_result* r, const zlb_item* seg, size_t n, bool 
     return reaches ? SPLIT_WINDOW : SPLIT_OK;
 }
 
-// result of an item whose n pieces passed the checks, the last one starting at input byte last_start of the item
-static zlb_result split_result(const zlb_result* r, size_t n, unsigned long long last_start)
+// result of item big[k], whose pieces' results r[0 .. job.pieces(k)) passed the checks
+static zlb_result split_result(const SplitJob& job, size_t k, const zlb_result* r)
 {
+    const size_t n = job.pieces(k);
     zlb_result o;
     memset(&o, 0, sizeof o);
     unsigned long long blocks = 0;
@@ -1037,17 +1047,18 @@ static zlb_result split_result(const zlb_result* r, size_t n, unsigned long long
         blocks += r[j].blocks & 0x7FFFFFFFu;
     }
     o.status = ZLB_ST_OK;
-    o.in_used = last_start + r[n - 1].in_used;
+    o.in_used = job.last_start(k) + r[n - 1].in_used;
     o.blocks = (uint32_t)blocks;
     return o;
 }
 
 // split_result, checked against the item's slot; the pieces' bytes (r[j].out_len at scratch offset seg[j].out_off)
 // are queued for the gather when they fit
-static void split_finish(const zlb_item& it, const zlb_result* r, const zlb_item* seg, size_t n, unsigned long long last_start,
-                         zlb_result& o, std::vector<ZtsGather>& gath)
+static zlb_result split_finish(const SplitJob& job, size_t k, const zlb_result* r, std::vector<ZtsGather>& gath)
 {
-    o = split_result(r, n, last_start);
+    const zlb_item& it = job.items[job.big[k]];
+    const zlb_item* seg = &job.seg[job.first[k]];
+    zlb_result o = split_result(job, k, r);
     const unsigned long long total = o.out_len;
     if (total > it.out_cap) {
         o.status = ZLB_ST_OUT_OVERFLOW;
@@ -1055,11 +1066,12 @@ static void split_finish(const zlb_item& it, const zlb_result* r, const zlb_item
     }
     if (total <= it.out_cap && total) {
         unsigned long long at = 0;
-        for (size_t j = 0; j < n; ++j) {
+        for (size_t j = 0; j < job.pieces(k); ++j) {
             if (r[j].out_len) gath.push_back({seg[j].out_off, it.out_off + at, r[j].out_len});
             at += r[j].out_len;
         }
     }
+    return o;
 }
 
 // Scratch budget of an arena of the split stage: a quarter of what the device has free plus what the arena already
@@ -1090,15 +1102,53 @@ static int split_reserve(zlb_ctx* ctx, ZtsDevBuf* arena, size_t bytes, bool* got
     return ZLB_OK;
 }
 
-// Window mode for the items big[cand[*]] (pieces as laid out by inflate_split_batch, byte slots at seg[j].out_off of
-// d_scratch): all of them in one decode launch and one scan; done[k] / res[k] / gath as there. h_dicts / d_dict: the
-// preset dictionaries of h_items (NULL: none).
-static int inflate_split_window(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_scratch, const zlb_item* h_items,
-                                const zlb_dict* h_dicts, const uint8_t* d_dict,
-                                const std::vector<size_t>& big, uint32_t flags, const std::vector<SplitPiece>& pieces,
-                                const std::vector<size_t>& first, const std::vector<zlb_item>& seg,
-                                const std::vector<size_t>& cand, std::vector<zlb_result>& res, std::vector<char>& done,
-                                std::vector<ZtsGather>& gath)
+// One segment-mode launch of the decoder over the piece table seg, whose copy and results go to d_seg / d_res in the
+// caller's arena; res = the pieces' results. MODE INF_BYTES writes byte slots at d_out, INF_WINDOW word slots at
+// d_out, INF_SIZE nothing (d_out NULL).
+template <int MODE>
+static int split_segments(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const std::vector<zlb_item>& seg,
+                          zlb_item* d_seg, zlb_result* d_res, uint32_t flags, std::vector<zlb_result>& res)
+{
+    cudaStream_t st = ctx->stream;
+    const size_t np = seg.size();
+    ZTS_CUDA(ctx, cudaMemcpyAsync(d_seg, seg.data(), np * sizeof(zlb_item), cudaMemcpyHostToDevice, st));
+    ZTS_CUDA(ctx, cudaMemsetAsync(d_res, 0, np * sizeof(zlb_result), st));
+    const int rc = inflate_launch_mode<MODE>(ctx, st, d_in, d_out, d_seg, d_res, np,
+                                             (flags & ZLB_INFLATE_CHECK_NLEN) | ZLB_INFLATE_SEGMENT, nullptr, nullptr);
+    if (rc) return rc;
+    res.assign(np, zlb_result());
+    ZTS_CUDA(ctx, cudaMemcpyAsync(res.data(), d_res, np * sizeof(zlb_result), cudaMemcpyDeviceToHost, st));
+    ZTS_CUDA(ctx, cudaStreamSynchronize(st));
+    return ZLB_OK;
+}
+
+// The window arena, as byte offsets: word slots (each behind its window, `words` bytes in all) | a map per run: the
+// aggregates, the prefixes | per piece: the decode's item and result | the resolve's pieces, runs and items | a fail
+// flag per item
+struct WinLayout {
+    size_t agg, prefix, seg, res, pieces, runs, items, fail, total;
+};
+static WinLayout win_layout(size_t words, size_t np, size_t nr, size_t ni)
+{
+    WinLayout l;
+    l.agg = words;
+    l.prefix = l.agg + nr * WIN_WORDS * 2;
+    l.seg = l.prefix + nr * WIN_WORDS * 2;
+    l.res = l.seg + np * sizeof(zlb_item);
+    l.pieces = l.res + np * sizeof(zlb_result);
+    l.runs = l.pieces + np * sizeof(ZtsWinPiece);
+    l.items = l.runs + nr * sizeof(ZtsWinRun);
+    l.fail = l.items + ni * sizeof(ZtsWinItem);
+    l.total = l.fail + ni * 4 + 256;
+    return l;
+}
+
+// Window mode for the items big[cand[*]] (byte slots at seg[j].out_off of d_scratch, as inflate_split_batch laid them
+// out): all of them in one decode launch and one scan; h_results / done / gath as there. d_dict: the blob of the
+// job's preset dictionaries.
+static int inflate_split_window(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_scratch, const uint8_t* d_dict,
+                                const SplitJob& job, uint32_t flags, const std::vector<size_t>& cand,
+                                zlb_result* h_results, std::vector<char>& done, std::vector<ZtsGather>& gath)
 {
     cudaStream_t st = ctx->stream;
     // runs of about sqrt(n) pieces: the scan's depth is then about 3 sqrt(n) compositions
@@ -1108,88 +1158,68 @@ static int inflate_split_window(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_sc
         return g;
     };
     const size_t map_b = (size_t)WIN_WORDS * 2;
-    // arena: word slots (each behind its window) | aggregates | prefixes | items | results | pieces | runs | items | fail
-    auto layout = [&](size_t words, size_t np, size_t nr, size_t ni, size_t* off) {
-        off[0] = words;
-        off[1] = off[0] + nr * map_b;
-        off[2] = off[1] + nr * map_b;
-        off[3] = off[2] + np * sizeof(zlb_item);
-        off[4] = off[3] + np * sizeof(zlb_result);
-        off[5] = off[4] + np * sizeof(ZtsWinPiece);
-        off[6] = off[5] + nr * sizeof(ZtsWinRun);
-        off[7] = off[6] + ni * sizeof(ZtsWinItem);
-        return off[7] + ni * 4 + 256;
-    };
     // The scratch is bounded like the byte slots', with three times their bound by input (two bytes per word, the
     // windows, the maps).
     const SplitBudget budget(ctx->d_window);
     std::vector<size_t> take;
-    size_t words = 0, np = 0, nr = 0, in_b = 0, need = 0, off[8];
+    size_t words = 0, np = 0, nr = 0, in_b = 0;
     for (size_t k : cand) {
-        const size_t a = first[k], b = first[k + 1], n = b - a;
+        const size_t a = job.first[k], n = job.pieces(k), in_k = job.items[job.big[k]].in_len;
         size_t w = 0;
-        for (size_t j = a; j < b; ++j) w += map_b + 2 * (size_t)seg[j].out_cap;  // (out_cap: a multiple of 256)
+        for (size_t j = a; j < a + n; ++j) w += map_b + 2 * (size_t)job.seg[j].out_cap;  // (out_cap: a multiple of 256)
         const size_t g = run_len(n);
-        const size_t need_k = layout(words + w, np + n, nr + (n + g - 1) / g, take.size() + 1, off);
-        if (need_k > budget(in_b + h_items[big[k]].in_len, 3)) continue;
+        if (win_layout(words + w, np + n, nr + (n + g - 1) / g, take.size() + 1).total > budget(in_b + in_k, 3)) continue;
         take.push_back(k);
         words += w;
         np += n;
         nr += (n + g - 1) / g;
-        in_b += h_items[big[k]].in_len;
-        need = need_k;
+        in_b += in_k;
     }
     if (take.empty()) return ZLB_OK;
+    const WinLayout lay = win_layout(words, np, nr, take.size());
     bool got = false;
-    int rc = split_reserve(ctx, &ctx->d_window, need, &got);
+    int rc = split_reserve(ctx, &ctx->d_window, lay.total, &got);
     if (rc || !got) return rc;
-    layout(words, np, nr, take.size(), off);
     uint8_t* arena = (uint8_t*)ctx->d_window.p;
-    uint16_t* d_agg = (uint16_t*)(arena + off[0]);
-    uint16_t* d_prefix = (uint16_t*)(arena + off[1]);
-    zlb_item* d_wseg = (zlb_item*)(arena + off[2]);
-    zlb_result* d_wres = (zlb_result*)(arena + off[3]);
-    ZtsWinPiece* d_pieces = (ZtsWinPiece*)(arena + off[4]);
-    ZtsWinRun* d_runs = (ZtsWinRun*)(arena + off[5]);
-    ZtsWinItem* d_witems = (ZtsWinItem*)(arena + off[6]);
-    uint32_t* d_fail = (uint32_t*)(arena + off[7]);
+    uint16_t* d_agg = (uint16_t*)(arena + lay.agg);
+    uint16_t* d_prefix = (uint16_t*)(arena + lay.prefix);
+    ZtsWinPiece* d_pieces = (ZtsWinPiece*)(arena + lay.pieces);
+    ZtsWinRun* d_runs = (ZtsWinRun*)(arena + lay.runs);
+    ZtsWinItem* d_witems = (ZtsWinItem*)(arena + lay.items);
+    uint32_t* d_fail = (uint32_t*)(arena + lay.fail);
     // 1. every piece of those items in window mode, one launch
     std::vector<zlb_item> wseg;
     wseg.reserve(np);
     size_t at = 0;
     for (size_t k : take)
-        for (size_t j = first[k]; j < first[k + 1]; ++j) {
-            zlb_item w = seg[j];
+        for (size_t j = job.first[k]; j < job.first[k + 1]; ++j) {
+            zlb_item w = job.seg[j];
             w.out_off = at + map_b;  // the window's words in front
-            at += map_b + 2 * (size_t)seg[j].out_cap;
+            at += map_b + 2 * (size_t)w.out_cap;
             wseg.push_back(w);
         }
-    ZTS_CUDA(ctx, cudaMemcpyAsync(d_wseg, wseg.data(), np * sizeof(zlb_item), cudaMemcpyHostToDevice, st));
-    ZTS_CUDA(ctx, cudaMemsetAsync(d_wres, 0, np * sizeof(zlb_result), st));
-    rc = inflate_launch_mode<INF_WINDOW>(ctx, st, d_in, arena, d_wseg, d_wres, np,
-                                         (flags & ZLB_INFLATE_CHECK_NLEN) | ZLB_INFLATE_SEGMENT, nullptr, nullptr);
+    std::vector<zlb_result> wres;
+    rc = split_segments<INF_WINDOW>(ctx, d_in, arena, wseg, (zlb_item*)(arena + lay.seg), (zlb_result*)(arena + lay.res),
+                                    flags, wres);
     if (rc) return rc;
-    std::vector<zlb_result> wres(np);
-    ZTS_CUDA(ctx, cudaMemcpyAsync(wres.data(), d_wres, np * sizeof(zlb_result), cudaMemcpyDeviceToHost, st));
-    ZTS_CUDA(ctx, cudaStreamSynchronize(st));
     // 2. the chain checks; the items that pass are resolved
     std::vector<ZtsWinPiece> wp;
     std::vector<ZtsWinRun> runs;
     std::vector<ZtsWinItem> witems;
     std::vector<size_t> wk, wfirst;  // per resolved item: its k, its first piece in wseg / wres
     for (size_t t = 0, wj = 0; t < take.size(); ++t) {
-        const size_t k = take[t], a = first[k], n = first[k + 1] - a;
+        const size_t k = take[t], a = job.first[k], n = job.pieces(k);
         const size_t w0 = wj;
         wj += n;
-        if (split_chain(&wres[w0], &seg[a], n, false, false) != SPLIT_OK) continue;
+        if (split_chain(&wres[w0], &job.seg[a], n, false, false) != SPLIT_OK) continue;
         const size_t g = run_len(n);
-        const zlb_dict d = h_dicts ? h_dicts[big[k]] : zlb_dict{0, 0};
+        const zlb_dict d = job.dicts ? job.dicts[job.big[k]] : zlb_dict{0, 0};
         const uint32_t dl = d.len < WIN_WORDS ? (uint32_t)d.len : WIN_WORDS;
         witems.push_back({(uint32_t)runs.size(), (uint32_t)((n + g - 1) / g), dl ? d_dict + d.off + d.len - dl : nullptr, dl, 0u});
         for (size_t s = 0; s < n; s += g)
             runs.push_back({(uint32_t)(wp.size() + s), (uint32_t)std::min(g, n - s), (uint32_t)wk.size(), 0u});
         for (size_t j = 0; j < n; ++j)
-            wp.push_back({wseg[w0 + j].out_off, seg[a + j].out_off, (uint32_t)wres[w0 + j].out_len, (uint32_t)seg[a + j].out_cap});
+            wp.push_back({wseg[w0 + j].out_off, job.seg[a + j].out_off, (uint32_t)wres[w0 + j].out_len, (uint32_t)job.seg[a + j].out_cap});
         wk.push_back(k);
         wfirst.push_back(w0);
     }
@@ -1214,27 +1244,19 @@ static int inflate_split_window(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_sc
     ZTS_CUDA(ctx, cudaStreamSynchronize(st));
     for (size_t i = 0; i < wk.size(); ++i) {
         if (fail[i]) continue;  // a byte before the start of the stream
-        const size_t k = wk[i], a = first[k], n = first[k + 1] - a;
-        split_finish(h_items[big[k]], &wres[wfirst[i]], &seg[a], n, pieces[a + n - 1].start, res[k], gath);
-        done[k] = 1;
+        h_results[job.big[wk[i]]] = split_finish(job, wk[i], &wres[wfirst[i]], gath);
+        done[job.big[wk[i]]] = 1;
     }
     return ZLB_OK;
 }
 
-// The pieces of the items h_items[big[*]]: one marker scan per item (queued back to back, one read-back for all), a
-// piece starting at 0 and behind every marker that leaves at least one byte. Pieces of item k: [first[k], first[k + 1]),
-// none when it has no marker inside; seg[j] = piece j's input span (out_off / out_cap 0). res / done are reset for
-// nb items, none done. No pieces at all: nothing to split. < 0 on API errors.
+// The pieces of the job's large items (job.first / job.seg): one marker scan per item (queued back to back, one
+// read-back for all), a piece starting at 0 and behind every marker that leaves at least one byte; none for an item
+// without a marker inside. A piece's out_off / out_cap are 0. No pieces at all: nothing to split. < 0 on API errors.
 #define SPLIT_TAG_SHIFT 40  // marks carry the item's index above the byte offset (offsets < 1 TiB, < 16 M large items)
-static int split_layout(zlb_ctx* ctx, const uint8_t* d_in, const zlb_item* h_items, const std::vector<size_t>& big,
-                        std::vector<zlb_result>& res, std::vector<char>& done, std::vector<SplitPiece>& pieces,
-                        std::vector<size_t>& first, std::vector<zlb_item>& seg)
+static int split_layout(zlb_ctx* ctx, const uint8_t* d_in, SplitJob& job)
 {
-    const size_t nb = big.size();
-    res.assign(nb, zlb_result());
-    done.assign(nb, 0);
-    for (size_t k = 0; k < nb; ++k) memset(&res[k], 0, sizeof(zlb_result));
-    pieces.clear();
+    const size_t nb = job.big.size();
     if (nb >= (1ull << 24)) return ZLB_OK;
     cudaStream_t st = ctx->stream;
     int rc = zts_reserve(ctx, &ctx->d_misc, (size_t)SPLIT_MAX_MARKS * 8 + 256);
@@ -1243,7 +1265,7 @@ static int split_layout(zlb_ctx* ctx, const uint8_t* d_in, const zlb_item* h_ite
     uint32_t* d_count = (uint32_t*)ctx->d_misc.p;
     ZTS_CUDA(ctx, cudaMemsetAsync(d_count, 0, 4, st));
     for (size_t k = 0; k < nb; ++k) {
-        const zlb_item& it = h_items[big[k]];
+        const zlb_item& it = job.items[job.big[k]];
         if (it.in_len >= (1ull << SPLIT_TAG_SHIFT)) continue;
         const unsigned grid = (unsigned)((it.in_len / 16 + 255) / 256 + 1);
         ZTS_LAUNCH(ctx, ZK_MARKER_SCAN,
@@ -1258,93 +1280,75 @@ static int split_layout(zlb_ctx* ctx, const uint8_t* d_in, const zlb_item* h_ite
     ZTS_CUDA(ctx, cudaMemcpyAsync(marks.data(), d_marks, (size_t)count * 8, cudaMemcpyDeviceToHost, st));
     ZTS_CUDA(ctx, cudaStreamSynchronize(st));
     std::sort(marks.begin(), marks.end());  // by item, then by offset
-    first.assign(nb + 1, 0);
+    std::vector<zlb_item>& seg = job.seg;
+    job.first.assign(nb + 1, 0);
     size_t mi = 0;
     for (size_t k = 0; k < nb; ++k) {
-        first[k] = pieces.size();
-        const unsigned long long n = h_items[big[k]].in_len;
-        pieces.push_back({(uint32_t)k, 0ull});
+        const zlb_item& it = job.items[job.big[k]];
+        const size_t a = job.first[k] = seg.size();
+        seg.push_back({it.in_off, 0, 0, 0});
         for (; mi < marks.size() && (marks[mi] >> SPLIT_TAG_SHIFT) == k; ++mi) {
             const unsigned long long m = marks[mi] & ((1ull << SPLIT_TAG_SHIFT) - 1);
             // a piece of this engine's streams holds a whole block: never closer than SPLIT_MIN_PIECE bytes to the
             // previous cut (a hostile stream of empty stored blocks would otherwise ask for a slot per 5 bytes)
-            if (m < n && m >= pieces.back().start + SPLIT_MIN_PIECE) pieces.push_back({(uint32_t)k, m});
+            if (m < it.in_len && m >= seg.back().in_off - it.in_off + SPLIT_MIN_PIECE) seg.push_back({it.in_off + m, 0, 0, 0});
         }
-        if (pieces.size() - first[k] < 2) pieces.resize(first[k]);  // no marker inside: nothing to gain
+        if (seg.size() - a < 2) seg.resize(a);  // no marker inside: nothing to gain
+        for (size_t j = a; j < seg.size(); ++j)
+            seg[j].in_len = (j + 1 < seg.size() ? seg[j + 1].in_off : it.in_off + it.in_len) - seg[j].in_off;
     }
-    first[nb] = pieces.size();
-    seg.assign(pieces.size(), zlb_item{0, 0, 0, 0});
-    for (size_t k = 0; k < nb; ++k) {
-        const zlb_item& it = h_items[big[k]];
-        for (size_t j = first[k]; j < first[k + 1]; ++j) {
-            seg[j].in_off = it.in_off + pieces[j].start;
-            seg[j].in_len = (j + 1 < first[k + 1] ? pieces[j + 1].start : it.in_len) - pieces[j].start;
-        }
-    }
+    job.first[nb] = seg.size();
     return ZLB_OK;
 }
 
-// Tries to decode the items h_items[big[*]] piecewise, all of them in one pass: the marker scan (split_layout), one
-// segment-mode launch over the pieces of every item, one window-mode pass for the items whose pieces reach into their
-// predecessors, one gather. done[k] tells whether big[k] worked (then res[k] is filled); the others have to go through
-// the serial decoder. < 0 on API errors.
-static int inflate_split_batch(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const zlb_item* h_items,
-                               const zlb_dict* h_dicts, const uint8_t* d_dict, const std::vector<size_t>& big,
-                               uint32_t flags, std::vector<zlb_result>& res, std::vector<char>& done)
+// Decodes the job's large items piecewise, all of them in one pass: one segment-mode launch over the pieces of every
+// item, one window-mode pass for the items whose pieces reach into their predecessors, one gather. An item that
+// worked gets its result in h_results and done set; the others have to go through the serial decoder. < 0 on API
+// errors.
+static int inflate_split_batch(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const uint8_t* d_dict, SplitJob& job,
+                               uint32_t flags, zlb_result* h_results, std::vector<char>& done)
 {
-    std::vector<SplitPiece> pieces;
-    std::vector<size_t> first;
-    std::vector<zlb_item> seg;
-    int rc = split_layout(ctx, d_in, h_items, big, res, done, pieces, first, seg);
-    if (rc || pieces.empty()) return rc;
-    const size_t nb = big.size(), np = pieces.size();
+    const size_t nb = job.big.size(), np = job.seg.size();
     cudaStream_t st = ctx->stream;
     // slots: a piece of L compressed bytes cannot inflate to more than ~1032 L (258 bytes per 2 bits at best), and a
     // piece of this engine's streams holds at most one 64 KiB chunk
     size_t scratch = 0, big_in = 0;
-    for (size_t k = 0; k < nb; ++k) {
-        if (first[k + 1] > first[k]) big_in += h_items[big[k]].in_len;
-        for (size_t j = first[k]; j < first[k + 1]; ++j) {
-            size_t slot = (size_t)seg[j].in_len * 1032u + 512u;
-            if (slot > SPLIT_SLOT) slot = SPLIT_SLOT;
-            slot = (slot + 255) & ~(size_t)255;
-            seg[j].out_off = scratch;
-            seg[j].out_cap = slot;
-            scratch += slot;
-        }
+    for (size_t k = 0; k < nb; ++k)
+        if (job.pieces(k)) big_in += job.items[job.big[k]].in_len;
+    for (zlb_item& s : job.seg) {
+        size_t slot = (size_t)s.in_len * 1032u + 512u;
+        if (slot > SPLIT_SLOT) slot = SPLIT_SLOT;
+        slot = (slot + 255) & ~(size_t)255;
+        s.out_off = scratch;
+        s.out_cap = slot;
+        scratch += slot;
     }
     const size_t need = ((scratch + 255) & ~(size_t)255) + np * (sizeof(zlb_item) + sizeof(zlb_result) + sizeof(ZtsGather)) + 1024;
     if (need > SplitBudget(ctx->d_split)(big_in, 1)) return ZLB_OK;
     bool got = false;
-    if ((rc = split_reserve(ctx, &ctx->d_split, need, &got)) || !got) return rc;
+    int rc = split_reserve(ctx, &ctx->d_split, need, &got);
+    if (rc || !got) return rc;
     uint8_t* d_scratch = (uint8_t*)ctx->d_split.p;
     zlb_item* d_seg = (zlb_item*)(d_scratch + ((scratch + 255) & ~(size_t)255));
     zlb_result* d_segres = (zlb_result*)(d_seg + np);
     ZtsGather* d_gather = (ZtsGather*)(d_segres + np);
-    ZTS_CUDA(ctx, cudaMemcpyAsync(d_seg, seg.data(), np * sizeof(zlb_item), cudaMemcpyHostToDevice, st));
-    ZTS_CUDA(ctx, cudaMemsetAsync(d_segres, 0, np * sizeof(zlb_result), st));
-    rc = inflate_launch(ctx, st, d_in, d_scratch, d_seg, d_segres, np,
-                        (flags & ZLB_INFLATE_CHECK_NLEN) | ZLB_INFLATE_SEGMENT);
-    if (rc) return rc;
-    std::vector<zlb_result> sres(np);
-    ZTS_CUDA(ctx, cudaMemcpyAsync(sres.data(), d_segres, np * sizeof(zlb_result), cudaMemcpyDeviceToHost, st));
-    ZTS_CUDA(ctx, cudaStreamSynchronize(st));
+    std::vector<zlb_result> sres;
+    if ((rc = split_segments<INF_BYTES>(ctx, d_in, d_scratch, job.seg, d_seg, d_segres, flags, sres))) return rc;
     // validate every item's chain of pieces; the valid ones are gathered in one launch, together with those that
     // window mode decodes
     std::vector<ZtsGather> gath;
     std::vector<size_t> window;
     for (size_t k = 0; k < nb; ++k) {
-        const size_t a = first[k], b = first[k + 1];
-        if (b - a < 2) continue;
-        const int chain = split_chain(&sres[a], &seg[a], b - a, true, h_dicts && h_dicts[big[k]].len);
+        const size_t a = job.first[k], n = job.pieces(k);
+        if (n < 2) continue;
+        const int chain = split_chain(&sres[a], &job.seg[a], n, true, job.dicts && job.dicts[job.big[k]].len);
         if (chain == SPLIT_WINDOW) window.push_back(k);
         if (chain != SPLIT_OK) continue;
-        split_finish(h_items[big[k]], &sres[a], &seg[a], b - a, pieces[b - 1].start, res[k], gath);
-        done[k] = 1;
+        h_results[job.big[k]] = split_finish(job, k, &sres[a], gath);
+        done[job.big[k]] = 1;
     }
     if (!window.empty()) {
-        rc = inflate_split_window(ctx, d_in, d_scratch, h_items, h_dicts, d_dict, big, flags, pieces, first, seg, window, res,
-                                  done, gath);
+        rc = inflate_split_window(ctx, d_in, d_scratch, d_dict, job, flags, window, h_results, done, gath);
         if (rc) return rc;
     }
     if (!gath.empty()) {
@@ -1355,47 +1359,34 @@ static int inflate_split_batch(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out
     return ZLB_OK;
 }
 
-// The marker split of a size call: the items h_items[big[*]] are cut as inflate_split_batch cuts them and every piece of
-// every item is sized by one segment-mode launch of the size decoder. A piece's size does not depend on the bytes in
-// front of it, only whether a distance reaches before the stream (or before its dictionary) does, and a piece tells
-// how far in front of its first byte it reached (crc32). So an item is settled when its chain passes and no piece
-// reaches further than the output of the pieces in front of it plus the dictionary's reachable bytes; it then gets
-// the one-warp decoder's result by construction. No byte slots and no window scratch: the piece tables take the place
-// of the marks. done / res as for inflate_split_batch.
-static int inflate_split_sizes(zlb_ctx* ctx, const uint8_t* d_in, const zlb_item* h_items, const zlb_dict* h_dicts,
-                               const std::vector<size_t>& big, uint32_t flags, std::vector<zlb_result>& res,
-                               std::vector<char>& done)
+// The marker split of a size call: the job's pieces are sized by one segment-mode launch of the size decoder. A
+// piece's size does not depend on the bytes in front of it, only whether a distance reaches before the stream (or
+// before its dictionary) does, and a piece tells how far in front of its first byte it reached (crc32). So an item is
+// settled when its chain passes and no piece reaches further than the output of the pieces in front of it plus the
+// dictionary's reachable bytes; it then gets the one-warp decoder's result by construction. No byte slots and no
+// window scratch: the piece tables take the place of the marks. h_results / done as for inflate_split_batch.
+static int inflate_split_sizes(zlb_ctx* ctx, const uint8_t* d_in, const SplitJob& job, uint32_t flags,
+                               zlb_result* h_results, std::vector<char>& done)
 {
-    std::vector<SplitPiece> pieces;
-    std::vector<size_t> first;
-    std::vector<zlb_item> seg;
-    int rc = split_layout(ctx, d_in, h_items, big, res, done, pieces, first, seg);
-    if (rc || pieces.empty()) return rc;
-    const size_t nb = big.size(), np = pieces.size();
-    cudaStream_t st = ctx->stream;
-    if ((rc = zts_reserve(ctx, &ctx->d_misc, np * (sizeof(zlb_item) + sizeof(zlb_result)) + 256))) return rc;
-    zlb_item* d_seg = (zlb_item*)ctx->d_misc.p;
-    zlb_result* d_segres = (zlb_result*)(d_seg + np);
-    ZTS_CUDA(ctx, cudaMemcpyAsync(d_seg, seg.data(), np * sizeof(zlb_item), cudaMemcpyHostToDevice, st));
-    ZTS_CUDA(ctx, cudaMemsetAsync(d_segres, 0, np * sizeof(zlb_result), st));
-    rc = inflate_launch(ctx, st, d_in, nullptr, d_seg, d_segres, np, (flags & ZLB_INFLATE_CHECK_NLEN) | ZLB_INFLATE_SEGMENT);
+    const size_t np = job.seg.size();
+    int rc = zts_reserve(ctx, &ctx->d_misc, np * (sizeof(zlb_item) + sizeof(zlb_result)) + 256);
     if (rc) return rc;
-    std::vector<zlb_result> sres(np);
-    ZTS_CUDA(ctx, cudaMemcpyAsync(sres.data(), d_segres, np * sizeof(zlb_result), cudaMemcpyDeviceToHost, st));
-    ZTS_CUDA(ctx, cudaStreamSynchronize(st));
-    for (size_t k = 0; k < nb; ++k) {
-        const size_t a = first[k], b = first[k + 1];
-        if (b - a < 2 || split_chain(&sres[a], &seg[a], b - a, false, false) != SPLIT_OK) continue;
-        const unsigned long long dl = h_dicts ? std::min(h_dicts[big[k]].len, (uint64_t)WIN_WORDS) : 0;
+    zlb_item* d_seg = (zlb_item*)ctx->d_misc.p;
+    std::vector<zlb_result> sres;
+    if ((rc = split_segments<INF_SIZE>(ctx, d_in, nullptr, job.seg, d_seg, (zlb_result*)(d_seg + np), flags, sres))) return rc;
+    for (size_t k = 0; k < job.big.size(); ++k) {
+        const size_t a = job.first[k], n = job.pieces(k);
+        if (n < 2 || split_chain(&sres[a], &job.seg[a], n, false, false) != SPLIT_OK) continue;
+        const unsigned long long dl = job.dicts ? std::min(job.dicts[job.big[k]].len, (uint64_t)WIN_WORDS) : 0;
         unsigned long long before = 0;  // output of the pieces in front
         bool fits = true;
-        for (size_t j = a; j < b && fits; ++j) {
+        for (size_t j = a; j < a + n && fits; ++j) {
             fits = sres[j].crc32 <= before + dl;
             before += sres[j].out_len;
         }
         if (!fits) continue;
-        res[k] = split_result(&sres[a], b - a, pieces[b - 1].start);
-        done[k] = 1;
+        h_results[job.big[k]] = split_result(job, k, &sres[a]);
+        done[job.big[k]] = 1;
     }
     return ZLB_OK;
 }
@@ -1509,8 +1500,9 @@ static int inflate_waves(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, cons
 }
 
 // Decodes n items on device buffers; results land in h_results after the final synchronise. The item table goes to the
-// device with the dictionary table beside it. With ZLB_INFLATE_SPLIT the large items are tried piecewise first
-// (inflate_split_batch); the items left go through one decoder launch, over a compacted table when the split did some.
+// device with the dictionary table beside it. With ZLB_INFLATE_SPLIT the large items are cut at markers (split_layout)
+// and tried piecewise first (inflate_split_batch), which settles some of them in h_results and in the mask `done`;
+// the items left go through one decoder launch, over a compacted table when the split settled any.
 // Then one tail: checksums, the result read-back and, on a "_host" call, the copy-back of the outputs. A "_host" call
 // without a split runs in waves instead (inflate_waves).
 // d_dict / h_dicts: the preset dictionaries (h_dicts == NULL: none; checked by the caller)
@@ -1522,13 +1514,13 @@ static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
                           const ZtsHostIO* hio)
 {
     // large items that may be cut at sync-flush markers (each is massively parallel by itself)
-    std::vector<size_t> big;
+    SplitJob job{h_items, h_dicts, {}, {}, {}};
     if ((flags & ZLB_INFLATE_SPLIT) && !(flags & ZLB_INFLATE_SEGMENT))
         for (size_t i = 0; i < n; ++i)
-            if (h_items[i].in_len >= SPLIT_MIN_BYTES) big.push_back(i);
+            if (h_items[i].in_len >= SPLIT_MIN_BYTES) job.big.push_back(i);
     // d_items holds the call's per-item tables: items | dictionaries, and with a split the same for the items left
     const size_t row = sizeof(zlb_item) + (h_dicts ? sizeof(zlb_dict) : 0);
-    int rc = zts_reserve(ctx, &ctx->d_items, (big.empty() ? 1 : 2) * n * row + 64);
+    int rc = zts_reserve(ctx, &ctx->d_items, (job.big.empty() ? 1 : 2) * n * row + 64);
     if (rc) return rc;
     rc = zts_reserve(ctx, &ctx->d_results, n * sizeof(zlb_result) + 64);
     if (rc) return rc;
@@ -1549,7 +1541,7 @@ static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
     if (flags & ZLB_INFLATE_WANT_CRC32) kinds |= ZLB_SUM_CRC32;
     if (flags & ZLB_INFLATE_WANT_ADLER32) kinds |= ZLB_SUM_ADLER32;
     const bool sizes = d_out == nullptr;
-    if (hio && big.empty() && !sizes)
+    if (hio && job.big.empty() && !sizes)
         return inflate_waves(ctx, d_in, d_out, d_dict, d_items, d_dicts, d_results, h_items, h_results, n, flags, kinds, *hio);
 
     // the split: the items it decodes get their results in h_results; when it decoded any, rest lists the others
@@ -1564,18 +1556,14 @@ static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
         zts_stage_wait_in(hio->stage, 0, hio->in_bytes);
         ZTS_CUDA(ctx, cudaMemcpyAsync((void*)d_in, hio->h_in, hio->in_bytes, cudaMemcpyHostToDevice, ctx->stream));
     }
-    if (!big.empty()) {
-        std::vector<zlb_result> bres;
-        std::vector<char> bdone, done(n, 0);
-        rc = sizes ? inflate_split_sizes(ctx, d_in, h_items, h_dicts, big, flags, bres, bdone)
-                   : inflate_split_batch(ctx, d_in, d_out, h_items, h_dicts, d_dict, big, flags, bres, bdone);
+    if (!job.big.empty()) {
+        std::vector<char> done(n, 0);
+        rc = split_layout(ctx, d_in, job);
+        if (!rc && !job.seg.empty())
+            rc = sizes ? inflate_split_sizes(ctx, d_in, job, flags, h_results, done)
+                       : inflate_split_batch(ctx, d_in, d_out, d_dict, job, flags, h_results, done);
         if (rc) return rc;
-        for (size_t k = 0; k < big.size(); ++k)
-            if (bdone[k]) {
-                done[big[k]] = 1;
-                h_results[big[k]] = bres[k];
-                split_any = true;
-            }
+        split_any = std::find(done.begin(), done.end(), 1) != done.end();
         if (split_any) {
             for (size_t i = 0; i < n; ++i)
                 if (!done[i]) {
