@@ -109,11 +109,15 @@ enum {
     ZLB_INFLATE_WANT_ADLER32 = 1u << 1, /* results[i].adler32 = Adler-32 of item output */
     ZLB_INFLATE_CHECK_NLEN = 1u << 2,   /* verify NLEN == ~LEN in stored blocks (the reference
                                            never does: src/RawInflate.ts:277 is always false) */
-    ZLB_INFLATE_SPLIT = 1u << 3,        /* large items may be cut at sync-flush markers (empty stored blocks,
-                                           `00 00 FF FF`) and their pieces decoded side by side: independent
-                                           pieces (what zlb_deflate_batch emits) directly, pieces that reach up to
-                                           32 KiB into the ones before (ZLB_MODE_PRIMED, zlib's Z_SYNC_FLUSH) in
-                                           window mode; anything else falls back to the one-warp decoder. Results
+    ZLB_INFLATE_SPLIT = 1u << 3,        /* large items are cut where the engine can prove a block boundary and
+                                           their pieces decoded side by side: at sync-flush markers (empty stored
+                                           blocks, `00 00 FF FF`), and in any stream -- gzip, zlib.compress, any
+                                           encoder -- at block starts found on the device in stretches of more than
+                                           1 MiB without markers. Independent pieces (what zlb_deflate_batch
+                                           emits) are decoded directly, pieces that reach up to 32 KiB into the ones
+                                           before (ZLB_MODE_PRIMED, zlib's Z_SYNC_FLUSH, found block starts) in
+                                           window mode; a cut is used only once the piece in front of it ended
+                                           exactly there, anything else falls back to the one-warp decoder. Results
                                            are identical. */
     ZLB_INFLATE_SEGMENT = 1u << 4       /* internal: an item may end at a block boundary without BFINAL */
 };
@@ -224,8 +228,8 @@ int zlb_inflate_batch_dict_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes,
  * no bytes to sum), as is a NULL input with items. results[i].status / out_len / in_used / blocks equal those
  * zlb_inflate_batch_dict returns for the same item, flags and dictionary with out_cap >= the item's size (never
  * ZLB_ST_OUT_OVERFLOW); crc32 = adler32 = 0. A size-only decode stores nothing and skips stored data; with
- * ZLB_INFLATE_SPLIT every stream the marker split can cut, primed and Z_SYNC_FLUSH ones included, is sized piecewise
- * without scratch for its bytes.                                                                                 */
+ * ZLB_INFLATE_SPLIT every stream the split can cut, primed, Z_SYNC_FLUSH and marker-less ones included, is sized
+ * piecewise without scratch for its bytes.                                                                                 */
 int zlb_inflate_size_batch(zlb_ctx* ctx, const void* d_in, const zlb_dict* dicts, const zlb_item* items,
                            zlb_result* results, size_t n_items, uint32_t flags);
 int zlb_inflate_size_batch_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes, const zlb_dict* dicts,
@@ -302,6 +306,12 @@ int zlb_debug_lz77(zlb_ctx* ctx, const void* d_in, uint32_t n, uint32_t* h_token
                    uint32_t* n_tokens, uint32_t* h_hist_out);
 /* code lengths for one histogram (src/RawDeflate.ts:440-474): freqs[nsym] -> lengths[nsym]     */
 int zlb_debug_code_lengths(zlb_ctx* ctx, const uint32_t* h_freqs, int nsym, int limit, uint8_t* h_lengths);
+/* the block finder of ZLB_INFLATE_SPLIT on the n input bytes at d_in, taken as one item: for each byte position
+ * h_cuts[c] (< n), h_bits_out[c] = the first candidate bit offset b in [8 h_cuts[c], 8 h_cuts[c] + span) -- a dynamic
+ * block header as an encoder writes it (the offset itself), or a stored block with LEN == ~NLEN (the offset of the
+ * block behind it) -- or UINT64_MAX when there is none. One kernel launch; synchronises.                         */
+int zlb_debug_block_starts(zlb_ctx* ctx, const void* d_in, uint64_t n, const uint64_t* h_cuts, size_t n_cuts,
+                           uint64_t span, uint64_t* h_bits_out);
 
 #ifdef __cplusplus
 }

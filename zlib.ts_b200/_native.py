@@ -43,7 +43,7 @@ EXPORTS = [
     "zlb_checksum_batch", "zlb_checksum_batch_host", "zlb_crc32_combine", "zlb_adler32_combine",
     "zlb_archive", "zlb_archive_host", "zlb_archive_bound",
     "zlb_profile_enable", "zlb_profile_read", "zlb_profile_reset", "zlb_launch_count",
-    "zlb_debug_lz77", "zlb_debug_code_lengths",
+    "zlb_debug_lz77", "zlb_debug_code_lengths", "zlb_debug_block_starts",
     "zlb_host_alloc", "zlb_host_free", "zlb_host_is_pinned",
     "zlb_deflate_batch_dict", "zlb_deflate_batch_dict_host", "zlb_inflate_batch_dict", "zlb_inflate_batch_dict_host",
     "zlb_inflate_size_batch", "zlb_inflate_size_batch_host",
@@ -121,6 +121,8 @@ def load_library():
     lib.zlb_debug_lz77.restype = i32
     lib.zlb_debug_code_lengths.argtypes = [vp, vp, i32, i32, vp]
     lib.zlb_debug_code_lengths.restype = i32
+    lib.zlb_debug_block_starts.argtypes = [vp, vp, u64, vp, sz, u64, vp]
+    lib.zlb_debug_block_starts.restype = i32
     lib.zlb_host_alloc.argtypes = [sz, ctypes.POINTER(vp)]
     lib.zlb_host_alloc.restype = i32
     lib.zlb_host_free.argtypes = [vp]
@@ -433,6 +435,16 @@ class Engine:
         rc = self.lib.zlb_debug_code_lengths(self.h, freqs.ctypes.data, len(freqs), limit, lengths.ctypes.data)
         self._check(rc, "zlb_debug_code_lengths")
         return lengths
+
+    def debug_block_starts(self, d_in, cuts, span):
+        """The split's block finder on the bytes of d_in (a CUDA uint8 tensor) as one item: per byte position in
+        `cuts`, the first candidate bit offset in [8 cut, 8 cut + span) (a stored block: where it ends), or -1."""
+        cuts = np.ascontiguousarray(cuts, dtype=np.uint64)
+        out = np.zeros(len(cuts), dtype=np.uint64)
+        rc = self.lib.zlb_debug_block_starts(self.h, d_in.data_ptr(), d_in.numel(), cuts.ctypes.data, len(cuts), span,
+                                             out.ctypes.data)
+        self._check(rc, "zlb_debug_block_starts")
+        return np.where(out == np.uint64(2**64 - 1), -1, out.astype(np.int64))
 
 
 _default_engines = {}

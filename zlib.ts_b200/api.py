@@ -204,7 +204,8 @@ def inflate_blob(blob, offs, lens, size_hints=None, want_crc32=False, want_adler
     for i in range(n):
         hint = None if size_hints is None else size_hints[i]
         caps[i] = int(hint) if hint is not None else max(0x8000, 4 * int(lens[i]))  # DefaultInflateBufferSize
-    # large streams written by this engine decode piecewise at their sync-flush markers (same result, see the header)
+    # large streams decode piecewise wherever the engine can prove a block boundary: at sync-flush markers, and in any
+    # other stream (gzip, zlib.compress, ...) at block starts found on the device (same result, see the header)
     flags = ((N.INFLATE_WANT_CRC32 if want_crc32 else 0) | (N.INFLATE_WANT_ADLER32 if want_adler32 else 0) |
              (N.INFLATE_SPLIT if split else 0))
     if blob.size == 0:
@@ -656,16 +657,30 @@ class GUnzip:
         caps = np.maximum(0x8000, 4 * gaps)
         index_of = {c: i for i, c in enumerate(starts)}
         outs, res = [None] * len(starts), np.zeros(len(starts), dtype=N.RESULT_DTYPE)
+
+        def decode(idx):
+            """inflates the candidates idx (ascending). The first member (candidate 0, at offset 0) goes through the
+            split, which decodes one large stream in parallel from whatever wrote it (its item reaches to the end of the
+            buffer, the split stops where its stream does); the other candidates' items reach to the end as well, so
+            they are inflated in one call without the split, which would scan the rest of the buffer once per candidate."""
+            idx = list(idx)
+            if idx and idx[0] == 0:
+                o, r = inflate_blob(inp, offs[:1], lens[:1], [int(caps[0])], want_crc32=True, tolerant=True)
+                outs[0], res[0] = o[0], r[0]
+                idx = idx[1:]
+            if idx:
+                o, r = inflate_blob(inp, offs[idx], lens[idx], list(caps[idx]), want_crc32=True, split=False,
+                                    tolerant=True)
+                for k, i in enumerate(idx):
+                    outs[i], res[i] = o[k], r[k]
+
         g0 = 0
         while g0 < len(starts):  # groups of candidates whose output slots stay below 2 GiB together
             g1, tot = g0, 0
             while g1 < len(starts) and (g1 == g0 or tot + int(caps[g1]) <= (2 << 30)):
                 tot += int(caps[g1])
                 g1 += 1
-            o1, r1 = inflate_blob(inp, offs[g0:g1], lens[g0:g1], list(caps[g0:g1]), want_crc32=True, split=False,
-                                  tolerant=True)
-            outs[g0:g1] = o1
-            res[g0:g1] = r1
+            decode(range(g0, g1))
             g0 = g1
         for _ in range(6):  # candidates on the chain whose slot was too small are decoded again, larger
             pos, retry = 0, None
@@ -682,10 +697,7 @@ class GUnzip:
                 break
             again = [i for i in range(retry, len(starts)) if int(res["status"][i]) == N.ST_OUT_OVERFLOW]
             caps[again] *= 4
-            o2, r2 = inflate_blob(inp, offs[again], lens[again], list(caps[again]), want_crc32=True, split=False,
-                                  tolerant=True)
-            for k, i in enumerate(again):
-                outs[i], res[i] = o2[k], r2[k]
+            decode(again)
         while self.ip < inp.size and self.ip in index_of:
             i = index_of[self.ip]
             if int(res["status"][i]) != N.ST_OK:

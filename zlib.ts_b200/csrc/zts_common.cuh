@@ -33,6 +33,7 @@ enum ZtsKernelSlot {
     ZK_DICT_STAGE,      // preset dictionaries (zts_deflate.cu, zts_inflate.cu)
     ZK_INFLATE_DICT,
     ZK_INFLATE_SIZE,    // zlb_inflate_size_batch (zts_inflate.cu)
+    ZK_BLOCK_FIND,      // block starts in streams without markers (zts_inflate.cu)
     ZK_COUNT
 };
 
@@ -43,7 +44,12 @@ static const char* const kZtsKernelNames[ZK_COUNT] = {
     "marker_scan_kernel",  "segment_gather_kernel",
     "frame_body_kernel",   "frame_header_kernel",
     "inflate_warp_kernel_window", "window_run_kernel", "window_scan_kernel", "window_resolve_kernel",
-    "dict_stage_kernel", "inflate_warp_kernel_dict", "inflate_warp_kernel_size"};
+    "dict_stage_kernel", "inflate_warp_kernel_dict", "inflate_warp_kernel_size",
+    "block_find_kernel"};
+
+// internal inflate flag beside ZLB_INFLATE_SEGMENT (not in the public header): an item's in_off / in_len and its
+// result's in_used count bits, so that a piece of a stream may start and end inside a byte (the searched split)
+#define ZLB_INFLATE_BITS (1u << 5)
 
 struct ZtsDevBuf {
     void* p = nullptr;

@@ -342,7 +342,9 @@ __device__ uint32_t inf_classify_symbols(const InfWarpSmem* S, const uint8_t* sr
 // it decodes and checks exactly like INF_BYTES but stores no byte, copies no match, skips stored data after its LEN
 // check and has no capacity; only the dictionary's length is read (dicts may be NULL). In segment mode a distance that
 // reaches before the piece's first byte does not fail it: results[item].crc32 tells how far in front the piece
-// reached, at most 32768 (the marker split compares that with the output of the pieces in front).
+// reached, at most 32768 (the marker split compares that with the output of the pieces in front). INF_SIZE and
+// INF_WINDOW read ZLB_INFLATE_BITS (the searched split): in_off / in_len / in_used count bits. Positions then count
+// from the piece's first byte, its first bits consumed at the start, so that a stored block's byte alignment holds.
 #define WIN_WORDS 32768u
 enum { INF_BYTES = 0, INF_WINDOW = 1, INF_DICT = 2, INF_SIZE = 3 };
 template <int MODE>
@@ -360,7 +362,11 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
     if (item >= n_items) return;
 
     const zlb_item it = items[item];
-    const uint8_t* src = in + it.in_off;
+    constexpr bool BITS_OK = MODE == INF_SIZE || MODE == INF_WINDOW;
+    const bool bits = BITS_OK && (flags & ZLB_INFLATE_BITS);
+    const uint32_t sb = bits ? (uint32_t)(it.in_off & 7u) : 0u;  // bits of the first byte in front of the piece
+    const uint8_t* src = in + (bits ? it.in_off >> 3 : it.in_off);
+    const unsigned long long in_len = bits ? (sb + it.in_len + 7) >> 3 : it.in_len;  // bytes the piece touches
     T* dst = reinterpret_cast<T*>(out + it.out_off);
     uint32_t reach = MODE == INF_WINDOW ? WIN_WORDS : 0u;  // how far a distance may reach in front of the output
     const uint8_t* dtail = nullptr;                       // INF_DICT: the `reach` bytes in front of the output
@@ -386,12 +392,14 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
         }
         __syncwarp();
     }
-    const unsigned long long in_bits = it.in_len * 8ull;
+    const unsigned long long in_bits = bits ? sb + it.in_len : it.in_len * 8ull;
     const unsigned long long cap = it.out_cap;
 
     BitReader br;
     br.ring_s = (uint32_t)__cvta_generic_to_shared(S->ring);
-    br_init(br, src, src + it.in_len, 0);
+    br_init(br, src, src + in_len, 0);
+    if constexpr (BITS_OK)
+        if (sb) br_take(br, (int)sb);
 
     unsigned long long op = 0;
     uint32_t status = ZLB_ST_OK;
@@ -416,9 +424,9 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
             // ---- stored block (src/RawInflate.ts:251-318): drop to the byte boundary, LEN, NLEN
             unsigned long long used = br_bits_used(br);
             unsigned long long byte_pos = (used + 7) >> 3;
-            if (byte_pos + 4 > it.in_len) {
+            if (byte_pos + 4 > in_len) {
                 // src/RawInflate.ts:266 (LEN) / :272 (NLEN): which of the two 16-bit fields is cut short
-                status = byte_pos + 2 > it.in_len ? ZLB_ST_STORED_LEN : (ZLB_ST_STORED_LEN | (1u << 8));
+                status = byte_pos + 2 > in_len ? ZLB_ST_STORED_LEN : (ZLB_ST_STORED_LEN | (1u << 8));
                 break;
             }
             const uint8_t* p = src + byte_pos;
@@ -429,7 +437,7 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
                 break;
             }
             byte_pos += 4;
-            if (byte_pos + len > it.in_len) {
+            if (byte_pos + len > in_len) {
                 status = ZLB_ST_INPUT_BROKEN;
                 break;
             }
@@ -440,7 +448,7 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
             if constexpr (MODE != INF_SIZE)
                 for (uint32_t k = lane; k < len; k += 32) dst[op + k] = src[byte_pos + k];
             op += len;
-            br_init(br, src + byte_pos + len, src + it.in_len, (byte_pos + len) * 8ull);
+            br_init(br, src + byte_pos + len, src + in_len, (byte_pos + len) * 8ull);
             __syncwarp();
             continue;
         }
@@ -514,7 +522,7 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
                     if (i + k < total) S->stage[i + k] = (uint8_t)val;
                 i += rep;
                 prev = val;
-                if (br_bits_used(br) > in_bits) status = inf_classify_cl(S, src, it.in_len, cl_pos);
+                if (br_bits_used(br) > in_bits) status = inf_classify_cl(S, src, in_len, cl_pos);
             }
             if (status != ZLB_ST_OK) break;
             __syncwarp();
@@ -645,7 +653,7 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
             if (br_bits_used(br) > in_bits) {
                 // the batch ran past the end of the input: nothing of it is trusted; which error it is -- a code or
                 // extra bits cut short -- is found by replaying the batch
-                status = inf_classify_symbols(S, src, it.in_len, batch_pos);
+                status = inf_classify_symbols(S, src, in_len, batch_pos);
                 break;
             }
             // -- output positions: exclusive prefix sum of the token lengths
@@ -768,7 +776,7 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
         r.status = status;
         r.blocks = blocks | ((flags & ZLB_INFLATE_SEGMENT) && bfinal ? 0x80000000u : 0u);  // segment mode: saw BFINAL
         r.out_len = op;
-        r.in_used = (br_bits_used(br) + 7) >> 3;  // whole unread bytes are given back (:511-514)
+        r.in_used = bits ? br_bits_used(br) - sb : (br_bits_used(br) + 7) >> 3;  // whole unread bytes are given back (:511-514)
         results[item] = r;
     }
 }
@@ -828,6 +836,176 @@ marker_scan_kernel(const uint8_t* __restrict__ in, unsigned long long n, unsigne
             if (slot < cap) marks[slot] = tag | (base + k + 4);  // first byte after the marker (+ the item's tag)
         }
     }
+}
+
+// ---- block finder: where a stream without markers may be cut ----------------------------------------------------
+// An ordinary zlib / gzip stream has no markers; its blocks start at arbitrary bit offsets. block_find_kernel tests
+// the bit offsets of a span, one warp per span and one offset per lane, for a block header that an encoder would
+// write: BFINAL = 0 and a dynamic header whose three codes are ones an encoder writes (zlib's own rules, stricter than
+// the decoder), or a stored block whose LEN / NLEN agree. A span's answer is the first offset that passes. Nothing
+// depends on it being right: the split uses a cut only once the piece in front of it decoded cleanly and ended exactly
+// there (split_chain), so a false candidate costs time, never a result. A stored block is proposed by where it ends:
+// the block behind it starts exactly there, while its own header may be preceded by zero bits that pass the same test.
+struct ZtsFindCut {
+    unsigned long long first, last, end;  // bits of the input: offsets [first, last) are tested; a block ends by `end`
+};
+#define FIND_WARPS 4
+#define FIND_NONE (~0ull)
+
+// 32 bits of the input at bit `pos` (aligned word loads of words that overlap [.., end_byte); zero behind)
+__device__ __forceinline__ uint32_t find_peek(const uint8_t* in, unsigned long long pos, const uint8_t* end)
+{
+    const uintptr_t a = (uintptr_t)(in + (pos >> 3));
+    const uint32_t* p = (const uint32_t*)(a & ~(uintptr_t)3);
+    const uint32_t w0 = (const uint8_t*)p < end ? __ldg(p) : 0u;
+    const uint32_t w1 = (const uint8_t*)(p + 1) < end ? __ldg(p + 1) : 0u;
+    return (uint32_t)((((unsigned long long)w1 << 32) | w0) >> ((a & 3u) * 8u + (uint32_t)(pos & 7u)));
+}
+
+// the dynamic block header at bit b (its first 17 bits passed the prefilter): the code-length code is complete, the
+// HLIT + HDIST lengths decode without a leading repeat and without overrunning, the literal / length code is complete
+// and codes symbol 256, the distance code is complete, one code of length 1 or empty, and all of it ends by `end`.
+// tab: this lane's 128-entry table of the code-length code (symbol | length << 5).
+__device__ bool find_dynamic(const uint8_t* in, unsigned long long b, unsigned long long end, const uint8_t* in_end,
+                             uint8_t* tab)
+{
+    const uint32_t h = find_peek(in, b, in_end);
+    const uint32_t hlit = ((h >> 3) & 31u) + 257u, hdist = ((h >> 8) & 31u) + 1u, hclen = ((h >> 13) & 15u) + 4u;
+    unsigned long long pos = b + 17;
+    if (pos + 3 * hclen > end) return false;
+    const unsigned long long lo = find_peek(in, pos, in_end), hi = find_peek(in, pos + 32, in_end);
+    const unsigned long long v = lo | (hi << 32);
+    unsigned long long lens = 0;  // 3 bits per code-length symbol
+    uint32_t kraft = 0;
+    for (uint32_t i = 0; i < hclen; ++i) {
+        const uint32_t l = (uint32_t)(v >> (3 * i)) & 7u;
+        lens |= (unsigned long long)l << (3 * c_huff_order[i]);
+        kraft += l ? 128u >> l : 0u;
+    }
+    if (kraft != 128u) return false;
+    pos += 3 * hclen;
+    uint32_t code = 0;
+    for (uint32_t L = 1; L <= 7; ++L) {
+        for (uint32_t s = 0; s < 19; ++s) {
+            if (((lens >> (3 * s)) & 7u) != L) continue;
+            for (uint32_t j = __brev(code) >> (32 - L); j < 128u; j += 1u << L) tab[j] = (uint8_t)(s | (L << 5));
+            ++code;
+        }
+        code <<= 1;
+    }
+    const uint32_t total = hlit + hdist;
+    uint32_t i = 0, prev = 0, lit_k = 0, dist_k = 0, dist_n = 0;
+    bool has_eob = false;
+    while (i < total) {
+        uint32_t x = find_peek(in, pos, in_end);
+        const uint32_t e = tab[x & 127u], L = e >> 5, sym = e & 31u;
+        pos += L;
+        x >>= L;
+        uint32_t rep = 1, val = sym;
+        if (sym == 16) {
+            if (i == 0) return false;
+            rep = 3 + (x & 3u);
+            pos += 2;
+            val = prev;
+        } else if (sym == 17) {
+            rep = 3 + (x & 7u);
+            pos += 3;
+            val = 0;
+        } else if (sym == 18) {
+            rep = 11 + (x & 127u);
+            pos += 7;
+            val = 0;
+        }
+        if (i + rep > total || pos > end) return false;
+        const uint32_t nl = i < hlit ? min(rep, hlit - i) : 0u, nd = rep - nl;
+        if (val) {
+            lit_k += nl << (15 - val);
+            dist_k += nd << (15 - val);
+            dist_n += nd;
+        }
+        if (i <= 256u && 256u < i + nl) has_eob = val != 0;
+        prev = val;
+        i += rep;
+    }
+    return lit_k == (1u << 15) && has_eob && (dist_k == (1u << 15) || dist_n == 0 || (dist_n == 1 && dist_k == (1u << 14)));
+}
+
+// the stored block at bit b (its 3 header bits are zero): zero padding, LEN == ~NLEN, the block ends before `end`,
+// and the block behind it is a stored one (LEN == ~NLEN) or passes the dynamic test (BFINAL either): 3 zero bits and
+// two 16-bit fields that agree turn up in compressed data every few hundred KB, this second header makes such a
+// chance hit rare. Returns the bit where it ends, FIND_NONE if it is not one.
+__device__ unsigned long long find_stored(const uint8_t* in, unsigned long long b, uint32_t h, unsigned long long end,
+                                          const uint8_t* in_end, uint8_t* tab)
+{
+    const unsigned long long a = (b + 3 + 7) & ~7ull;  // the byte boundary LEN starts at
+    const uint32_t pad = (uint32_t)(a - b - 3);
+    if (((h >> 3) & ((1u << pad) - 1u)) != 0) return FIND_NONE;
+    if (a + 32 > end) return FIND_NONE;
+    const uint32_t w = find_peek(in, a, in_end);
+    if (((w & 0xFFFFu) ^ (w >> 16)) != 0xFFFFu) return FIND_NONE;
+    const unsigned long long stop = a + 32 + 8ull * (w & 0xFFFFu);
+    if (stop + 40 > end) return FIND_NONE;
+    const uint32_t h2 = find_peek(in, stop, in_end);
+    if ((h2 & 0xFEu) == 0u) {  // stored, starting on the byte boundary
+        const uint32_t w2 = find_peek(in, stop + 8, in_end);
+        return ((w2 & 0xFFFFu) ^ (w2 >> 16)) == 0xFFFFu ? stop : FIND_NONE;
+    }
+    if ((h2 & 6u) == 4u && ((h2 >> 3) & 31u) <= 29u && ((h2 >> 8) & 31u) <= 29u && find_dynamic(in, stop, end, in_end, tab))
+        return stop;
+    return FIND_NONE;
+}
+
+// out[c] = the first candidate of span c (a stored block: where it ends), FIND_NONE if there is none
+__global__ void __launch_bounds__(FIND_WARPS * 32)
+block_find_kernel(const uint8_t* __restrict__ in, const ZtsFindCut* __restrict__ cuts, uint32_t n,
+                  unsigned long long* __restrict__ out)
+{
+    __shared__ uint8_t tabs[FIND_WARPS * 32][128];
+    const unsigned lane = zts_lane();
+    const uint32_t c = blockIdx.x * FIND_WARPS + (threadIdx.x >> 5);
+    if (c >= n) return;
+    const ZtsFindCut cut = cuts[c];
+    const uint8_t* in_end = in + ((cut.end + 7) >> 3);
+    unsigned long long found = FIND_NONE;
+    for (unsigned long long base = cut.first; base < cut.last; base += 32) {
+        const unsigned long long b = base + lane;
+        unsigned long long prop = FIND_NONE;
+        if (b < cut.last && b + 17 <= cut.end) {
+            const uint32_t h = find_peek(in, b, in_end);
+            // prefilter on 17 bits: BFINAL = 0, BTYPE = 2, HLIT <= 286, HDIST <= 30 (or BTYPE = 0)
+            if ((h & 7u) == 4u) {
+                if (((h >> 3) & 31u) <= 29u && ((h >> 8) & 31u) <= 29u && find_dynamic(in, b, cut.end, in_end, tabs[threadIdx.x]))
+                    prop = b;
+            } else if ((h & 7u) == 0u) {
+                prop = find_stored(in, b, h, cut.end, in_end, tabs[threadIdx.x]);
+            }
+        }
+        const unsigned m = __ballot_sync(0xFFFFFFFFu, prop != FIND_NONE);
+        if (m) {
+            found = __shfl_sync(0xFFFFFFFFu, prop, __ffs((int)m) - 1);
+            break;
+        }
+    }
+    if (lane == 0) out[c] = found;
+}
+
+// one launch of the finder over h_cuts; results in h_out. The tables go to ctx->d_misc.
+static int block_find(zlb_ctx* ctx, const uint8_t* d_in, const std::vector<ZtsFindCut>& h_cuts, unsigned long long* h_out)
+{
+    const size_t n = h_cuts.size();
+    if (!n) return ZLB_OK;
+    cudaStream_t st = ctx->stream;
+    int rc = zts_reserve(ctx, &ctx->d_misc, n * (sizeof(ZtsFindCut) + 8) + 256);
+    if (rc) return rc;
+    ZtsFindCut* d_cuts = (ZtsFindCut*)ctx->d_misc.p;
+    unsigned long long* d_found = (unsigned long long*)(d_cuts + n);
+    ZTS_CUDA(ctx, cudaMemcpyAsync(d_cuts, h_cuts.data(), n * sizeof(ZtsFindCut), cudaMemcpyHostToDevice, st));
+    ZTS_LAUNCH(ctx, ZK_BLOCK_FIND,
+               block_find_kernel<<<(unsigned)((n + FIND_WARPS - 1) / FIND_WARPS), FIND_WARPS * 32, 0, st>>>(d_in, d_cuts,
+                                                                                                         (uint32_t)n, d_found));
+    ZTS_CUDA(ctx, cudaMemcpyAsync(h_out, d_found, n * 8, cudaMemcpyDeviceToHost, st));
+    ZTS_CUDA(ctx, cudaStreamSynchronize(st));
+    return ZLB_OK;
 }
 
 struct ZtsGather {
@@ -1000,18 +1178,23 @@ window_resolve_kernel(const uint8_t* __restrict__ arena, uint8_t* __restrict__ s
     if (__syncthreads_or((int)(seen & 0x8000u)) && threadIdx.x == 0) fail[r.item] = 1u;
 }
 
-// One call's marker split: the caller's items and preset dictionaries (dicts == NULL: none), the indices of its large
-// items, and the pieces of item big[k], seg[first[k] .. first[k + 1]) (split_layout). seg[j] is piece j's input span;
-// the decode split gives it a byte slot of its scratch (out_off / out_cap).
+// One call's split: the caller's items and preset dictionaries (dicts == NULL: none), the indices of its large items,
+// and the pieces of item big[k], seg[first[k] .. first[k + 1]) (split_layout). seg[j] is piece j's input span, in bytes
+// or, with `bits` (the searched split), in bits of the input; the decode split gives it a byte slot of its scratch
+// (out_off / out_cap).
 struct SplitJob {
     const zlb_item* items;
     const zlb_dict* dicts;
     std::vector<size_t> big;
     std::vector<size_t> first;
     std::vector<zlb_item> seg;
+    bool bits = false;
     size_t pieces(size_t k) const { return first[k + 1] - first[k]; }
-    // where the last piece of big[k] starts, from the item's first input byte
-    unsigned long long last_start(size_t k) const { return seg[first[k + 1] - 1].in_off - items[big[k]].in_off; }
+    // where the last piece of big[k] starts, from the item's first input byte (bit)
+    unsigned long long last_start(size_t k) const
+    {
+        return seg[first[k + 1] - 1].in_off - items[big[k]].in_off * (bits ? 8u : 1u);
+    }
 };
 
 // The chain checks of the pieces r[0 .. n) of an item: each one decoded cleanly, ended exactly where the next one
@@ -1047,7 +1230,7 @@ static zlb_result split_result(const SplitJob& job, size_t k, const zlb_result* 
         blocks += r[j].blocks & 0x7FFFFFFFu;
     }
     o.status = ZLB_ST_OK;
-    o.in_used = job.last_start(k) + r[n - 1].in_used;
+    o.in_used = job.bits ? (job.last_start(k) + r[n - 1].in_used + 7) >> 3 : job.last_start(k) + r[n - 1].in_used;
     o.blocks = (uint32_t)blocks;
     return o;
 }
@@ -1104,17 +1287,19 @@ static int split_reserve(zlb_ctx* ctx, ZtsDevBuf* arena, size_t bytes, bool* got
 
 // One segment-mode launch of the decoder over the piece table seg, whose copy and results go to d_seg / d_res in the
 // caller's arena; res = the pieces' results. MODE INF_BYTES writes byte slots at d_out, INF_WINDOW word slots at
-// d_out, INF_SIZE nothing (d_out NULL).
+// d_out, INF_SIZE nothing (d_out NULL). bits: the table's spans count bits (ZLB_INFLATE_BITS).
 template <int MODE>
 static int split_segments(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const std::vector<zlb_item>& seg,
-                          zlb_item* d_seg, zlb_result* d_res, uint32_t flags, std::vector<zlb_result>& res)
+                          zlb_item* d_seg, zlb_result* d_res, uint32_t flags, std::vector<zlb_result>& res,
+                          bool bits = false)
 {
     cudaStream_t st = ctx->stream;
     const size_t np = seg.size();
     ZTS_CUDA(ctx, cudaMemcpyAsync(d_seg, seg.data(), np * sizeof(zlb_item), cudaMemcpyHostToDevice, st));
     ZTS_CUDA(ctx, cudaMemsetAsync(d_res, 0, np * sizeof(zlb_result), st));
     const int rc = inflate_launch_mode<MODE>(ctx, st, d_in, d_out, d_seg, d_res, np,
-                                             (flags & ZLB_INFLATE_CHECK_NLEN) | ZLB_INFLATE_SEGMENT, nullptr, nullptr);
+                                             (flags & ZLB_INFLATE_CHECK_NLEN) | ZLB_INFLATE_SEGMENT |
+                                                 (bits ? ZLB_INFLATE_BITS : 0u), nullptr, nullptr);
     if (rc) return rc;
     res.assign(np, zlb_result());
     ZTS_CUDA(ctx, cudaMemcpyAsync(res.data(), d_res, np * sizeof(zlb_result), cudaMemcpyDeviceToHost, st));
@@ -1200,7 +1385,7 @@ static int inflate_split_window(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_sc
         }
     std::vector<zlb_result> wres;
     rc = split_segments<INF_WINDOW>(ctx, d_in, arena, wseg, (zlb_item*)(arena + lay.seg), (zlb_result*)(arena + lay.res),
-                                    flags, wres);
+                                    flags, wres, job.bits);
     if (rc) return rc;
     // 2. the chain checks; the items that pass are resolved
     std::vector<ZtsWinPiece> wp;
@@ -1251,10 +1436,30 @@ static int inflate_split_window(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_sc
 }
 
 // The pieces of the job's large items (job.first / job.seg): one marker scan per item (queued back to back, one
-// read-back for all), a piece starting at 0 and behind every marker that leaves at least one byte; none for an item
-// without a marker inside. A piece's out_off / out_cap are 0. No pieces at all: nothing to split. < 0 on API errors.
+// read-back for all), a piece starting at 0 and behind every marker that leaves at least one byte. An item with a
+// stretch longer than SPLIT_SEARCH_GAP between its start, markers and end is searched instead (sjob, in bits): every
+// such stretch gets a nominal cut every SPLIT_SEARCH_STEP bytes, the block finder runs on all of them in one launch,
+// and its proposals join the markers as cuts. Items whose pieces are all shorter keep the marker route (no finder
+// launch when no item is searched). An item goes to one of the two jobs or to neither (no cut inside); the other job
+// lists no pieces for it. A piece's out_off / out_cap are 0. < 0 on API errors.
 #define SPLIT_TAG_SHIFT 40  // marks carry the item's index above the byte offset (offsets < 1 TiB, < 16 M large items)
-static int split_layout(zlb_ctx* ctx, const uint8_t* d_in, SplitJob& job)
+// Far above the longest piece this engine's own streams have (a 64 KiB chunk, at most 64 KiB + 5 bytes compressed),
+// and above the pieces of streams flushed at least every 1 MiB of input (zlib Z_SYNC_FLUSH / Z_FULL_FLUSH, pigz): all
+// of those keep the marker route, which already decodes their pieces side by side. A stretch this long holds dozens
+// of blocks of any encoder.
+#define SPLIT_SEARCH_GAP (1u << 20)
+// Nominal cut spacing of a searched stretch, about one cut per zlib block (16 K symbols at its default memLevel,
+// ~15-30 KB compressed). Chosen on a B200 at 1000 W (profiles/r03d_split_step.json, both builds in one session, 256 MiB
+// through zlib -6, decompressed GB/s): 32 KiB against 16 KiB gave mixed 9.4 / 9.2, text 9.2 / 7.8, random data
+// 15.7 / 9.3. A finer step finds more block starts (mixed: 6338 against 3863), but each costs the finder a search up
+// to the next block, many cuts of text land on the same block (3118 starts from 5826 cuts), and every piece costs the
+// size and window passes a table build and a 64 KiB map. 64 KiB was measured with the finder alone (finder_step in
+// profiles/r03d_split_search.json): it halves the block starts found again (1931 on mixed), which lengthens the
+// longest piece. (-DSPLIT_SEARCH_STEP=... builds another step for such a comparison.)
+#ifndef SPLIT_SEARCH_STEP
+#define SPLIT_SEARCH_STEP (32u << 10)
+#endif
+static int split_layout(zlb_ctx* ctx, const uint8_t* d_in, SplitJob& job, SplitJob& sjob)
 {
     const size_t nb = job.big.size();
     if (nb >= (1ull << 24)) return ZLB_OK;
@@ -1275,29 +1480,76 @@ static int split_layout(zlb_ctx* ctx, const uint8_t* d_in, SplitJob& job)
     uint32_t count = 0;
     ZTS_CUDA(ctx, cudaMemcpyAsync(&count, d_count, 4, cudaMemcpyDeviceToHost, st));
     ZTS_CUDA(ctx, cudaStreamSynchronize(st));
-    if (count == 0 || count > SPLIT_MAX_MARKS) return ZLB_OK;
+    if (count > SPLIT_MAX_MARKS) return ZLB_OK;
     std::vector<unsigned long long> marks(count);
-    ZTS_CUDA(ctx, cudaMemcpyAsync(marks.data(), d_marks, (size_t)count * 8, cudaMemcpyDeviceToHost, st));
-    ZTS_CUDA(ctx, cudaStreamSynchronize(st));
+    if (count) {
+        ZTS_CUDA(ctx, cudaMemcpyAsync(marks.data(), d_marks, (size_t)count * 8, cudaMemcpyDeviceToHost, st));
+        ZTS_CUDA(ctx, cudaStreamSynchronize(st));
+    }
     std::sort(marks.begin(), marks.end());  // by item, then by offset
-    std::vector<zlb_item>& seg = job.seg;
-    job.first.assign(nb + 1, 0);
+    // marker cuts of every item (byte offsets from its start, 0 first); the searched items get nominal cuts
+    std::vector<std::vector<unsigned long long>> cuts(nb);
+    std::vector<char> searched(nb, 0);
+    std::vector<ZtsFindCut> find;
+    std::vector<size_t> find_first(nb + 1, 0);
     size_t mi = 0;
     for (size_t k = 0; k < nb; ++k) {
         const zlb_item& it = job.items[job.big[k]];
-        const size_t a = job.first[k] = seg.size();
-        seg.push_back({it.in_off, 0, 0, 0});
+        std::vector<unsigned long long>& c = cuts[k];
+        find_first[k] = find.size();
+        if (it.in_len >= (1ull << SPLIT_TAG_SHIFT)) continue;
+        c.push_back(0);
         for (; mi < marks.size() && (marks[mi] >> SPLIT_TAG_SHIFT) == k; ++mi) {
             const unsigned long long m = marks[mi] & ((1ull << SPLIT_TAG_SHIFT) - 1);
             // a piece of this engine's streams holds a whole block: never closer than SPLIT_MIN_PIECE bytes to the
             // previous cut (a hostile stream of empty stored blocks would otherwise ask for a slot per 5 bytes)
-            if (m < it.in_len && m >= seg.back().in_off - it.in_off + SPLIT_MIN_PIECE) seg.push_back({it.in_off + m, 0, 0, 0});
+            if (m < it.in_len && m >= c.back() + SPLIT_MIN_PIECE) c.push_back(m);
         }
-        if (seg.size() - a < 2) seg.resize(a);  // no marker inside: nothing to gain
-        for (size_t j = a; j < seg.size(); ++j)
-            seg[j].in_len = (j + 1 < seg.size() ? seg[j + 1].in_off : it.in_off + it.in_len) - seg[j].in_off;
+        for (size_t j = 0; j < c.size(); ++j) {
+            const unsigned long long g0 = c[j], g1 = j + 1 < c.size() ? c[j + 1] : it.in_len;
+            if (g1 - g0 <= SPLIT_SEARCH_GAP) continue;
+            searched[k] = 1;
+            const unsigned long long base = 8ull * it.in_off;
+            for (unsigned long long p = g0 + SPLIT_SEARCH_STEP; p < g1; p += SPLIT_SEARCH_STEP)
+                find.push_back({base + 8 * p, base + 8 * std::min(p + SPLIT_SEARCH_STEP, g1), base + 8 * it.in_len});
+        }
     }
-    job.first[nb] = seg.size();
+    find_first[nb] = find.size();
+    std::vector<unsigned long long> found(find.size());
+    if ((rc = block_find(ctx, d_in, find, found.data()))) return rc;
+    job.first.assign(nb + 1, 0);
+    sjob.first.assign(nb + 1, 0);
+    for (size_t k = 0; k < nb; ++k) {
+        const zlb_item& it = job.items[job.big[k]];
+        job.first[k] = job.seg.size();
+        sjob.first[k] = sjob.seg.size();
+        if (cuts[k].size() < (searched[k] ? 1u : 2u)) continue;  // no marker inside: nothing to gain
+        if (!searched[k]) {
+            for (unsigned long long m : cuts[k]) job.seg.push_back({it.in_off + m, 0, 0, 0});
+            job.seg.back().in_len = it.in_len - cuts[k].back();
+            for (size_t j = job.first[k]; j + 1 < job.seg.size(); ++j) job.seg[j].in_len = job.seg[j + 1].in_off - job.seg[j].in_off;
+            continue;
+        }
+        // bit offsets: the markers' and the finder's proposals, in order, each at least SPLIT_MIN_PIECE bytes behind
+        // the one in front
+        const unsigned long long b0 = 8ull * it.in_off, b1 = 8ull * (it.in_off + it.in_len);
+        std::vector<unsigned long long> bc;
+        for (unsigned long long m : cuts[k]) bc.push_back(b0 + 8 * m);
+        for (size_t f = find_first[k]; f < find_first[k + 1]; ++f)
+            if (found[f] != FIND_NONE && found[f] > b0 && found[f] < b1) bc.push_back(found[f]);
+        std::sort(bc.begin(), bc.end());
+        std::vector<zlb_item>& seg = sjob.seg;
+        const size_t a = seg.size();
+        for (unsigned long long x : bc)
+            if (seg.size() == a || x >= seg.back().in_off + 8ull * SPLIT_MIN_PIECE) seg.push_back({x, 0, 0, 0});
+        if (seg.size() - a < 2) {
+            seg.resize(a);
+            continue;
+        }
+        for (size_t j = a; j < seg.size(); ++j) seg[j].in_len = (j + 1 < seg.size() ? seg[j + 1].in_off : b1) - seg[j].in_off;
+    }
+    job.first[nb] = job.seg.size();
+    sjob.first[nb] = sjob.seg.size();
     return ZLB_OK;
 }
 
@@ -1359,12 +1611,39 @@ static int inflate_split_batch(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out
     return ZLB_OK;
 }
 
+// Whether the segment-mode size results sres of item big[k]'s pieces reach no further than the output of the pieces
+// in front of each plus the dictionary's reachable bytes (crc32: how far a piece reached in front of its first byte):
+// the one-warp decoder's own condition, so it then fails no distance either.
+static bool split_reach_ok(const SplitJob& job, size_t k, const std::vector<zlb_result>& sres)
+{
+    const size_t a = job.first[k], n = job.pieces(k);
+    const unsigned long long dl = job.dicts ? std::min(job.dicts[job.big[k]].len, (uint64_t)WIN_WORDS) : 0;
+    unsigned long long before = 0;  // output of the pieces in front
+    for (size_t j = a; j < a + n; ++j) {
+        if (sres[j].crc32 > before + dl) return false;
+        before += sres[j].out_len;
+    }
+    return true;
+}
+
+// An item of a size call is settled when its chain passes and no piece reaches too far (split_reach_ok); it then gets
+// the one-warp decoder's result by construction.
+static void split_settle_sizes(const SplitJob& job, const std::vector<zlb_result>& sres, zlb_result* h_results,
+                               std::vector<char>& done)
+{
+    for (size_t k = 0; k < job.big.size(); ++k) {
+        const size_t a = job.first[k], n = job.pieces(k);
+        if (n < 2 || split_chain(&sres[a], &job.seg[a], n, false, false) != SPLIT_OK) continue;
+        if (!split_reach_ok(job, k, sres)) continue;
+        h_results[job.big[k]] = split_result(job, k, &sres[a]);
+        done[job.big[k]] = 1;
+    }
+}
+
 // The marker split of a size call: the job's pieces are sized by one segment-mode launch of the size decoder. A
 // piece's size does not depend on the bytes in front of it, only whether a distance reaches before the stream (or
-// before its dictionary) does, and a piece tells how far in front of its first byte it reached (crc32). So an item is
-// settled when its chain passes and no piece reaches further than the output of the pieces in front of it plus the
-// dictionary's reachable bytes; it then gets the one-warp decoder's result by construction. No byte slots and no
-// window scratch: the piece tables take the place of the marks. h_results / done as for inflate_split_batch.
+// before its dictionary) does, and a piece tells how far in front of its first byte it reached (crc32). No byte slots
+// and no window scratch: the piece tables take the place of the marks. h_results / done as for inflate_split_batch.
 static int inflate_split_sizes(zlb_ctx* ctx, const uint8_t* d_in, const SplitJob& job, uint32_t flags,
                                zlb_result* h_results, std::vector<char>& done)
 {
@@ -1374,19 +1653,147 @@ static int inflate_split_sizes(zlb_ctx* ctx, const uint8_t* d_in, const SplitJob
     zlb_item* d_seg = (zlb_item*)ctx->d_misc.p;
     std::vector<zlb_result> sres;
     if ((rc = split_segments<INF_SIZE>(ctx, d_in, nullptr, job.seg, d_seg, (zlb_result*)(d_seg + np), flags, sres))) return rc;
+    split_settle_sizes(job, sres, h_results, done);
+    return ZLB_OK;
+}
+
+// ---- the searched split: size first, then window ----------------------------------------------------------------
+// Almost every piece of a searched item reaches into its predecessor, so there is no byte-slot pass: the size decoder
+// runs over the pieces in segment mode (the chain check, and each piece's exact output size), broken chains are
+// repaired, and the window pass decodes the pieces into exact slots.
+#define SPLIT_REPAIR_ROUNDS 3
+
+// Sizes the pieces of sjob; res = their results. Where a chain breaks, each maximal run of broken pieces is merged with
+// the piece behind it (a cut the piece in front did not end at is dropped) and only the merged pieces are sized again,
+// for at most SPLIT_REPAIR_ROUNDS rounds. A chain that reaches a clean BFINAL before its last piece is kept up to that
+// piece: the one-warp decoder stops there too. On return every item left with pieces passes split_chain; the others
+// have none (the one-warp decoder takes them).
+static int split_search_size(zlb_ctx* ctx, const uint8_t* d_in, SplitJob& job, uint32_t flags, std::vector<zlb_result>& res)
+{
+    const size_t nb = job.big.size();
+    res.assign(job.seg.size(), zlb_result());
+    std::vector<size_t> todo(job.seg.size());
+    for (size_t j = 0; j < todo.size(); ++j) todo[j] = j;
+    for (int round = 0;; ++round) {
+        if (!todo.empty()) {
+            std::vector<zlb_item> part(todo.size());
+            for (size_t t = 0; t < todo.size(); ++t) part[t] = job.seg[todo[t]];
+            int rc = zts_reserve(ctx, &ctx->d_misc, part.size() * (sizeof(zlb_item) + sizeof(zlb_result)) + 256);
+            if (rc) return rc;
+            zlb_item* d_seg = (zlb_item*)ctx->d_misc.p;
+            std::vector<zlb_result> pres;
+            rc = split_segments<INF_SIZE>(ctx, d_in, nullptr, part, d_seg, (zlb_result*)(d_seg + part.size()), flags, pres,
+                                          true);
+            if (rc) return rc;
+            for (size_t t = 0; t < todo.size(); ++t) res[todo[t]] = pres[t];
+        }
+        todo.clear();
+        std::vector<zlb_item> nseg;
+        std::vector<zlb_result> nres;
+        std::vector<size_t> nfirst(nb + 1, 0);
+        for (size_t k = 0; k < nb; ++k) {
+            const size_t a = job.first[k], n = job.pieces(k);
+            nfirst[k] = nseg.size();
+            if (n < 2) continue;
+            const zlb_item* g = &job.seg[a];
+            const zlb_result* r = &res[a];
+            auto fin = [&](size_t j) { return r[j].status == ZLB_ST_OK && (r[j].blocks & 0x80000000u); };
+            auto good = [&](size_t j) {
+                return r[j].status == ZLB_ST_OK && (j + 1 == n ? fin(j) : !fin(j) && r[j].in_used == g[j].in_len);
+            };
+            size_t ok = 0;  // pieces in front that are good
+            while (ok < n && good(ok)) ++ok;
+            if (ok == n || (ok < n && fin(ok))) {  // the whole chain, or up to a clean BFINAL
+                const size_t keep = ok == n ? n : ok + 1;
+                nseg.insert(nseg.end(), g, g + keep);
+                nres.insert(nres.end(), r, r + keep);
+                continue;
+            }
+            if (round == SPLIT_REPAIR_ROUNDS) continue;
+            bool progress = false;
+            const size_t b0 = nseg.size();
+            for (size_t j = 0; j < n;) {
+                if (good(j)) {
+                    nseg.push_back(g[j]);
+                    nres.push_back(r[j]);
+                    ++j;
+                    continue;
+                }
+                size_t e = j;
+                while (e + 1 < n && !good(e + 1)) ++e;
+                const size_t last = std::min(e + 1, n - 1);  // the run and the piece behind it
+                progress |= last > j;
+                nseg.push_back({g[j].in_off, g[last].in_off + g[last].in_len - g[j].in_off, 0, 0});
+                nres.push_back(zlb_result());
+                todo.push_back(nseg.size() - 1);
+                j = last + 1;
+            }
+            if (!progress || nseg.size() - b0 < 2) {  // nothing left to merge, or one piece: the one-warp decoder
+                while (!todo.empty() && todo.back() >= b0) todo.pop_back();
+                nseg.resize(b0);
+                nres.resize(b0);
+            }
+        }
+        nfirst[nb] = nseg.size();
+        job.seg.swap(nseg);
+        job.first.swap(nfirst);
+        res.swap(nres);
+        if (todo.empty()) return ZLB_OK;
+    }
+}
+
+// The decode of the searched items, sized by split_search_size (res): exact byte slots, the window pass, one gather.
+// An item whose pieces do not fit ZtsWinPiece's 32-bit sizes, or whose scratch exceeds the budget, is left to the
+// one-warp decoder; one whose output exceeds its slot gets ZLB_ST_OUT_OVERFLOW without a decode, but only when no
+// distance reaches before the stream or its dictionary (split_reach_ok) -- the one-warp decoder would stop at such a
+// distance with ZLB_ST_BAD_CODE if it came before the slot filled, so such an item is left to it.
+static int inflate_split_search(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const uint8_t* d_dict, SplitJob& job,
+                                const std::vector<zlb_result>& res, uint32_t flags, zlb_result* h_results,
+                                std::vector<char>& done)
+{
+    cudaStream_t st = ctx->stream;
+    std::vector<ZtsGather> gath;
+    std::vector<size_t> cand;
+    size_t scratch = 0, big_in = 0;
     for (size_t k = 0; k < job.big.size(); ++k) {
         const size_t a = job.first[k], n = job.pieces(k);
-        if (n < 2 || split_chain(&sres[a], &job.seg[a], n, false, false) != SPLIT_OK) continue;
-        const unsigned long long dl = job.dicts ? std::min(job.dicts[job.big[k]].len, (uint64_t)WIN_WORDS) : 0;
-        unsigned long long before = 0;  // output of the pieces in front
+        if (n < 2) continue;
+        unsigned long long total = 0;
         bool fits = true;
-        for (size_t j = a; j < a + n && fits; ++j) {
-            fits = sres[j].crc32 <= before + dl;
-            before += sres[j].out_len;
+        for (size_t j = a; j < a + n; ++j) {
+            total += res[j].out_len;
+            fits &= res[j].out_len <= 0xFFFFFF00ull;
         }
         if (!fits) continue;
-        h_results[job.big[k]] = split_result(job, k, &sres[a]);
-        done[job.big[k]] = 1;
+        if (total > job.items[job.big[k]].out_cap) {
+            if (!split_reach_ok(job, k, res)) continue;
+            std::vector<ZtsGather> none;
+            h_results[job.big[k]] = split_finish(job, k, &res[a], none);
+            done[job.big[k]] = 1;
+            continue;
+        }
+        for (size_t j = a; j < a + n; ++j) {
+            job.seg[j].out_off = scratch;
+            job.seg[j].out_cap = (res[j].out_len + 255) & ~255ull;
+            scratch += job.seg[j].out_cap;
+        }
+        big_in += job.items[job.big[k]].in_len;
+        cand.push_back(k);
+    }
+    if (cand.empty()) return ZLB_OK;
+    const size_t np = job.seg.size();
+    const size_t need = scratch + np * sizeof(ZtsGather) + 256;
+    if (need > SplitBudget(ctx->d_split)(big_in, 1)) return ZLB_OK;
+    bool got = false;
+    int rc = split_reserve(ctx, &ctx->d_split, need, &got);
+    if (rc || !got) return rc;
+    uint8_t* d_scratch = (uint8_t*)ctx->d_split.p;
+    ZtsGather* d_gather = (ZtsGather*)(d_scratch + scratch);
+    if ((rc = inflate_split_window(ctx, d_in, d_scratch, d_dict, job, flags, cand, h_results, done, gath))) return rc;
+    if (!gath.empty()) {
+        ZTS_CUDA(ctx, cudaMemcpyAsync(d_gather, gath.data(), gath.size() * sizeof(ZtsGather), cudaMemcpyHostToDevice, st));
+        ZTS_LAUNCH(ctx, ZK_GATHER, segment_gather_kernel<<<(unsigned)gath.size(), 256, 0, st>>>(d_scratch, d_out, d_gather));
+        ZTS_CUDA(ctx, cudaStreamSynchronize(st));  // gath goes out of scope
     }
     return ZLB_OK;
 }
@@ -1514,6 +1921,7 @@ static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
                           const ZtsHostIO* hio)
 {
     // large items that may be cut at sync-flush markers (each is massively parallel by itself)
+    flags &= ~ZLB_INFLATE_BITS;  // (internal)
     SplitJob job{h_items, h_dicts, {}, {}, {}};
     if ((flags & ZLB_INFLATE_SPLIT) && !(flags & ZLB_INFLATE_SEGMENT))
         for (size_t i = 0; i < n; ++i)
@@ -1558,10 +1966,17 @@ static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
     }
     if (!job.big.empty()) {
         std::vector<char> done(n, 0);
-        rc = split_layout(ctx, d_in, job);
+        SplitJob sjob{h_items, h_dicts, job.big, {}, {}, true};  // the searched items
+        rc = split_layout(ctx, d_in, job, sjob);
         if (!rc && !job.seg.empty())
             rc = sizes ? inflate_split_sizes(ctx, d_in, job, flags, h_results, done)
                        : inflate_split_batch(ctx, d_in, d_out, d_dict, job, flags, h_results, done);
+        if (!rc && !sjob.seg.empty()) {
+            std::vector<zlb_result> sres;
+            rc = split_search_size(ctx, d_in, sjob, flags, sres);
+            if (!rc && sizes) split_settle_sizes(sjob, sres, h_results, done);
+            if (!rc && !sizes) rc = inflate_split_search(ctx, d_in, d_out, d_dict, sjob, sres, flags, h_results, done);
+        }
         if (rc) return rc;
         split_any = std::find(done.begin(), done.end(), 1) != done.end();
         if (split_any) {
@@ -1676,4 +2091,18 @@ extern "C" int zlb_inflate_size_batch_host(zlb_ctx* ctx, const void* h_in, size_
                          [&](ZtsHostIO& io, const zlb_dict* d) {
         return inflate_device(ctx, (const uint8_t*)ctx->d_stage_in.p, nullptr, nullptr, d, items, results, n, flags, &io);
     }, ZTS_HOST_SIZES);
+}
+
+extern "C" int zlb_debug_block_starts(zlb_ctx* ctx, const void* d_in, uint64_t n, const uint64_t* h_cuts, size_t n_cuts,
+                                      uint64_t span, uint64_t* h_bits_out)
+{
+    if (!ctx || (n_cuts && (!d_in || !h_cuts || !h_bits_out)) || n_cuts >= (1ull << 32)) return ZLB_E_ARG;
+    ZTS_CUDA(ctx, cudaSetDevice(ctx->device));
+    std::vector<ZtsFindCut> cuts(n_cuts);
+    for (size_t c = 0; c < n_cuts; ++c) {
+        if (h_cuts[c] >= n) return zts_fail(ctx, ZLB_E_ARG, "cut %zu lies behind the input", c);
+        cuts[c] = {8 * h_cuts[c], std::min(8 * h_cuts[c] + span, 8 * n), 8 * n};
+    }
+    static_assert(sizeof(unsigned long long) == sizeof(uint64_t), "");
+    return block_find(ctx, (const uint8_t*)d_in, cuts, (unsigned long long*)h_bits_out);
 }
