@@ -235,6 +235,64 @@ int zlb_inflate_size_batch(zlb_ctx* ctx, const void* d_in, const zlb_dict* dicts
 int zlb_inflate_size_batch_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes, const zlb_dict* dicts,
                                 const zlb_item* items, zlb_result* results, size_t n_items, uint32_t flags);
 
+/* ---- random access through an index of access points (what zlib's zran.c, indexed_gzip and rapidgzip offer) -----
+ * An access point is a block start of a stream that a decode proved: its bit offset from the stream's first byte
+ * (items[i].in_off), the decompressed bytes in front of it, and where its window -- the min(out_pos, 32768) bytes in
+ * front of it -- lies in a window blob. A read of [pos, pos + len) starts at the last point at or before pos instead
+ * of the start of the stream, and a long read is cut at every point inside it, each piece decoded by its own warp.
+ *
+ * zlb_inflate_index[_host]: a decode that also reports access points. Output bytes and results are those of
+ * zlb_inflate_batch[_host] with flags | ZLB_INFLATE_SPLIT (flags: ZLB_INFLATE_WANT_CRC32 / _ADLER32 / _CHECK_NLEN;
+ * no preset dictionaries). Item i's points go to points[point_first[i] .. point_first[i + 1]) (point_first has
+ * n_items + 1 nondecreasing entries; when the slots run out later points are dropped: the index is only sparser) and
+ * their number to point_count[i]; an item that failed gets 0. Points ascend in in_bit and out_pos, the first is
+ * {0, 0}. The candidates are the block starts the decode proved: the split's piece starts, or every block header
+ * when one warp decodes the item. The choice is greedy: the first candidate whose out_pos is at least the previous
+ * point's out_pos + spacing (0 = ZLB_INDEX_DEFAULT_SPACING). win_off = items[i].out_off + out_pos -
+ * min(out_pos, 32768): the call's output blob is the window blob (a caller that keeps only the windows compacts them
+ * and rewrites win_off).
+ *
+ * zlb_inflate_ranges[_host]: batched reads. Range i wants out_cap bytes from decompressed position pos of the stream
+ * at in_off / in_len of the input, whose points are points[pt_first .. pt_first + pt_count). The range is cut at the
+ * points inside [pos, pos + out_cap); every piece is decoded by one warp from its point with that point's window (in
+ * d_win / h_win). results[i].out_len = min(out_cap, size - pos) (0 at or past the end: a short read is ZLB_ST_OK),
+ * status = the decoder's status for a data error inside the stretch decoded, crc32 / adler32 of the bytes written
+ * when requested (flags: ZLB_INFLATE_WANT_CRC32 / _ADLER32 / _CHECK_NLEN), in_used = blocks = 0. Nothing is written
+ * outside [out_off, out_off + out_cap), whatever the windows hold: a wrong window gives wrong bytes or
+ * ZLB_ST_BAD_CODE (zlib's inflateSetDictionary contract). The bytes do not depend on which of a stream's points are
+ * passed as long as the first one is; only the speed does. ZLB_E_ARG: pt_count == 0, a first point that is not
+ * {0, 0}, points that do not ascend, a point behind 8 * in_len, pos + out_cap beyond 2^64, a point with a window and
+ * a NULL window blob, a window span outside win_bytes or a range slot outside out_bytes (_host), any other flag.
+ * A range's first piece decodes the bytes between its point and pos into scratch (at most what the rest of the
+ * stream can give: 258 bytes per bit); ZLB_E_NOMEM when that alone exceeds what a call may take -- pass the points
+ * between. A pos beyond what the stream can give from its point is a read past the end (out_len 0), decoded not at
+ * all.                                                                                                           */
+#define ZLB_INDEX_DEFAULT_SPACING (1u << 20)
+typedef struct {
+    uint64_t in_bit;   /* a block start: bit offset from the stream's first byte; 0 for the first point           */
+    uint64_t out_pos;  /* decompressed bytes in front of it                                                        */
+    uint64_t win_off;  /* its window, the min(out_pos, 32768) decompressed bytes in front of it, in the window blob */
+} zlb_point;
+
+typedef struct {
+    uint64_t in_off, in_len;     /* the stream, as the index build saw it                                  */
+    uint64_t pt_first, pt_count; /* its points: points[pt_first .. pt_first + pt_count)                    */
+    uint64_t pos;                /* first decompressed byte wanted                                          */
+    uint64_t out_off, out_cap;   /* where the bytes go; out_cap bytes are wanted                            */
+} zlb_range;
+
+int zlb_inflate_index(zlb_ctx* ctx, const void* d_in, void* d_out, const zlb_item* items, zlb_result* results,
+                      size_t n_items, uint32_t flags, uint64_t spacing, zlb_point* points, const uint64_t* point_first,
+                      uint64_t* point_count);
+int zlb_inflate_index_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes, void* h_out, size_t out_bytes,
+                           const zlb_item* items, zlb_result* results, size_t n_items, uint32_t flags, uint64_t spacing,
+                           zlb_point* points, const uint64_t* point_first, uint64_t* point_count);
+int zlb_inflate_ranges(zlb_ctx* ctx, const void* d_in, const void* d_win, void* d_out, const zlb_point* points,
+                       size_t n_points, const zlb_range* ranges, zlb_result* results, size_t n_ranges, uint32_t flags);
+int zlb_inflate_ranges_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes, const void* h_win, size_t win_bytes,
+                            void* h_out, size_t out_bytes, const zlb_point* points, size_t n_points,
+                            const zlb_range* ranges, zlb_result* results, size_t n_ranges, uint32_t flags);
+
 /* ---- checksums (replace CRC32.create src/CRC32.ts:13, Adler32.create src/Adler32.ts:13) ----- */
 int zlb_checksum_batch(zlb_ctx* ctx, const void* d_in, const zlb_item* items, zlb_result* results,
                        size_t n_items, uint32_t kinds);

@@ -17,6 +17,12 @@
 //   inflateSizes(input: Uint8Array, offsets: number[], lengths: number[], flags, dictionary?)
 //                                                          -> {status: number[], outLen: number[], inUsed: number[], blocks: number[]}
 //     decompressed sizes without writing them (exact `caps` for inflateBatch)
+//   inflateIndex(input: Uint8Array, offset, length, cap, flags, spacing)
+//                              -> {output, status, inUsed, crc32, adler32, inBit: number[], outPos: number[], winOff: number[]}
+//     one stream decoded (as inflateBatch with ZLB_INFLATE_SPLIT) with its access points; winOff counts from output
+//   inflateRanges(input: Uint8Array, offset, length, windows: Uint8Array, inBit[], outPos[], winOff[], pos[], len[], flags)
+//                                                          -> {outputs, status: number[], crc32, adler32}
+//     reads of one indexed stream (the points and the window blob an inflateIndex gave, or a compacted blob)
 //   checksumBatch(inputs: Uint8Array[], kinds)             -> {crc32: number[], adler32: number[]}
 //   crc32Combine(a, b, lenB), adler32Combine(a, b, lenB)
 //   hostAlloc(bytes) -> Uint8Array over page-locked memory (build inputs in it: they then travel without a copy)
@@ -356,6 +362,126 @@ static napi_value InflateSizes(napi_env env, napi_callback_info info)
     return result;
 }
 
+// inflateIndex(input, offset, length, cap, flags, spacing): one stream decoded, and its access points
+static napi_value InflateIndex(napi_env env, napi_callback_info info)
+{
+    size_t argc = 6;
+    napi_value argv[6];
+    napi_get_cb_info(env, info, &argc, argv, nullptr, nullptr);
+    if (!ensure_ctx(env)) return nullptr;
+    Bytes in;
+    if (!get_u8(env, argv[0], &in)) {
+        napi_throw_type_error(env, nullptr, "input must be Uint8Array");
+        return nullptr;
+    }
+    double off = 0, len = 0, cap = 0, spacing = 0;
+    uint32_t flags = 0;
+    napi_get_value_double(env, argv[1], &off);
+    napi_get_value_double(env, argv[2], &len);
+    napi_get_value_double(env, argv[3], &cap);
+    napi_get_value_uint32(env, argv[4], &flags);
+    napi_get_value_double(env, argv[5], &spacing);
+    zlb_item item = {(uint64_t)off, (uint64_t)len, 0, (uint64_t)cap};
+    zlb_result res;
+    const uint64_t sp = spacing > 0 ? (uint64_t)spacing : ZLB_INDEX_DEFAULT_SPACING;
+    std::vector<zlb_point> pts(item.out_cap / sp + 2);
+    const uint64_t first[2] = {0, (uint64_t)pts.size()};
+    uint64_t count = 0;
+    HostBuf out(item.out_cap);
+    if (!out.p) {
+        napi_throw_error(env, nullptr, "zlib.ts-b200: out of host memory");
+        return nullptr;
+    }
+    int rc = zlb_inflate_index_host(g_ctx, in.p, in.n, out.p, item.out_cap, &item, &res, 1, flags, sp, pts.data(), first,
+                                    &count);
+    if (rc != ZLB_OK) {
+        napi_throw_error(env, nullptr, zlb_last_error(g_ctx));
+        return nullptr;
+    }
+    std::vector<double> bit(count), pos(count), win(count);
+    for (uint64_t k = 0; k < count; ++k) {
+        bit[k] = (double)pts[k].in_bit;
+        pos[k] = (double)pts[k].out_pos;
+        win[k] = (double)pts[k].win_off;
+    }
+    napi_value result, v;
+    napi_create_object(env, &result);
+    const uint8_t* out_base = out.p;
+    Outputs views(env, out);
+    napi_set_named_property(env, result, "output", views.at(out_base, 0, (size_t)res.out_len));
+    napi_create_double(env, res.status, &v);
+    napi_set_named_property(env, result, "status", v);
+    napi_create_double(env, (double)res.in_used, &v);
+    napi_set_named_property(env, result, "inUsed", v);
+    napi_create_double(env, res.crc32, &v);
+    napi_set_named_property(env, result, "crc32", v);
+    napi_create_double(env, res.adler32, &v);
+    napi_set_named_property(env, result, "adler32", v);
+    napi_set_named_property(env, result, "inBit", num_array(env, bit));
+    napi_set_named_property(env, result, "outPos", num_array(env, pos));
+    napi_set_named_property(env, result, "winOff", num_array(env, win));
+    return result;
+}
+
+// inflateRanges(input, offset, length, windows, inBit, outPos, winOff, pos, len, flags): reads through access points
+static napi_value InflateRanges(napi_env env, napi_callback_info info)
+{
+    size_t argc = 10;
+    napi_value argv[10];
+    napi_get_cb_info(env, info, &argc, argv, nullptr, nullptr);
+    if (!ensure_ctx(env)) return nullptr;
+    Bytes in, win;
+    if (!get_u8(env, argv[0], &in) || !get_u8(env, argv[3], &win)) {
+        napi_throw_type_error(env, nullptr, "input and windows must be Uint8Array");
+        return nullptr;
+    }
+    double off = 0, len = 0;
+    uint32_t flags = 0;
+    napi_get_value_double(env, argv[1], &off);
+    napi_get_value_double(env, argv[2], &len);
+    std::vector<double> bit = get_numbers(env, argv[4]), opos = get_numbers(env, argv[5]), woff = get_numbers(env, argv[6]);
+    std::vector<double> pos = get_numbers(env, argv[7]), want = get_numbers(env, argv[8]);
+    napi_get_value_uint32(env, argv[9], &flags);
+    std::vector<zlb_point> pts(bit.size());
+    for (size_t k = 0; k < pts.size(); ++k) pts[k] = {(uint64_t)bit[k], (uint64_t)opos[k], (uint64_t)woff[k]};
+    const size_t n = pos.size();
+    std::vector<zlb_range> rg(n);
+    std::vector<zlb_result> res(n);
+    uint64_t out_total = 0;
+    for (size_t i = 0; i < n; ++i) {
+        rg[i] = {(uint64_t)off, (uint64_t)len, 0, (uint64_t)pts.size(), (uint64_t)pos[i], out_total, (uint64_t)want[i]};
+        out_total += rg[i].out_cap;
+    }
+    HostBuf out(out_total);
+    if (!out.p) {
+        napi_throw_error(env, nullptr, "zlib.ts-b200: out of host memory");
+        return nullptr;
+    }
+    int rc = zlb_inflate_ranges_host(g_ctx, in.p, in.n, win.p, win.n, out.p, out_total, pts.data(), pts.size(), rg.data(),
+                                     res.data(), n, flags);
+    if (rc != ZLB_OK) {
+        napi_throw_error(env, nullptr, zlb_last_error(g_ctx));
+        return nullptr;
+    }
+    napi_value result, outs;
+    napi_create_object(env, &result);
+    napi_create_array_with_length(env, n, &outs);
+    std::vector<double> st(n), crc(n), adler(n);
+    const uint8_t* out_base = out.p;
+    Outputs views(env, out);
+    for (size_t i = 0; i < n; ++i) {
+        napi_set_element(env, outs, (uint32_t)i, views.at(out_base, rg[i].out_off, (size_t)res[i].out_len));
+        st[i] = res[i].status;
+        crc[i] = res[i].crc32;
+        adler[i] = res[i].adler32;
+    }
+    napi_set_named_property(env, result, "outputs", outs);
+    napi_set_named_property(env, result, "status", num_array(env, st));
+    napi_set_named_property(env, result, "crc32", num_array(env, crc));
+    napi_set_named_property(env, result, "adler32", num_array(env, adler));
+    return result;
+}
+
 // checksumBatch(inputs, kinds)  <- CRC32.create / Adler32.create
 static napi_value ChecksumBatch(napi_env env, napi_callback_info info)
 {
@@ -545,6 +671,8 @@ static napi_value Init(napi_env env, napi_value exports)
         {"deflateBatch", nullptr, DeflateBatch, nullptr, nullptr, nullptr, napi_default, nullptr},
         {"inflateBatch", nullptr, InflateBatch, nullptr, nullptr, nullptr, napi_default, nullptr},
         {"inflateSizes", nullptr, InflateSizes, nullptr, nullptr, nullptr, napi_default, nullptr},
+        {"inflateIndex", nullptr, InflateIndex, nullptr, nullptr, nullptr, napi_default, nullptr},
+        {"inflateRanges", nullptr, InflateRanges, nullptr, nullptr, nullptr, napi_default, nullptr},
         {"checksumBatch", nullptr, ChecksumBatch, nullptr, nullptr, nullptr, napi_default, nullptr},
         {"archive", nullptr, Archive, nullptr, nullptr, nullptr, napi_default, nullptr},
         {"crc32Combine", nullptr, Crc32Combine, nullptr, nullptr, nullptr, napi_default, nullptr},

@@ -149,6 +149,35 @@ export const inflateSizes = (input: Uint8Array, offsets: number[], lengths: numb
     native.inflateSizes(input, offsets, lengths, flags, dictionary) as
     { status: number[]; outLen: number[]; inUsed: number[]; blocks: number[] };
 
+// Random access into one raw deflate stream (input[offset .. offset + length)): InflateIndex.build decodes it once and
+// keeps access points about every `spacing` output bytes with the 32 KiB window in front of each; read() decodes only
+// from the last point in front of a range (zlb_inflate_index / zlb_inflate_ranges). zlib / gzip framing and trailer
+// checks stay with the caller (api.py's inflate_index does them).
+export class InflateIndex {
+    private constructor(public input: Uint8Array, public offset: number, public length: number, public windows: Uint8Array,
+                        public inBit: number[], public outPos: number[], public winOff: number[]) {}
+    static build(input: Uint8Array, offset: number, length: number, size: number, spacing = 1 << 20):
+        { output: Uint8Array; index: InflateIndex } {
+        const r = native.inflateIndex(input, offset, length, size, 0, spacing);
+        if (r.status !== 0) throw new Error(statusText(r.status));
+        // keep only the windows, back to back
+        const lens = (r.outPos as number[]).map((p: number) => Math.min(p, 32768));
+        const windows = new Uint8Array(lens.reduce((a: number, b: number) => a + b, 0));
+        const winOff: number[] = [];
+        let at = 0;
+        (r.outPos as number[]).forEach((p: number, k: number) => {
+            windows.set(r.output.subarray(p - lens[k], p), at); winOff.push(at); at += lens[k]; });
+        return { output: r.output, index: new InflateIndex(input, offset, r.inUsed, windows, r.inBit, r.outPos, winOff) };
+    }
+    readMany(spans: [number, number][]): Uint8Array[] {
+        const r = native.inflateRanges(this.input, this.offset, this.length, this.windows, this.inBit, this.outPos, this.winOff,
+                                       spans.map(s => s[0]), spans.map(s => s[1]), 0);
+        (r.status as number[]).forEach((st: number) => { if (st !== 0) throw new Error(statusText(st)); });
+        return r.outputs;
+    }
+    read(pos: number, length: number): Uint8Array { return this.readMany([[pos, length]])[0]; }
+}
+
 // Whole containers in one call (what GZip.compress / Zip.compress do entry by entry, src/GZip.ts:96-194,
 // src/Zip.ts:117-372): every entry checksummed + deflated in one batch, headers / trailers / central directory / end
 // record written and packed on the device. heads / cdirs / tail are the byte templates described in the header.

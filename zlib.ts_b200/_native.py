@@ -17,7 +17,12 @@ RESULT_DTYPE = np.dtype([("status", "<u4"), ("crc32", "<u4"), ("adler32", "<u4")
 ENTRY_DTYPE = np.dtype([("in_off", "<u8"), ("in_len", "<u8"), ("head_off", "<u8"), ("head_len", "<u4"),
                         ("method", "<u4"), ("cdir_off", "<u8"), ("cdir_len", "<u4"), ("reserved", "<u4")])
 DICT_DTYPE = np.dtype([("off", "<u8"), ("len", "<u8")])   # zlb_dict: an item's preset dictionary in the dictionary blob
+POINT_DTYPE = np.dtype([("in_bit", "<u8"), ("out_pos", "<u8"), ("win_off", "<u8")])   # zlb_point: an access point
+RANGE_DTYPE = np.dtype([("in_off", "<u8"), ("in_len", "<u8"), ("pt_first", "<u8"), ("pt_count", "<u8"), ("pos", "<u8"),
+                        ("out_off", "<u8"), ("out_cap", "<u8")])                     # zlb_range: one read
 assert ITEM_DTYPE.itemsize == 32 and RESULT_DTYPE.itemsize == 32 and ENTRY_DTYPE.itemsize == 48 and DICT_DTYPE.itemsize == 16
+assert POINT_DTYPE.itemsize == 24 and RANGE_DTYPE.itemsize == 56
+INDEX_DEFAULT_SPACING = 1 << 20
 
 # CompressionType (src/RawDeflate.ts:12-17)
 NONE, FIXED, DYNAMIC = 0, 1, 2
@@ -47,6 +52,7 @@ EXPORTS = [
     "zlb_host_alloc", "zlb_host_free", "zlb_host_is_pinned",
     "zlb_deflate_batch_dict", "zlb_deflate_batch_dict_host", "zlb_inflate_batch_dict", "zlb_inflate_batch_dict_host",
     "zlb_inflate_size_batch", "zlb_inflate_size_batch_host",
+    "zlb_inflate_index", "zlb_inflate_index_host", "zlb_inflate_ranges", "zlb_inflate_ranges_host",
 ]
 
 _lib = None
@@ -94,6 +100,14 @@ def load_library():
     lib.zlb_inflate_size_batch.restype = i32
     lib.zlb_inflate_size_batch_host.argtypes = [vp, vp, sz, vp, vp, vp, sz, u32]
     lib.zlb_inflate_size_batch_host.restype = i32
+    lib.zlb_inflate_index.argtypes = [vp, vp, vp, vp, vp, sz, u32, u64, vp, vp, vp]
+    lib.zlb_inflate_index.restype = i32
+    lib.zlb_inflate_index_host.argtypes = [vp, vp, sz, vp, sz, vp, vp, sz, u32, u64, vp, vp, vp]
+    lib.zlb_inflate_index_host.restype = i32
+    lib.zlb_inflate_ranges.argtypes = [vp, vp, vp, vp, vp, sz, vp, vp, sz, u32]
+    lib.zlb_inflate_ranges.restype = i32
+    lib.zlb_inflate_ranges_host.argtypes = [vp, vp, sz, vp, sz, vp, sz, vp, sz, vp, vp, sz, u32]
+    lib.zlb_inflate_ranges_host.restype = i32
     lib.zlb_checksum_batch.argtypes = [vp, vp, vp, vp, sz, u32]
     lib.zlb_checksum_batch.restype = i32
     lib.zlb_checksum_batch_host.argtypes = [vp, vp, sz, vp, vp, sz, u32]
@@ -199,6 +213,10 @@ def make_dicts(n):
 
 def make_items(n):
     return np.zeros(n, dtype=ITEM_DTYPE)
+
+
+def make_ranges(n):
+    return np.zeros(n, dtype=RANGE_DTYPE)
 
 
 def make_entries(n):
@@ -321,6 +339,36 @@ class Engine:
         self._check(rc, "zlb_inflate_size_batch")
         return results
 
+    @staticmethod
+    def _index_tables(n, point_first):
+        """(point_first as uint64 with n + 1 entries, point table, point counts) of an index build."""
+        first = np.ascontiguousarray(point_first, dtype=np.uint64)
+        if first.size != n + 1:
+            raise ValueError("point_first needs n_items + 1 entries")
+        return first, np.zeros(max(int(first[-1]), 1), dtype=POINT_DTYPE), np.zeros(n, dtype=np.uint64)
+
+    def inflate_index(self, d_in, d_out, items, point_first, spacing=0, flags=0):
+        """zlb_inflate_index: the decode of inflate_batch(..., flags | INFLATE_SPLIT) that also reports access points.
+        Item i's points are points[point_first[i] : point_first[i] + counts[i]]. Returns (results, points, counts)."""
+        items, results = self._tables(items)
+        first, points, counts = self._index_tables(len(items), point_first)
+        rc = self.lib.zlb_inflate_index(self.h, d_in.data_ptr(), d_out.data_ptr(), items.ctypes.data, results.ctypes.data,
+                                        len(items), flags, spacing, points.ctypes.data, first.ctypes.data,
+                                        counts.ctypes.data)
+        self._check(rc, "zlb_inflate_index")
+        return results, points, counts
+
+    def inflate_ranges(self, d_in, d_win, d_out, points, ranges, flags=0):
+        """zlb_inflate_ranges: reads through access points (RANGE_DTYPE table; device blobs d_in, d_win, d_out)."""
+        points = np.ascontiguousarray(points, dtype=POINT_DTYPE)
+        ranges = np.ascontiguousarray(ranges, dtype=RANGE_DTYPE)
+        results = np.zeros(len(ranges), dtype=RESULT_DTYPE)
+        rc = self.lib.zlb_inflate_ranges(self.h, d_in.data_ptr(), d_win.data_ptr() if d_win is not None else None,
+                                         d_out.data_ptr(), points.ctypes.data, len(points), ranges.ctypes.data,
+                                         results.ctypes.data, len(ranges), flags)
+        self._check(rc, "zlb_inflate_ranges")
+        return results
+
     def checksum_batch(self, d_in, items, kinds=SUM_CRC32 | SUM_ADLER32):
         items, results = self._tables(items)
         rc = self.lib.zlb_checksum_batch(self.h, d_in.data_ptr(), items.ctypes.data, results.ctypes.data,
@@ -380,6 +428,30 @@ class Engine:
         rc = self.lib.zlb_inflate_size_batch_host(self.h, pi, ni, None if dicts is None else dicts.ctypes.data,
                                                   items.ctypes.data, results.ctypes.data, len(items), flags)
         self._check(rc, "zlb_inflate_size_batch_host")
+        return results
+
+    def inflate_index_host(self, h_in, h_out, items, point_first, spacing=0, flags=0):
+        """zlb_inflate_index_host (see inflate_index)."""
+        items, results = self._tables(items)
+        first, points, counts = self._index_tables(len(items), point_first)
+        pi, ni, ki = self._host_ptr(h_in)
+        po, no, ko = self._host_ptr(h_out)
+        rc = self.lib.zlb_inflate_index_host(self.h, pi, ni, po, no, items.ctypes.data, results.ctypes.data, len(items),
+                                             flags, spacing, points.ctypes.data, first.ctypes.data, counts.ctypes.data)
+        self._check(rc, "zlb_inflate_index_host")
+        return results, points, counts
+
+    def inflate_ranges_host(self, h_in, h_win, h_out, points, ranges, flags=0):
+        """zlb_inflate_ranges_host (see inflate_ranges)."""
+        points = np.ascontiguousarray(points, dtype=POINT_DTYPE)
+        ranges = np.ascontiguousarray(ranges, dtype=RANGE_DTYPE)
+        results = np.zeros(len(ranges), dtype=RESULT_DTYPE)
+        pi, ni, ki = self._host_ptr(h_in)
+        pw, nw, kw = self._host_ptr(h_win) if h_win is not None else (None, 0, None)
+        po, no, ko = self._host_ptr(h_out)
+        rc = self.lib.zlb_inflate_ranges_host(self.h, pi, ni, pw, nw, po, no, points.ctypes.data, len(points),
+                                              ranges.ctypes.data, results.ctypes.data, len(ranges), flags)
+        self._check(rc, "zlb_inflate_ranges_host")
         return results
 
     def checksum_batch_host(self, h_in, items, kinds=SUM_CRC32 | SUM_ADLER32):

@@ -27,6 +27,10 @@ Deviations from the reference, all deliberate (SURVEY.md Appendix B):
   * decompressed sizes without decoding the bytes: `inflate_sizes` (zlb_inflate_size_batch) returns what each stream
     inflates to, so that the output slots of `inflate_many(..., size_hints=sizes)` or RawInflate's `bufferSize` are
     exact and that call needs no retry. The reference has no such query (its buffer grows while it decodes).
+  * random access (zlb_inflate_index / zlb_inflate_ranges): `inflate_index` decodes a raw, zlib or gzip stream once and
+    keeps access points -- proven block starts with the 32 KiB window in front of each -- in an `InflateIndex`, whose
+    `read` / `read_many` (and `read_ranges` across streams) decode only from the last point in front of a range. What
+    zlib's zran.c and indexed_gzip offer; the reference has nothing of the kind.
 """
 import datetime
 import struct
@@ -704,6 +708,174 @@ class GUnzip:
                 return
             m, p = heads[self.ip]
             self._finish_member(dict(m), p, outs[i], res[i])
+
+
+# ------------------------------------------------------------------------------------------------------------
+# random access: an index of access points (zlb_inflate_index / zlb_inflate_ranges)
+# ------------------------------------------------------------------------------------------------------------
+_INDEX_KINDS = ("raw", "zlib", "gzip")
+_INDEX_MAGIC = b"ZLBINDEX"
+_INDEX_VERSION = 1
+# magic, version, kind, deflate start, container bytes, deflate bytes, decompressed bytes, spacing, points, window bytes
+_INDEX_HEAD = struct.Struct("<8sIIQQQQQQQ")
+
+
+class InflateIndex:
+    """Access points into one raw deflate, zlib or gzip stream (made by inflate_index). A read of any decompressed
+    range decodes from the last point at or before it, not from the start of the stream; a long one is cut at every
+    point inside it and its pieces are decoded side by side. Holds the points and, compacted, the window of each (the
+    up to 32 KiB of output in front of it): about 32 KiB per point. The compressed data is not part of it: every read
+    is given the same bytes the index was built over."""
+
+    def __init__(self, kind, start, data_len, deflate_len, size, spacing, points, windows):
+        if kind not in _INDEX_KINDS:
+            raise ZlibError("unknown index kind: %s" % kind)
+        self.kind, self.start, self.data_len, self.deflate_len = kind, int(start), int(data_len), int(deflate_len)
+        self.size, self.spacing = int(size), int(spacing)
+        self.points = np.ascontiguousarray(points, dtype=N.POINT_DTYPE)
+        self.windows = np.ascontiguousarray(windows, dtype=np.uint8).reshape(-1)
+
+    def __len__(self):
+        return len(self.points)
+
+    @property
+    def nbytes(self):
+        """bytes of the serialized index"""
+        return _INDEX_HEAD.size + self.points.nbytes + self.windows.nbytes
+
+    def read(self, data, pos, length):
+        """data[...] decompressed, bytes [pos, pos + length) (fewer at the end of the stream) as a uint8 array."""
+        return read_ranges([(data, self, pos, length)])[0]
+
+    def read_many(self, data, spans):
+        """read() of every (pos, length) in spans, in one GPU call."""
+        return read_ranges([(data, self, pos, length) for pos, length in spans])
+
+    def to_bytes(self):
+        head = _INDEX_HEAD.pack(_INDEX_MAGIC, _INDEX_VERSION, _INDEX_KINDS.index(self.kind), self.start, self.data_len,
+                                self.deflate_len, self.size, self.spacing, len(self.points), self.windows.size)
+        return head + self.points.tobytes() + self.windows.tobytes()
+
+    @classmethod
+    def from_bytes(cls, blob):
+        b = bytes(blob)
+        if len(b) < _INDEX_HEAD.size or b[:8] != _INDEX_MAGIC:
+            raise ZlibError("not an inflate index")
+        magic, version, kind, start, data_len, deflate_len, size, spacing, n, wbytes = _INDEX_HEAD.unpack_from(b)
+        if version != _INDEX_VERSION:
+            raise ZlibError("unsupported inflate index version: %d" % version)
+        if kind >= len(_INDEX_KINDS) or len(b) != _INDEX_HEAD.size + n * N.POINT_DTYPE.itemsize + wbytes:
+            raise ZlibError("inflate index is corrupt")
+        at = _INDEX_HEAD.size
+        points = np.frombuffer(b, dtype=N.POINT_DTYPE, count=n, offset=at).copy()
+        windows = np.frombuffer(b, dtype=np.uint8, count=wbytes, offset=at + points.nbytes).copy()
+        return cls(_INDEX_KINDS[kind], start, data_len, deflate_len, size, spacing, points, windows)
+
+    def _deflate(self, data):
+        """the stream's deflate bytes in data, which must be as long as what the index was built over"""
+        a = _u8(data)
+        if a.size != self.data_len:
+            raise ZlibError("data of %d bytes does not belong to this index (built over %d bytes)" % (a.size, self.data_len))
+        return a[self.start:self.start + self.deflate_len]
+
+
+def inflate_index(data, kind="raw", spacing=N.INDEX_DEFAULT_SPACING):
+    """Decompresses one raw deflate, zlib or gzip stream and indexes it: returns (output, InflateIndex) with an access
+    point about every `spacing` decompressed bytes. zlib and gzip headers are read as Inflate / GUnzip read them, with
+    their error texts, and the Adler-32, or CRC-32 and ISIZE, are always checked. Preset dictionaries (FDICT) and
+    multi-member gzip files are refused."""
+    if kind not in _INDEX_KINDS:
+        raise ZlibError("unknown index kind: %s" % kind)
+    a = _u8(data)
+    start = 0
+    if kind == "zlib":
+        cmf, flg = int(a[0]), int(a[1])
+        if (cmf & 0x0F) != 8:
+            raise ZlibError("unsupported compression method")  # src/Inflate.ts:47
+        if ((cmf << 8) + flg) % 31 != 0:
+            raise ZlibError("invalid fcheck flag:%d" % (((cmf << 8) + flg) % 31))  # :52
+        if flg & 0x20:
+            raise ZlibError("fdict flag is not supported")  # :57
+        start = 2
+    elif kind == "gzip":
+        _, start = GUnzip(a)._parse_header(0)
+    body = a[start:]
+    size = int(inflate_sizes([body])[0])  # exact slot: no retry
+    out = np.zeros(max(size, 1), dtype=np.uint8)
+    items = N.make_items(1)
+    items["in_len"], items["out_cap"] = body.size, size
+    slots = size // max(int(spacing), 1) + 2
+    flags = {"raw": 0, "zlib": N.INFLATE_WANT_ADLER32, "gzip": N.INFLATE_WANT_CRC32}[kind]
+    res, points, counts = engine().inflate_index_host(body if body.size else np.zeros(1, dtype=np.uint8), out, items,
+                                                      [0, slots], int(spacing), flags)
+    if int(res["status"][0]) != N.ST_OK:
+        raise ZlibError(status_text(res["status"][0]))
+    out = out[:int(res["out_len"][0])]
+    used = int(res["in_used"][0])
+    p = start + used
+    if kind == "zlib":
+        stored = struct.unpack(">I", a[p:p + 4].tobytes().ljust(4, b"\0"))[0]
+        if int(res["adler32"][0]) != stored:
+            raise ZlibError("invalid adler-32 checksum")  # src/Inflate.ts:88
+    elif kind == "gzip":  # src/GUnzip.ts:160-176
+        crc32, isize = struct.unpack("<II", a[p:p + 8].tobytes().ljust(8, b"\0"))
+        if int(res["crc32"][0]) != crc32:
+            raise ZlibError("invalid CRC-32 checksum: 0x%x / 0x%x" % (int(res["crc32"][0]), crc32))
+        if (out.size & 0xFFFFFFFF) != isize:
+            raise ZlibError("invalid input size: %d / %d" % (out.size & 0xFFFFFFFF, isize))
+        if p + 8 < a.size:
+            raise ZlibError("multi-member gzip files cannot be indexed")
+    points = points[:int(counts[0])].copy()
+    # keep only the windows, back to back
+    wl = np.minimum(points["out_pos"], 32768)
+    windows = np.concatenate([out[int(q) - int(w):int(q)] for q, w in zip(points["out_pos"], wl)] or [out[:0]])
+    points["win_off"] = np.concatenate([[0], np.cumsum(wl)[:-1]]).astype(np.uint64)
+    return out, InflateIndex(kind, start, a.size, used, out.size, spacing, points, windows)
+
+
+def read_ranges(reads, want_crc32=False, want_adler32=False):
+    """Reads of (data, InflateIndex, pos, length) -- any streams, any number of each -- in one GPU call
+    (zlb_inflate_ranges_host). Returns a uint8 array per read: bytes [pos, pos + length) of the decompressed stream,
+    fewer where it ends. With want_crc32 / want_adler32, (arrays, results table) with the checksums of each read."""
+    reads = list(reads)
+    if not reads:
+        return ([], np.zeros(0, dtype=N.RESULT_DTYPE)) if want_crc32 or want_adler32 else []
+    blobs, where, pts, wins, pbase = [], {}, [], [], {}
+    at = wat = pat = out_at = 0
+    ranges = N.make_ranges(len(reads))
+    for i, (data, idx, pos, length) in enumerate(reads):
+        pos, length = int(pos), int(length)
+        if pos < 0 or length < 0:
+            raise ZlibError("negative position or length")
+        key = (id(data), id(idx))
+        if key not in where:
+            blobs.append(idx._deflate(data))
+            where[key] = at
+            at += idx.deflate_len
+        if id(idx) not in pbase:
+            p = idx.points.copy()
+            p["win_off"] += np.uint64(wat)
+            pts.append(p)
+            wins.append(idx.windows)
+            pbase[id(idx)] = pat
+            pat += len(p)
+            wat += idx.windows.size
+        cap = max(0, min(length, idx.size - pos))
+        ranges[i] = (where[key], idx.deflate_len, pbase[id(idx)], len(idx.points), pos, out_at, cap)
+        out_at += cap
+    blob = np.concatenate(blobs + [np.zeros(1, dtype=np.uint8)])
+    win = np.concatenate(wins + [np.zeros(1, dtype=np.uint8)])
+    out = np.zeros(max(out_at, 1), dtype=np.uint8)
+    flags = (N.INFLATE_WANT_CRC32 if want_crc32 else 0) | (N.INFLATE_WANT_ADLER32 if want_adler32 else 0)
+    res = engine().inflate_ranges_host(blob, win, out, np.concatenate(pts), ranges, flags)
+    outs = []
+    for r, rg in zip(res, ranges):
+        if int(r["status"]) != N.ST_OK:
+            raise ZlibError(status_text(r["status"]))
+        if int(r["out_len"]) != int(rg["out_cap"]):
+            raise ZlibError("input buffer is broken")  # the stream ended before the index said it would
+        outs.append(out[int(rg["out_off"]):int(rg["out_off"]) + int(rg["out_cap"])])
+    return (outs, res) if flags else outs
 
 
 # ------------------------------------------------------------------------------------------------------------

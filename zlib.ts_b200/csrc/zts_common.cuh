@@ -34,6 +34,8 @@ enum ZtsKernelSlot {
     ZK_INFLATE_DICT,
     ZK_INFLATE_SIZE,    // zlb_inflate_size_batch (zts_inflate.cu)
     ZK_BLOCK_FIND,      // block starts in streams without markers (zts_inflate.cu)
+    ZK_INFLATE_POINTS,  // zlb_inflate_index / zlb_inflate_ranges (zts_inflate.cu)
+    ZK_INFLATE_RANGE,
     ZK_COUNT
 };
 
@@ -45,7 +47,7 @@ static const char* const kZtsKernelNames[ZK_COUNT] = {
     "frame_body_kernel",   "frame_header_kernel",
     "inflate_warp_kernel_window", "window_run_kernel", "window_scan_kernel", "window_resolve_kernel",
     "dict_stage_kernel", "inflate_warp_kernel_dict", "inflate_warp_kernel_size",
-    "block_find_kernel"};
+    "block_find_kernel", "inflate_warp_kernel_points", "inflate_warp_kernel_range"};
 
 // internal inflate flag beside ZLB_INFLATE_SEGMENT (not in the public header): an item's in_off / in_len and its
 // result's in_used count bits, so that a piece of a stream may start and end inside a byte (the searched split)

@@ -26,7 +26,10 @@
 #include <stdlib.h>
 
 #include <algorithm>
+#include <array>
+#include <climits>
 #include <cstddef>
+#include <set>
 #include <chrono>
 #include <type_traits>
 
@@ -345,13 +348,29 @@ __device__ uint32_t inf_classify_symbols(const InfWarpSmem* S, const uint8_t* sr
 // reached, at most 32768 (the marker split compares that with the output of the pieces in front). INF_SIZE and
 // INF_WINDOW read ZLB_INFLATE_BITS (the searched split): in_off / in_len / in_used count bits. Positions then count
 // from the piece's first byte, its first bits consumed at the start, so that a stored block's byte alignment holds.
+// INF_POINTS (zlb_inflate_index): INF_BYTES that also records access points into `sink` (ZtsPointSink). INF_RANGE
+// (zlb_inflate_ranges): INF_DICT -- the window of an access point is the dictionary -- that starts at a bit offset
+// (ZLB_INFLATE_BITS) and stops, without an error, once out_cap bytes are written: a match or stored copy that crosses
+// the cap is clamped, so exactly the bytes up to the cap are written and nothing behind it.
 #define WIN_WORDS 32768u
-enum { INF_BYTES = 0, INF_WINDOW = 1, INF_DICT = 2, INF_SIZE = 3 };
+enum { INF_BYTES = 0, INF_WINDOW = 1, INF_DICT = 2, INF_SIZE = 3, INF_POINTS = 4, INF_RANGE = 5 };
+// Where INF_POINTS puts the access points of item i: slots points[first[i] .. first[i + 1]), its count in count[i]. A
+// block start becomes a point when its output position is at least the last point's plus `spacing` (the first block
+// always): the greedy rule of zlb_inflate_index, the same as the host applies to the split's piece starts.
+struct ZtsPointSink {
+    zlb_point* points;
+    const unsigned long long* first;
+    unsigned long long* count;
+    unsigned long long spacing;
+};
+// `out`: the output base of items[*].out_off. INF_RANGE is launched with out == NULL and device addresses in out_off
+// (a range's pieces write into the caller's slots and into scratch in one launch): the slot address is only ever
+// out + out_off, never compared with or offset from `out` otherwise.
 template <int MODE>
 __global__ void __launch_bounds__(INF_WARPS_PER_CTA * 32, INF_MIN_CTAS)
 inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, const zlb_item* __restrict__ items,
                     zlb_result* __restrict__ results, uint32_t n_items, uint32_t flags,
-                    const zlb_dict* __restrict__ dicts, const uint8_t* __restrict__ dict)
+                    const zlb_dict* __restrict__ dicts, const uint8_t* __restrict__ dict, ZtsPointSink sink)
 {
     using T = typename std::conditional<MODE == INF_WINDOW, uint16_t, uint8_t>::type;
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -362,7 +381,8 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
     if (item >= n_items) return;
 
     const zlb_item it = items[item];
-    constexpr bool BITS_OK = MODE == INF_SIZE || MODE == INF_WINDOW;
+    constexpr bool BITS_OK = MODE == INF_SIZE || MODE == INF_WINDOW || MODE == INF_RANGE;
+    constexpr bool DICT = MODE == INF_DICT || MODE == INF_RANGE;  // a window in front of the output, from the blob
     const bool bits = BITS_OK && (flags & ZLB_INFLATE_BITS);
     const uint32_t sb = bits ? (uint32_t)(it.in_off & 7u) : 0u;  // bits of the first byte in front of the piece
     const uint8_t* src = in + (bits ? it.in_off >> 3 : it.in_off);
@@ -370,7 +390,7 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
     T* dst = reinterpret_cast<T*>(out + it.out_off);
     uint32_t reach = MODE == INF_WINDOW ? WIN_WORDS : 0u;  // how far a distance may reach in front of the output
     const uint8_t* dtail = nullptr;                       // INF_DICT: the `reach` bytes in front of the output
-    if constexpr (MODE == INF_DICT) {
+    if constexpr (DICT) {
         const zlb_dict d = dicts[item];
         reach = d.len < WIN_WORDS ? (uint32_t)d.len : WIN_WORDS;
         dtail = dict + d.off + d.len - reach;
@@ -406,14 +426,28 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
     uint32_t blocks = 0;
     int have_fixed = 0;
     bool bfinal = false;
+    bool full = false;  // INF_RANGE: out_cap bytes written
+    // INF_POINTS: the item's next slot, its end, and the output position the next point needs at least
+    unsigned long long pt_next = 0, pt_end = 0, pt_due = 0;
+    if constexpr (MODE == INF_POINTS) {
+        pt_next = sink.first[item];
+        pt_end = sink.first[item + 1];
+    }
 
-    while (!bfinal && status == ZLB_ST_OK) {
+    while (!bfinal && status == ZLB_ST_OK && !full) {
         // segment mode: a piece of a larger stream ends cleanly where a block ends and its input is used up
         if ((flags & ZLB_INFLATE_SEGMENT) && blocks > 0 && br_bits_used(br) == in_bits) break;
         br_refill(br);
         if (br_bits_used(br) + 3 > in_bits) {
             status = ZLB_ST_INPUT_BROKEN;
             break;
+        }
+        if constexpr (MODE == INF_POINTS) {
+            if (op >= pt_due) {
+                if (lane == 0 && pt_next < pt_end) sink.points[pt_next] = {br_bits_used(br), op, 0};
+                pt_next++;
+                pt_due = op + sink.spacing;
+            }
         }
         uint32_t hdr = br_take(br, 3);  // src/RawInflate.ts:146-152
         bfinal = hdr & 1u;
@@ -440,6 +474,10 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
             if (byte_pos + len > in_len) {
                 status = ZLB_ST_INPUT_BROKEN;
                 break;
+            }
+            if (MODE == INF_RANGE && op + len >= cap) {
+                len = (uint32_t)(cap - op);  // (the cap is reached: what is left of the block is not wanted)
+                full = true;
             }
             if (MODE != INF_SIZE && op + len > cap) {
                 status = ZLB_ST_OUT_OVERFLOW;
@@ -537,7 +575,7 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
 
         // ---- symbol loop (src/RawInflate.ts:466-516), 32 symbols per batch
         bool eob = false;
-        while (!eob && status == ZLB_ST_OK) {
+        while (!eob && status == ZLB_ST_OK && !full) {
             // -- decode: token of symbol i ends up in lane i: literal = byte << 16 | junk < 256, match = INF_TOK_MATCH | len << 16 | dist.
             //    The tables are addressed through 32-bit shared-window addresses held in registers (a generic
             //    pointer to the per-warp slice gets rematerialised from %tid on every look-up otherwise).
@@ -677,13 +715,18 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
             // a distance beyond the start of the output (the reference would copy `undefined` -> 0) or an
             // output slot that is too small ends the batch before the offending token
             const bool bad_dist = is_match && dist > behind + rel + reach;
-            const bool over = MODE != INF_SIZE && mine && rel + len > room;
+            // (INF_RANGE: a token that starts at or behind the cap is not wanted, one that crosses it is clamped)
+            const bool over = MODE != INF_SIZE && mine && (MODE == INF_RANGE ? rel >= room : rel + len > room);
+            const uint32_t wlen = MODE == INF_RANGE ? min(len, room - min(rel, room)) : len;  // bytes the token writes
             const unsigned bad_mask = __ballot_sync(0xFFFFFFFFu, bad_dist || over);
             uint32_t nvalid = ntok;
             if (bad_mask) {
                 nvalid = (uint32_t)__ffs((int)bad_mask) - 1u;
                 const bool first_is_dist = __shfl_sync(0xFFFFFFFFu, (int)bad_dist, (int)nvalid) != 0;
-                status = first_is_dist ? ZLB_ST_BAD_CODE : ZLB_ST_OUT_OVERFLOW;
+                if (MODE == INF_RANGE && __shfl_sync(0xFFFFFFFFu, (int)over, (int)nvalid))
+                    full = true;  // (a bad distance behind the cap is not looked at)
+                else
+                    status = first_is_dist ? ZLB_ST_BAD_CODE : ZLB_ST_OUT_OVERFLOW;
             }
             const bool live = lane < nvalid;
             if constexpr (MODE == INF_SIZE) {
@@ -694,7 +737,7 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
                 continue;
             }
             // -- literals: one store
-            ZTS_ASSERT(!live || (op + rel + len <= cap && (!is_match || dist <= op + rel + reach)));
+            ZTS_ASSERT(!live || (op + rel + wlen <= cap && (!is_match || dist <= op + rel + reach)));
             if (live && !is_match) bdst[rel] = (uint8_t)(mytok >> 16);
             __syncwarp();  // (a match may read the literals of its own batch)
             // -- matches, sub-batch by sub-batch: a sub-batch ends in front of the first match that reads what a match
@@ -712,28 +755,28 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
                 const unsigned dep_mask = __ballot_sync(0xFFFFFFFFu, dep);
                 const uint32_t cut = dep_mask ? (uint32_t)__ffs((int)dep_mask) - 1u : 32u;  // behind the first match always
                 const bool in_sub = live && is_match && lane >= start && lane < cut;
-                const bool small = in_sub && len <= 8u && dist >= len && (MODE != INF_DICT || dist <= behind + rel);
+                const bool small = in_sub && len <= 8u && dist >= len && (!DICT || dist <= behind + rel);
                 if (__any_sync(0xFFFFFFFFu, small)) {
                     // short non-overlapping matches: every lane copies its own, loads first, then stores
                     T v[8];
                     T* dp = bdst + rel;
                     const T* sp = dp - dist;
 #pragma unroll
-                    for (int k = 0; k < 8; ++k) v[k] = (small && (uint32_t)k < len) ? sp[k] : (T)0;
+                    for (int k = 0; k < 8; ++k) v[k] = (small && (uint32_t)k < wlen) ? sp[k] : (T)0;
 #pragma unroll
                     for (int k = 0; k < 8; ++k)
-                        if (small && (uint32_t)k < len) dp[k] = v[k];
+                        if (small && (uint32_t)k < wlen) dp[k] = v[k];
                 }
                 unsigned big_mask = __ballot_sync(0xFFFFFFFFu, in_sub && !small);
                 while (big_mask) {
                     const int j = __ffs((int)big_mask) - 1;
                     big_mask &= big_mask - 1;
-                    const uint32_t jl = __shfl_sync(0xFFFFFFFFu, len, j);
+                    const uint32_t jl = __shfl_sync(0xFFFFFFFFu, wlen, j);
                     const uint32_t jd = __shfl_sync(0xFFFFFFFFu, dist, j);
                     const uint32_t jr = __shfl_sync(0xFFFFFFFFu, rel, j);
                     T* o = bdst + jr;
                     const T* s0 = o - jd;
-                    if (MODE == INF_DICT && jd > behind + jr) {
+                    if (DICT && jd > behind + jr) {
                         // the source starts in the dictionary (then behind == op): byte k is byte
                         // op + jr - jd + (k mod jd) of dictionary || output, which lies in front of the match
                         const int x0 = (int)(behind + jr) - (int)jd;
@@ -764,12 +807,18 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
             }
             // bytes of the tokens that were written (all of them unless the batch was cut short)
             op += nvalid ? __shfl_sync(0xFFFFFFFFu, inc, (int)nvalid - 1) : 0u;
+            if (MODE == INF_RANGE && op >= cap) {
+                op = cap;
+                full = true;
+            }
             __syncwarp();
         }
         if (status == ZLB_ST_OK && br_bits_used(br) > in_bits) status = ZLB_ST_INPUT_BROKEN;
     }
 
     if constexpr (MODE == INF_SIZE) reached = __reduce_max_sync(0xFFFFFFFFu, reached);
+    if constexpr (MODE == INF_POINTS)
+        if (lane == 0) sink.count[item] = pt_next < pt_end ? pt_next - sink.first[item] : pt_end - sink.first[item];
     if (lane == 0) {
         zlb_result r = results[item];
         if (MODE == INF_SIZE && (flags & ZLB_INFLATE_SEGMENT)) r.crc32 = reached;
@@ -784,15 +833,16 @@ inflate_warp_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, c
 template <int MODE>
 static int inflate_launch_mode(zlb_ctx* ctx, cudaStream_t st, const uint8_t* d_in, uint8_t* d_out, const zlb_item* d_items,
                                zlb_result* d_results, size_t n, uint32_t flags, const zlb_dict* d_dicts,
-                               const uint8_t* d_dict)
+                               const uint8_t* d_dict, ZtsPointSink sink = ZtsPointSink{})
 {
     const size_t smem = sizeof(InfWarpSmem) * INF_WARPS_PER_CTA;
     ZTS_CUDA(ctx, cudaFuncSetAttribute(inflate_warp_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     unsigned grid = (unsigned)((n + INF_WARPS_PER_CTA - 1) / INF_WARPS_PER_CTA);
     ZTS_LAUNCH(ctx,
-               MODE == INF_WINDOW ? ZK_INFLATE_WINDOW : MODE == INF_DICT ? ZK_INFLATE_DICT : MODE == INF_SIZE ? ZK_INFLATE_SIZE : ZK_INFLATE,
+               MODE == INF_WINDOW ? ZK_INFLATE_WINDOW : MODE == INF_DICT ? ZK_INFLATE_DICT : MODE == INF_SIZE ? ZK_INFLATE_SIZE
+               : MODE == INF_POINTS ? ZK_INFLATE_POINTS : MODE == INF_RANGE ? ZK_INFLATE_RANGE : ZK_INFLATE,
                inflate_warp_kernel<MODE><<<grid, INF_WARPS_PER_CTA * 32, smem, st>>>(d_in, d_out, d_items, d_results,
-                                                                                    (uint32_t)n, flags, d_dicts, d_dict));
+                                                                                    (uint32_t)n, flags, d_dicts, d_dict, sink));
     return ZLB_OK;
 }
 // the decoder: with a dictionary table (d_dicts[i] belongs to d_items[i]) the dictionary instantiation; without an
@@ -1178,6 +1228,36 @@ window_resolve_kernel(const uint8_t* __restrict__ arena, uint8_t* __restrict__ s
     if (__syncthreads_or((int)(seen & 0x8000u)) && threadIdx.x == 0) fail[r.item] = 1u;
 }
 
+// The access points a zlb_inflate_index call collects (inflate_device with a sink): the caller's host tables. The
+// split's routes offer the starts of an item's pieces, the one-warp route (INF_POINTS) its block headers; both take
+// them by the same greedy rule (ZtsPointSink).
+struct ZtsIndexSink {
+    unsigned long long spacing;
+    zlb_point* points;
+    const uint64_t* first;  // n + 1 entries
+    uint64_t* count;
+};
+
+// window of a point: the min(out_pos, 32768) output bytes in front of it, in the item's output slot
+static unsigned long long index_win_off(const zlb_item& it, unsigned long long out_pos)
+{
+    return it.out_off + out_pos - std::min(out_pos, (unsigned long long)WIN_WORDS);
+}
+
+// the greedy choice over the ascending candidates c[0 .. n) of item i, into its slots
+static void index_select(const ZtsIndexSink& s, size_t i, const zlb_item& it, const zlb_point* c, size_t n)
+{
+    const uint64_t slots = s.first[i + 1] - s.first[i];
+    uint64_t taken = 0;
+    unsigned long long due = 0;
+    for (size_t j = 0; j < n && taken < slots; ++j) {
+        if (c[j].out_pos < due) continue;
+        s.points[s.first[i] + taken++] = {c[j].in_bit, c[j].out_pos, index_win_off(it, c[j].out_pos)};
+        due = c[j].out_pos + s.spacing;
+    }
+    s.count[i] = taken;
+}
+
 // One call's split: the caller's items and preset dictionaries (dicts == NULL: none), the indices of its large items,
 // and the pieces of item big[k], seg[first[k] .. first[k + 1]) (split_layout). seg[j] is piece j's input span, in bytes
 // or, with `bits` (the searched split), in bits of the input; the decode split gives it a byte slot of its scratch
@@ -1189,6 +1269,7 @@ struct SplitJob {
     std::vector<size_t> first;
     std::vector<zlb_item> seg;
     bool bits = false;
+    ZtsIndexSink* sink = nullptr;  // zlb_inflate_index: where the piece starts of a decoded item go
     size_t pieces(size_t k) const { return first[k + 1] - first[k]; }
     // where the last piece of big[k] starts, from the item's first input byte (bit)
     unsigned long long last_start(size_t k) const
@@ -1253,6 +1334,15 @@ static zlb_result split_finish(const SplitJob& job, size_t k, const zlb_result* 
             if (r[j].out_len) gath.push_back({seg[j].out_off, it.out_off + at, r[j].out_len});
             at += r[j].out_len;
         }
+    }
+    if (job.sink && o.status == ZLB_ST_OK) {  // the pieces' starts, in bits from the item's first byte
+        std::vector<zlb_point> cand(job.pieces(k));
+        unsigned long long at = 0;
+        for (size_t j = 0; j < cand.size(); ++j) {
+            cand[j] = {job.bits ? seg[j].in_off - 8 * it.in_off : 8 * (seg[j].in_off - it.in_off), at, 0};
+            at += r[j].out_len;
+        }
+        index_select(*job.sink, job.big[k], it, cand.data(), cand.size());
     }
     return o;
 }
@@ -1916,13 +2006,19 @@ static int inflate_waves(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, cons
 // d_out == NULL: a size call (zlb_inflate_size_batch). The same route with the size decoder, the split's sizing stage
 // (inflate_split_sizes) and no checksums (refused by the caller); nothing is written, d_dict is not read, a "_host"
 // call copies its input over in one piece and nothing back.
+// sink (zlb_inflate_index, no dictionaries): the split's routes report the piece starts of the items they decode,
+// and the items left go through INF_POINTS instead of the plain decoder (never in waves); without a sink the call
+// launches what it launched before.
 static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, const uint8_t* d_dict,
                           const zlb_dict* h_dicts, const zlb_item* h_items, zlb_result* h_results, size_t n, uint32_t flags,
-                          const ZtsHostIO* hio)
+                          const ZtsHostIO* hio, ZtsIndexSink* sink = nullptr)
 {
     // large items that may be cut at sync-flush markers (each is massively parallel by itself)
     flags &= ~ZLB_INFLATE_BITS;  // (internal)
     SplitJob job{h_items, h_dicts, {}, {}, {}};
+    job.sink = sink;
+    if (sink)
+        for (size_t i = 0; i < n; ++i) sink->count[i] = 0;
     if ((flags & ZLB_INFLATE_SPLIT) && !(flags & ZLB_INFLATE_SEGMENT))
         for (size_t i = 0; i < n; ++i)
             if (h_items[i].in_len >= SPLIT_MIN_BYTES) job.big.push_back(i);
@@ -1949,7 +2045,7 @@ static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
     if (flags & ZLB_INFLATE_WANT_CRC32) kinds |= ZLB_SUM_CRC32;
     if (flags & ZLB_INFLATE_WANT_ADLER32) kinds |= ZLB_SUM_ADLER32;
     const bool sizes = d_out == nullptr;
-    if (hio && job.big.empty() && !sizes)
+    if (hio && job.big.empty() && !sizes && !sink)
         return inflate_waves(ctx, d_in, d_out, d_dict, d_items, d_dicts, d_results, h_items, h_results, n, flags, kinds, *hio);
 
     // the split: the items it decodes get their results in h_results; when it decoded any, rest lists the others
@@ -1966,7 +2062,7 @@ static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
     }
     if (!job.big.empty()) {
         std::vector<char> done(n, 0);
-        SplitJob sjob{h_items, h_dicts, job.big, {}, {}, true};  // the searched items
+        SplitJob sjob{h_items, h_dicts, job.big, {}, {}, true, sink};  // the searched items
         rc = split_layout(ctx, d_in, job, sjob);
         if (!rc && !job.seg.empty())
             rc = sizes ? inflate_split_sizes(ctx, d_in, job, flags, h_results, done)
@@ -1993,7 +2089,31 @@ static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
     }
     // the items left, in one launch; after a split their results come back to the host, join the split's there, and
     // the whole table goes to d_results in one copy (the checksums read out_len from it)
-    if (m) {
+    // (with a sink: the launched items' slots, compacted, in ctx->d_misc; read back behind the results)
+    std::vector<unsigned long long> pt_first, pt_count;
+    std::vector<zlb_point> pts;
+    if (m && sink) {
+        pt_first.assign(m + 1, 0);
+        for (size_t j = 0; j < m; ++j) {
+            const size_t i = split_any ? rest[j] : j;
+            pt_first[j + 1] = pt_first[j] + (sink->first[i + 1] - sink->first[i]);
+        }
+        pts.resize(pt_first[m]);
+        pt_count.resize(m);
+        rc = zts_reserve(ctx, &ctx->d_misc, (2 * m + 1) * 8 + pts.size() * sizeof(zlb_point) + 256);
+        if (rc) return rc;
+        ZtsPointSink ds;
+        ds.first = (const unsigned long long*)ctx->d_misc.p;
+        ds.count = (unsigned long long*)ctx->d_misc.p + m + 1;
+        ds.points = (zlb_point*)(ds.count + m);
+        ds.spacing = sink->spacing;
+        ZTS_CUDA(ctx, cudaMemcpyAsync((void*)ds.first, pt_first.data(), (m + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
+        rc = inflate_launch_mode<INF_POINTS>(ctx, ctx->stream, d_in, d_out, d_rest, d_results, m, flags, nullptr, nullptr, ds);
+        if (rc) return rc;
+        ZTS_CUDA(ctx, cudaMemcpyAsync(pt_count.data(), ds.count, m * 8, cudaMemcpyDeviceToHost, ctx->stream));
+        if (!pts.empty())
+            ZTS_CUDA(ctx, cudaMemcpyAsync(pts.data(), ds.points, pts.size() * sizeof(zlb_point), cudaMemcpyDeviceToHost, ctx->stream));
+    } else if (m) {
         rc = inflate_launch(ctx, ctx->stream, d_in, d_out, d_rest, d_results, m, flags, d_rest_dicts, d_dict);
         if (rc) return rc;
     }
@@ -2009,6 +2129,19 @@ static int inflate_device(zlb_ctx* ctx, const uint8_t* d_in, uint8_t* d_out, con
         if (rc) return rc;
     }
     ZTS_CUDA(ctx, cudaMemcpyAsync(h_results, d_results, n * sizeof(zlb_result), cudaMemcpyDeviceToHost, ctx->stream));
+    if (!pt_first.empty()) {  // the one-warp items' points, for those that decoded
+        ZTS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        for (size_t j = 0; j < m; ++j) {
+            const size_t i = split_any ? rest[j] : j;
+            if (h_results[i].status != ZLB_ST_OK) continue;
+            for (unsigned long long c = 0; c < pt_count[j]; ++c) {
+                zlb_point p = pts[pt_first[j] + c];
+                p.win_off = index_win_off(h_items[i], p.out_pos);
+                sink->points[sink->first[i] + c] = p;
+            }
+            sink->count[i] = pt_count[j];
+        }
+    }
     if (hio && !sizes) {
         ZTS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // the sizes decide what travels
         rc = zts_copy_back(ctx, hio->stage, ctx->stream, d_out, hio->h_out, h_items, h_results, d_items, d_results, 0, n);
@@ -2105,4 +2238,265 @@ extern "C" int zlb_debug_block_starts(zlb_ctx* ctx, const void* d_in, uint64_t n
     }
     static_assert(sizeof(unsigned long long) == sizeof(uint64_t), "");
     return block_find(ctx, (const uint8_t*)d_in, cuts, (unsigned long long*)h_bits_out);
+}
+
+// ---- random access: an index of access points ------------------------------------------------------------------
+#define ZTS_INDEX_FLAGS (ZLB_INFLATE_WANT_CRC32 | ZLB_INFLATE_WANT_ADLER32 | ZLB_INFLATE_CHECK_NLEN)
+
+static int index_check(zlb_ctx* ctx, uint32_t flags, const zlb_point* points, const uint64_t* first, const uint64_t* count,
+                       size_t n)
+{
+    if (!ctx) return ZLB_E_ARG;
+    if (flags & ~ZTS_INDEX_FLAGS)
+        return zts_fail(ctx, ZLB_E_ARG, "an index build takes ZLB_INFLATE_WANT_CRC32 / _ADLER32 / _CHECK_NLEN only");
+    if (!n) return ZLB_OK;
+    if (!first || !count) return zts_fail(ctx, ZLB_E_ARG, "point_first / point_count is NULL");
+    for (size_t i = 0; i < n; ++i)
+        if (first[i + 1] < first[i]) return zts_fail(ctx, ZLB_E_ARG, "point_first decreases at item %zu", i);
+    if (first[n] > first[0] && !points) return zts_fail(ctx, ZLB_E_ARG, "the point table is NULL");
+    return ZLB_OK;
+}
+
+extern "C" int zlb_inflate_index(zlb_ctx* ctx, const void* d_in, void* d_out, const zlb_item* items, zlb_result* results,
+                                 size_t n, uint32_t flags, uint64_t spacing, zlb_point* points, const uint64_t* point_first,
+                                 uint64_t* point_count)
+{
+    int rc = index_check(ctx, flags, points, point_first, point_count, n);
+    if (rc) return rc;
+    bool any = false;
+    rc = zts_entry_begin(ctx, (d_in && d_out) || !n, items, results, n, 0x7FFFFFFFull, nullptr, SIZE_MAX, nullptr, &any);
+    if (rc) return rc > 0 ? ZLB_OK : rc;
+    ZtsIndexSink sink{spacing ? spacing : ZLB_INDEX_DEFAULT_SPACING, points, point_first, point_count};
+    rc = inflate_device(ctx, (const uint8_t*)d_in, (uint8_t*)d_out, nullptr, nullptr, items, results, n,
+                        flags | ZLB_INFLATE_SPLIT, nullptr, &sink);
+    if (rc) return rc;
+    ZTS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return ZLB_OK;
+}
+
+extern "C" int zlb_inflate_index_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes, void* h_out, size_t out_bytes,
+                                      const zlb_item* items, zlb_result* results, size_t n, uint32_t flags, uint64_t spacing,
+                                      zlb_point* points, const uint64_t* point_first, uint64_t* point_count)
+{
+    const int rc = index_check(ctx, flags, points, point_first, point_count, n);
+    if (rc) return rc;
+    ZtsIndexSink sink{spacing ? spacing : ZLB_INDEX_DEFAULT_SPACING, points, point_first, point_count};
+    return zts_host_call(ctx, h_in, in_bytes, h_out, out_bytes, nullptr, 0, nullptr, items, results, n, 0x7FFFFFFFull,
+                         [&](ZtsHostIO& io, const zlb_dict*) {
+        return inflate_device(ctx, (const uint8_t*)ctx->d_stage_in.p, (uint8_t*)ctx->d_stage_out.p, nullptr, nullptr, items,
+                              results, n, flags | ZLB_INFLATE_SPLIT, &io, &sink);
+    });
+}
+
+// The checks of a ranges call, with a text. in_bytes / win_bytes / out_bytes == SIZE_MAX: device buffers, whose sizes
+// are not known; win_given: the window blob is not NULL. A stream's points (pt_first, pt_count, in_len) are checked
+// once per call however many ranges name them.
+static int ranges_check(zlb_ctx* ctx, const zlb_point* points, size_t n_points, const zlb_range* ranges, size_t n,
+                        uint32_t flags, size_t in_bytes, size_t win_bytes, size_t out_bytes, bool win_given)
+{
+    if (flags & ~ZTS_INDEX_FLAGS)
+        return zts_fail(ctx, ZLB_E_ARG, "a ranges call takes ZLB_INFLATE_WANT_CRC32 / _ADLER32 / _CHECK_NLEN only");
+    if (n && !points) return zts_fail(ctx, ZLB_E_ARG, "the point table is NULL");
+    std::set<std::array<uint64_t, 3>> checked;
+    for (size_t i = 0; i < n; ++i) {
+        const zlb_range& r = ranges[i];
+        if (in_bytes != SIZE_MAX && (r.in_off > in_bytes || r.in_len > in_bytes - r.in_off))
+            return zts_fail(ctx, ZLB_E_ARG, "range %zu: its stream lies outside the input", i);
+        if (r.in_len >= (1ull << 60) || r.in_off >= (1ull << 60))
+            return zts_fail(ctx, ZLB_E_ARG, "range %zu: its stream lies beyond 2^60 bytes", i);  // (bit offsets fit)
+        if (out_bytes != SIZE_MAX && (r.out_off > out_bytes || r.out_cap > out_bytes - r.out_off))
+            return zts_fail(ctx, ZLB_E_ARG, "range %zu: its slot lies outside the output", i);
+        if (r.pos > UINT64_MAX - r.out_cap) return zts_fail(ctx, ZLB_E_ARG, "range %zu: pos + out_cap overflows", i);
+        if (!checked.insert({r.pt_first, r.pt_count, r.in_len}).second) continue;
+        if (r.pt_count == 0) return zts_fail(ctx, ZLB_E_ARG, "range %zu has no access points", i);
+        if (r.pt_first > n_points || r.pt_count > n_points - r.pt_first)
+            return zts_fail(ctx, ZLB_E_ARG, "range %zu: its points lie outside the point table", i);
+        const zlb_point* p = points + r.pt_first;
+        if (p[0].in_bit || p[0].out_pos) return zts_fail(ctx, ZLB_E_ARG, "range %zu: its first point is not {0, 0}", i);
+        for (uint64_t k = 0; k < r.pt_count; ++k) {
+            if (k && (p[k].in_bit <= p[k - 1].in_bit || p[k].out_pos <= p[k - 1].out_pos))
+                return zts_fail(ctx, ZLB_E_ARG, "range %zu: its points do not ascend (point %llu)", i, (unsigned long long)k);
+            if (p[k].in_bit >= 8 * r.in_len)
+                return zts_fail(ctx, ZLB_E_ARG, "range %zu: point %llu lies behind the stream", i, (unsigned long long)k);
+            const uint64_t wl = std::min(p[k].out_pos, (uint64_t)WIN_WORDS);
+            if (wl && !win_given)
+                return zts_fail(ctx, ZLB_E_ARG, "range %zu: point %llu has a window but the window blob is NULL", i,
+                                (unsigned long long)k);
+            if (win_bytes != SIZE_MAX && (p[k].win_off > win_bytes || wl > win_bytes - p[k].win_off))
+                return zts_fail(ctx, ZLB_E_ARG, "range %zu: the window of point %llu lies outside the window blob", i,
+                                (unsigned long long)k);
+        }
+    }
+    return ZLB_OK;
+}
+
+// A piece of a range: one warp from one point. The first piece of a range that starts behind its point decodes the
+// `skip` bytes in front of pos as well, into scratch; the others decode into the range's slot.
+struct ZtsRangePiece {
+    size_t range;
+    unsigned long long skip, want;  // bytes in front of pos; bytes of the range it is to give
+    zlb_item item;                  // bits from the input's first byte; out_off: a device address
+    zlb_dict win;
+};
+
+// Output bytes a stream can still give from bit `in_bit` of its `in_len` bytes on: a match of at most 258 bytes takes
+// at least two bits (a length and a distance code), a literal one, a stored byte eight; saturates.
+static unsigned long long range_reach(const zlb_range& r, const zlb_point& p)
+{
+    const unsigned long long bits = 8 * r.in_len - p.in_bit;
+    return bits > ULLONG_MAX / 258 ? ULLONG_MAX : 258 * bits;
+}
+
+// The reads of zlb_inflate_ranges[_host] on device buffers: pieces planned here, INF_RANGE over a wave of them per
+// launch (a wave's scratch within SplitBudget), the gather of the first pieces, then the results, the checksum tail and
+// on a "_host" call the copy-back. h_results is final on return. A range whose pos lies beyond what the stream can give
+// from the point in front of it gets no piece (out_len 0); a first piece whose scratch -- the bytes in front of pos
+// plus its part, at most what the stream can give -- exceeds the budget by itself fails the call with ZLB_E_NOMEM.
+static int ranges_device(zlb_ctx* ctx, const uint8_t* d_in, const uint8_t* d_win, uint8_t* d_out, const zlb_point* points,
+                         const zlb_range* ranges, zlb_result* h_results, size_t n, uint32_t flags, const ZtsHostIO* hio)
+{
+    cudaStream_t st = ctx->stream;
+    const size_t budget = SplitBudget(ctx->d_split).device;
+    std::vector<ZtsRangePiece> pieces;
+    for (size_t i = 0; i < n; ++i) {
+        const zlb_range& r = ranges[i];
+        const zlb_point* p = points + r.pt_first;
+        const unsigned long long end = r.pos + r.out_cap;  // (no overflow: ranges_check)
+        // the last point at or before pos, then every point inside [pos, end)
+        size_t j = std::upper_bound(p, p + r.pt_count, r.pos, [](unsigned long long v, const zlb_point& q) { return v < q.out_pos; }) - p - 1;
+        if (r.pos - p[j].out_pos >= range_reach(r, p[j])) continue;  // past the end of the stream: no byte to give
+        for (bool first = true; r.out_cap && j < r.pt_count && (first || p[j].out_pos < end); ++j, first = false) {
+            const unsigned long long from = std::max((unsigned long long)r.pos, (unsigned long long)p[j].out_pos);
+            const unsigned long long to = j + 1 < r.pt_count ? std::min(end, (unsigned long long)p[j + 1].out_pos) : end;
+            ZtsRangePiece q;
+            q.range = i;
+            q.skip = from - p[j].out_pos;
+            q.want = to - from;
+            q.item = {8 * r.in_off + p[j].in_bit, 8 * r.in_len - p[j].in_bit, (uintptr_t)(d_out + r.out_off + (from - r.pos)),
+                      std::min(q.skip + q.want, range_reach(r, p[j]))};
+            q.win = {p[j].win_off, std::min(p[j].out_pos, (uint64_t)WIN_WORDS)};
+            if (q.skip && q.item.out_cap > budget)
+                return zts_fail(ctx, ZLB_E_NOMEM,
+                                "range %zu: %llu bytes in front of pos would be decoded into scratch, more than the %zu a "
+                                "call may take: pass the access points between",
+                                i, q.skip, budget);
+            pieces.push_back(q);
+        }
+    }
+    const size_t np = pieces.size();
+    int rc = zts_reserve(ctx, &ctx->d_items, (n + np) * sizeof(zlb_item) + np * (sizeof(zlb_dict) + sizeof(ZtsGather)) + 256);
+    if (rc) return rc;
+    rc = zts_reserve(ctx, &ctx->d_results, std::max(n, np) * sizeof(zlb_result) + 64);
+    if (rc) return rc;
+    zlb_item* d_slots = (zlb_item*)ctx->d_items.p;
+    zlb_item* d_pitems = d_slots + n;
+    zlb_dict* d_pwin = (zlb_dict*)(d_pitems + np);
+    ZtsGather* d_gather = (ZtsGather*)(d_pwin + np);
+    zlb_result* d_results = (zlb_result*)ctx->d_results.p;
+    std::vector<zlb_result> pres(np);
+    // waves: pieces in order, a new wave where the first pieces' scratch would exceed the budget (a piece's scratch is
+    // at most the budget, so the rounding below cannot wrap)
+    std::vector<unsigned long long> soff(np, 0);
+    for (size_t a = 0; a < np;) {
+        size_t b = a, scratch = 0;
+        for (; b < np; ++b) {
+            if (!pieces[b].skip) continue;
+            const size_t s = (pieces[b].item.out_cap + 255) & ~(size_t)255;
+            if (scratch && scratch + s > budget) break;
+            soff[b] = scratch;
+            scratch += s;
+        }
+        if (scratch) {
+            bool got = false;
+            if ((rc = split_reserve(ctx, &ctx->d_split, scratch, &got))) return rc;
+            if (!got) return zts_fail(ctx, ZLB_E_NOMEM, "no device memory for %zu bytes of range scratch", scratch);
+        }
+        std::vector<zlb_item> it(b - a);
+        std::vector<zlb_dict> win(b - a);
+        for (size_t k = a; k < b; ++k) {
+            it[k - a] = pieces[k].item;
+            if (pieces[k].skip) it[k - a].out_off = (uintptr_t)ctx->d_split.p + soff[k];
+            win[k - a] = pieces[k].win;
+        }
+        ZTS_CUDA(ctx, cudaMemcpyAsync(d_pitems + a, it.data(), (b - a) * sizeof(zlb_item), cudaMemcpyHostToDevice, st));
+        ZTS_CUDA(ctx, cudaMemcpyAsync(d_pwin + a, win.data(), (b - a) * sizeof(zlb_dict), cudaMemcpyHostToDevice, st));
+        ZTS_CUDA(ctx, cudaMemsetAsync(d_results, 0, (b - a) * sizeof(zlb_result), st));
+        // (the slots' out_off are device addresses: the output base is NULL)
+        rc = inflate_launch_mode<INF_RANGE>(ctx, st, d_in, nullptr, d_pitems + a, d_results, b - a,
+                                            (flags & ZLB_INFLATE_CHECK_NLEN) | ZLB_INFLATE_BITS, d_pwin + a, d_win);
+        if (rc) return rc;
+        ZTS_CUDA(ctx, cudaMemcpyAsync(pres.data() + a, d_results, (b - a) * sizeof(zlb_result), cudaMemcpyDeviceToHost, st));
+        ZTS_CUDA(ctx, cudaStreamSynchronize(st));
+        std::vector<ZtsGather> gath;
+        for (size_t k = a; k < b; ++k) {
+            const ZtsRangePiece& q = pieces[k];
+            if (q.skip && pres[k].out_len > q.skip)
+                gath.push_back({soff[k] + q.skip, ranges[q.range].out_off, pres[k].out_len - q.skip});
+        }
+        if (!gath.empty()) {
+            ZTS_CUDA(ctx, cudaMemcpyAsync(d_gather, gath.data(), gath.size() * sizeof(ZtsGather), cudaMemcpyHostToDevice, st));
+            ZTS_LAUNCH(ctx, ZK_GATHER, segment_gather_kernel<<<(unsigned)gath.size(), 256, 0, st>>>(
+                                           (const uint8_t*)ctx->d_split.p, d_out, d_gather));
+            ZTS_CUDA(ctx, cudaStreamSynchronize(st));  // gath goes out of scope, the next wave reuses the scratch
+        }
+        a = b;
+    }
+    // a range's result: its pieces in order, up to the first that failed or came short (the stream ended there)
+    for (size_t i = 0; i < n; ++i) memset(&h_results[i], 0, sizeof(zlb_result));
+    std::vector<char> closed(n, 0);
+    for (size_t k = 0; k < np; ++k) {
+        const ZtsRangePiece& q = pieces[k];
+        if (closed[q.range]) continue;
+        zlb_result& o = h_results[q.range];
+        const unsigned long long got = pres[k].out_len > q.skip ? pres[k].out_len - q.skip : 0;
+        o.out_len += std::min(got, q.want);
+        if (pres[k].status != ZLB_ST_OK) o.status = pres[k].status;
+        if (pres[k].status != ZLB_ST_OK || got < q.want) closed[q.range] = 1;
+    }
+    std::vector<zlb_item> slots(n);
+    for (size_t i = 0; i < n; ++i) slots[i] = {ranges[i].in_off, ranges[i].in_len, ranges[i].out_off, ranges[i].out_cap};
+    ZTS_CUDA(ctx, cudaMemcpyAsync(d_slots, slots.data(), n * sizeof(zlb_item), cudaMemcpyHostToDevice, st));
+    ZTS_CUDA(ctx, cudaMemcpyAsync(d_results, h_results, n * sizeof(zlb_result), cudaMemcpyHostToDevice, st));
+    uint32_t kinds = 0;
+    if (flags & ZLB_INFLATE_WANT_CRC32) kinds |= ZLB_SUM_CRC32;
+    if (flags & ZLB_INFLATE_WANT_ADLER32) kinds |= ZLB_SUM_ADLER32;
+    if (kinds) {
+        rc = zts_checksum_device(ctx, d_out, d_slots, d_results, slots.data(), n, kinds, 1);
+        if (rc) return rc;
+        ZTS_CUDA(ctx, cudaMemcpyAsync(h_results, d_results, n * sizeof(zlb_result), cudaMemcpyDeviceToHost, st));
+    }
+    ZTS_CUDA(ctx, cudaStreamSynchronize(st));  // (slots goes out of scope; the copy-back needs the sizes)
+    if (hio) return zts_copy_back(ctx, hio->stage, st, d_out, hio->h_out, slots.data(), h_results, d_slots, d_results, 0, n);
+    return ZLB_OK;
+}
+
+extern "C" int zlb_inflate_ranges(zlb_ctx* ctx, const void* d_in, const void* d_win, void* d_out, const zlb_point* points,
+                                  size_t n_points, const zlb_range* ranges, zlb_result* results, size_t n, uint32_t flags)
+{
+    if (!ctx || (n && (!d_in || !d_out || !ranges || !results))) return ZLB_E_ARG;
+    int rc = ranges_check(ctx, points, n_points, ranges, n, flags, SIZE_MAX, SIZE_MAX, SIZE_MAX, d_win != nullptr);
+    if (rc || !n) return rc;
+    ZTS_CUDA(ctx, cudaSetDevice(ctx->device));
+    return ranges_device(ctx, (const uint8_t*)d_in, (const uint8_t*)d_win, (uint8_t*)d_out, points, ranges, results, n, flags,
+                         nullptr);
+}
+
+extern "C" int zlb_inflate_ranges_host(zlb_ctx* ctx, const void* h_in, size_t in_bytes, const void* h_win, size_t win_bytes,
+                                       void* h_out, size_t out_bytes, const zlb_point* points, size_t n_points,
+                                       const zlb_range* ranges, zlb_result* results, size_t n, uint32_t flags)
+{
+    if (!ctx || (n && (!ranges || !results))) return ZLB_E_ARG;
+    int rc = ranges_check(ctx, points, n_points, ranges, n, flags, in_bytes, win_bytes, out_bytes, h_win != nullptr);
+    if (rc || !n) return rc;
+    // the window blob travels the way a dictionary blob does (one table entry naming all of it)
+    std::vector<zlb_item> slots(n);
+    for (size_t i = 0; i < n; ++i) slots[i] = {ranges[i].in_off, ranges[i].in_len, ranges[i].out_off, ranges[i].out_cap};
+    const std::vector<zlb_dict> whole(n, zlb_dict{0, win_bytes});
+    return zts_host_call(ctx, h_in, in_bytes, h_out, out_bytes, h_win, win_bytes, whole.data(), slots.data(), results, n,
+                         SIZE_MAX, [&](ZtsHostIO& io, const zlb_dict*) {
+        zts_stage_wait_in(io.stage, 0, io.in_bytes);
+        ZTS_CUDA(ctx, cudaMemcpyAsync(ctx->d_stage_in.p, io.h_in, io.in_bytes, cudaMemcpyHostToDevice, ctx->stream));
+        return ranges_device(ctx, (const uint8_t*)ctx->d_stage_in.p, (const uint8_t*)ctx->d_dict.p,
+                             (uint8_t*)ctx->d_stage_out.p, points, ranges, results, n, flags, &io);
+    });
 }
